@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            (ours; torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K --warmup W
     python bench.py --gpus N --native-dist ...               (ours, ONE process driving N GPUs through the C ABI)
+    python bench.py ... --dump-outputs DIR                   (also write the last timed frame to DIR/*.npy)
 
 Metric: Mrays/s (primary + shadow rays of one frame / frame time).  A "step" is one frame
 of the hot path over synthetic input.  Default workload = BASELINE.json configs[3]:
@@ -56,6 +57,22 @@ WORKLOADS = {
 }
 WORKLOAD_SPP = {"c5": 16}
 GOLDEN_MODELS = {"c1": "cornell_original.npz", "c3": "cornell_water.npz"}
+DUMP_BYTES = 64 << 20   # --dump-outputs writes at most this much
+DUMP_SAMPLE_PIXELS = 1 << 21
+
+
+def dump_outputs(out_dir, frame):
+    """Write the frame [H, W, 3] (uint8, PPM row order) of the last timed step as float32 .npy files: whole as
+    frame.npy when it fits DUMP_BYTES, else a fixed seeded sample of DUMP_SAMPLE_PIXELS pixels as frame_sample.npy
+    [k, 3] beside their flat pixel indices (h * W + w in PPM row order) as frame_sample_pixel.npy (float64, exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    rgb = np.asarray(frame).reshape(-1, 3)
+    if rgb.size * 4 <= DUMP_BYTES:
+        np.save(os.path.join(out_dir, "frame.npy"), np.asarray(frame, np.float32))
+        return
+    idx = np.sort(np.random.default_rng(0).choice(len(rgb), DUMP_SAMPLE_PIXELS, replace=False))
+    np.save(os.path.join(out_dir, "frame_sample.npy"), rgb[idx].astype(np.float32))
+    np.save(os.path.join(out_dir, "frame_sample_pixel.npy"), idx.astype(np.float64))
 
 
 def make_scene(name, args):
@@ -293,7 +310,13 @@ def main():
     ap.add_argument("--native-dist", action="store_true",
                     help="ONE process drives --gpus N GPUs through the library's own multi-GPU entry points (NCCL inside the C ABI) "
                          "instead of one rank per GPU under torchrun")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the frame the last timed step rendered to DIR/*.npy (float32), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU frame; --impl reference times a pixel sample and renders no frame")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -385,6 +408,8 @@ def main():
     ms = t_wall * 1e3 if native else ev0.elapsed_time(ev1)
     clocks = sampler.stop() if rank == 0 else None
     frame_sha = hashlib.sha256(frame.cpu().numpy().tobytes()).hexdigest() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, frame.cpu().numpy())
     flop_primary = float(st.get("flop_primary") or 0.0)  # FP32 flops executed per swept pair (same on every rank)
     flop_shadow = float(st.get("flop_shadow") or 0.0)
     flop_primary_e = float(st.get("flop_primary_edges") or 0.0)

@@ -77,11 +77,32 @@ def test_mt19937_rejection_path(restated):
     assert np.array_equal(a, b) and a.max() == 9
 
 
-def test_mt19937_replay_equals_libstdcxx_for_any_face_count(ref_oracle):
+def test_mt19937_replay_equals_libstdcxx_for_any_face_count(restated, tmp_path):
     """lights of 100-250 faces (not powers of two): tracer_mt19937_faceids against the draws the reference's own scan_row made
-    with std::uniform_int_distribution (libstdc++'s Lemire mapping), generator state equality asserted by the harness"""
-    from conftest import to_flat
+    with std::uniform_int_distribution (libstdc++'s Lemire mapping), generator state equality asserted by the harness.
+    Without the reference tree the same draws come from libstdc++ itself: tests/libstdcxx_faceids.cpp runs the harness'
+    replay loop over the restatement's hit mask (held bit-equal to the reference's intersect() by test_oracle_pin.py)."""
+    import subprocess
 
+    from conftest import to_flat
+    from oracle import REF_ROOT, RefOracle, build, ref_available
+
+    if os.path.exists(os.path.join(REF_ROOT, "src", "main.cpp")):
+        build()
+    ref = RefOracle() if ref_available() else None
+    exe = tmp_path / "libstdcxx_faceids"
+
+    def libstdcxx_faceids(W, H, seed, faces, hit):
+        r = subprocess.run([str(exe), str(W), str(H), str(seed)] + [str(int(f)) for f in faces],
+                           input=np.asarray(hit, np.uint8).tobytes(), capture_output=True, check=True)
+        return np.frombuffer(r.stdout, np.int32).reshape(W * H, len(faces))
+
+    if ref is None:
+        subprocess.check_call(["g++", "-std=c++17", "-O2", os.path.join(ROOT, "tests", "libstdcxx_faceids.cpp"), "-o", str(exe)])
+        for name in ("cornell_box_ks", "cornell_original_3lights"):  # the draws the reference's scan_row made, stored
+            fs, fr = load_golden(name)
+            faces = fs.geom_tri_offset[fs.light_geom + 1] - fs.geom_tri_offset[fs.light_geom]
+            assert np.array_equal(libstdcxx_faceids(fr["W"], fr["H"], fr["seed"], faces, fr["tri"] >= 0), fr["faceid"])
     rng = np.random.default_rng(3)
     seen = set()
     for _ in range(5):
@@ -90,13 +111,19 @@ def test_mt19937_replay_equals_libstdcxx_for_any_face_count(ref_oracle):
         s2 = Scene(s.geom_tri_offset, s.tri_verts, s.geom_material, lg, tri_normals=s.tri_normals, geom_has_normals=s.geom_has_normals)
         seen.update(int(f) for f in s2.faces_per_light)
         W, H, seed = 48, 36, int(rng.integers(1, 2 ** 31))
-        h = ref_oracle.from_flat(to_flat(s2))
-        try:
-            fr, exact = ref_oracle.render_frame(h, W, H, (0, 1, 3), (0, 1, 0), seed=seed)
-        finally:
-            ref_oracle.free(h)
-        assert exact
-        assert np.array_equal(mt19937_faceids(s2, W, H, seed, fr["faceid"][:, 0] >= 0), fr["faceid"])
+        if ref is not None:
+            h = ref.from_flat(to_flat(s2))
+            try:
+                fr, exact = ref.render_frame(h, W, H, (0, 1, 3), (0, 1, 0), seed=seed)
+            finally:
+                ref.free(h)
+            assert exact
+            want = fr["faceid"]
+        else:
+            hit = restated.render(to_flat(s2), restated.camera((0, 1, 3), (0, 1, 0), W, H), W, H, seed=seed).tri >= 0
+            want = libstdcxx_faceids(W, H, seed, s2.faces_per_light, hit)
+            assert hit.any() and (want[hit] >= 0).all() and (want[~hit] == -1).all()
+        assert np.array_equal(mt19937_faceids(s2, W, H, seed, want[:, 0] >= 0), want)
     assert any(f & (f - 1) for f in seen)  # face counts that are not powers of two were exercised
 
 

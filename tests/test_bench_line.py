@@ -82,8 +82,11 @@ def test_bench_line_has_the_contract_keys_and_consistent_arithmetic(dry_bench):
 
 
 def test_bench_refuses_to_run_without_a_gpu(monkeypatch):
+    import torch
+
     import bench
 
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)  # also on a machine that has one
     monkeypatch.setattr(sys, "argv", ["bench.py", "--no-cpu-baseline"])
     for k in ("RANK", "WORLD_SIZE", "LOCAL_RANK"):
         monkeypatch.delenv(k, raising=False)
@@ -105,6 +108,56 @@ def test_bench_flag_combinations_produce_one_line(dry_bench, argv):
         assert d["e2e"] is None
     if "c5" in argv:
         assert d["config"]["spp"] == 16
+
+
+@pytest.mark.parametrize("size,sampled", [((64, 48), False), ((3840, 2160), True)])
+def test_bench_dump_outputs_writes_the_last_timed_frame(dry_bench, monkeypatch, tmp_path, size, sampled):
+    """--steps sets the number of timed renders; --dump-outputs writes the last one's frame as float32 (a fixed pixel sample
+    when the whole frame would exceed 64 MB), the same files on every run"""
+    import numpy as np
+    import torch
+
+    from esctp1raytracer_b200 import dist as tdist
+
+    fake = tdist.render_frame
+    calls = []
+
+    def render_frame(renderer, rs, cam, W, H, **kw):
+        frame, st = fake(renderer, rs, cam, W, H, **kw)
+        calls.append(1)
+        frame = torch.from_numpy(np.random.default_rng(len(calls)).integers(0, 256, (H, W, 3), dtype=np.uint8))
+        return frame, st
+
+    monkeypatch.setattr(tdist, "render_frame", render_frame)
+    W, H = size
+    dumps = []
+    for run in range(2):
+        calls.clear()
+        out = tmp_path / f"run{run}"
+        dry_bench("--workload", "small", "--tris", "2000", "--width", str(W), "--height", str(H), "--steps", "5", "--warmup", "2",
+                  "--no-cpu-baseline", "--no-e2e", "--no-cull", "--dump-outputs", str(out))
+        assert len(calls) == 2 + 5
+        files = sorted(p.name for p in out.iterdir())
+        dumps.append({f: np.load(out / f) for f in files})
+    last = np.random.default_rng(7).integers(0, 256, (H, W, 3), dtype=np.uint8)  # the frame of the 7th call
+    a, b = dumps
+    assert a.keys() == b.keys() and all(np.array_equal(a[k], b[k]) for k in a)
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20 and all(v.dtype in (np.float32, np.float64) for v in a.values())
+    if sampled:
+        assert sorted(a) == ["frame_sample.npy", "frame_sample_pixel.npy"]
+        idx = a["frame_sample_pixel.npy"].astype(np.int64)
+        assert len(np.unique(idx)) == len(idx) and np.array_equal(a["frame_sample.npy"], last.reshape(-1, 3)[idx].astype(np.float32))
+    else:
+        assert sorted(a) == ["frame.npy"] and np.array_equal(a["frame.npy"], last.astype(np.float32))
+
+
+def test_bench_refuses_dump_outputs_with_the_reference_arm(monkeypatch, tmp_path, capsys):
+    import bench
+
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--impl", "reference", "--dump-outputs", str(tmp_path / "d")])
+    with pytest.raises(SystemExit) as ei:
+        bench.main()
+    assert ei.value.code == 2 and "--dump-outputs" in capsys.readouterr().err and not (tmp_path / "d").exists()
 
 
 def test_bench_torchrun_path_two_ranks_on_gloo():

@@ -54,8 +54,26 @@ def test_host_code_clean_under_asan_ubsan_on_hostile_input(driver, tmp_path):
 
 
 def test_host_code_clean_under_asan_ubsan_on_the_reference_models(driver, tmp_path):
+    """the reference's models when its tree is present, and always the stored geometry of the ones in tests/golden (as
+    the reference's loader flattened them) written back as OBJ + MTL"""
+    from conftest import golden_names, load_golden, write_obj
+
+    def counts(out):  # (scenes loaded, refused)
+        return tuple(int(x) for x in out.split("host_san_driver:")[1].replace(",", "").split() if x.isdigit())
+
+    def scratch(name):
+        d = tmp_path / name
+        d.mkdir()
+        return d
+
+    base = counts(run(driver, scratch("base"), []))  # the driver's own cases alone
+    golden = []
+    for name in golden_names():
+        obj = scratch(name) / "scene.obj"
+        write_obj(load_golden(name)[0], obj)
+        golden.append(str(obj))
+    assert counts(run(driver, scratch("golden"), golden)) == (base[0] + len(golden), base[1])  # every one of them loads
     models = sorted(glob.glob(os.path.join(MODELS, "**", "*.obj"), recursive=True))
-    if not models:
-        pytest.skip("reference models not present")
-    out = run(driver, tmp_path, models)
-    assert "scenes loaded" in out
+    if models:
+        out = run(driver, scratch("models"), models)
+        assert "scenes loaded" in out
