@@ -510,9 +510,6 @@ __host__ __device__ __forceinline__ int hash_faceid(uint32_t seed, uint32_t imag
     return (int)(((unsigned long long)h * F) >> 32);
 }
 
-// glibc powf is computed in double and rounded once; do the same on the device
-__device__ __forceinline__ float powf_like_glibc(float x, float y) { return (float)pow((double)x, (double)y); }
-
 __global__ void __launch_bounds__(256) light_step_kernel(const LightStepParams p) {
     const int kpx = blockIdx.x * blockDim.x + threadIdx.x;
     const bool in_range = kpx < p.bands.n_px;
@@ -581,7 +578,7 @@ __global__ void __launch_bounds__(256) light_step_kernel(const LightStepParams p
                         const float Ns = mat[12];
                         f3 c = strict::div(strict::add(strict::mul(ka, 0.5f), ke), fL);
                         const f3 Hh = strict::normalize(strict::mul(strict::add(N, Lv), 2.f));
-                        const float pw = powf_like_glibc(strict::dot(N, Hh), Ns);
+                        const float pw = strict::powf_glibc(strict::dot(N, Hh), Ns); // glibc powf, bit for bit
                         c = strict::add(c, strict::div(strict::add(strict::mul(kd, d), strict::mul(ks, pw)), fL));
                         acc = strict::add(acc, c);
                     }

@@ -64,6 +64,19 @@ extern "C" void tracer__filter_pass(const float *rows20, int n, const float *p, 
     }
 }
 
+// Internal (tests only): strict::powf_glibc as the device computes it, for every stride-th float bit pattern x from
+// lo_bits up to hi_bits (inclusive) -> host_out[(hi_bits - lo_bits) / stride + 1], or for n (x, y) pairs.  Runs on the
+// current device (tracer_cuda_init first) in chunks; tests/test_gpu_specular.py compares with the host build.
+__global__ void powf_range_kernel(uint32_t lo_bits, uint32_t stride, uint32_t n, float y, float *out) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        out[i] = strict::powf_glibc(__uint_as_float(lo_bits + i * stride), y);
+}
+__global__ void powf_pairs_kernel(const float *x, const float *y, uint32_t n, float *out) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) out[i] = strict::powf_glibc(x[i], y[i]);
+}
+extern "C" int tracer__device_powf(uint32_t lo_bits, uint32_t hi_bits, uint32_t stride, float y, float *host_out);
+extern "C" int tracer__device_powf_pairs(int64_t n, const float *x, const float *y, float *host_out);
+
 extern "C" int tracer__mt19937_scan(uint32_t seed, int32_t n_lights, const int32_t *faces_per_light, int64_t n_px,
                                     const uint8_t *hit_scan, int32_t *faceid_scan);
 
@@ -82,6 +95,14 @@ int fail(int code, const std::string &msg) {
         if (e_ != cudaSuccess)                                                                              \
             return fail(TRACER_ERR_CUDA, std::string(#call) + " failed (tracer_cuda.cu:" + std::to_string(__LINE__) + "): " + cudaGetErrorString(e_)); \
     } while (0)
+
+// A cudaMalloc'ed buffer of the test hooks, freed on every return path.
+struct DevBuf {
+    void *p = nullptr;
+    ~DevBuf() {
+        if (p) cudaFree(p);
+    }
+};
 
 // Device-memory pool: the drop-in call (tracer_cuda_render) creates and destroys a resident scene per
 // frame; cudaMalloc/cudaFree of a few GB of tables and workspace would cost more than the upload itself.
@@ -497,6 +518,44 @@ int tracer_cuda_device_info(tracer_device_info *out) {
     out->clock_khz = khz;
     out->total_mem = (int64_t)g.prop.totalGlobalMem;
     out->l2_bytes = g.prop.l2CacheSize;
+    return TRACER_OK;
+}
+
+int tracer__device_powf(uint32_t lo_bits, uint32_t hi_bits, uint32_t stride, float y, float *host_out) {
+    if (!g_cur) return fail(TRACER_ERR_NO_DEVICE, "tracer_cuda_init not called");
+    if (!host_out || stride == 0 || hi_bits < lo_bits) return fail(TRACER_ERR_INVALID, "tracer__device_powf: bad range");
+    const int64_t n = ((int64_t)hi_bits - lo_bits) / stride + 1;
+    const int64_t chunk = std::min<int64_t>(n, 1 << 24);
+    DevBuf out;
+    CK_CUDA(cudaMalloc(&out.p, chunk * sizeof(float)));
+    for (int64_t b = 0; b < n; b += chunk) {
+        const uint32_t m = (uint32_t)std::min(chunk, n - b);
+        powf_range_kernel<<<(m + 255) / 256, 256, 0, g_cur->stream>>>(lo_bits + (uint32_t)(b * stride), stride, m, y, (float *)out.p);
+        CK_CUDA(cudaGetLastError());
+        CK_CUDA(cudaMemcpyAsync(host_out + b, out.p, m * sizeof(float), cudaMemcpyDeviceToHost, g_cur->stream));
+        CK_CUDA(cudaStreamSynchronize(g_cur->stream));
+    }
+    return TRACER_OK;
+}
+
+int tracer__device_powf_pairs(int64_t n, const float *x, const float *y, float *host_out) {
+    if (!g_cur) return fail(TRACER_ERR_NO_DEVICE, "tracer_cuda_init not called");
+    if (n < 0 || (n && (!x || !y || !host_out))) return fail(TRACER_ERR_INVALID, "tracer__device_powf_pairs: bad arguments");
+    const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(n, 1 << 24));
+    DevBuf dx, dy, dout;
+    CK_CUDA(cudaMalloc(&dx.p, chunk * sizeof(float)));
+    CK_CUDA(cudaMalloc(&dy.p, chunk * sizeof(float)));
+    CK_CUDA(cudaMalloc(&dout.p, chunk * sizeof(float)));
+    cudaStream_t st = g_cur->stream;
+    for (int64_t b = 0; b < n; b += chunk) {
+        const uint32_t m = (uint32_t)std::min(chunk, n - b);
+        CK_CUDA(cudaMemcpyAsync(dx.p, x + b, m * sizeof(float), cudaMemcpyHostToDevice, st));
+        CK_CUDA(cudaMemcpyAsync(dy.p, y + b, m * sizeof(float), cudaMemcpyHostToDevice, st));
+        powf_pairs_kernel<<<(m + 255) / 256, 256, 0, st>>>((const float *)dx.p, (const float *)dy.p, m, (float *)dout.p);
+        CK_CUDA(cudaGetLastError());
+        CK_CUDA(cudaMemcpyAsync(host_out + b, dout.p, m * sizeof(float), cudaMemcpyDeviceToHost, st));
+        CK_CUDA(cudaStreamSynchronize(st));
+    }
     return TRACER_OK;
 }
 

@@ -82,6 +82,5 @@ def test_restatement_equals_reference_at_configured_size(restated, name):
         restated.set_simd(False)
     assert np.array_equal(o.tri, z["tri"])
     assert sha(o.t) == str(z["sha_t"]) and sha(o.v) == str(z["sha_v"])
-    if not sc.geom_material[:, 6:9].any():
-        assert sha(o.rgb) == str(z["sha_rgb"])
+    assert sha(o.rgb) == str(z["sha_rgb"])  # specular frames too: libm powf is what the reference called
     assert np.array_equal(o.rgb8, z["q"])

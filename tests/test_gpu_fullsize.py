@@ -53,7 +53,7 @@ def _image(a, W, H):
     return _ppm(a, W, H)
 
 
-def _check_against_reference(out, z, W, H, has_pow):
+def _check_against_reference(out, z, W, H):
     assert np.array_equal(out.tri, _ppm(z["tri"], W, H)), "hit ids differ from the reference's intersect()"
     stride = int(z["stride"])
     t, v, rgb = _image(out.t, W, H), _image(out.v, W, H), _image(out.rgb, W, H)
@@ -61,14 +61,10 @@ def _check_against_reference(out, z, W, H, has_pow):
     assert np.array_equal(bits(t[::stride]), bits(z["t_s"])), "closest-hit t differs"
     assert np.array_equal(bits(v[::stride]), bits(z["v_s"])), "closest-hit v differs"
     assert sha(t) == str(z["sha_t"]) and sha(v) == str(z["sha_v"])
-    q = z["q"].reshape(-1, 3)
-    if not has_pow:
-        assert np.array_equal(bits(rgb[::stride]), bits(z["rgb_s"])), "float accumulator differs"
-        assert sha(rgb) == str(z["sha_rgb"]), "float accumulator differs from scan_row's"
-        assert np.array_equal(out.rgb8.reshape(-1, 3), q), "PPM bytes differ"
-    d = np.abs(out.rgb8.reshape(-1, 3).astype(int) - q.astype(int))
-    assert (d.max(axis=1) <= 1).mean() >= 0.999, "PPM channels: more than 0.1 % of pixels off by > 1 LSB"
-    assert np.array_equal(out.tri, _ppm(z["tri"], W, H))
+    # specular frames (C3: ks != 0) included: the device's powf is glibc's own (strict::powf_glibc)
+    assert np.array_equal(bits(rgb[::stride]), bits(z["rgb_s"])), "float accumulator differs"
+    assert sha(rgb) == str(z["sha_rgb"]), "float accumulator differs from scan_row's"
+    assert np.array_equal(out.rgb8.reshape(-1, 3), z["q"].reshape(-1, 3)), "PPM bytes differ"
 
 
 @pytest.mark.parametrize("name", FULL)
@@ -80,10 +76,9 @@ def test_reference_frame_at_configured_size(renderer, name):
     W, H = int(z["W"]), int(z["H"])
     cam = Camera.for_frame(z["eye"], z["look"], W, H)
     assert np.array_equal(cam.as_array(), z["cam"])
-    has_pow = bool(sc.geom_material[:, 6:9].any())
     rs = renderer.upload(sc)
     out = renderer.trace(rs, cam, W, H, rng_mode=RNG_MT19937, seed=int(z["seed"]), debug=True)
-    _check_against_reference(out, z, W, H, has_pow)
+    _check_against_reference(out, z, W, H)
     assert out.stats["tests_primary"] == W * H * sc.n_tris
     # explicit faceIDs (the replay the harness recorded) and the optional bundle-cull mode give the same bytes
     fid = z["faceid"].astype(np.int32)
