@@ -136,6 +136,7 @@ __host__ __device__ __forceinline__ float4 project_row(const TableParam &tp, dou
 // area of the (p,q) box; dropping a bound only loosens the filter.  Rows that are not finite make the triangle "always
 // candidate" (the strict path decides).
 constexpr double SPAN_PMAX = 1.0625, SPAN_QMAX = 1.0625; // |p|, |q| of every ray swept in span form (image plane: [0,1]; cube faces: [-1,1])
+static_assert((double)sweep::SPAN_BOX == (double)sweep::SPAN_S * SPAN_PMAX + 1.0, "the interval form's clamp box is S * PMAX + 1");
 
 struct SpanBound {
     double beta, gamma;

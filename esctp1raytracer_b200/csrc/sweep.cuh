@@ -3,8 +3,8 @@
 //
 // What the reference does per (ray, triangle) pair: full Moller-Trumbore with
 // a double-precision divide (ray_triangle.h:7-57, ~52 flop).  What this kernel
-// does per pair: two saturating adds and half a packed multiply-add (4.), plus
-// 4-8 FFMA per thread and triangle.  The saving comes from these observations.
+// does per pair: half a packed add and half a three-input min (4., interval form),
+// plus ~15 ops per thread and triangle.  The saving comes from these observations.
 //
 //  1. Every sweep is a bundle of rays through ONE common point.  Primary rays
 //     all start at the eye (camera.h:31-34).  A shadow ray runs from the hit
@@ -60,14 +60,12 @@
 //  * every lane of every warp reads the SAME row at the same time, so the two LDS.128 per
 //    triangle are pure broadcasts, amortised over R rays per thread held in registers
 //    (R = 32 closest hit, 16 any-hit);
-//  * the conjunction is decided IN THE FMA PIPE: bounds carry the +1 of a saturating test, so
-//    x = sat(S*p + ax) and y = sat(ay - S*p) are both exactly 1 for a pair the reference could
-//    accept, and acc += x*y runs on ray pairs as one packed FFMA2: 2 FFMA.SAT-slot instructions
-//    + half an FFMA2 per pair, no integer op.  History on this part (cycles per pair, closest hit):
-//    round 1 sign bits through LOP3 on the half-rate ALU pipe 7.9, three saturating rows with a
-//    product accumulate 6.8, span form 4.0;
-//  * the inner loop has NO per-triangle branch: an accumulator group of 4 triangles is
-//    tested once; candidates (a few per ray per sweep) are then re-evaluated one by one;
+//  * each pair is ONE interval test |S*p - c| <= h (interval form, below): per two pairs one packed
+//    FADD2 and one FMNMX3 running minimum, no saturation, no integer op.  History on this part
+//    (cycles per pair, closest hit): round 1 sign bits through LOP3 on the half-rate ALU pipe 7.9,
+//    three saturating rows with a product accumulate 6.8, span form with two saturating adds 4.0;
+//  * the inner loop has NO per-triangle branch: a batch of 16 triangles yields one verdict bit per
+//    triangle; candidates (a few per ray per sweep) are then re-evaluated one by one;
 //  * NO block-wide barrier per tile in either sweep: every warp counts itself out of a
 //    tile stage (shared-memory atomicAdd) and the last one issues the refill, so warps
 //    run up to STAGES-1 tiles apart.  An any-hit warp whose rays all have their occluder
@@ -92,7 +90,7 @@
 namespace sweep {
 
 constexpr int TILE = 256;          // triangles per shared-memory stage (48-byte rows: 12 KB)
-constexpr int BATCH = 16;          // triangles between candidate checks
+constexpr int BATCH = 16;          // triangles between candidate checks of the three-row form
 constexpr int STAGES = SWEEP_STAGES; // TMA pipeline depth
 constexpr int THREADS = 512;       // threads per CTA of the bundle-cull kernels (cull.cuh)
 constexpr int NT = SWEEP_NT;       // threads per CTA of the default sweeps
@@ -296,35 +294,74 @@ __host__ __device__ __forceinline__ bool span_pass(const float4 lo, const float4
     return fminf(ps + ax, ay - ps) >= 1.f;
 }
 
-// BATCH triangles of a staged span tile against the R rays of this thread (ps[r] = p_r * SPAN_S).  A candidate pair
-// contributes exactly 1 to its accumulator, any other pair something in [0,1).  Returns bit g set = triangles
-// [g*GROUP, (g+1)*GROUP) may hold a candidate.
+// ---- INTERVAL form of the span test (the hot loop of MODE_SHAREDQ and MODE_QBAR) -----------------------------------------
+// For one thread's shared q a triangle's span row is ONE interval of S*p:  x = y = 1  <=>  1 - ax <= S*p <= ay - 1, i.e.
+// |S*p - c| <= h with c the interval's centre and h its half width.  Per thread and triangle (span_interval):
+//     lo = max(1 - ax, -SPAN_BOX)   hi = min(ay - 1, SPAN_BOX)   nc = -(lo + hi)/2   h = (hi - lo)/2 + SPAN_DELTA
+// and per ray PAIR one packed FADD2 {S*p_r, S*p_r+1} + nc and one three-input FMNMX3 m = min(m, |e_r|, |e_r+1|) (|.| is
+// an operand modifier): 1 FMA-pipe instruction per two pairs, against 2 FFMA.SAT + half an FFMA2 per pair of the
+// saturating form, whose .sat has no packed f32x2 form on sm_100a.  After the R rays, m <= h is the triangle's verdict.
+//
+// SPAN_DELTA makes the interval test pass every pair the saturating test passes (which the table's margins make pass every
+// pair the reference accepts).  Let u = 2^-24 (float unit roundoff), P = SPAN_BOX, |S*p| <= S*SPAN_PMAX = P - 1 for every
+// ray swept in span form (kernels.cuh).  A pair with fl(S*p + ax) >= 1 and fl(ay - S*p) >= 1 has, exactly,
+// S*p >= (1 - ax) - u/2 and S*p <= (ay - 1) + u/2 (a sum rounds up to 1 from 1 - u/2 at the least).  Then:
+//   lo: either -P (< S*p) or fl(1 - ax) > -P, and then 1 - ax lies in (-P, P): lo <= S*p + e, e = u/2 + u*P; same for hi.
+//       So lo, hi lie in [-P, P] and S*p in [lo - e, hi + e]: |S*p - (lo+hi)/2| <= (hi-lo)/2 + e.
+//   nc: one rounding of a sum of magnitude <= 2P (the halving is exact): |nc + (lo+hi)/2| <= u*P.
+//   h:  fl(hi - lo) is off by <= 2u*P, the fma's one rounding by <= u*(P + SPAN_DELTA): h >= (hi-lo)/2 + SPAN_DELTA - 2.1u*P.
+//   e = fl(S*p + nc): S*p + nc has magnitude <= 2P + 1, one rounding <= 2.1u*P.
+// so |e| <= (hi-lo)/2 + u/2 + u*P + u*P + 2.1u*P <= h whenever SPAN_DELTA >= 6.3u*P; SPAN_DELTA = 8 FLT_EPSILON * P = 16u*P
+// (0.066 row units, 1/250 of a 3840-wide frame's pixel).  The clamp is what bounds every term by P: without it an open
+// bound (SPAN_OPEN = 1e30) would put c near 5e29 and round S*p away.  Padding rows (ax = -SPAN_OPEN) give lo = 1e30 > hi, so
+// h ~ -5e29 and the triangle is never a candidate; always-candidate rows (ax = ay = SPAN_OPEN) give c = 0, h > P > |S*p|.
+// NaN cannot reach h (fminf/fmaxf drop it) and a NaN |e| is ignored by the minimum, so neither can hide a candidate.
+constexpr float SPAN_BOX = SPAN_S * 1.0625f + 1.f;                  // S * SPAN_PMAX + 1 (kernels.cuh checks the match)
+constexpr float SPAN_DELTA = 8.f * 1.1920928955078125e-7f * SPAN_BOX; // 8 FLT_EPSILON * SPAN_BOX
+#ifndef SWEEP_SPAN_BATCH
+#define SWEEP_SPAN_BATCH 16
+#endif
+constexpr int SPAN_BATCH = SWEEP_SPAN_BATCH; // triangles between candidate checks of the interval form (<= 32: a bit each)
+static_assert(SPAN_BATCH <= 32 && TILE % SPAN_BATCH == 0, "one verdict bit per triangle of a batch");
+
+// (ax, ay) from span_terms / span_terms_qbar -> the negated centre and the widened half width of the interval of S*p
+// (box, delta: SPAN_BOX, SPAN_DELTA; other values only in the test hook tracer__interval_pass)
+__host__ __device__ __forceinline__ void span_interval(float ax, float ay, float &nc, float &h, float box = SPAN_BOX,
+                                                      float delta = SPAN_DELTA) {
+    const float lo = fmaxf(1.f - ax, -box), hi = fminf(ay - 1.f, box);
+    nc = -0.5f * (lo + hi);
+    h = fmaf(0.5f, hi - lo, delta);
+}
+// the interval test of one pair, as the hot loop evaluates it (ps = p * SPAN_S)
+__host__ __device__ __forceinline__ bool interval_pass(float nc, float h, float ps) { return fabsf(ps + nc) <= h; }
+
+// min(m, |a|, |b|): one FMNMX3 with both absolute values as operand modifiers (sm_100)
+__device__ __forceinline__ float fmin3_abs(float m, float a, float b) {
+    float d;
+    asm("min.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(m), "f"(fabsf(a)), "f"(fabsf(b)));
+    return d;
+}
+
+// SPAN_BATCH triangles of a staged span tile against the R rays of this thread (ps[r] = p_r * SPAN_S).  One minimum
+// chain per triangle: the SPAN_BATCH chains are independent, which is the loop's instruction-level parallelism.
+// Returns bit k set = triangle k may hold a candidate.
 template <int R, int MODE>
-__device__ __forceinline__ unsigned eval_span(const float4 *__restrict__ tp, const float (&ps)[R], float q, float qdelta) {
-    constexpr int GROUP = Batch<R>::GROUP, NA = Batch<R>::NACC;
+__device__ __forceinline__ unsigned eval_interval(const float4 *__restrict__ tp, const float (&ps)[R], float q, float qdelta) {
+    static_assert(R % 2 == 0, "rays are evaluated in pairs");
     unsigned cand = 0;
 #pragma unroll
-    for (int g = 0; g < BATCH / GROUP; ++g) {
-        float2 acc[NA];
+    for (int k = 0; k < SPAN_BATCH; ++k) {
+        float ax, ay, nc, h;
+        if (MODE == MODE_QBAR) span_terms_qbar(tp[2 * k], tp[2 * k + 1], q, qdelta, ax, ay);
+        else span_terms(tp[2 * k], tp[2 * k + 1], q, ax, ay);
+        span_interval(ax, ay, nc, h);
+        float m = __int_as_float(0x7f800000); // +inf
 #pragma unroll
-        for (int a = 0; a < NA; ++a) acc[a] = make_float2(0.f, 0.f);
-#pragma unroll
-        for (int kk = 0; kk < GROUP; ++kk) {
-            const int k = g * GROUP + kk;
-            float ax, ay;
-            if (MODE == MODE_QBAR) span_terms_qbar(tp[2 * k], tp[2 * k + 1], q, qdelta, ax, ay);
-            else span_terms(tp[2 * k], tp[2 * k + 1], q, ax, ay);
-#pragma unroll
-            for (int r = 0; r < R; r += 2) {
-                const float2 x = make_float2(__saturatef(ps[r] + ax), __saturatef(ps[r + 1] + ax));
-                const float2 y = make_float2(__saturatef(ay - ps[r]), __saturatef(ay - ps[r + 1]));
-                acc[(r / 2) % NA] = __ffma2_rn(x, y, acc[(r / 2) % NA]);
-            }
+        for (int r = 0; r < R; r += 2) {
+            const float2 e = __fadd2_rn(make_float2(ps[r], ps[r + 1]), make_float2(nc, nc));
+            m = fmin3_abs(m, e.x, e.y);
         }
-        float sum = 0.f;
-#pragma unroll
-        for (int a = 0; a < NA; ++a) sum += acc[a].x + acc[a].y;
-        if (sum >= 1.f) cand |= 1u << g;
+        cand |= (unsigned)(m <= h) << k;
     }
     return cand;
 }
@@ -409,28 +446,30 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
         if (!idle) {
             ++n_tiles_swept;
             const float4 *__restrict__ tp = sm.tile[s];
+            // triangles per hot-loop call, and per bit of its verdict: the interval form (span rows) flags single
+            // triangles, the three-row form groups of GROUP
+            constexpr int NB = SPAN ? SPAN_BATCH : BATCH, UNIT = SPAN ? 1 : Batch<R>::GROUP;
 #pragma unroll 1
-            for (int b0 = 0; b0 < TILE; b0 += BATCH) {
+            for (int b0 = 0; b0 < TILE; b0 += NB) {
                 unsigned cand;
-                if (SPAN) cand = eval_span<R, MODE>(tp + ROWS * b0, ps, qhot, qdelta);
+                if (SPAN) cand = eval_interval<R, MODE>(tp + ROWS * b0, ps, qhot, qdelta);
                 else cand = eval_batch<R, MODE>(tp + ROWS * b0, rp, rq, qbar, qdelta);
 #ifdef SWEEP_NO_STRICT // development microbenchmark only (tools/sweep_mb2.cu): timing without the strict path
                 if (cand) ++done;
 #else
-                constexpr int GROUP = Batch<R>::GROUP;
-                // validation mode: every group goes to the strict path; the hot loop's own verdict is kept so that an
-                // accepted pair whose group it would have skipped counts as a filter miss too
+                // validation mode: every triangle goes to the strict path; the hot loop's own verdict is kept so that an
+                // accepted pair whose triangle (group) it would have skipped counts as a filter miss too
                 const unsigned cand_hot = cand;
-                if (EXHAUSTIVE) cand = (1u << (BATCH / GROUP)) - 1u;
+                if (EXHAUSTIVE) cand = NB / UNIT == 32 ? 0xffffffffu : (1u << (NB / UNIT)) - 1u;
                 while (cand) {
-                    // rare: a group of GROUP triangles may hold a candidate.  Rebuild the per-ray candidate mask of each
-                    // of its triangles (each ray's own q, exact threshold), then the reference's own arithmetic.  The rows
-                    // are re-read through opaque loads so that the compiler cannot merge this with the hot evaluation.
+                    // rare: a triangle (group of UNIT triangles) may hold a candidate.  Rebuild the per-ray candidate mask
+                    // of each of its triangles (exact threshold), then the reference's own arithmetic.  The rows are re-read
+                    // through opaque loads so that the compiler cannot merge this with the hot evaluation.
                     const int gq = __ffs(cand) - 1; // ascending triangle order
                     cand &= cand - 1;
 #pragma unroll 1
-                    for (int kk = 0; kk < GROUP; ++kk) {
-                        const int k = b0 + gq * GROUP + kk;
+                    for (int kk = 0; kk < UNIT; ++kk) {
+                        const int k = b0 + gq * UNIT + kk;
                         const int tri = (tile_lo + it) * TILE + k;
                         unsigned filt = 0;
                         if (SPAN) {

@@ -63,6 +63,24 @@ extern "C" void tracer__filter_pass(const float *rows20, int n, const float *p, 
                                  (fminf(ps + ax, ay - ps) >= 1.f ? 4 : 0));
     }
 }
+// n rays (p) of one thread against one span row (row8 = lo.xyzw, hi.xyzw) in the hot loop's shared-q form: qdelta < 0 = one
+// exact q (MODE_SHAREDQ), else q = qbar and the bounds widened by |B| * qdelta (MODE_QBAR).  bit 0 = the interval form with
+// clamp box and margin delta (sweep::SPAN_BOX, sweep::SPAN_DELTA in the sweeps), bit 1 = the saturating form it replaces
+// (x = sat(S p + ax) and y = sat(ay - S p) both 1), bit 2 = the candidate path's span_pass with q as the ray's own q.
+extern "C" void tracer__interval_pass(const float *row8, int n, const float *p, float q, float qdelta, float box, float delta,
+                                      unsigned char *out) {
+    const float4 lo = make_float4(row8[0], row8[1], row8[2], row8[3]), hi = make_float4(row8[4], row8[5], row8[6], row8[7]);
+    float ax, ay, nc, h;
+    if (qdelta < 0.f) sweep::span_terms(lo, hi, q, ax, ay);
+    else sweep::span_terms_qbar(lo, hi, q, qdelta, ax, ay);
+    sweep::span_interval(ax, ay, nc, h, box, delta);
+    for (int i = 0; i < n; ++i) {
+        const float ps = p[i] * sweep::SPAN_S;
+        out[i] = (unsigned char)((sweep::interval_pass(nc, h, ps) ? 1 : 0) | (fminf(ps + ax, ay - ps) >= 1.f ? 2 : 0) |
+                                 (sweep::span_pass(lo, hi, ps, q) ? 4 : 0));
+    }
+}
+extern "C" void tracer__interval_consts(float *out2) { out2[0] = sweep::SPAN_BOX, out2[1] = sweep::SPAN_DELTA; }
 
 // Internal (tests only): strict::powf_glibc as the device computes it, for every stride-th float bit pattern x from
 // lo_bits up to hi_bits (inclusive) -> host_out[(hi_bits - lo_bits) / stride + 1], or for n (x, y) pairs.  Runs on the
@@ -860,6 +878,7 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     const char *cand_env = std::getenv("TRACER_CAND_CAP");
     const unsigned long long em_cap = cand_env ? std::min<unsigned long long>((unsigned long long)std::atoll(cand_env), s->cand_cap) : (unsigned long long)s->cand_cap;
     double flop_primary = 0.0; // executed FP32 flops per swept pair of the closest-hit sweep (default mode)
+    double flop_primary_edges = 0.0; // of which bound-evaluating multiply-adds
     const bool two_phase = cull && o.bundle_cull != 2;
     int64_t host_tests_primary = 0, host_tests_shadow = 0; // pairs considered by two-phase sweeps (every block x every triangle)
     auto ensure_boxes = [&](size_t n_blocks) -> int {
@@ -961,9 +980,11 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
         if (p.n_blocks < want_items) // same sizing rule as pick_decomp, on the real block count
             p.n_slices = std::max(1, std::min((want_items + p.n_blocks - 1) / p.n_blocks, std::max(1, n_tiles / 4)));
         const int grid = std::min(p.n_blocks * p.n_slices, sweep::MINB * g.n_sms);
-        // executed FP32 flops per pair: span form 2 FADD + 1 FFMA per pair and 4 FFMA per thread and triangle; three-row
-        // form with every ray its own q: 6 FFMA.SAT + FMUL + FFMA
-        flop_primary = qmode == sweep::MODE_OWNQ ? 15.0 : 4.0 + (qmode == sweep::MODE_QBAR ? 16.0 : 8.0) / d.R;
+        // executed FP32 flops per pair: interval form half a packed FADD2 per pair (the three-input min is no flop), and
+        // per thread and triangle 4 FFMA for the bounds + the interval's 3 FADD, FMUL and FFMA (15 flops; 8 more FFMA-flops
+        // with a mean q); three-row form with every ray its own q: 6 FFMA.SAT + FMUL + FFMA
+        flop_primary = qmode == sweep::MODE_OWNQ ? 15.0 : 1.0 + (qmode == sweep::MODE_QBAR ? 23.0 : 15.0) / d.R;
+        flop_primary_edges = qmode == sweep::MODE_OWNQ ? 12.0 : (qmode == sweep::MODE_QBAR ? 16.0 : 8.0) / d.R;
         if (int rc = launch_primary(d.R, o.exhaustive_strict != 0, qmode, p, grid, st)) return rc;
         trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(dc, bands, s->best, s->tri_verts, s->n_tris, s->spheres,
                                                                         s->n_spheres, s->hit_tri, s->hit_t, s->hit_v);
@@ -1281,12 +1302,12 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     s->stats.filter_misses = (int64_t)hc.filter_misses;
     s->stats.pipeline_errors = (int64_t)hc.pipeline_errors;
     s->stats.kernel_launches = launches;
-    // FP32 flops the sweeps' formulation needs per swept pair (all in the FMA pipe; FFMA = 2, FADD = 1).  Span form: two
-    // saturating adds + one multiply-add per pair, plus the bound FFMAs per thread and triangle: 4 (one exact q) or 8 (mean q
-    // + |B| * spread: shadow sweeps, jittered primary samples) over the R rays of the thread.
-    s->stats.flop_primary = cull ? 0.0 : flop_primary, s->stats.flop_shadow = cull ? 0.0 : 4.0 + 16.0 / trk::SHADOW_R;
-    // of which multiply-adds that evaluate bounds (the rest is the two saturating adds and the accumulate of each pair)
-    s->stats.flop_primary_edges = cull ? 0.0 : (flop_primary >= 15.0 ? 12.0 : flop_primary - 4.0);
+    // FP32 flops the sweeps' formulation needs per swept pair (FFMA = 2, FADD = FMUL = 1, a minimum 0).  Interval form: half
+    // a packed FADD2 per pair, plus per thread and triangle the bound FFMAs, 4 (one exact q) or 8 (mean q + |B| * spread:
+    // shadow sweeps, jittered primary samples), and the interval's centre and half width (7 flops), over the R rays.
+    s->stats.flop_primary = cull ? 0.0 : flop_primary, s->stats.flop_shadow = cull ? 0.0 : 1.0 + 23.0 / trk::SHADOW_R;
+    // of which multiply-adds that evaluate bounds (the rest is each pair's interval test and the per-triangle interval)
+    s->stats.flop_primary_edges = cull ? 0.0 : flop_primary_edges;
     s->stats.flop_shadow_edges = cull ? 0.0 : 16.0 / trk::SHADOW_R;
     if (hc.cull_overflow) {
         // the optional mode's candidate buffer (24 per ray + slack) was too small for this scene's depth complexity: render
