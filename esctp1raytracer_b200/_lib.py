@@ -52,7 +52,7 @@ class RenderOpts(C.Structure):
         ("exhaustive_strict", C.c_int32), ("samples_per_pixel", C.c_int32),
         ("rays_per_thread", C.c_int32), ("shadow_chunks", C.c_int32), ("bundle_cull", C.c_int32),
         ("out_tri", C.POINTER(C.c_int32)), ("out_t", C.POINTER(C.c_float)), ("out_v", C.POINTER(C.c_float)),
-        ("out_occ_tri", C.POINTER(C.c_int32)), ("out_rgb", C.POINTER(C.c_float)),
+        ("out_occ_tri", C.POINTER(C.c_int32)), ("out_rgb", C.POINTER(C.c_float)), ("accel", C.c_int32),
     ]
 
 

@@ -241,8 +241,9 @@ class MultiRenderer:
         return _MultiScene(self, scene, h)
 
     def trace(self, scene, camera: "Camera", width: int, height: int, *, rng_mode=RNG_HASH, seed=1, faceid=None,
-              samples_per_pixel=0, bundle_cull=False, band_rows=0, out_device_ptr=None) -> "Frame":
-        """``out_device_ptr``: leave the assembled frame in HBM on GPU 0 at that address instead of copying it to the host."""
+              samples_per_pixel=0, bundle_cull=False, band_rows=0, out_device_ptr=None, bvh=False) -> "Frame":
+        """``out_device_ptr``: leave the assembled frame in HBM on GPU 0 at that address instead of copying it to the host.
+        ``bvh``: the optional BVH mode (opts.accel = 1; every GPU builds its replica's tree), same bytes."""
         sc = scene.scene if isinstance(scene, _MultiScene) else scene
         o = _lib.RenderOpts()
         o.struct_size = C.sizeof(_lib.RenderOpts)
@@ -252,6 +253,7 @@ class MultiRenderer:
             keep = np.ascontiguousarray(faceid, np.int32)
             o.faceid = _ptr(keep, C.c_int32)
         o.samples_per_pixel, o.bundle_cull, o.band_rows = samples_per_pixel, int(bundle_cull), band_rows
+        o.accel = int(bool(bvh))
         if out_device_ptr is not None:
             out, dst, o.rgb_out_is_device = None, C.c_void_p(out_device_ptr), 1
         else:
@@ -315,7 +317,7 @@ class Renderer:
         if bands is not None:
             o.band_rows, o.band_index, o.band_count = bands
         o.exhaustive_strict = int(exhaustive)
-        o.rays_per_thread, o.shadow_chunks, o.samples_per_pixel, o.bundle_cull = tuning
+        o.rays_per_thread, o.shadow_chunks, o.samples_per_pixel, o.bundle_cull, o.accel = tuning
         dbg = {}
         if debug:
             L = scene.n_lights
@@ -327,9 +329,10 @@ class Renderer:
 
     def trace(self, scene, camera: Camera, width: int, height: int, *, rng_mode=RNG_HASH, seed=1, faceid=None,
               bands=None, exhaustive_strict=False, debug=False, out_device_ptr=None, stream=None,
-              rays_per_thread=0, shadow_chunks=0, samples_per_pixel=0, bundle_cull=False, out=None) -> Frame:
+              rays_per_thread=0, shadow_chunks=0, samples_per_pixel=0, bundle_cull=False, out=None, bvh=False) -> Frame:
         """Render; ``scene`` is a Scene (one-shot: upload + render, the drop-in call) or a
-        ResidentScene.  ``bands`` = (band_rows, band_index, band_count).  With
+        ResidentScene.  ``bvh``: the optional BVH mode (opts.accel = 1): the resident scene builds its tree on the
+        first such render and keeps it; same bytes as the default mode.  ``bands`` = (band_rows, band_index, band_count).  With
         ``out_device_ptr`` the packed rows are left in HBM at that address; ``out`` is an optional
         caller-owned uint8 [rows, W, 3] host array (e.g. pinned) to receive them."""
         sc = scene.scene if isinstance(scene, ResidentScene) else scene
@@ -337,7 +340,7 @@ class Renderer:
         n_px = rows * width
         keep = []
         o, dbg = self._opts(sc, width, height, rng_mode, seed, faceid, bands, exhaustive_strict, debug, n_px, keep,
-                            (rays_per_thread, shadow_chunks, samples_per_pixel, int(bundle_cull)))
+                            (rays_per_thread, shadow_chunks, samples_per_pixel, int(bundle_cull), int(bool(bvh))))
         if out_device_ptr is not None:
             out = None
             o.rgb_out_is_device = 1

@@ -1073,7 +1073,15 @@ __global__ void __launch_bounds__(sweep::NT, sweep::MINB) shadow_light_kernel(co
     }
 }
 
-// extension: spheres are tested after all triangles, in order, by the rays that found no triangle
+// extension: spheres are tested after all triangles, in order, by a shadow ray that found no triangle; the first one that
+// accepts is the occluder (key index << 32 | t2, object index n_tris + s), KEY_NONE if none
+__device__ __forceinline__ unsigned long long sphere_occluder(f3 o, f3 d, float t, const float4 *__restrict__ spheres, int n_spheres,
+                                                              int n_tris) {
+    for (int s = 0; s < n_spheres; ++s)
+        if (strict::intersect_sphere(o, d, __ldg(&spheres[s]), t)) return ((unsigned long long)(unsigned)(n_tris + s) << 32) | __float_as_uint(t);
+    return KEY_NONE;
+}
+
 __global__ void shadow_spheres_kernel(const int *__restrict__ list, const int *__restrict__ seg_off, const int *__restrict__ cnt,
                                       int F, PixelState px, int n_px, const float4 *__restrict__ spheres, int n_spheres,
                                       int n_tris) {
@@ -1085,12 +1093,8 @@ __global__ void shadow_spheres_kernel(const int *__restrict__ list, const int *_
         if (px.best_occ[k] != KEY_NONE) continue;
         const f3 o = strict::mk(px.ro[k], px.ro[n_px + k], px.ro[2 * n_px + k]);
         const f3 d = strict::mk(px.rd[k], px.rd[n_px + k], px.rd[2 * n_px + k]);
-        float t = px.rt[k];
-        for (int s = 0; s < n_spheres; ++s)
-            if (strict::intersect_sphere(o, d, __ldg(&spheres[s]), t)) {
-                px.best_occ[k] = ((unsigned long long)(unsigned)(n_tris + s) << 32) | __float_as_uint(t);
-                break;
-            }
+        const unsigned long long key = sphere_occluder(o, d, px.rt[k], spheres, n_spheres, n_tris);
+        if (key != KEY_NONE) px.best_occ[k] = key;
     }
 }
 

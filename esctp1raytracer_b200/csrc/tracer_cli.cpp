@@ -2,7 +2,9 @@
 // place of its accelerator call:  arg parse -> model::loadobj -> camera -> render -> PPM.
 // Same flags as the reference where they exist (-m -o -v -l, main.cpp:467-529); `-w W,H` really sets
 // the window here (in the reference it overwrites `look`, main.cpp:515-529); `--cuda` is accepted
-// for symmetry with `--ispc`.  The CPU modes (--thread, --bvh, --ispc) do not exist in this build.
+// for symmetry with `--ispc`.  The CPU/ISPC modes (--thread, --ispc) do not exist in this build.  `--bvh` does what the
+// reference's --bvh intends (main.cpp:566-567 flatten + sort, then a BVH render): the flatten+sort pass of --sorted, then
+// the optional BVH mode (opts.accel = 1), so its output is the bytes of --sorted.
 // `--gpus N` renders the frame on N GPUs of the box (interleaved 8-row bands, NCCL gather: tracer_cuda_init_multi);
 // `--spp S` = S stratified jittered samples per pixel (extension); `--sorted` runs the reference's optional
 // flatten+sort pass (src/simplify/flatten.cpp:50-82) before rendering.
@@ -29,6 +31,7 @@ int main(int argc, char *argv[]) {
         int W = 1024, H = 768;                          // main.cpp:427
         int device = 0, p6 = 0, bundle_cull = 0, gpus = 1, spp = 0;
         bool sorted = false;
+        int accel = 0;
         bool have_seed = false;
         unsigned seed = 0;
         int rng = TRACER_RNG_MT19937; // the serial path's generator
@@ -39,7 +42,7 @@ int main(int argc, char *argv[]) {
                 return argv[++a];
             };
             if (f == "--cuda" || f == "--debug" || f == "--trace" || f == "--test") continue;
-            if (f == "--thread" || f == "--bvh" || f == "--ispc")
+            if (f == "--thread" || f == "--ispc")
                 throw std::runtime_error(f + ": CPU/ISPC modes are not part of this build (GPU renderer only)");
             if (f == "-m") model = need("-m");
             else if (f == "-o") output = need("-o");
@@ -57,6 +60,7 @@ int main(int argc, char *argv[]) {
             else if (f == "--gpus") gpus = std::atoi(need("--gpus"));
             else if (f == "--spp") spp = std::atoi(need("--spp"));
             else if (f == "--sorted") sorted = true;
+            else if (f == "--bvh") sorted = true, accel = 1;
             else throw std::runtime_error("Unknown argument: " + f); // main.cpp:531-534
         }
         tracer_scene_host *scene = nullptr;
@@ -87,6 +91,7 @@ int main(int argc, char *argv[]) {
         o.struct_size = sizeof o;
         o.rng_mode = rng;
         o.bundle_cull = bundle_cull;
+        o.accel = accel;
         o.samples_per_pixel = spp;
         if (spp > 1 && rng == TRACER_RNG_MT19937) o.rng_mode = rng = TRACER_RNG_HASH; // the serial replay is 1 spp only
         o.seed = have_seed ? seed : std::random_device{}(); // main.cpp:587-588

@@ -17,7 +17,7 @@
 #include <nccl.h>
 #include <thread>
 
-#include "kernels.cuh"
+#include "bvh.cuh" // (includes kernels.cuh)
 
 // Internal (tests only, no GPU needed): the row construction of build_origin_table and the sweeps' per-ray tests,
 // compiled for the host from the same source.  rows9 = three exact rows (A, B, C); row8 = lo.xyzw, hi.xyzw.
@@ -256,6 +256,12 @@ struct tracer_scene_dev {
         *n_slices = nullptr;
     int maxF = 0;
     sweep::Counters *counters = nullptr;
+    // optional BVH mode: built on the first BVH render, kept until the scene is destroyed
+    bool bvh_built = false;
+    bvh::Node *bvh_nodes = nullptr;
+    unsigned long long *bvh_keys = nullptr; // sorted keys; the always-test list is the tail from bvh_tree.n_in on
+    bvh::Tree bvh_tree{};
+    double bvh_ext = 0.0; // largest |coordinate| of the tree's triangles
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
     std::vector<cudaEvent_t> ev_shadow;
     tracer_frame_stats stats{};
@@ -460,6 +466,72 @@ int build_table(const tracer_scene_dev *s, const trk::TableParam &tp, float4 *ta
     return 0;
 }
 
+// The BVH of the optional mode (bvh.cuh), on stream st: prep (boxes, sigma, bounds) -> Morton keys -> radix sort ->
+// Karras nodes -> bottom-up refit.  One read-back when it is built (tree size and bounds, for the per-frame margin).
+int ensure_bvh(tracer_scene_dev *s, cudaStream_t st) {
+    if (s->bvh_built) return 0;
+    const int n = s->n_tris;
+    float4 *tlo = nullptr, *thi = nullptr;
+    unsigned long long *keys = nullptr;
+    int *parent = nullptr, *leaf_parent = nullptr, *flags = nullptr;
+    bvh::BuildHdr *hdr = nullptr;
+    void *tmp = nullptr;
+    struct Scratch { // build-only buffers, back to the pool on every return path
+        float4 *&a, *&b;
+        unsigned long long *&k;
+        int *&p, *&lp, *&f;
+        bvh::BuildHdr *&h;
+        void *&t;
+        ~Scratch() { dev_free(a), dev_free(b), dev_free(k), dev_free(p), dev_free(lp), dev_free(f), dev_free(h), t_pool->release(t); }
+    } scratch{tlo, thi, keys, parent, leaf_parent, flags, hdr, tmp};
+    const size_t N = (size_t)std::max(n, 1);
+    dev_free(s->bvh_nodes), dev_free(s->bvh_keys);
+    if (dev_alloc(&tlo, N) || dev_alloc(&thi, N) || dev_alloc(&keys, N) || dev_alloc(&s->bvh_keys, N) || dev_alloc(&parent, N) ||
+        dev_alloc(&leaf_parent, N) || dev_alloc(&flags, N) || dev_alloc(&s->bvh_nodes, N) || dev_alloc(&hdr, 1))
+        return TRACER_ERR_NOMEM;
+    bvh::BuildHdr h0{};
+    for (int c = 0; c < 6; ++c) h0.cb[c] = h0.bb[c] = c < 3 ? 0xffffffffu : 0u;
+    CK_CUDA(cudaMemcpyAsync(hdr, &h0, sizeof h0, cudaMemcpyHostToDevice, st));
+    const int th = 256, blocks = (int)((N + th - 1) / th);
+    if (n > 0) {
+        bvh::prep_kernel<<<blocks, th, 0, st>>>(s->tri_verts, n, tlo, thi, hdr);
+        CK_CUDA(cudaGetLastError());
+        bvh::key_kernel<<<blocks, th, 0, st>>>(tlo, thi, n, hdr, keys);
+        CK_CUDA(cudaGetLastError());
+        size_t tmp_bytes = 0;
+        CK_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, keys, s->bvh_keys, n, 0, 64, st));
+        if (!(tmp = t_pool->alloc(tmp_bytes))) return fail(TRACER_ERR_NOMEM, "BVH sort scratch");
+        CK_CUDA(cub::DeviceRadixSort::SortKeys(tmp, tmp_bytes, keys, s->bvh_keys, n, 0, 64, st));
+    }
+    bvh::BuildHdr hh{};
+    CK_CUDA(cudaMemcpyAsync(&hh, hdr, sizeof hh, cudaMemcpyDeviceToHost, st));
+    CK_CUDA(cudaStreamSynchronize(st));
+    const int n_in = hh.n_in;
+    if (n_in >= 2) {
+        bvh::nodes_kernel<<<(n_in - 1 + th - 1) / th, th, 0, st>>>(s->bvh_keys, n_in, s->bvh_nodes, parent, leaf_parent, flags);
+        CK_CUDA(cudaGetLastError());
+        bvh::refit_kernel<<<(n_in + th - 1) / th, th, 0, st>>>(s->bvh_keys, n_in, tlo, thi, s->bvh_nodes, parent, leaf_parent, flags);
+        CK_CUDA(cudaGetLastError());
+    }
+    int root_leaf = -1;
+    if (n_in == 1) {
+        unsigned long long k0 = 0;
+        CK_CUDA(cudaMemcpyAsync(&k0, s->bvh_keys, sizeof k0, cudaMemcpyDeviceToHost, st));
+        CK_CUDA(cudaStreamSynchronize(st));
+        root_leaf = (int)(k0 & 0xffffffffull);
+    }
+    CK_CUDA(cudaStreamSynchronize(st)); // the scratch buffers go back to the pool when this returns
+    s->bvh_tree = bvh::Tree{s->bvh_nodes, n_in, root_leaf, s->bvh_keys + n_in, n - n_in};
+    s->bvh_ext = 0.0;
+    if (n_in > 0)
+        for (int c = 0; c < 6; ++c) s->bvh_ext = std::max(s->bvh_ext, (double)std::fabs(bvh::unord(hh.bb[c])));
+    s->bvh_built = true;
+    if (std::getenv("TRACER_BVH_DIAG"))
+        std::fprintf(stderr, "bvh: %d triangles in the tree, %d on the always-test list (non-finite or sigma >= %g)\n", n_in, n - n_in,
+                     (double)bvh::SIGMA_MAX);
+    return 0;
+}
+
 // cube face f around point o: d' = p*e_a + q*e_b + sg*e_c, c = f/2, a = (c+1)%3, b = (c+2)%3, |d'| <= sqrt(3)
 trk::TableParam face_param(const float *o, int f, double lmax) {
     trk::TableParam tp{};
@@ -598,6 +670,7 @@ void tracer_cuda_scene_destroy(tracer_scene_dev *s) {
     dev_free(s->boxes), dev_free(s->blk_cnt);
     t_pool->release(s->sort_tmp), t_pool->release(s->pair_tmp);
     dev_free(s->counters);
+    dev_free(s->bvh_nodes), dev_free(s->bvh_keys);
     for (auto &e : s->ev)
         if (e) cudaEventDestroy(e);
     for (auto &e : s->ev_shadow) cudaEventDestroy(e);
@@ -792,6 +865,10 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     if (o.rng_mode == TRACER_RNG_EXPLICIT && !o.faceid && s->n_lights > 0)
         return fail(TRACER_ERR_INVALID, "TRACER_RNG_EXPLICIT needs opts->faceid");
     if (o.rng_mode < 0 || o.rng_mode > 2) return fail(TRACER_ERR_INVALID, "bad rng_mode");
+    if (o.accel < 0 || o.accel > 1) return fail(TRACER_ERR_INVALID, "bad accel (0 = sweeps, 1 = BVH)");
+    const bool use_bvh = o.accel == 1;
+    if (use_bvh && (o.bundle_cull != 0 || o.exhaustive_strict != 0))
+        return fail(TRACER_ERR_INVALID, "accel = 1 (BVH) does not combine with bundle_cull or exhaustive_strict (a debug mode of the sweeps' filter)");
     const int n_rows = tracer_band_row_count(H, band_rows, band_count > 1 ? o.band_index : 0, band_count);
     const int n_px = n_rows * W;
     const int L = s->n_lights;
@@ -819,7 +896,9 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     // shadow segments of light k are bounded by len_k <= (k+1) * diag: t carries over lights (main.cpp:764)
     const double diag = std::sqrt(diag2) * 1.001 + 1e-30;
     CK_CUDA(cudaEventRecord(s->ev[0], st));
-    {   // eye table on the image plane: d'(s,t) = (llc - origin) + s*horizontal + t*vertical (camera.h:31-34)
+    if (use_bvh) {
+        if (int rc = ensure_bvh(s, st)) return rc;
+    } else {   // eye table on the image plane: d'(s,t) = (llc - origin) + s*horizontal + t*vertical (camera.h:31-34)
         trk::TableParam tp{};
         for (int c = 0; c < 3; ++c) {
             tp.o[c] = cam->origin[c], tp.U[c] = cam->horizontal[c], tp.V[c] = cam->vertical[c];
@@ -845,7 +924,7 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     // faster of the two (tiny scenes: the mode has a fixed cost of a few ms in sorts and count read-backs)
     const double est_default_ms = (double)n_px * (double)s->n_tris * (1.0 + 0.25 * L) / 4.0e9;
     // (the optional mode keeps every light vertex's tables resident; a light too big for that renders in the default mode)
-    const bool cull = s->tables_resident && (o.bundle_cull == 3 ? est_default_ms > 6.0 : o.bundle_cull != 0);
+    const bool cull = !use_bvh && s->tables_resident && (o.bundle_cull == 3 ? est_default_ms > 6.0 : o.bundle_cull != 0);
     if (cull) { // candidate buffers: 24 per ray + slack (a few per ray are typical), sorted with a radix sort
         const size_t cap = (size_t)n_px * 24 * (size_t)s->cull_grow + ((size_t)1 << 22);
         if (cap > s->cand_cap) {
@@ -860,7 +939,7 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     }
     // default mode: shadow rays ordered by (group, q) so that the rays of a thread can share a q-term (sweep::MODE_QBAR);
     // bundle-cull mode: ordered by (group, Morton code of (p,q)).  Either way a radix sort of (key, pixel) pairs.
-    if (s->rkey_npx < n_px) {
+    if (!use_bvh && s->rkey_npx < n_px) {
         dev_free(s->rkey), dev_free(s->rkey_sorted), dev_free(s->iota);
         t_pool->release(s->pair_tmp);
         s->pair_tmp = nullptr;
@@ -924,7 +1003,19 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     CK_CUDA(cudaMemsetAsync(s->work, 0, sizeof(int), st));
     CK_CUDA(cudaMemsetAsync(s->best, 0xff, sizeof(unsigned long long) * (size_t)n_px, st));
     CK_CUDA(cudaEventRecord(s->ev[1], st));
-    if (cull) { // OPTIONAL bundle-cull mode: screen tiles of 128 x 32 pixels -> candidates -> sort -> strict
+    // BVH mode: the tree's dilation m (bvh.cuh frame_margin) from the largest |coordinate| of the tree and the eye, with
+    // the reach bound diag of the primary rays' hit points, (k+1) diag for light k
+    double bvh_ext = s->bvh_ext;
+    for (int c = 0; c < 3; ++c) bvh_ext = std::max(bvh_ext, (double)std::fabs(cam->origin[c]));
+    if (use_bvh) {
+        bvh::primary_kernel<<<(n_px + 127) / 128, 128, 0, st>>>(dc, bands, s->bvh_tree, bvh::frame_margin(bvh_ext, diag), s->tri_verts,
+                                                                 s->best, s->counters);
+        CK_CUDA(cudaGetLastError());
+        trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(dc, bands, s->best, s->tri_verts, s->n_tris, s->spheres,
+                                                                        s->n_spheres, s->hit_tri, s->hit_t, s->hit_v);
+        CK_CUDA(cudaGetLastError());
+        launches += 2;
+    } else if (cull) { // OPTIONAL bundle-cull mode: screen tiles of 128 x 32 pixels -> candidates -> sort -> strict
         trk::PrimaryCullParams p{};
         const int c_tiles = s->n_pad / cull::CTILE;
         p.cam = dc, p.bands = bands, p.table = s->eye_table, p.n_tiles = c_tiles, p.n_tris = s->n_tris, p.n_rows = n_rows;
@@ -1054,12 +1145,21 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
         lp.rng_mode = o.rng_mode, lp.seed = seed_s, lp.faceid = s->faceid, lp.lmax = (k + 1) * diag;
         lp.seg_count = s->seg_count, lp.counters = s->counters;
         lp.dbg_occ = o.out_occ_tri ? s->dbg_occ : nullptr;
-        lp.cull_cells = cull ? 1 : 2, lp.rkey = s->rkey;
+        lp.cull_cells = use_bvh ? 0 : (cull ? 1 : 2), lp.rkey = s->rkey;
         if (k < L) CK_CUDA(cudaMemsetAsync(s->seg_count, 0, sizeof(int) * ((size_t)s->maxF * trk::NFACE + 1), st));
         trk::light_step_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(lp);
         CK_CUDA(cudaGetLastError());
         ++launches;
         if (k == L) break;
+        if (use_bvh) { // one thread per pixel: first occluder through the tree, then the spheres
+            CK_CUDA(cudaEventRecord(s->ev_shadow[2 * k], st));
+            bvh::shadow_kernel<<<(n_px + 127) / 128, 128, 0, st>>>(s->bvh_tree, px, n_px, bvh::frame_margin(bvh_ext, (k + 1) * diag),
+                                                                    s->tri_verts, s->spheres, s->n_spheres, s->n_tris, s->counters);
+            CK_CUDA(cudaGetLastError());
+            ++launches;
+            CK_CUDA(cudaEventRecord(s->ev_shadow[2 * k + 1], st));
+            continue;
+        }
         const int F = s->h_light_F[k] * trk::NFACE; // ray groups: (light vertex, cube face)
         if (cull) {
             // OPTIONAL bundle-cull mode: rays sorted by (group, Morton code of (p,q)), one culled sweep over all triangles per light
@@ -1305,10 +1405,11 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     // FP32 flops the sweeps' formulation needs per swept pair (FFMA = 2, FADD = FMUL = 1, a minimum 0).  Interval form: half
     // a packed FADD2 per pair, plus per thread and triangle the bound FFMAs, 4 (one exact q) or 8 (mean q + |B| * spread:
     // shadow sweeps, jittered primary samples), and the interval's centre and half width (7 flops), over the R rays.
-    s->stats.flop_primary = cull ? 0.0 : flop_primary, s->stats.flop_shadow = cull ? 0.0 : 1.0 + 23.0 / trk::SHADOW_R;
+    const bool no_flops = cull || use_bvh; // the optional modes: no fixed per-pair cost
+    s->stats.flop_primary = no_flops ? 0.0 : flop_primary, s->stats.flop_shadow = no_flops ? 0.0 : 1.0 + 23.0 / trk::SHADOW_R;
     // of which multiply-adds that evaluate bounds (the rest is each pair's interval test and the per-triangle interval)
-    s->stats.flop_primary_edges = cull ? 0.0 : flop_primary_edges;
-    s->stats.flop_shadow_edges = cull ? 0.0 : 16.0 / trk::SHADOW_R;
+    s->stats.flop_primary_edges = no_flops ? 0.0 : flop_primary_edges;
+    s->stats.flop_shadow_edges = no_flops ? 0.0 : 16.0 / trk::SHADOW_R;
     if (hc.cull_overflow) {
         // the optional mode's candidate buffer (24 per ray + slack) was too small for this scene's depth complexity: render
         // the frame again with a 4x larger one while that fits comfortably, else by the default sweeps, which need no such
@@ -1337,6 +1438,24 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
 int tracer_cuda_last_stats(tracer_scene_dev *s, tracer_frame_stats *out) {
     if (!s || !out) return fail(TRACER_ERR_INVALID, "null argument");
     *out = s->stats;
+    return TRACER_OK;
+}
+
+// Internal (measurement): (re)build the scene's BVH on its context's stream, timed with CUDA events around the build and
+// a synchronise; *ms_out = the build's device time.  The next BVH render uses this tree.
+int tracer__bvh_prepare(tracer_scene_dev *s, double *ms_out) {
+    if (!s || !s->ctx || !s->ctx->inited) return fail(TRACER_ERR_INVALID, "null scene");
+    t_pool = &s->ctx->pool;
+    CK_CUDA(cudaSetDevice(s->ctx->device));
+    cudaStream_t st = s->ctx->stream;
+    s->bvh_built = false;
+    CK_CUDA(cudaEventRecord(s->ev[0], st));
+    if (int rc = ensure_bvh(s, st)) return rc;
+    CK_CUDA(cudaEventRecord(s->ev[3], st));
+    CK_CUDA(cudaEventSynchronize(s->ev[3]));
+    float ms = 0.f;
+    CK_CUDA(cudaEventElapsedTime(&ms, s->ev[0], s->ev[3]));
+    if (ms_out) *ms_out = ms;
     return TRACER_OK;
 }
 

@@ -56,7 +56,7 @@ def torch_stream_handle():
 
 
 def render_frame(renderer, resident_scene, camera, width, height, *, rank=0, world=1, band_rows=DEFAULT_BAND_ROWS,
-                 rng_mode=0, seed=1, group=None, bundle_cull=False, samples_per_pixel=0):
+                 rng_mode=0, seed=1, group=None, bundle_cull=False, samples_per_pixel=0, bvh=False):
     """Render this rank's bands into HBM, gather to rank 0, assemble.  Returns
     (frame uint8 CUDA tensor [H, W, 3] on rank 0 else None, per-rank stats dict)."""
     import torch
@@ -66,7 +66,7 @@ def render_frame(renderer, resident_scene, camera, width, height, *, rank=0, wor
     stream = torch_stream_handle()
     bands = (band_rows, rank, world) if world > 1 else None
     fr = renderer.trace(resident_scene, camera, width, height, rng_mode=rng_mode, seed=seed, bands=bands,
-                        out_device_ptr=local.data_ptr(), stream=stream, bundle_cull=bundle_cull,
+                        out_device_ptr=local.data_ptr(), stream=stream, bundle_cull=bundle_cull, bvh=bvh,
                         samples_per_pixel=samples_per_pixel)
     if world == 1:
         return local, fr.stats

@@ -125,6 +125,14 @@ typedef struct tracer_render_opts {
     float *out_v;         /* closest-hit v */
     int32_t *out_occ_tri; /* [n_px*n_lights] first in-order occluder, -1 none, -2 no shadow ray */
     float *out_rgb;       /* [n_px*3] float accumulator before quantisation */
+
+    int32_t accel;        /* OPTIONAL mode: 0 = the modes above; 1 = BVH: a linear BVH over the triangles (built on the
+                             device on the first BVH render of a scene, kept until the scene is destroyed) with a
+                             conservative traversal in front of the reference's own test; identical results.  Not
+                             combinable with bundle_cull or exhaustive_strict (TRACER_ERR_INVALID); rays_per_thread and
+                             shadow_chunks are ignored.  In this mode tests_primary / tests_shadow = strict_evals = the
+                             triangle tests done at leaves, flop_* = 0, and the tree's build time is part of ms_other.
+                             Appended last: callers with an older struct_size get 0. */
 } tracer_render_opts;
 
 typedef struct tracer_frame_stats {
