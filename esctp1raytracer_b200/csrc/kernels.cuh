@@ -270,7 +270,8 @@ __host__ __device__ __forceinline__ void origin_rows(const float *__restrict__ p
     if (want_span) span_rows(rows, slo, shi);
 }
 
-// table: the 48-byte three-row table (MODE_OWNQ sweeps, bundle-cull mode) or null; span: the 32-byte span table or null
+// table: the 48-byte three-row table (MODE_OWNQ sweeps, bundle-cull mode) or null; span: the 32-byte span table or null,
+// stored in the hot form of the sweeps (sweep::hot_row)
 __global__ void build_origin_table(const float *__restrict__ tri_verts, int n_tris, int n_pad, const TableParam tp,
                                    float4 *__restrict__ table, float4 *__restrict__ span) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -288,6 +289,7 @@ __global__ void build_origin_table(const float *__restrict__ tri_verts, int n_tr
         table[3 * (size_t)i + 2] = rd;
     }
     if (span) {
+        sweep::hot_row(slo, shi);
         span[2 * (size_t)i] = slo;
         span[2 * (size_t)i + 1] = shi;
     }
@@ -300,8 +302,10 @@ __global__ void build_allcand_table(int n_tris, int n_pad, float4 *__restrict__ 
     const float4 r = make_float4(0.f, 0.f, i < n_tris ? 1.f : -1.f, 0.f);
     table[3 * (size_t)i] = table[3 * (size_t)i + 1] = table[3 * (size_t)i + 2] = r;
     const float lo = i < n_tris ? sweep::SPAN_OPEN : -sweep::SPAN_OPEN;
-    span[2 * (size_t)i] = make_float4(0.f, lo, 0.f, lo);
-    span[2 * (size_t)i + 1] = make_float4(0.f, sweep::SPAN_OPEN, 0.f, sweep::SPAN_OPEN);
+    float4 slo = make_float4(0.f, lo, 0.f, lo), shi = make_float4(0.f, sweep::SPAN_OPEN, 0.f, sweep::SPAN_OPEN);
+    sweep::hot_row(slo, shi);
+    span[2 * (size_t)i] = slo;
+    span[2 * (size_t)i + 1] = shi;
 }
 
 // ---------------------------------------------------------------------------------
@@ -335,7 +339,8 @@ struct PrimaryParams {
 // rejects, ray_triangle.h:49, so among equal t the lowest index stays), whatever the order of evaluation.
 // k0: local pixel index of the thread's ray 0 (ray r = pixel k0 + r).  filt: rays the filter passed (validation).
 // Returns evaluations | filter misses << 16.
-__device__ __noinline__ unsigned strict_primary(const PrimaryParams &p, int k0, unsigned mask, int tri, unsigned filt) {
+template <class Mask>
+__device__ __noinline__ unsigned strict_primary(const PrimaryParams &p, int k0, Mask mask, int tri, Mask filt) {
     const float *q = p.tri_verts + 9 * (size_t)tri;
     const f3 v0 = strict::mk(__ldg(q), __ldg(q + 1), __ldg(q + 2));
     const f3 v1 = strict::mk(__ldg(q + 3), __ldg(q + 4), __ldg(q + 5));
@@ -343,7 +348,7 @@ __device__ __noinline__ unsigned strict_primary(const PrimaryParams &p, int k0, 
     const f3 o = strict::ld(p.cam.o);
     unsigned ret = 0;
     while (mask) {
-        const int r = __ffs(mask) - 1;
+        const int r = sweep::lowest_ray(mask);
         mask &= mask - 1;
         int w, h;
         p.bands.map(k0 + r, w, h);
@@ -358,6 +363,12 @@ __device__ __noinline__ unsigned strict_primary(const PrimaryParams &p, int k0, 
     return ret;
 }
 
+// CTAs per SM of the closest-hit sweep: 64 rays per thread need more registers than sweep::MINB leaves
+#ifndef SWEEP_MINB64
+#define SWEEP_MINB64 2
+#endif
+constexpr int primary_minb(int R) { return R > 32 ? SWEEP_MINB64 : sweep::MINB; }
+
 // Ray block = screen tile, each thread holding R horizontally consecutive pixels of ONE image row.  Without
 // jitter those R rays share the filter parameter q exactly (MODE_SHAREDQ): the four bounds of a triangle's span row are
 // evaluated once per thread and triangle.  With jittered samples (extension) the rays of a thread are the same sample
@@ -365,8 +376,9 @@ __device__ __noinline__ unsigned strict_primary(const PrimaryParams &p, int k0, 
 // the thread's mean q plus |B| x spread (MODE_QBAR, as the shadow sweeps do); the candidate path uses each ray's own q.
 // MODE_OWNQ (three-row table, every ray its own q) remains for frames too small for the span rows' |p|,|q| range.
 template <int R, bool EXHAUSTIVE, int MODE>
-__global__ void __launch_bounds__(sweep::NT, sweep::MINB) primary_kernel(const __grid_constant__ PrimaryParams p) {
+__global__ void __launch_bounds__(sweep::NT, primary_minb(R)) primary_kernel(const __grid_constant__ PrimaryParams p) {
     constexpr bool SHAREDQ = MODE == sweep::MODE_SHAREDQ;
+    using Mask = sweep::RayMask<R>;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     using Smem = sweep::SmemT<sweep::Rows<MODE>::N>;
     Smem &sm = *reinterpret_cast<Smem *>(smem_raw);
@@ -389,10 +401,10 @@ __global__ void __launch_bounds__(sweep::NT, sweep::MINB) primary_kernel(const _
         const int txn = 1 << p.tx_log2;
         const int x0 = (tile_x * txn + (tid & (txn - 1))) * R, ly = tile_y * (sweep::NT >> p.tx_log2) + (tid >> p.tx_log2);
         float rp[R], rq[R];
-        unsigned valid = 0;
+        Mask valid = 0;
 #pragma unroll
         for (int r = 0; r < R; ++r) {
-            if (x0 + r < W && ly < p.n_rows) valid |= 1u << r;
+            if (x0 + r < W && ly < p.n_rows) valid |= (Mask)1 << r;
             int w, h;
             p.bands.map(min(ly, p.n_rows - 1) * W + min(x0 + r, W - 1), w, h);
             // filter parameters: the ray's own (s,t) on the image plane (main.cpp:709-710)
@@ -404,7 +416,7 @@ __global__ void __launch_bounds__(sweep::NT, sweep::MINB) primary_kernel(const _
             for (int r = 1; r < R; ++r) rq[r] = q0;
         }
         const int k0 = ly * W + x0; // valid rays are pixels k0 + r
-        unsigned done = 0;
+        Mask done = 0;
         float qbar = 0.f, qdelta = 0.f;
         if (MODE == sweep::MODE_QBAR) { // (rays past the frame's edge are duplicates of edge pixels: all R values count)
             float qmin = rq[0], qmax = rq[0];
@@ -416,14 +428,14 @@ __global__ void __launch_bounds__(sweep::NT, sweep::MINB) primary_kernel(const _
         }
         sweep::sweep_table<R, MODE, false, EXHAUSTIVE>(
             sm, p.table, tile_lo, tile_hi, p.n_tris, rp, rq, qbar, qdelta, valid, done, gtile, n_swept,
-            [&](unsigned mask, int tri, unsigned filt) {
+            [&](Mask mask, int tri, Mask filt) {
                 const unsigned c = strict_primary(p, k0, mask, tri, filt);
                 n_strict += c & 0xffffu, n_miss += c >> 16;
-                return 0u;
+                return (Mask)0;
             },
             &n_pipe_err);
         const int t_lo = min(tile_lo * sweep::TILE, p.n_tris), t_hi = min(tile_hi * sweep::TILE, p.n_tris);
-        tests += (unsigned long long)__popc(valid) * (unsigned)(t_hi - t_lo);
+        tests += (unsigned long long)__popcll(valid) * (unsigned)(t_hi - t_lo);
         __syncthreads(); // sm.blk is rewritten by the next item
     }
     atomicAdd(&p.counters->tests_primary, tests);

@@ -3,8 +3,8 @@
 //
 // What the reference does per (ray, triangle) pair: full Moller-Trumbore with
 // a double-precision divide (ray_triangle.h:7-57, ~52 flop).  What this kernel
-// does per pair: half a packed add and half a three-input min (4., interval form),
-// plus ~15 ops per thread and triangle.  The saving comes from these observations.
+// does per pair: half a packed add and half a three-input min (4., hot rows), plus
+// 8 ops per thread and triangle (12 with a mean q).  The saving comes from these observations.
 //
 //  1. Every sweep is a bundle of rays through ONE common point.  Primary rays
 //     all start at the eye (camera.h:31-34).  A shadow ray runs from the hit
@@ -51,7 +51,9 @@
 //     p >= q*beta_i + gamma_i where A_i > 0 and p <= q*beta_i + gamma_i where A_i < 0.  A
 //     triangle has two lower bounds and one upper bound or the reverse, so the table row is
 //     two lower + two upper bounds = 32 bytes, the thread evaluates the four at its q and keeps
-//     the binding ones (4 FFMA + 2 FMNMX), and each PAIR is a two-sided span test (below).
+//     the binding ones, and each PAIR is a two-sided span test (below).  The tables store the rows
+//     in HOT form (hot_row): the test's +1s, the clamp and the margin folded into the constants, so
+//     the thread's set-up is 4 FFMA + 2 FMNMX3 + 2 FADD per triangle.
 //     MODE_OWNQ (every ray its own q) keeps the 48-byte three-row table: 3 x (A,B,C,-).
 //
 // Mapping to the SM (choices measured with tools/sweep_mb2-4.cu, see DESIGN.md):
@@ -59,8 +61,8 @@
 //    (cp.async.bulk + mbarrier complete_tx, UBLKCP in SASS), STAGES deep;
 //  * every lane of every warp reads the SAME row at the same time, so the two LDS.128 per
 //    triangle are pure broadcasts, amortised over R rays per thread held in registers
-//    (R = 32 closest hit, 16 any-hit);
-//  * each pair is ONE interval test |S*p - c| <= h (interval form, below): per two pairs one packed
+//    (R = 64 closest hit, 16 any-hit);
+//  * each pair is ONE interval test |2*S*p + nc2| <= h2 (hot rows, below): per two pairs one packed
 //    FADD2 and one FMNMX3 running minimum, no saturation, no integer op.  History on this part
 //    (cycles per pair, closest hit): round 1 sign bits through LOP3 on the half-rate ALU pipe 7.9,
 //    three saturating rows with a product accumulate 6.8, span form with two saturating adds 4.0;
@@ -70,9 +72,12 @@
 //    tile stage (shared-memory atomicAdd) and the last one issues the refill, so warps
 //    run up to STAGES-1 tiles apart.  An any-hit warp whose rays all have their occluder
 //    stops evaluating (it only keeps the stage counts going);
-//  * SWEEP_NT threads per CTA, SWEEP_MINB CTAs per SM (launch bounds cap the registers).
+//  * SWEEP_NT threads per CTA, SWEEP_MINB CTAs per SM (launch bounds cap the registers; the 64-ray closest-hit
+//    kernel has its own, SWEEP_MINB64 in kernels.cuh).
 #pragma once
+#include <cmath>
 #include <cstdint>
+#include <type_traits>
 #include <cuda_runtime.h>
 
 #include "strict_math.cuh"
@@ -217,7 +222,7 @@ struct Batch {
     static_assert(R % 2 == 0, "rays are evaluated in pairs");
     static constexpr int GROUP = R >= 12 ? 4 : 8;                   // triangles per accumulator group
     static constexpr int NACC = R >= 16 ? 4 : R >= 12 ? 3 : (R >= 4 ? 2 : 1); // independent packed accumulators (FFMA2 chains) per group
-    static_assert(R <= 32, "ray masks are 32 bits wide");
+    static_assert(R <= 32, "ray masks of the three-row form are 32 bits wide");
     static constexpr int NGROUPS = BATCH / GROUP;
 };
 
@@ -326,6 +331,8 @@ static_assert(SPAN_BATCH <= 32 && TILE % SPAN_BATCH == 0, "one verdict bit per t
 
 // (ax, ay) from span_terms / span_terms_qbar -> the negated centre and the widened half width of the interval of S*p
 // (box, delta: SPAN_BOX, SPAN_DELTA; other values only in the test hook tracer__interval_pass)
+// span_terms, span_pass and span_interval are the reference form of the span test: the tables store the HOT form of the
+// same rows (hot_row below), which is proven against them.
 __host__ __device__ __forceinline__ void span_interval(float ax, float ay, float &nc, float &h, float box = SPAN_BOX,
                                                       float delta = SPAN_DELTA) {
     const float lo = fmaxf(1.f - ax, -box), hi = fminf(ay - 1.f, box);
@@ -335,6 +342,16 @@ __host__ __device__ __forceinline__ void span_interval(float ax, float ay, float
 // the interval test of one pair, as the hot loop evaluates it (ps = p * SPAN_S)
 __host__ __device__ __forceinline__ bool interval_pass(float nc, float h, float ps) { return fabsf(ps + nc) <= h; }
 
+// min(a, b, c): one FMNMX3 on sm_100 (NaN inputs are dropped, as fminf drops them)
+__host__ __device__ __forceinline__ float fmin3(float a, float b, float c) {
+#ifdef __CUDA_ARCH__
+    float d;
+    asm("min.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
+    return d;
+#else
+    return fminf(fminf(a, b), c);
+#endif
+}
 // min(m, |a|, |b|): one FMNMX3 with both absolute values as operand modifiers (sm_100)
 __device__ __forceinline__ float fmin3_abs(float m, float a, float b) {
     float d;
@@ -342,26 +359,92 @@ __device__ __forceinline__ float fmin3_abs(float m, float a, float b) {
     return d;
 }
 
-// SPAN_BATCH triangles of a staged span tile against the R rays of this thread (ps[r] = p_r * SPAN_S).  One minimum
+// ---- HOT rows: the span row as the tables store it (the hot loop of MODE_SHAREDQ and MODE_QBAR) ---------------------------
+// The +1 of the saturating test, the clamp and the interval's margin are folded into the row.  build_origin_table stores
+// span_rows' row with both constants of every bound shifted:  C' = C - (1 - HOT_DELTA), rounded toward +inf (hot_row), the
+// q coefficients unchanged.  A thread with shared q then forms, per triangle,
+//     A = min3(q*Bl1 + Cl1', q*Bl2 + Cl2', HOT_CLAMP) ~ -lo + delta     B = min3(q*Bu1 + Cu1', q*Bu2 + Cu2', HOT_CLAMP) ~ hi + delta
+//     nc2 = A - B  (the negated centre of the interval of 2*S*p)          h2 = A + B  (its full width, 2*delta included)
+// and per ray pair |2*S*p_r + nc2| <= h2: the two 1s cancel, delta is in the row and the clamp is the third input of the
+// FMNMX3.  Rays hold 2*S*p (exact: a power of two).  Per thread and triangle 4 FFMA + 2 FMNMX3 + 2 FADD (MODE_QBAR: 8 FFMA,
+// the |B|*qdelta widening kept, with qdelta scaled by HOT_QD_SCALE), against 4 FFMA + 2 FMNMX + 8 for span_interval.
+//
+// Why every pair the saturating test passes (fl(S*p + ax) >= 1 and fl(ay - S*p) >= 1, ax and ay from span_terms or
+// span_terms_qbar on the unshifted row) passes the hot test.  u = 2^-24, C = HOT_CLAMP, s = 1 - delta, P0 = S*SPAN_PMAX =
+// C - 1 >= |S*p|, Q = C + 2.  Take one lower bound, a = fl(G) its saturating value, G = |Bl|*qd + t0 exactly, t0 = fl(z),
+// z = q*Bl + Cl (qd = 0 and t0 = z with a shared q), and its hot value A_i = fl(G'), G' = |Bl|*qd' + t, t = fl(q*Bl + Cl').
+//   the pass: a >= ax and fl(S*p + ax) >= 1 give a >= 1 - u/2 - S*p (a sum rounds to 1 from 1 - u/2 at the least).
+//   shift:    Cl' >= Cl - s exactly (rounded up), so t >= fl(z - s) >= z - s - u|z| - u, and t0 <= z + u|z|.
+//   qdelta:   qd' = fl(qd * (1 + 2^-20)) >= qd (1 + 14u), and |z| <= (1 + 2u)(|G| + |Bl|*qd), so
+//             G' - G >= 14u|Bl|qd - s - u - 2(1 + 2u)u(|G| + |Bl|qd) >= -s - u - 2.1u|G|.
+//   a <= Q:   |G - a| <= uQ, G' >= a - s - 3.2uQ - u, and A_i = fl(G') >= min(C, a - s - 4.2uQ - 3u).
+//   a > Q:    G > Q(1 - u), G' > C + 1 - 4.3uQ > C, A_i >= C.
+// So A = min3(A_1, A_2, C) >= min(C, -S*p + delta - e) = -S*p + delta - e, e = 4.2uQ + 3.5u (C >= P0 + delta); the same
+// for B >= S*p + delta - e, and |A|, |B| <= C.  Then, with one rounding each (u times a magnitude <= 2C):
+//   h2 >= A + B - 2uC;   |2*S*p + A - B| <= A + B - 2*delta + 2e;   nc2 is off by <= 2uC and the FADD2 by <= 2uC(1 + u),
+// so |fl(2*S*p + nc2)| <= h2 whenever delta >= e + 3uC + u^2 C ~ 7.2uC = 0.030 row units.  HOT_DELTA = 8 FLT_EPSILON * C
+// (0.066, as SPAN_DELTA) and HOT_CLAMP = SPAN_BOX >= P0 + HOT_DELTA.  The FMNMX3 and the final compare are exact.
+// Padding rows (Cl = -SPAN_OPEN, shifted: still -1e30) give A = -1e30, B = C, h2 = -1e30 < 0: never a candidate;
+// always-candidate rows (every constant SPAN_OPEN) give A = B = C, nc2 = 0, h2 = 2C > |2*S*p|.  A NaN bound is dropped by
+// the min3 (the clamp stays), a NaN |e| by the running minimum: neither can hide a candidate.
+constexpr float HOT_CLAMP = SPAN_BOX;
+constexpr float HOT_DELTA = 8.f * 1.1920928955078125e-7f * HOT_CLAMP;
+constexpr float HOT_QD_SCALE = 1.f + 0x1p-20f;
+static_assert((double)HOT_CLAMP >= (double)SPAN_S * 1.0625 + (double)HOT_DELTA, "the clamp lies outside every swept ray");
+
+// C - (1 - delta) rounded toward +inf: an exact sum in FP64 (TwoSum), then the nearest float, moved up if below
+__host__ __device__ __forceinline__ float hot_shift(float c, float delta) {
+    const double a = (double)c, b = (double)delta - 1.0; // exact
+    const double d = a + b, bb = d - a, err = (a - (d - bb)) + (b - bb); // a + b = d + err exactly
+    float f = (float)d;
+    if ((double)f < d || ((double)f == d && err > 0.0)) f = nextafterf(f, INFINITY);
+    return f;
+}
+// span_rows' row (lo, hi) -> its hot form, in place (build_origin_table, build_allcand_table; delta: tests only)
+__host__ __device__ __forceinline__ void hot_row(float4 &lo, float4 &hi, float delta = HOT_DELTA) {
+    lo.y = hot_shift(lo.y, delta), lo.w = hot_shift(lo.w, delta);
+    hi.y = hot_shift(hi.y, delta), hi.w = hot_shift(hi.w, delta);
+}
+__host__ __device__ __forceinline__ float hot_qdelta(float qdelta) { return qdelta * HOT_QD_SCALE; }
+// (nc2, h2) of a hot row at q: a shared exact q, or q = qbar with the bounds widened by |B| * qdh, qdh = hot_qdelta(qdelta)
+__host__ __device__ __forceinline__ void hot_terms(const float4 lo, const float4 hi, float q, float &nc2, float &h2) {
+    const float A = fmin3(fmaf(q, lo.x, lo.y), fmaf(q, lo.z, lo.w), HOT_CLAMP);
+    const float B = fmin3(fmaf(q, hi.x, hi.y), fmaf(q, hi.z, hi.w), HOT_CLAMP);
+    nc2 = A - B, h2 = A + B;
+}
+__host__ __device__ __forceinline__ void hot_terms_qbar(const float4 lo, const float4 hi, float qbar, float qdh, float &nc2, float &h2) {
+    const float A = fmin3(fmaf(fabsf(lo.x), qdh, fmaf(qbar, lo.x, lo.y)), fmaf(fabsf(lo.z), qdh, fmaf(qbar, lo.z, lo.w)), HOT_CLAMP);
+    const float B = fmin3(fmaf(fabsf(hi.x), qdh, fmaf(qbar, hi.x, hi.y)), fmaf(fabsf(hi.z), qdh, fmaf(qbar, hi.z, hi.w)), HOT_CLAMP);
+    nc2 = A - B, h2 = A + B;
+}
+// the hot test of one pair (ps2 = p * 2 * SPAN_S)
+__host__ __device__ __forceinline__ bool hot_pass(float nc2, float h2, float ps2) { return fabsf(ps2 + nc2) <= h2; }
+
+// ray masks of the sweeps: a bit per ray of a thread
+template <int R>
+using RayMask = typename std::conditional<(R > 32), unsigned long long, unsigned>::type;
+template <class M>
+__device__ __forceinline__ int lowest_ray(M m) { return sizeof(M) == 8 ? __ffsll((long long)m) - 1 : __ffs((int)m) - 1; }
+
+// SPAN_BATCH triangles of a staged hot-row tile against the R rays of this thread (ps2[r] = p_r * 2 * SPAN_S).  One minimum
 // chain per triangle: the SPAN_BATCH chains are independent, which is the loop's instruction-level parallelism.
-// Returns bit k set = triangle k may hold a candidate.
+// qdh: hot_qdelta(qdelta) (MODE_QBAR).  Returns bit k set = triangle k may hold a candidate.
 template <int R, int MODE>
-__device__ __forceinline__ unsigned eval_interval(const float4 *__restrict__ tp, const float (&ps)[R], float q, float qdelta) {
+__device__ __forceinline__ unsigned eval_interval(const float4 *__restrict__ tp, const float (&ps2)[R], float q, float qdh) {
     static_assert(R % 2 == 0, "rays are evaluated in pairs");
     unsigned cand = 0;
 #pragma unroll
     for (int k = 0; k < SPAN_BATCH; ++k) {
-        float ax, ay, nc, h;
-        if (MODE == MODE_QBAR) span_terms_qbar(tp[2 * k], tp[2 * k + 1], q, qdelta, ax, ay);
-        else span_terms(tp[2 * k], tp[2 * k + 1], q, ax, ay);
-        span_interval(ax, ay, nc, h);
+        float nc2, h2;
+        if (MODE == MODE_QBAR) hot_terms_qbar(tp[2 * k], tp[2 * k + 1], q, qdh, nc2, h2);
+        else hot_terms(tp[2 * k], tp[2 * k + 1], q, nc2, h2);
         float m = __int_as_float(0x7f800000); // +inf
 #pragma unroll
         for (int r = 0; r < R; r += 2) {
-            const float2 e = __fadd2_rn(make_float2(ps[r], ps[r + 1]), make_float2(nc, nc));
+            const float2 e = __fadd2_rn(make_float2(ps2[r], ps2[r + 1]), make_float2(nc2, nc2));
             m = fmin3_abs(m, e.x, e.y);
         }
-        cand |= (unsigned)(m <= h) << k;
+        cand |= (unsigned)(m <= h2) << k;
     }
     return cand;
 }
@@ -396,15 +479,17 @@ __device__ __forceinline__ unsigned eval_batch_lop3(const float4 *__restrict__ t
 // ---- the sweep over tiles [tile_lo, tile_hi) of one origin table, for the R rays of each thread ---
 // rp/rq: the rays' parameters in the table's direction parametrisation (rq is read by MODE_OWNQ and by the candidate path
 //        of the any-hit sweeps; MODE_SHAREDQ takes the common q from rq[0], MODE_QBAR from qbar/qdelta)
-// valid: bit r set = ray r exists; done: bit r set = ray r needs no more tests
+// valid: bit r set = ray r exists; done: bit r set = ray r needs no more tests (RayMask<R>: 64 bits for R > 32)
 // gtile: running tile counter of this CTA (mbarrier phase bookkeeping across work items)
 // strict(mask, tri, filt) -> newly done rays: the reference's own test on the surviving pairs (kernels.cuh);
 //        mask = rays to test, filt = rays the filter passed (differs from mask only in EXHAUSTIVE validation mode)
 template <int R, int MODE, bool ANYHIT, bool EXHAUSTIVE, class Strict>
 __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const float4 *__restrict__ table, int tile_lo, int tile_hi, int n_tris,
-                                            const float (&rp)[R], const float (&rq)[R], float qbar, float qdelta, unsigned valid,
-                                            unsigned &done, unsigned &gtile, unsigned &n_tiles_swept, Strict &&strict,
+                                            const float (&rp)[R], const float (&rq)[R], float qbar, float qdelta, RayMask<R> valid,
+                                            RayMask<R> &done, unsigned &gtile, unsigned &n_tiles_swept, Strict &&strict,
                                             unsigned *n_pipe_err = nullptr) {
+    using Mask = RayMask<R>;
+    static_assert(R <= 32 || MODE != MODE_OWNQ, "the three-row form's rays fit one 32-bit mask");
     constexpr int ROWS = Rows<MODE>::N;
     constexpr uint32_t BYTES = Rows<MODE>::BYTES;
     constexpr bool SPAN = MODE != MODE_OWNQ;
@@ -419,10 +504,10 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
             tma_load_1d(sm.tile[g % STAGES], src + (size_t)i * TILE * ROWS, BYTES, &sm.full_bar[g % STAGES]);
         }
     }
-    float ps[R]; // span form: the rays' p in row units (exact: SPAN_S is a power of two)
+    float ps2[R]; // span form: the rays' 2 p in row units (exact: SPAN_S is a power of two)
 #pragma unroll
-    for (int r = 0; r < R; ++r) ps[r] = rp[r] * SPAN_S;
-    const float qhot = MODE == MODE_QBAR ? qbar : rq[0];
+    for (int r = 0; r < R; ++r) ps2[r] = rp[r] * (2.f * SPAN_S);
+    const float qhot = MODE == MODE_QBAR ? qbar : rq[0], qdh = hot_qdelta(qdelta);
     for (int it = 0; it < n_tiles; ++it) {
         const unsigned g = gtile + it;
         const int s = g % STAGES;
@@ -442,17 +527,17 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
         };
         if (EXHAUSTIVE && n_pipe_err && tile_differs() && (tid & 31) == 0) ++*n_pipe_err;
         // any-hit: a warp whose rays all have their occluder has nothing left to evaluate
-        const bool idle = ANYHIT && __all_sync(0xffffffffu, (done | ~valid) == 0xffffffffu);
+        const bool idle = ANYHIT && __all_sync(0xffffffffu, (Mask)(done | ~valid) == (Mask)~(Mask)0);
         if (!idle) {
             ++n_tiles_swept;
             const float4 *__restrict__ tp = sm.tile[s];
             // triangles per hot-loop call, and per bit of its verdict: the interval form (span rows) flags single
             // triangles, the three-row form groups of GROUP
-            constexpr int NB = SPAN ? SPAN_BATCH : BATCH, UNIT = SPAN ? 1 : Batch<R>::GROUP;
+            constexpr int NB = SPAN ? SPAN_BATCH : BATCH, UNIT = SPAN ? 1 : Batch<SPAN ? 2 : R>::GROUP;
 #pragma unroll 1
             for (int b0 = 0; b0 < TILE; b0 += NB) {
                 unsigned cand;
-                if (SPAN) cand = eval_interval<R, MODE>(tp + ROWS * b0, ps, qhot, qdelta);
+                if constexpr (SPAN) cand = eval_interval<R, MODE>(tp + ROWS * b0, ps2, qhot, qdh);
                 else cand = eval_batch<R, MODE>(tp + ROWS * b0, rp, rq, qbar, qdelta);
 #ifdef SWEEP_NO_STRICT // development microbenchmark only (tools/sweep_mb2.cu): timing without the strict path
                 if (cand) ++done;
@@ -463,7 +548,7 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
                 if (EXHAUSTIVE) cand = NB / UNIT == 32 ? 0xffffffffu : (1u << (NB / UNIT)) - 1u;
                 while (cand) {
                     // rare: a triangle (group of UNIT triangles) may hold a candidate.  Rebuild the per-ray candidate mask
-                    // of each of its triangles (exact threshold), then the reference's own arithmetic.  The rows are re-read
+                    // of each of its triangles, then the reference's own arithmetic.  The rows are re-read
                     // through opaque loads so that the compiler cannot merge this with the hot evaluation.
                     const int gq = __ffs(cand) - 1; // ascending triangle order
                     cand &= cand - 1;
@@ -471,34 +556,39 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
                     for (int kk = 0; kk < UNIT; ++kk) {
                         const int k = b0 + gq * UNIT + kk;
                         const int tri = (tile_lo + it) * TILE + k;
-                        unsigned filt = 0;
+                        Mask filt = 0;
                         if (SPAN) {
+                            // the hot test on the stored row, ray by ray: it passes every pair span_pass passes (hot_row)
                             const float4 lo = lds128_opaque(&tp[2 * k]), hi = lds128_opaque(&tp[2 * k + 1]);
                             if (MODE == MODE_QBAR && ANYHIT) {
                                 // shadow rays: each ray's own q (the widening of the shared-q bounds, ~10 % of a pixel over
                                 // 16 consecutive rays of a q-sorted list, would cost ~5 % more strict evaluations)
 #pragma unroll
-                                for (int r = 0; r < R; ++r) filt |= (unsigned)span_pass(lo, hi, ps[r], rq[r]) << r;
+                                for (int r = 0; r < R; ++r) {
+                                    float nc2, h2;
+                                    hot_terms(lo, hi, rq[r], nc2, h2);
+                                    filt |= (Mask)hot_pass(nc2, h2, ps2[r]) << r;
+                                }
                             } else {
                                 // closest hit: the hot loop's own test, ray by ray — exact with a common q; with jittered samples
                                 // (mean q + |B| * qdelta, 1/8 pixel) it saves keeping 32 q values in registers during the sweep
                                 // for ~2 % more strict evaluations
-                                float ax, ay;
-                                if (MODE == MODE_QBAR) span_terms_qbar(lo, hi, qhot, qdelta, ax, ay);
-                                else span_terms(lo, hi, qhot, ax, ay);
+                                float nc2, h2;
+                                if (MODE == MODE_QBAR) hot_terms_qbar(lo, hi, qhot, qdh, nc2, h2);
+                                else hot_terms(lo, hi, qhot, nc2, h2);
 #pragma unroll
-                                for (int r = 0; r < R; ++r) filt |= (unsigned)(fminf(ps[r] + ax, ay - ps[r]) >= 1.f) << r;
+                                for (int r = 0; r < R; ++r) filt |= (Mask)hot_pass(nc2, h2, ps2[r]) << r;
                             }
                         } else {
                             const float4 rb = lds128_opaque(&tp[3 * k]), rc = lds128_opaque(&tp[3 * k + 1]), rd = lds128_opaque(&tp[3 * k + 2]);
 #pragma unroll
-                            for (int r = 0; r < R; ++r) filt |= (unsigned)edge_pass(rb, rc, rd, rp[r], rq[r]) << r;
+                            for (int r = 0; r < R; ++r) filt |= (Mask)edge_pass(rb, rc, rd, rp[r], rq[r]) << r;
                         }
                         if (EXHAUSTIVE && !((cand_hot >> gq) & 1u)) filt = 0;
-                        const unsigned live = valid & ~done;
-                        const unsigned mask = EXHAUSTIVE ? live : (filt & live);
+                        const Mask live = valid & ~done;
+                        const Mask mask = EXHAUSTIVE ? live : (filt & live);
                         if (mask && tri < n_tris) {
-                            const unsigned nw = strict(mask, tri, filt);
+                            const Mask nw = strict(mask, tri, filt);
                             if (ANYHIT) done |= nw;
                         }
                     }

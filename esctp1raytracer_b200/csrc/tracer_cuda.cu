@@ -81,6 +81,32 @@ extern "C" void tracer__interval_pass(const float *row8, int n, const float *p, 
     }
 }
 extern "C" void tracer__interval_consts(float *out2) { out2[0] = sweep::SPAN_BOX, out2[1] = sweep::SPAN_DELTA; }
+// n rays (p, own q) of one thread against one span row (row8 = lo.xyzw, hi.xyzw as span_rows makes it), stored in the hot form
+// with margin delta (sweep::hot_row; sweep::HOT_DELTA in the tables).  Shared-q form: qdelta < 0 = one exact q = qbar
+// (MODE_SHAREDQ), else q = qbar with the bounds widened by |B| * qdelta (MODE_QBAR).  bit 0 = the hot loop's test in the
+// shared-q form, bit 1 = the candidate path's hot test with the ray's own q, bit 2 = the saturating form in the same shared-q
+// form, bit 3 = span_pass with the ray's own q, bit 4 = the interval form (span_interval, SPAN_BOX, SPAN_DELTA) it replaces.
+// hot8 (may be null) receives the stored hot row.
+extern "C" void tracer__hot_row_pass(const float *row8, int n, const float *p, const float *q, float qbar, float qdelta, float delta,
+                                     unsigned char *out, float *hot8) {
+    const float4 lo = make_float4(row8[0], row8[1], row8[2], row8[3]), hi = make_float4(row8[4], row8[5], row8[6], row8[7]);
+    float4 hlo = lo, hhi = hi;
+    sweep::hot_row(hlo, hhi, delta);
+    if (hot8) hot8[0] = hlo.x, hot8[1] = hlo.y, hot8[2] = hlo.z, hot8[3] = hlo.w, hot8[4] = hhi.x, hot8[5] = hhi.y, hot8[6] = hhi.z, hot8[7] = hhi.w;
+    float nc2, h2, ax, ay, nc, h;
+    if (qdelta < 0.f) sweep::hot_terms(hlo, hhi, qbar, nc2, h2), sweep::span_terms(lo, hi, qbar, ax, ay);
+    else sweep::hot_terms_qbar(hlo, hhi, qbar, sweep::hot_qdelta(qdelta), nc2, h2), sweep::span_terms_qbar(lo, hi, qbar, qdelta, ax, ay);
+    sweep::span_interval(ax, ay, nc, h);
+    for (int i = 0; i < n; ++i) {
+        const float ps = p[i] * sweep::SPAN_S, ps2 = p[i] * (2.f * sweep::SPAN_S);
+        float rnc2, rh2;
+        sweep::hot_terms(hlo, hhi, q[i], rnc2, rh2);
+        out[i] = (unsigned char)((sweep::hot_pass(nc2, h2, ps2) ? 1 : 0) | (sweep::hot_pass(rnc2, rh2, ps2) ? 2 : 0) |
+                                 (fminf(ps + ax, ay - ps) >= 1.f ? 4 : 0) | (sweep::span_pass(lo, hi, ps, q[i]) ? 8 : 0) |
+                                 (sweep::interval_pass(nc, h, ps) ? 16 : 0));
+    }
+}
+extern "C" void tracer__hot_consts(float *out3) { out3[0] = sweep::HOT_CLAMP, out3[1] = sweep::HOT_DELTA, out3[2] = sweep::HOT_QD_SCALE; }
 
 // Internal (tests only): strict::powf_glibc as the device computes it, for every stride-th float bit pattern x from
 // lo_bits up to hi_bits (inclusive) -> host_out[(hi_bits - lo_bits) / stride + 1], or for n (x, y) pairs.  Runs on the
@@ -409,6 +435,7 @@ int launch_primary(int R, bool ex, int qmode, const trk::PrimaryParams &p, int g
         if (R == 4) return ex ? launch_primary_q<4, true, QB>(p, grid, st) : launch_primary_q<4, false, QB>(p, grid, st);
         return ex ? launch_primary_q<2, true, QB>(p, grid, st) : launch_primary_q<2, false, QB>(p, grid, st);
     }
+    if (R == 64) return ex ? launch_primary_q<64, true, SQ>(p, grid, st) : launch_primary_q<64, false, SQ>(p, grid, st);
     if (R == 32) return ex ? launch_primary_q<32, true, SQ>(p, grid, st) : launch_primary_q<32, false, SQ>(p, grid, st);
     if (R == 24) return ex ? launch_primary_q<24, true, SQ>(p, grid, st) : launch_primary_q<24, false, SQ>(p, grid, st);
     if (R == 16) return ex ? launch_primary_q<16, true, SQ>(p, grid, st) : launch_primary_q<16, false, SQ>(p, grid, st);
@@ -438,20 +465,22 @@ Decomp pick_decomp(int64_t n_rays, int n_tiles, int n_sms, int forced_R, int ext
         return (int)((n_rays + (int64_t)sweep::NT * R - 1) / ((int64_t)sweep::NT * R)) + extra_blocks;
     };
     Decomp d{2, blocks_for(2), 1};
-    // rays per thread: span form with one exact q (no jitter) 32, 16, 8, 4 or 2 (24 on request); span form with a shared
-    // mean q (jittered samples) 16, 8, 4 or 2; three-row form (own q) 12, 8, 4 or 2
-    // (C4 closest-hit sweep on one B200: 997 ms at 16, 944 at 24, 905 at 32)
-    const bool own_q = qmode == sweep::MODE_OWNQ;
-    const int big = own_q ? 12 : 32, mid = own_q ? 8 : 16;
-    if (forced_R == 2 || forced_R == 4 || forced_R == 8 || forced_R == mid || forced_R == big || (qmode == sweep::MODE_SHAREDQ && forced_R == 24)) {
+    // rays per thread: span form with one exact q (no jitter) 64, 32, 16, 8, 4 or 2 (24 on request); span form with a
+    // shared mean q (jittered samples) 32, 16, 8, 4 or 2; three-row form (own q) 12, 8, 4 or 2
+    // (C4 closest-hit sweep on one B200: 997 ms at 16, 944 at 24, 905 at 32 with the saturating span loop)
+    const bool own_q = qmode == sweep::MODE_OWNQ, shared_q = qmode == sweep::MODE_SHAREDQ;
+    const int huge = shared_q ? 64 : 0, big = own_q ? 12 : 32, mid = own_q ? 8 : 16;
+    if (forced_R == 2 || forced_R == 4 || forced_R == 8 || forced_R == mid || forced_R == big ||
+        (shared_q && (forced_R == 24 || forced_R == 64))) {
         d.R = forced_R, d.n_blocks = blocks_for(forced_R);
     } else {
-        for (int R : {big, mid, 8, 4, 2}) {
+        for (int R : {huge, big, mid, 8, 4, 2}) {
+            if (!R) continue;
             d.R = R, d.n_blocks = blocks_for(R);
             if ((int64_t)d.n_blocks * slices_possible >= 4 * (int64_t)n_sms) break;
         }
     }
-    const int64_t ips = (int64_t)items_per_cta() * sweep::MINB;
+    const int64_t ips = (int64_t)items_per_cta() * trk::primary_minb(d.R);
     const int64_t want = (ips * (int64_t)n_sms + d.n_blocks - 1) / std::max(1, d.n_blocks);
     d.n_slices = d.n_blocks >= ips * n_sms ? 1 : (int)std::max<int64_t>(1, std::min<int64_t>(want, slices_possible));
     return d;
@@ -1061,20 +1090,21 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
         p.tri_verts = s->tri_verts;
         p.best = s->best, p.counters = s->counters, p.work = s->work;
         p.n_rows = n_rows, p.n_blocks = 0; // ray blocks = screen tiles of (TX R) x (NT / TX) pixels: least edge waste wins
-        for (int lg = 3; lg <= 6; ++lg) {
+        for (int lg = d.R > 32 ? 2 : 3; lg <= 6; ++lg) { // (64 rays per thread: from 4 x 64 = 256 pixels wide)
             const int tw = (1 << lg) * d.R, th = sweep::NT >> lg;
             const int tx = (W + tw - 1) / tw, nb = tx * ((n_rows + th - 1) / th);
             if (!p.n_blocks || nb < p.n_blocks) p.n_blocks = nb, p.tiles_x = tx, p.tx_log2 = lg;
         }
         p.n_slices = d.n_slices;
-        const int want_items = items_per_cta() * sweep::MINB * g.n_sms;
+        const int minb = trk::primary_minb(d.R);
+        const int want_items = items_per_cta() * minb * g.n_sms;
         if (p.n_blocks < want_items) // same sizing rule as pick_decomp, on the real block count
             p.n_slices = std::max(1, std::min((want_items + p.n_blocks - 1) / p.n_blocks, std::max(1, n_tiles / 4)));
-        const int grid = std::min(p.n_blocks * p.n_slices, sweep::MINB * g.n_sms);
-        // executed FP32 flops per pair: interval form half a packed FADD2 per pair (the three-input min is no flop), and
-        // per thread and triangle 4 FFMA for the bounds + the interval's 3 FADD, FMUL and FFMA (15 flops; 8 more FFMA-flops
-        // with a mean q); three-row form with every ray its own q: 6 FFMA.SAT + FMUL + FFMA
-        flop_primary = qmode == sweep::MODE_OWNQ ? 15.0 : 1.0 + (qmode == sweep::MODE_QBAR ? 23.0 : 15.0) / d.R;
+        const int grid = std::min(p.n_blocks * p.n_slices, minb * g.n_sms);
+        // executed FP32 flops per pair: hot form half a packed FADD2 per pair (the three-input mins are no flops), and
+        // per thread and triangle 4 FFMA for the bounds + the 2 FADD of nc2 and h2 (10 flops; 8 more FFMA-flops with a
+        // mean q); three-row form with every ray its own q: 6 FFMA.SAT + FMUL + FFMA
+        flop_primary = qmode == sweep::MODE_OWNQ ? 15.0 : 1.0 + (qmode == sweep::MODE_QBAR ? 18.0 : 10.0) / d.R;
         flop_primary_edges = qmode == sweep::MODE_OWNQ ? 12.0 : (qmode == sweep::MODE_QBAR ? 16.0 : 8.0) / d.R;
         if (int rc = launch_primary(d.R, o.exhaustive_strict != 0, qmode, p, grid, st)) return rc;
         trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(dc, bands, s->best, s->tri_verts, s->n_tris, s->spheres,
@@ -1406,7 +1436,7 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     // a packed FADD2 per pair, plus per thread and triangle the bound FFMAs, 4 (one exact q) or 8 (mean q + |B| * spread:
     // shadow sweeps, jittered primary samples), and the interval's centre and half width (7 flops), over the R rays.
     const bool no_flops = cull || use_bvh; // the optional modes: no fixed per-pair cost
-    s->stats.flop_primary = no_flops ? 0.0 : flop_primary, s->stats.flop_shadow = no_flops ? 0.0 : 1.0 + 23.0 / trk::SHADOW_R;
+    s->stats.flop_primary = no_flops ? 0.0 : flop_primary, s->stats.flop_shadow = no_flops ? 0.0 : 1.0 + 18.0 / trk::SHADOW_R;
     // of which multiply-adds that evaluate bounds (the rest is each pair's interval test and the per-triangle interval)
     s->stats.flop_primary_edges = no_flops ? 0.0 : flop_primary_edges;
     s->stats.flop_shadow_edges = no_flops ? 0.0 : 16.0 / trk::SHADOW_R;

@@ -110,7 +110,7 @@ typedef struct tracer_render_opts {
 
     int32_t exhaustive_strict; /* debug: bypass the conservative filter, strict-test every pair */
     int32_t samples_per_pixel; /* extension (parity unpinned): 0/1 = reference; n*n stratified jitter */
-    int32_t rays_per_thread;   /* tuning: 0 = auto, else 2, 4, 8, 16, 24 or 32 rays per thread in the closest-hit sweep
+    int32_t rays_per_thread;   /* tuning: 0 = auto, else 2, 4, 8, 16, 24, 32 or 64 rays per thread in the closest-hit sweep
                                   (2, 4, 8 or 12 with jittered samples) */
     int32_t shadow_chunks;     /* tuning: 0 = auto; triangle chunks between shadow-ray compactions */
     int32_t bundle_cull;       /* OPTIONAL mode: hierarchical (bundle box -> warp box -> ray) evaluation of the same

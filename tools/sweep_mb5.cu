@@ -10,6 +10,8 @@
 // half an FFMA2 per pair (= 5 per two pairs) of the span loop (tools/sweep_mb4.cu, F_ADD: the library's form).
 // saturation has no packed form on sm_100a (ptxas rejects .sat on f32x2), so the span loop cannot pack its two adds.
 // The FMNMX3 chain kernel times the three-input min alone, to find its issue cost and pipe.
+// F_HOT is the loop on the HOT rows the tables store now (csrc/sweep.cuh, hot_row): the +1s, the clamp and the margin
+// folded into the row, per thread and triangle 4 FFMA + 2 FMNMX3 + 2 FADD (8 FFMA with a mean q), the rays holding 2*S*p.
 #include <cstdio>
 #include <cstdlib>
 #include <cuda_runtime.h>
@@ -17,7 +19,7 @@
 
 constexpr int TILE = 256, BATCH = 16;
 enum { MODE_SHAREDQ = 1, MODE_QBAR = 2 };
-enum { F_SPAN = 0, F_IV_FMA2 = 1, F_IV_ADD2 = 2 };
+enum { F_SPAN = 0, F_IV_FMA2 = 1, F_IV_ADD2 = 2, F_HOT = 3 };
 
 __device__ __forceinline__ float min3(float a, float b, float c) {
     float d;
@@ -73,8 +75,14 @@ __device__ __forceinline__ unsigned eval_interval(const float4 *__restrict__ tp,
             a1 = fmaf(fabsf(lo.x), qdelta, a1), a2 = fmaf(fabsf(lo.z), qdelta, a2);
             b1 = fmaf(fabsf(hi.x), qdelta, b1), b2 = fmaf(fabsf(hi.z), qdelta, b2);
         }
-        const float l = fmaxf(1.f - fminf(a1, a2), -P), u = fminf(fminf(b1, b2) - 1.f, P);
-        const float nc = -0.5f * (l + u), h = fmaf(0.5f, u - l, DELTA);
+        float nc, h;
+        if (FORM == F_HOT) { // (ps holds 2*S*p here)
+            const float A = min3(a1, a2, P), B = min3(b1, b2, P);
+            nc = A - B, h = A + B;
+        } else {
+            const float l = fmaxf(1.f - fminf(a1, a2), -P), u = fminf(fminf(b1, b2) - 1.f, P);
+            nc = -0.5f * (l + u), h = fmaf(0.5f, u - l, DELTA);
+        }
         float m[NCH];
 #pragma unroll
         for (int j = 0; j < NCH; ++j) m[j] = __int_as_float(0x7f800000);
@@ -100,7 +108,7 @@ __global__ void __launch_bounds__(NTH, MINBLK) k_loop(const float4 *tile_g, int 
     __syncthreads();
     float rp[R], ps[R];
 #pragma unroll
-    for (int r = 0; r < R; ++r) rp[r] = seed * (threadIdx.x + 1) * (r + 1), ps[r] = rp[r] * S;
+    for (int r = 0; r < R; ++r) rp[r] = seed * (threadIdx.x + 1) * (r + 1), ps[r] = rp[r] * (FORM == F_HOT ? 2.f * S : S);
     const float q = seed * (threadIdx.x + 7) * 3, qdelta = 1e-6f * (1 + (threadIdx.x & 3));
     int hits = 0;
     for (int rep = 0; rep < reps; ++rep) {
@@ -216,11 +224,17 @@ int main() {
     LOOP(32, MODE_SHAREDQ, F_IV_ADD2, 128, 4, 1, 1);
     LOOP(32, MODE_SHAREDQ, F_IV_ADD2, 128, 4, 1, 2);
     LOOP(32, MODE_SHAREDQ, F_IV_ADD2, 256, 2, 1, 1);
+    printf("-- shared q: hot rows (R = 32, 64) against the interval form\n");
+    LOOP(32, MODE_SHAREDQ, F_HOT, 128, 4, 1, 1);
+    LOOP(64, MODE_SHAREDQ, F_IV_ADD2, 128, 2, 1, 1);
+    LOOP(64, MODE_SHAREDQ, F_HOT, 128, 2, 1, 1);
+    LOOP(64, MODE_SHAREDQ, F_HOT, 128, 3, 1, 1);
     printf("-- any-hit (qbar + |B| qdelta): span loop vs interval form\n");
     LOOP(16, MODE_QBAR, F_SPAN, 128, 4, 4, 4);
     LOOP(16, MODE_QBAR, F_IV_FMA2, 128, 4, 1, 1);
     LOOP(16, MODE_QBAR, F_IV_ADD2, 128, 4, 1, 1);
     LOOP(16, MODE_QBAR, F_IV_ADD2, 128, 4, 1, 2);
     LOOP(32, MODE_QBAR, F_IV_ADD2, 128, 4, 1, 1);
+    LOOP(16, MODE_QBAR, F_HOT, 128, 4, 1, 1);
     return 0;
 }
