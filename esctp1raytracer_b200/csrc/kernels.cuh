@@ -333,34 +333,24 @@ struct PrimaryParams {
     int tx_log2;         // threads across a tile (the host picks the shape that wastes the fewest pixels at the frame's edges)
 };
 
-// The reference's own test for the rays (bits of mask) of one thread against triangle tri, eye rays
-// (cpp_intersect, main.cpp:176-192).  Every accepted pair is merged into the pixel's closest-hit key; the
-// lexicographic minimum of (t, index) over all accepted pairs is what the serial loop ends with (t2 >= t
-// rejects, ray_triangle.h:49, so among equal t the lowest index stays), whatever the order of evaluation.
-// k0: local pixel index of the thread's ray 0 (ray r = pixel k0 + r).  filt: rays the filter passed (validation).
-// Returns evaluations | filter misses << 16.
-template <class Mask>
-__device__ __noinline__ unsigned strict_primary(const PrimaryParams &p, int k0, Mask mask, int tri, Mask filt) {
+// The reference's own test for pixel kpx's eye ray against triangle tri (cpp_intersect, main.cpp:176-192).  An
+// accepted pair is merged into the pixel's closest-hit key; the lexicographic minimum of (t, index) over all accepted
+// pairs is what the serial loop ends with (t2 >= t rejects, ray_triangle.h:49, so among equal t the lowest index
+// stays), whatever the order of evaluation.  filt: the filter passed the pair (validation).  Returns true for a
+// filter miss: an accepted pair the filter did not pass.
+__device__ __noinline__ bool strict_primary(const PrimaryParams &p, int kpx, int tri, bool filt) {
     const float *q = p.tri_verts + 9 * (size_t)tri;
     const f3 v0 = strict::mk(__ldg(q), __ldg(q + 1), __ldg(q + 2));
     const f3 v1 = strict::mk(__ldg(q + 3), __ldg(q + 4), __ldg(q + 5));
     const f3 v2 = strict::mk(__ldg(q + 6), __ldg(q + 7), __ldg(q + 8));
     const f3 o = strict::ld(p.cam.o);
-    unsigned ret = 0;
-    while (mask) {
-        const int r = sweep::lowest_ray(mask);
-        mask &= mask - 1;
-        int w, h;
-        p.bands.map(k0 + r, w, h);
-        const f3 d = primary_dir(p.cam, p.bands, w, h);
-        float t = FLT_MAX, v = 0.f; // main.cpp:715-717
-        ++ret;
-        if (strict::intersect_triangle(o, d, v0, v1, v2, t, v)) {
-            atomicMin(&p.best[k0 + r], ((unsigned long long)__float_as_uint(t) << 32) | (unsigned)tri);
-            if (!((filt >> r) & 1u)) ret += 1u << 16;
-        }
-    }
-    return ret;
+    int w, h;
+    p.bands.map(kpx, w, h);
+    const f3 d = primary_dir(p.cam, p.bands, w, h);
+    float t = FLT_MAX, v = 0.f; // main.cpp:715-717
+    if (!strict::intersect_triangle(o, d, v0, v1, v2, t, v)) return false;
+    atomicMin(&p.best[kpx], ((unsigned long long)__float_as_uint(t) << 32) | (unsigned)tri);
+    return !filt;
 }
 
 // CTAs per SM of the closest-hit sweep: 64 rays per thread need more registers than sweep::MINB leaves
@@ -399,7 +389,10 @@ __global__ void __launch_bounds__(sweep::NT, primary_minb(R)) primary_kernel(con
         const int W = p.bands.W;
         const int tile_y = blk / p.tiles_x, tile_x = blk - tile_y * p.tiles_x;
         const int txn = 1 << p.tx_log2;
-        const int x0 = (tile_x * txn + (tid & (txn - 1))) * R, ly = tile_y * (sweep::NT >> p.tx_log2) + (tid >> p.tx_log2);
+        // first pixel (x, local row) of thread t's R rays
+        auto thread_x0 = [&](int t) { return (tile_x * txn + (t & (txn - 1))) * R; };
+        auto thread_ly = [&](int t) { return tile_y * (sweep::NT >> p.tx_log2) + (t >> p.tx_log2); };
+        const int x0 = thread_x0(tid), ly = thread_ly(tid);
         float rp[R], rq[R];
         Mask valid = 0;
 #pragma unroll
@@ -415,8 +408,7 @@ __global__ void __launch_bounds__(sweep::NT, primary_minb(R)) primary_kernel(con
 #pragma unroll
             for (int r = 1; r < R; ++r) rq[r] = q0;
         }
-        const int k0 = ly * W + x0; // valid rays are pixels k0 + r
-        Mask done = 0;
+        Mask done = 0; // valid rays are pixels ly * W + x0 + r
         float qbar = 0.f, qdelta = 0.f;
         if (MODE == sweep::MODE_QBAR) { // (rays past the frame's edge are duplicates of edge pixels: all R values count)
             float qmin = rq[0], qmax = rq[0];
@@ -428,10 +420,10 @@ __global__ void __launch_bounds__(sweep::NT, primary_minb(R)) primary_kernel(con
         }
         sweep::sweep_table<R, MODE, false, EXHAUSTIVE>(
             sm, p.table, tile_lo, tile_hi, p.n_tris, rp, rq, qbar, qdelta, valid, done, gtile, n_swept,
-            [&](Mask mask, int tri, Mask filt) {
-                const unsigned c = strict_primary(p, k0, mask, tri, filt);
-                n_strict += c & 0xffffu, n_miss += c >> 16;
-                return (Mask)0;
+            [&](int otid, int r, int tri, bool filt, const float4 *) {
+                ++n_strict;
+                n_miss += strict_primary(p, thread_ly(otid) * W + thread_x0(otid) + r, tri, filt);
+                return false;
             },
             &n_pipe_err);
         const int t_lo = min(tile_lo * sweep::TILE, p.n_tris), t_hi = min(tile_hi * sweep::TILE, p.n_tris);
@@ -717,9 +709,16 @@ __global__ void iota_kernel(int *a, int n) {
 // so the pairs actually swept track the reference's own early-exit count (main.cpp:324) and the host is not in
 // the loop at all: block offsets, slice counts, the chunk scheme and the early stop ("every ray has its occluder")
 // are decided on the device.  Round 1 ran A/B/C as 4 launches per chunk with host read-backs in between.
-constexpr int SHADOW_R = 16;    // rays per thread of a full shadow-ray block (blocks of NT * SHADOW_R consecutive list entries).
-                                // 32 measured slower (C4: 397 vs 330 ms): a thread's strict evaluations serialise over twice the
-                                // rays and the CTAs that hold them are the stragglers of every chunk barrier (23 % waiting)
+constexpr int SHADOW_R = 32;    // rays per thread of a full shadow-ray block (blocks of NT * SHADOW_R consecutive list entries).
+                                // Each thread pays 12 set-up instructions per triangle (mean q), amortised over R rays; with
+                                // the candidate pairs drained warp-wide (sweep.cuh) a thread's strict evaluations no longer
+                                // serialise over its rays, which is what made 32 slower than 16 in the per-thread form.
+                                // 64 measured slower (C4: 238 against 199 ms of shadow sweep, 2 CTAs per SM).
+// CTAs per SM of the shadow sweep: its launch bound, and the cooperative grid is sized from it.  32 rays per thread take 168
+// registers; at 4 CTAs per SM (128) the kernel spills and measured 3 % slower.
+#ifndef SHADOW_MINB
+#define SHADOW_MINB 3
+#endif
 constexpr int SL_MAXF = 1022;   // ray groups per launch (the host batches bigger lights: 146 vertices x NFACE)
 constexpr int SL_MAXCHUNK = 64;
 constexpr int CBLK = 1024;      // list entries per compaction block
@@ -749,55 +748,45 @@ struct ShadowLightParams {
                                   // ran out of sweep items / left the barrier after the sweep, or null
 };
 
-// The reference's own test for the rays (bits of mask) of one thread against triangle tri, shadow rays
-// (occlusion(), main.cpp:314-329): the first accepted face in order ends the ray and leaves t = t2 behind (the
-// multi-light carry).  Origin, direction and length stay in the pixel state and are fetched on demand: only a
-// few rays per work item ever get here.  Ray r of the thread is list entry min(e0 + r, e_last).
-// Returns newly occluded rays (bits 0-31) | evaluations << 32 | filter misses << 48.
-__device__ __noinline__ unsigned long long strict_shadow(const PixelState &px, const float *__restrict__ tri_verts, const int *__restrict__ list_in,
-                                               int n_px, int e0, int e_last, unsigned mask, int tri, unsigned filt) {
+// The reference's own test for shadow ray k (a pixel) against triangle tri (occlusion(), main.cpp:314-329): the first
+// accepted face in order ends the ray and leaves t = t2 behind (the multi-light carry).  Origin, direction and length
+// stay in the pixel state and are fetched on demand: only a few rays per work item ever get here.
+// Returns whether the ray has an occluder (it may hold a lower one from another triangle already).
+__device__ __noinline__ bool strict_shadow(const PixelState &px, const float *__restrict__ tri_verts, int n_px, int k, int tri) {
     const float *q = tri_verts + 9 * (size_t)tri;
     const f3 v0 = strict::mk(__ldg(q), __ldg(q + 1), __ldg(q + 2));
     const f3 v1 = strict::mk(__ldg(q + 3), __ldg(q + 4), __ldg(q + 5));
     const f3 v2 = strict::mk(__ldg(q + 6), __ldg(q + 7), __ldg(q + 8));
     const size_t n = (size_t)n_px;
-    unsigned long long ret = 0;
-    while (mask) {
-        const int r = __ffs(mask) - 1;
-        mask &= mask - 1;
-        const int k = list_in[min(e0 + r, e_last)];
-        const f3 o = strict::mk(px.ro[k], px.ro[n + k], px.ro[2 * n + k]);
-        const f3 d = strict::mk(px.rd[k], px.rd[n + k], px.rd[2 * n + k]);
-        float t = px.rt[k], v = 0.f; // the ray has no occluder yet, so t is its initial length (main.cpp:764)
-        ret += 1ull << 32;
-        if (strict::intersect_triangle(o, d, v0, v1, v2, t, v)) {
-            atomicMin(&px.best_occ[k], ((unsigned long long)(unsigned)tri << 32) | __float_as_uint(t));
-            ret |= 1ull << r;
-            if (!((filt >> r) & 1u)) ret += 1ull << 48;
-        }
-    }
-    return ret;
+    const f3 o = strict::mk(px.ro[k], px.ro[n + k], px.ro[2 * n + k]);
+    const f3 d = strict::mk(px.rd[k], px.rd[n + k], px.rd[2 * n + k]);
+    float t = px.rt[k], v = 0.f; // the ray has no occluder yet, so t is its initial length (main.cpp:764)
+    if (!strict::intersect_triangle(o, d, v0, v1, v2, t, v)) return false;
+    atomicMin(&px.best_occ[k], ((unsigned long long)(unsigned)tri << 32) | __float_as_uint(t));
+    return true;
 }
 
 // one (ray block, triangle slice) work item with RR rays per thread.  The list is ordered by q inside each group
 // (and compaction keeps it so); a thread takes RR CONSECUTIVE rays, whose q differ by ~1e-6, and evaluates them
-// with one q-term per edge row (sweep::MODE_QBAR).
+// with one q-term per edge row (sweep::MODE_QBAR).  Only 2*S*p stays in registers: the candidate path reads a
+// queued ray's own (p, q) back through the list.
 template <int RR, bool EXHAUSTIVE>
 __device__ __forceinline__ void shadow_item(sweep::SmemT<2> &sm, const ShadowLightParams &p, const int *__restrict__ list_in, int base,
                                             int seg_end, int lo, int hi, const float4 *__restrict__ tab, unsigned &gtile,
                                             unsigned &n_strict, unsigned &n_miss, unsigned long long &tests, unsigned &n_pipe_err) {
+    using Mask = sweep::RayMask<RR>;
     const int tid = threadIdx.x, n = p.n_px;
     float rp[RR], rq[RR];
-    unsigned valid = 0, done = 0;
+    Mask valid = 0, done = 0;
     const int e0 = base + tid * RR;
 #pragma unroll
     for (int r = 0; r < RR; ++r) {
-        if (e0 + r < seg_end) valid |= 1u << r;
+        if (e0 + r < seg_end) valid |= (Mask)1 << r;
         const int k = list_in[min(e0 + r, seg_end - 1)];
         rp[r] = p.px.re[k], rq[r] = p.px.re[n + k];
         // an earlier slice may already have published an occluder below this slice: nothing to do
         const unsigned long long seen = p.px.best_occ[k];
-        if (seen != KEY_NONE && (int)(unsigned)(seen >> 32) < lo * sweep::TILE) done |= 1u << r;
+        if (seen != KEY_NONE && (int)(unsigned)(seen >> 32) < lo * sweep::TILE) done |= (Mask)1 << r;
     }
     // rays past the end of the list are duplicates of the last one, so all RR values count
     float qmin = rq[0], qmax = rq[0];
@@ -808,13 +797,20 @@ __device__ __forceinline__ void shadow_item(sweep::SmemT<2> &sm, const ShadowLig
     const float qdelta = fmaxf(qmax - qbar, qbar - qmin) * 1.0001f + 2.4e-7f * (fabsf(qbar) + 1.f);
     unsigned swept = 0;
     sweep::sweep_table<RR, sweep::MODE_QBAR, true, EXHAUSTIVE>(
-        sm, tab, lo, hi, p.n_tris, rp, rq, qbar, qdelta, valid, done, gtile, swept, [&](unsigned mask, int tri, unsigned filt) {
-            const unsigned long long c = strict_shadow(p.px, p.tri_verts, list_in, n, e0, seg_end - 1, mask, tri, filt);
-            n_strict += (unsigned)(c >> 32) & 0xffffu, n_miss += (unsigned)(c >> 48);
-            return (unsigned)c;
+        sm, tab, lo, hi, p.n_tris, rp, rq, qbar, qdelta, valid, done, gtile, swept,
+        [&](int otid, int r, int tri, bool filt, const float4 *row) {
+            const int k = list_in[min(base + otid * RR + r, seg_end - 1)];
+            // each ray's own q: the widening of the shared-q bounds, ~10 % of a pixel over 16 consecutive rays of a
+            // q-sorted list, would cost ~5 % more strict evaluations
+            filt = filt && sweep::hot_row_pass(row, p.px.re[k], p.px.re[n + k]);
+            if (!EXHAUSTIVE && !filt) return false;
+            ++n_strict;
+            const bool acc = strict_shadow(p.px, p.tri_verts, n, k, tri);
+            n_miss += acc && !filt;
+            return acc;
         },
         &n_pipe_err);
-    tests += (unsigned long long)swept * sweep::TILE * __popc(valid);
+    tests += (unsigned long long)swept * sweep::TILE * __popcll((unsigned long long)valid);
 }
 
 // exclusive prefix over the F groups of ceil(cnt[j] / unit), by the whole CTA into shared memory; returns the total
@@ -880,7 +876,7 @@ __device__ __forceinline__ void grid_barrier(unsigned *bar, unsigned &epoch) {
 }
 
 template <bool EXHAUSTIVE>
-__global__ void __launch_bounds__(sweep::NT, sweep::MINB) shadow_light_kernel(const __grid_constant__ ShadowLightParams p, unsigned *bar) {
+__global__ void __launch_bounds__(sweep::NT, SHADOW_MINB) shadow_light_kernel(const __grid_constant__ ShadowLightParams p, unsigned *bar) {
     static_assert(CBLK % sweep::NT == 0, "compaction block must be a multiple of the CTA size");
     constexpr int R = SHADOW_R, CPT = CBLK / sweep::NT; // rays per thread of a full ray block; list entries per thread of a compaction block
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -948,8 +944,11 @@ __global__ void __launch_bounds__(sweep::NT, sweep::MINB) shadow_light_kernel(co
                 // The last block of a ray group is rarely full.  A block with at most NT*RR rays is swept with RR rays per
                 // thread instead of dragging empty lanes through every triangle (late chunks have few rays in many groups).
                 const int cnt = seg_end - base;
-                if (cnt > 8 * sweep::NT)
+                static_assert(SHADOW_R == 32, "the part-filled block sizes below follow SHADOW_R");
+                if (cnt > 16 * sweep::NT)
                     shadow_item<SHADOW_R, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err);
+                else if (cnt > 8 * sweep::NT)
+                    shadow_item<16, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err);
                 else if (cnt > 4 * sweep::NT)
                     shadow_item<8, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err);
                 else if (cnt > 2 * sweep::NT)

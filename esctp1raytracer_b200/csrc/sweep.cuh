@@ -61,13 +61,15 @@
 //    (cp.async.bulk + mbarrier complete_tx, UBLKCP in SASS), STAGES deep;
 //  * every lane of every warp reads the SAME row at the same time, so the two LDS.128 per
 //    triangle are pure broadcasts, amortised over R rays per thread held in registers
-//    (R = 64 closest hit, 16 any-hit);
+//    (R = 64 closest hit, 32 any-hit);
 //  * each pair is ONE interval test |2*S*p + nc2| <= h2 (hot rows, below): per two pairs one packed
 //    FADD2 and one FMNMX3 running minimum, no saturation, no integer op.  History on this part
 //    (cycles per pair, closest hit): round 1 sign bits through LOP3 on the half-rate ALU pipe 7.9,
 //    three saturating rows with a product accumulate 6.8, span form with two saturating adds 4.0;
 //  * the inner loop has NO per-triangle branch: a batch of 16 triangles yields one verdict bit per
-//    triangle; candidates (a few per ray per sweep) are then re-evaluated one by one;
+//    triangle; candidates (a few per ray per sweep) then go through a warp-wide pass: the flagged triangles'
+//    (owner lane, ray, triangle) pairs are queued in shared memory and drained one pair per lane, so the
+//    strict evaluations of a thread's R rays no longer serialise on that thread;
 //  * NO block-wide barrier per tile in either sweep: every warp counts itself out of a
 //    tile stage (shared-memory atomicAdd) and the last one issues the refill, so warps
 //    run up to STAGES-1 tiles apart.  An any-hit warp whose rays all have their occluder
@@ -150,13 +152,16 @@ __device__ __forceinline__ float4 lds128_opaque(const float4 *p) {
     return v;
 }
 
-// ---- shared memory of one sweep CTA: the table-tile pipeline and nothing else -------------------
+// ---- shared memory of one sweep CTA: the table-tile pipeline and each warp's candidate queue -------------------
+constexpr int QCAP = 32; // candidate pairs per warp queue: one per lane and drain
 template <int ROWS> // float4 per triangle of the table the kernel sweeps: 2 (span rows) or 3 (three-row table)
 struct __align__(128) SmemT {
     float4 tile[STAGES][TILE * ROWS];
     uint64_t full_bar[STAGES];
     int consumed[STAGES]; // warps that have finished the tile in this stage
     int blk, seg, slice;  // the work item the CTA is on
+    unsigned queue[NT / 32][QCAP];             // candidate pairs: ray | owner lane << 6 | triangle in tile << 11 | filt << 19
+    unsigned long long qdone[NT / 32][32];     // any-hit: rays of each owner lane accepted during a drain (zero between drains)
 };
 using Smem = SmemT<3>;
 
@@ -176,6 +181,7 @@ __device__ __forceinline__ void smem_init(SmemT<ROWS> &sm) {
         for (int s = 0; s < STAGES; ++s) mbar_init(&sm.full_bar[s], 1), sm.consumed[s] = 0;
         fence_barrier_init();
     }
+    if (threadIdx.x < NT) sm.qdone[threadIdx.x >> 5][threadIdx.x & 31] = 0;
     __syncthreads();
 }
 
@@ -419,6 +425,12 @@ __host__ __device__ __forceinline__ void hot_terms_qbar(const float4 lo, const f
 }
 // the hot test of one pair (ps2 = p * 2 * SPAN_S)
 __host__ __device__ __forceinline__ bool hot_pass(float nc2, float h2, float ps2) { return fabsf(ps2 + nc2) <= h2; }
+// the hot test of one ray (p, its own q) on a staged hot row (candidate path of the any-hit sweeps)
+__device__ __forceinline__ bool hot_row_pass(const float4 *row, float p, float q) {
+    float nc2, h2;
+    hot_terms(lds128_opaque(row), lds128_opaque(row + 1), q, nc2, h2);
+    return hot_pass(nc2, h2, p * (2.f * SPAN_S));
+}
 
 // ray masks of the sweeps: a bit per ray of a thread
 template <int R>
@@ -477,12 +489,13 @@ __device__ __forceinline__ unsigned eval_batch_lop3(const float4 *__restrict__ t
 }
 
 // ---- the sweep over tiles [tile_lo, tile_hi) of one origin table, for the R rays of each thread ---
-// rp/rq: the rays' parameters in the table's direction parametrisation (rq is read by MODE_OWNQ and by the candidate path
-//        of the any-hit sweeps; MODE_SHAREDQ takes the common q from rq[0], MODE_QBAR from qbar/qdelta)
+// rp/rq: the rays' parameters in the table's direction parametrisation (rq is read by MODE_OWNQ only; MODE_SHAREDQ takes
+//        the common q from rq[0], MODE_QBAR from qbar/qdelta; span forms keep only 2*S*p in registers)
 // valid: bit r set = ray r exists; done: bit r set = ray r needs no more tests (RayMask<R>: 64 bits for R > 32)
 // gtile: running tile counter of this CTA (mbarrier phase bookkeeping across work items)
-// strict(mask, tri, filt) -> newly done rays: the reference's own test on the surviving pairs (kernels.cuh);
-//        mask = rays to test, filt = rays the filter passed (differs from mask only in EXHAUSTIVE validation mode)
+// strict(otid, r, tri, filt, row) -> accepted: the reference's own test of ray r of thread otid (a thread of the calling
+//        lane's warp) against triangle tri (kernels.cuh), run by whichever lane drains the pair; filt = the filter passed
+//        the pair (false only in EXHAUSTIVE validation mode), row = the triangle's staged row (still resident)
 template <int R, int MODE, bool ANYHIT, bool EXHAUSTIVE, class Strict>
 __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const float4 *__restrict__ table, int tile_lo, int tile_hi, int n_tris,
                                             const float (&rp)[R], const float (&rq)[R], float qbar, float qdelta, RayMask<R> valid,
@@ -508,6 +521,27 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
 #pragma unroll
     for (int r = 0; r < R; ++r) ps2[r] = rp[r] * (2.f * SPAN_S);
     const float qhot = MODE == MODE_QBAR ? qbar : rq[0], qdh = hot_qdelta(qdelta);
+    const unsigned lane = tid & 31;
+    unsigned *queue = sm.queue[tid >> 5];
+#ifndef SWEEP_NO_STRICT
+    // the first n queued pairs, one per lane: the reference's own test, then (any-hit) the accepted rays into done
+    auto drain = [&](const float4 *__restrict__ tp, int it, int n) {
+        __syncwarp();
+        if ((int)lane < n) {
+            const unsigned e = queue[lane];
+            const int r = e & 63, owner = (e >> 6) & 31, k = (e >> 11) & 255;
+            const int otid = (tid & ~31) | owner;
+            if (strict(otid, r, (tile_lo + it) * TILE + k, (bool)(e >> 19), tp + ROWS * k) && ANYHIT)
+                atomicOr(&sm.qdone[tid >> 5][owner], 1ull << r);
+        }
+        __syncwarp();
+        if (ANYHIT) {
+            done |= (Mask)sm.qdone[tid >> 5][lane];
+            sm.qdone[tid >> 5][lane] = 0;
+        }
+        __syncwarp();
+    };
+#endif
     for (int it = 0; it < n_tiles; ++it) {
         const unsigned g = gtile + it;
         const int s = g % STAGES;
@@ -546,52 +580,62 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
                 // accepted pair whose triangle (group) it would have skipped counts as a filter miss too
                 const unsigned cand_hot = cand;
                 if (EXHAUSTIVE) cand = NB / UNIT == 32 ? 0xffffffffu : (1u << (NB / UNIT)) - 1u;
-                while (cand) {
-                    // rare: a triangle (group of UNIT triangles) may hold a candidate.  Rebuild the per-ray candidate mask
-                    // of each of its triangles, then the reference's own arithmetic.  The rows are re-read
-                    // through opaque loads so that the compiler cannot merge this with the hot evaluation.
-                    const int gq = __ffs(cand) - 1; // ascending triangle order
-                    cand &= cand - 1;
+                // rare: some lane flagged a triangle (group of UNIT triangles).  The warp rebuilds, lane by lane, the per-ray
+                // candidate mask of each flagged triangle, queues the (owner lane, ray, triangle) pairs and drains the queue one
+                // pair per lane, so a thread's candidates no longer serialise while the rest of the warp idles.
+                unsigned wcand = __reduce_or_sync(0xffffffffu, cand);
+                if (wcand) {
+                    int fill = 0;
+                    while (wcand) {
+                        const int gq = __ffs(wcand) - 1; // ascending triangle order
+                        wcand &= wcand - 1;
+                        const bool mine = (cand >> gq) & 1u;
 #pragma unroll 1
-                    for (int kk = 0; kk < UNIT; ++kk) {
-                        const int k = b0 + gq * UNIT + kk;
-                        const int tri = (tile_lo + it) * TILE + k;
-                        Mask filt = 0;
-                        if (SPAN) {
-                            // the hot test on the stored row, ray by ray: it passes every pair span_pass passes (hot_row)
-                            const float4 lo = lds128_opaque(&tp[2 * k]), hi = lds128_opaque(&tp[2 * k + 1]);
-                            if (MODE == MODE_QBAR && ANYHIT) {
-                                // shadow rays: each ray's own q (the widening of the shared-q bounds, ~10 % of a pixel over
-                                // 16 consecutive rays of a q-sorted list, would cost ~5 % more strict evaluations)
-#pragma unroll
-                                for (int r = 0; r < R; ++r) {
+                        for (int kk = 0; kk < UNIT; ++kk) {
+                            const int k = b0 + gq * UNIT + kk;
+                            if ((tile_lo + it) * TILE + k >= n_tris) break; // padding (warp-uniform)
+                            Mask filt = 0;
+                            if (mine) {
+                                // The rows are re-read through opaque loads so that the compiler cannot merge this with the
+                                // hot evaluation.
+                                if (SPAN) {
+                                    // the hot loop's own test, ray by ray: it passes every pair span_pass passes (hot_row); exact
+                                    // with a common q.  Shadow rays are tested again with their own q when the queue drains.
+                                    const float4 lo = lds128_opaque(&tp[2 * k]), hi = lds128_opaque(&tp[2 * k + 1]);
                                     float nc2, h2;
-                                    hot_terms(lo, hi, rq[r], nc2, h2);
-                                    filt |= (Mask)hot_pass(nc2, h2, ps2[r]) << r;
+                                    if (MODE == MODE_QBAR) hot_terms_qbar(lo, hi, qhot, qdh, nc2, h2);
+                                    else hot_terms(lo, hi, qhot, nc2, h2);
+#pragma unroll
+                                    for (int r = 0; r < R; ++r) filt |= (Mask)hot_pass(nc2, h2, ps2[r]) << r;
+                                } else {
+                                    const float4 rb = lds128_opaque(&tp[3 * k]), rc = lds128_opaque(&tp[3 * k + 1]), rd = lds128_opaque(&tp[3 * k + 2]);
+#pragma unroll
+                                    for (int r = 0; r < R; ++r) filt |= (Mask)edge_pass(rb, rc, rd, rp[r], rq[r]) << r;
                                 }
-                            } else {
-                                // closest hit: the hot loop's own test, ray by ray — exact with a common q; with jittered samples
-                                // (mean q + |B| * qdelta, 1/8 pixel) it saves keeping 32 q values in registers during the sweep
-                                // for ~2 % more strict evaluations
-                                float nc2, h2;
-                                if (MODE == MODE_QBAR) hot_terms_qbar(lo, hi, qhot, qdh, nc2, h2);
-                                else hot_terms(lo, hi, qhot, nc2, h2);
-#pragma unroll
-                                for (int r = 0; r < R; ++r) filt |= (Mask)hot_pass(nc2, h2, ps2[r]) << r;
+                                if (EXHAUSTIVE && !((cand_hot >> gq) & 1u)) filt = 0;
                             }
-                        } else {
-                            const float4 rb = lds128_opaque(&tp[3 * k]), rc = lds128_opaque(&tp[3 * k + 1]), rd = lds128_opaque(&tp[3 * k + 2]);
+                            const Mask live = valid & ~done;
+                            Mask pend = mine ? (EXHAUSTIVE ? live : filt & live) : (Mask)0;
+                            while (__any_sync(0xffffffffu, pend != 0)) {
+                                // this lane's pairs go to queue slots [fill + before, ...): as many as fit, the rest after a drain
+                                const int n = __popcll((unsigned long long)pend);
+                                int incl = n;
 #pragma unroll
-                            for (int r = 0; r < R; ++r) filt |= (Mask)edge_pass(rb, rc, rd, rp[r], rq[r]) << r;
-                        }
-                        if (EXHAUSTIVE && !((cand_hot >> gq) & 1u)) filt = 0;
-                        const Mask live = valid & ~done;
-                        const Mask mask = EXHAUSTIVE ? live : (filt & live);
-                        if (mask && tri < n_tris) {
-                            const Mask nw = strict(mask, tri, filt);
-                            if (ANYHIT) done |= nw;
+                                for (int o = 1; o < 32; o <<= 1) {
+                                    const int y = __shfl_up_sync(0xffffffffu, incl, o);
+                                    if (lane >= o) incl += y;
+                                }
+                                for (int slot = fill + incl - n; pend && slot < QCAP; ++slot) {
+                                    const int r = lowest_ray(pend);
+                                    pend &= pend - 1;
+                                    queue[slot] = (unsigned)r | lane << 6 | (unsigned)k << 11 | (unsigned)((filt >> r) & 1u) << 19;
+                                }
+                                fill = min(QCAP, fill + __shfl_sync(0xffffffffu, incl, 31));
+                                if (fill == QCAP) drain(tp, it, fill), fill = 0;
+                            }
                         }
                     }
+                    if (fill) drain(tp, it, fill);
                 }
 #endif
             }

@@ -410,7 +410,7 @@ int launch_shadow_light_t(Ctx &g, const trk::ShadowLightParams &p, unsigned *bar
         CK_CUDA(cudaFuncSetAttribute(trk::shadow_light_kernel<EX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         CK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, trk::shadow_light_kernel<EX>, sweep::NT, smem));
         if (ctas_per_sm < 1) return fail(TRACER_ERR_CUDA, "shadow_light_kernel does not fit on an SM");
-        ctas_per_sm = std::min(ctas_per_sm, sweep::MINB);
+        ctas_per_sm = std::min(ctas_per_sm, SHADOW_MINB);
     }
     void *args[] = {(void *)&p, (void *)&bar};
     CK_CUDA(cudaLaunchCooperativeKernel((const void *)trk::shadow_light_kernel<EX>, dim3((unsigned)(ctas_per_sm * g.n_sms)), dim3(sweep::NT), args, smem, st));
@@ -1280,13 +1280,14 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
         }
         // Triangle chunks: after each one the still-unoccluded rays are compacted (early exit, main.cpp:324).  Equal chunks
         // keep the pairs swept past a ray's occluder lowest (x1.056 at 64 chunks; x1.11 at 32) and win when a light has many
-        // shadow rays; with few rays (small frames, one band share of a multi-GPU frame) a chunk's fixed cost (three grid
-        // barriers, the compaction passes, the sweep's tail: ~0.1 ms) weighs more, and 20 chunks that start fine (1/64 of the
-        // triangles: most occluded rays find their occluder early) and coarsen win (x1.10).  The kernel picks the scheme from
+        // shadow rays.  32 of them: at 32 rays per thread an item is twice as long and so is each chunk's tail (C4: 189 ms
+        // of shadow sweep at 32 chunks, 192 at 48, 199 at 64; profiles/r05_d).  With few rays (small frames, one band share of
+        // a multi-GPU frame) a chunk's fixed cost (three grid barriers, the compaction passes, the sweep's tail: ~0.1 ms)
+        // weighs more, and 20 chunks that start fine (1/64 of the triangles: most occluded rays find their occluder early) and coarsen win (x1.10).  The kernel picks the scheme from
         // the live-ray count it finds.  opts.shadow_chunks asks for that many equal chunks.
         trk::ShadowLightParams sp{};
         {
-            const int nc = std::min({n_tiles, trk::SL_MAXCHUNK, o.shadow_chunks > 0 ? o.shadow_chunks : std::max(1, std::min(64, n_tiles / 8))});
+            const int nc = std::min({n_tiles, trk::SL_MAXCHUNK, o.shadow_chunks > 0 ? o.shadow_chunks : std::max(1, std::min(32, n_tiles / 8))});
             sp.n_chunks[1] = nc;
             for (int c = 0; c <= nc; ++c) sp.bounds[1][c] = (int)((int64_t)n_tiles * c / nc);
             if (o.shadow_chunks > 0 || n_tiles < 64) {

@@ -54,7 +54,7 @@ __global__ void __launch_bounds__(NTH, MINBLK) k_prod(const float4 *table, int n
         for (int r = 0; r < R; ++r) rp[r] = seed * (tid + 1) * (r + 1 + blk), rq[r] = seed * (tid + 7) * 3;
         unsigned done = 0;
         sweep_table<R, MODE, ANYHIT, false>(sm, table, 0, n_tiles, n_tiles * TILE, rp, rq, rq[0], 1e-6f, (1u << R) - 1u, done, gtile, n_swept,
-                                            [&](unsigned, int, unsigned) { return 0u; });
+                                            [&](int, int, int, bool, const float4 *) { return false; });
         acc += done;
         __syncthreads();
     }
