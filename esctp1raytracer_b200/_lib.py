@@ -44,6 +44,10 @@ class CameraC(C.Structure):
                 ("vertical", C.c_float * 3)]
 
 
+# int32_t (*row_hits_exchange)(void *user, int32_t height, int32_t *row_hits)
+ROW_HITS_EXCHANGE = C.CFUNCTYPE(C.c_int32, C.c_void_p, C.c_int32, C.POINTER(C.c_int32))
+
+
 class RenderOpts(C.Structure):
     _fields_ = [
         ("struct_size", C.c_uint32), ("rng_mode", C.c_int32), ("seed", C.c_uint32), ("faceid", C.POINTER(C.c_int32)),
@@ -53,6 +57,7 @@ class RenderOpts(C.Structure):
         ("rays_per_thread", C.c_int32), ("shadow_chunks", C.c_int32), ("bundle_cull", C.c_int32),
         ("out_tri", C.POINTER(C.c_int32)), ("out_t", C.POINTER(C.c_float)), ("out_v", C.POINTER(C.c_float)),
         ("out_occ_tri", C.POINTER(C.c_int32)), ("out_rgb", C.POINTER(C.c_float)), ("accel", C.c_int32),
+        ("row_hits_exchange", ROW_HITS_EXCHANGE), ("row_hits_user", C.c_void_p),
     ]
 
 

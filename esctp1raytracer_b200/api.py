@@ -329,12 +329,16 @@ class Renderer:
 
     def trace(self, scene, camera: Camera, width: int, height: int, *, rng_mode=RNG_HASH, seed=1, faceid=None,
               bands=None, exhaustive_strict=False, debug=False, out_device_ptr=None, stream=None,
-              rays_per_thread=0, shadow_chunks=0, samples_per_pixel=0, bundle_cull=False, out=None, bvh=False) -> Frame:
+              rays_per_thread=0, shadow_chunks=0, samples_per_pixel=0, bundle_cull=False, out=None, bvh=False,
+              row_hits_exchange=None) -> Frame:
         """Render; ``scene`` is a Scene (one-shot: upload + render, the drop-in call) or a
         ResidentScene.  ``bvh``: the optional BVH mode (opts.accel = 1): the resident scene builds its tree on the
         first such render and keeps it; same bytes as the default mode.  ``bands`` = (band_rows, band_index, band_count).  With
         ``out_device_ptr`` the packed rows are left in HBM at that address; ``out`` is an optional
-        caller-owned uint8 [rows, W, 3] host array (e.g. pinned) to receive them."""
+        caller-owned uint8 [rows, W, 3] host array (e.g. pinned) to receive them.  ``row_hits_exchange``: with
+        ``RNG_MT19937`` and bands, a callable ``(row_hits: np.ndarray[int32, H]) -> None`` that completes this call's
+        per-row hit counts into the frame's, in place (opts.row_hits_exchange; an all-reduce sum over the calls that render
+        the frame does it).  An exception inside it fails the render with TracerError."""
         sc = scene.scene if isinstance(scene, ResidentScene) else scene
         rows = height if bands is None else band_row_count(height, *bands)
         n_px = rows * width
@@ -352,6 +356,8 @@ class Renderer:
             dst = out.ctypes.data_as(C.c_void_p)
         if stream is not None:
             o.cuda_stream = C.c_void_p(stream)
+        if row_hits_exchange is not None:
+            o.row_hits_exchange = keep_cb = _row_hits_hook(row_hits_exchange)  # noqa: F841 (alive for the call)
         stats = {}
         if isinstance(scene, ResidentScene):
             _lib.check(self.lib.tracer_cuda_render_scene(scene.handle, C.byref(camera.c), width, height, C.byref(o), dst))
@@ -372,6 +378,23 @@ class Renderer:
         tf, ms = C.c_double(), C.c_double()
         _lib.check(self.lib.tracer_cuda_fp32_peak(variant, iters, C.byref(tf), C.byref(ms)))
         return tf.value, ms.value
+
+
+def _row_hits_hook(fn):
+    """opts.row_hits_exchange over a Python callable.  ctypes would print an exception raised in a callback and return 0,
+    which the library would read as success: it returns 1 instead."""
+
+    def hook(_user, height, rows):
+        try:
+            fn(np.ctypeslib.as_array(rows, (height,)))
+            return 0
+        except BaseException:  # noqa: BLE001 — any failure must reach the library as a non-zero return
+            import traceback
+
+            traceback.print_exc()
+            return 1
+
+    return _lib.ROW_HITS_EXCHANGE(hook)
 
 
 def write_ppm(path: str, rgb8: np.ndarray, binary: bool = False) -> None:

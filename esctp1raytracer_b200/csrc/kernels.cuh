@@ -1540,12 +1540,6 @@ __global__ void accumulate_kernel(const float *__restrict__ accum, float *__rest
     total[i] = v;
 }
 
-// hit mask in local pixel order (= the reference's scan order) for the mt19937 replay
-__global__ void hitmask_kernel(const int *__restrict__ hit_tri, int n_px, uint8_t *__restrict__ mask) {
-    const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k < n_px) mask[k] = hit_tri[k] >= 0;
-}
-
 // rank 0 after the gather: rank r's buffer holds its bands back to back
 __global__ void assemble_bands_kernel(const uint8_t *__restrict__ gathered, uint8_t *__restrict__ frame, int W, int H,
                                       int band_rows, int band_count, int rows_pad) {

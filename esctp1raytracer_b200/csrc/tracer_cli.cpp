@@ -5,7 +5,8 @@
 // for symmetry with `--ispc`.  The CPU/ISPC modes (--thread, --ispc) do not exist in this build.  `--bvh` does what the
 // reference's --bvh intends (main.cpp:566-567 flatten + sort, then a BVH render): the flatten+sort pass of --sorted, then
 // the optional BVH mode (opts.accel = 1), so its output is the bytes of --sorted.
-// `--gpus N` renders the frame on N GPUs of the box (interleaved 8-row bands, NCCL gather: tracer_cuda_init_multi);
+// `--gpus N` renders the frame on N GPUs of the box (interleaved 8-row bands, NCCL gather: tracer_cuda_init_multi), with the
+// same generator and, for a given --seed, the same bytes as one GPU;
 // `--spp S` = S stratified jittered samples per pixel (extension); `--sorted` runs the reference's optional
 // flatten+sort pass (src/simplify/flatten.cpp:50-82) before rendering.
 #include <chrono>
@@ -81,10 +82,6 @@ int main(int argc, char *argv[]) {
         const float vup[3] = {0, 1, 0};
         tracer_camera_lookat(eye, look, vup, 60.f, float(W) / H, &cam); // main.cpp:548-551
         if (gpus > 1) {
-            if (rng == TRACER_RNG_MT19937) {
-                if (have_seed) throw std::runtime_error("--gpus > 1 needs --rng hash: the mt19937 stream is sequential over the whole frame (main.cpp:587-589)");
-                rng = TRACER_RNG_HASH; // unseeded runs are random anyway (main.cpp:587-588)
-            }
             if (tracer_cuda_init_multi(gpus)) throw std::runtime_error(tracer_cuda_last_error());
         } else if (tracer_cuda_init(device)) throw std::runtime_error(tracer_cuda_last_error());
         tracer_render_opts o{};

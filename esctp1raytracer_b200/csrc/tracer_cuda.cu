@@ -4,6 +4,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
+#include <condition_variable>
 #include <cstring>
 #include <map>
 #include <mutex>
@@ -18,6 +19,7 @@
 #include <thread>
 
 #include "bvh.cuh" // (includes kernels.cuh)
+#include "mt19937.cuh"
 
 // Internal (tests only, no GPU needed): the row construction of build_origin_table and the sweeps' per-ray tests,
 // compiled for the host from the same source.  rows9 = three exact rows (A, B, C); row8 = lo.xyzw, hi.xyzw.
@@ -120,9 +122,6 @@ __global__ void powf_pairs_kernel(const float *x, const float *y, uint32_t n, fl
 }
 extern "C" int tracer__device_powf(uint32_t lo_bits, uint32_t hi_bits, uint32_t stride, float y, float *host_out);
 extern "C" int tracer__device_powf_pairs(int64_t n, const float *x, const float *y, float *host_out);
-
-extern "C" int tracer__mt19937_scan(uint32_t seed, int32_t n_lights, const int32_t *faces_per_light, int64_t n_px,
-                                    const uint8_t *hit_scan, int32_t *faceid_scan);
 
 namespace {
 
@@ -231,6 +230,28 @@ void dev_free(T *&p) {
     t_pool->release((void *)p);
     p = nullptr;
 }
+template <typename T>
+int dev_grow(T *&p, size_t &cap, size_t n) {
+    if (n <= cap) return 0;
+    dev_free(p);
+    cap = 0;
+    if (int rc = dev_alloc(&p, n)) return rc;
+    cap = n;
+    return 0;
+}
+
+// Buffers of the device replay of the seeded draws (mt19937.cuh), grown as frames need them
+struct MtWork {
+    int *rank = nullptr, *row_hits = nullptr, *maps = nullptr, *start = nullptr, *fid_ord = nullptr;
+    uint32_t *words = nullptr, *lights = nullptr;
+    int64_t *base = nullptr, *ord = nullptr;
+    size_t rank_cap = 0, rows_cap = 0, maps_cap = 0, start_cap = 0, fid_cap = 0, words_cap = 0, lights_cap = 0, base_cap = 0, ord_cap = 0;
+    void release() {
+        dev_free(rank), dev_free(row_hits), dev_free(maps), dev_free(start), dev_free(fid_ord), dev_free(words), dev_free(lights);
+        dev_free(base), dev_free(ord);
+        rank_cap = rows_cap = maps_cap = start_cap = fid_cap = words_cap = lights_cap = base_cap = ord_cap = 0;
+    }
+};
 
 }  // namespace
 
@@ -263,7 +284,8 @@ struct tracer_scene_dev {
     unsigned long long *best = nullptr, *best_occ = nullptr;
     float *hit_t = nullptr, *hit_v = nullptr, *carry = nullptr, *nrm = nullptr, *accum = nullptr, *ro = nullptr,
           *rd = nullptr, *re = nullptr, *rt = nullptr;
-    uint8_t *rgb8 = nullptr, *mask = nullptr;
+    uint8_t *rgb8 = nullptr;
+    MtWork mt;
     float *accum_total = nullptr;
     // bundle-cull mode: candidate (ray<<32|triangle) buffers, their count, radix-sort scratch
     unsigned long long *cand_a = nullptr, *cand_b = nullptr, *cand_count = nullptr, *rkey = nullptr, *rkey_sorted = nullptr;
@@ -300,7 +322,7 @@ int ensure_workspace(tracer_scene_dev *s, int n_px, bool want_dbg_occ) {
     if (n_px > s->ws_npx) {
         dev_free(s->hit_tri), dev_free(s->rj), dev_free(s->best), dev_free(s->best_occ), dev_free(s->list), dev_free(s->list_b);
         dev_free(s->faceid), dev_free(s->hit_t), dev_free(s->hit_v), dev_free(s->carry), dev_free(s->nrm), dev_free(s->accum);
-        dev_free(s->ro), dev_free(s->rd), dev_free(s->re), dev_free(s->rt), dev_free(s->rgb8), dev_free(s->mask);
+        dev_free(s->ro), dev_free(s->rd), dev_free(s->re), dev_free(s->rt), dev_free(s->rgb8);
         dev_free(s->dbg_occ), dev_free(s->accum_total);
         s->ws_npx = 0;
         const size_t n = (size_t)n_px;
@@ -312,7 +334,7 @@ int ensure_workspace(tracer_scene_dev *s, int n_px, bool want_dbg_occ) {
         rc |= dev_alloc(&s->hit_t, n) | dev_alloc(&s->hit_v, n) | dev_alloc(&s->carry, n);
         rc |= dev_alloc(&s->nrm, 3 * n) | dev_alloc(&s->accum, 3 * n + 16) | dev_alloc(&s->ro, 3 * n);
         rc |= dev_alloc(&s->rd, 3 * n) | dev_alloc(&s->re, 2 * n) | dev_alloc(&s->rt, n);
-        rc |= dev_alloc(&s->rgb8, 3 * n + 64) | dev_alloc(&s->mask, n);
+        rc |= dev_alloc(&s->rgb8, 3 * n + 64);
         if (rc) return TRACER_ERR_NOMEM;
         s->ws_npx = n_px;
     }
@@ -692,7 +714,7 @@ void tracer_cuda_scene_destroy(tracer_scene_dev *s) {
     dev_free(s->hit_tri), dev_free(s->rj), dev_free(s->best), dev_free(s->best_occ), dev_free(s->list), dev_free(s->list_b);
     dev_free(s->faceid), dev_free(s->dbg_occ), dev_free(s->cnt_b), dev_free(s->accum_total);
     dev_free(s->hit_t), dev_free(s->hit_v), dev_free(s->carry), dev_free(s->nrm), dev_free(s->accum);
-    dev_free(s->ro), dev_free(s->rd), dev_free(s->re), dev_free(s->rt), dev_free(s->rgb8), dev_free(s->mask);
+    dev_free(s->ro), dev_free(s->rd), dev_free(s->re), dev_free(s->rt), dev_free(s->rgb8);
     dev_free(s->seg_count), dev_free(s->seg_off), dev_free(s->blk_off), dev_free(s->cursor), dev_free(s->work);
     dev_free(s->n_slices);
     dev_free(s->cand_a), dev_free(s->cand_b), dev_free(s->cand_count), dev_free(s->rkey), dev_free(s->rkey_sorted), dev_free(s->iota);
@@ -700,6 +722,7 @@ void tracer_cuda_scene_destroy(tracer_scene_dev *s) {
     t_pool->release(s->sort_tmp), t_pool->release(s->pair_tmp);
     dev_free(s->counters);
     dev_free(s->bvh_nodes), dev_free(s->bvh_keys);
+    s->mt.release();
     for (auto &e : s->ev)
         if (e) cudaEventDestroy(e);
     for (auto &e : s->ev_shadow) cudaEventDestroy(e);
@@ -861,10 +884,97 @@ int scene_create_on(Ctx &g, const tracer_scene_flat *sc, tracer_scene_dev **out)
 }
 }  // namespace
 
+namespace {
+// ---- the seeded draws (TRACER_RNG_MT19937), replayed on the device: mt19937.cuh -------------------------------------------
+// In-row hit ranks of the n_rows local rows (on the device) and their hit counts (read back into `local`)
+int mt_count_rows(MtWork &m, const int *hit_tri, int W, int n_rows, cudaStream_t st, std::vector<int> &local) {
+    local.assign((size_t)n_rows, 0);
+    if (n_rows == 0) return 0;
+    if (dev_grow(m.rank, m.rank_cap, (size_t)n_rows * W) || dev_grow(m.row_hits, m.rows_cap, (size_t)n_rows)) return TRACER_ERR_NOMEM;
+    mt::row_rank_kernel<<<n_rows, mt::SCAN_THREADS, 0, st>>>(hit_tri, W, m.rank, m.row_hits);
+    CK_CUDA(cudaGetLastError());
+    CK_CUDA(cudaMemcpyAsync(local.data(), m.row_hits, sizeof(int) * (size_t)n_rows, cudaMemcpyDeviceToHost, st));
+    CK_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
+// The frame's [H] row hit counts from this call's own: the whole frame, or a band selection completed by the caller's hook
+int mt_frame_rows(const tracer_render_opts &o, int W, int H, int band_rows, int band_count, const std::vector<int> &local,
+                  std::vector<int> &frame) {
+    const int bi = band_count > 1 ? o.band_index : 0, n_rows = (int)local.size();
+    frame.assign((size_t)H, 0);
+    mt::own_rows(local.data(), n_rows, band_rows, bi, band_count, frame.data(), H);
+    if (band_count <= 1) return 0;
+    const int32_t r = o.row_hits_exchange(o.row_hits_user, H, frame.data());
+    if (r != 0) return fail(TRACER_ERR_STATE, "row_hits_exchange returned " + std::to_string(r));
+    if (!mt::rows_valid(local.data(), n_rows, band_rows, bi, band_count, frame.data(), H, W))
+        return fail(TRACER_ERR_INVALID, "row_hits_exchange changed this call's rows or gave a count outside [0, width]");
+    return 0;
+}
+
+// faceid[k*L + l] of every hit local pixel k, from the frame's row counts: the stream, the automaton, the gather
+int mt_replay(MtWork &m, uint32_t seed, const std::vector<int> &faces, const std::vector<int> &frame, int W, int band_rows,
+              int band_index, int band_count, int n_rows, const int *hit_tri, int *faceid, cudaStream_t st, int &launches) {
+    const int L = (int)faces.size(), S = 3 * L, n_px = n_rows * W;
+    if (L == 0 || n_rows == 0) return 0;
+    std::vector<int64_t> base((size_t)n_rows);
+    const int64_t T = mt::row_bases(frame.data(), (int)frame.size(), n_rows, band_rows, band_index, band_count, base.data());
+    if (T == 0) return 0;
+    std::vector<uint32_t> lights((size_t)2 * L);
+    for (int l = 0; l < L; ++l) lights[l] = (uint32_t)faces[l], lights[L + l] = mt::threshold((uint32_t)faces[l]);
+    if (dev_grow(m.lights, m.lights_cap, lights.size()) || dev_grow(m.base, m.base_cap, base.size()) ||
+        dev_grow(m.fid_ord, m.fid_cap, (size_t)T * L))
+        return TRACER_ERR_NOMEM;
+    CK_CUDA(cudaMemcpyAsync(m.lights, lights.data(), sizeof(uint32_t) * lights.size(), cudaMemcpyHostToDevice, st));
+    CK_CUDA(cudaMemcpyAsync(m.base, base.data(), sizeof(int64_t) * base.size(), cudaMemcpyHostToDevice, st));
+    // 3L words per hit pixel without rejections; when rejections leave the stream short, a longer one is generated
+    int64_t D = 3 * (int64_t)L * T, C = 0, n_chunks = 0;
+    for (;;) {
+        C = std::max<int64_t>(256, (D + 2047) / 2048), n_chunks = (D + C - 1) / C;
+        if (dev_grow(m.words, m.words_cap, (size_t)D) || dev_grow(m.maps, m.maps_cap, (size_t)(2 * n_chunks * S)) ||
+            dev_grow(m.start, m.start_cap, (size_t)n_chunks) || dev_grow(m.ord, m.ord_cap, (size_t)n_chunks + 1))
+            return TRACER_ERR_NOMEM;
+        mt::stream_kernel<<<1, mt::GEN_THREADS, 0, st>>>(seed, D, m.words);
+        CK_CUDA(cudaGetLastError());
+        const int64_t n_maps = n_chunks * S;
+        mt::chunk_map_kernel<<<(unsigned)((n_maps + mt::AUTO_THREADS - 1) / mt::AUTO_THREADS), mt::AUTO_THREADS, 0, st>>>(
+            m.words, D, C, n_chunks, L, m.lights, m.maps, m.maps + n_maps);
+        CK_CUDA(cudaGetLastError());
+        mt::chain_kernel<<<1, 1, 0, st>>>(n_chunks, L, m.maps, m.maps + n_maps, m.start, m.ord);
+        CK_CUDA(cudaGetLastError());
+        launches += 3;
+        int64_t done = 0;
+        CK_CUDA(cudaMemcpyAsync(&done, m.ord + n_chunks, sizeof done, cudaMemcpyDeviceToHost, st));
+        CK_CUDA(cudaStreamSynchronize(st));
+        if (done >= T) break;
+        D += 3 * (int64_t)L * (T - done) + D / 16;
+    }
+    mt::chunk_faceids_kernel<<<(unsigned)((n_chunks + mt::AUTO_THREADS - 1) / mt::AUTO_THREADS), mt::AUTO_THREADS, 0, st>>>(
+        m.words, D, C, n_chunks, T, L, m.lights, m.start, m.ord, m.fid_ord);
+    CK_CUDA(cudaGetLastError());
+    mt::gather_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(hit_tri, W, n_px, L, m.base, m.rank, m.fid_ord, faceid);
+    CK_CUDA(cudaGetLastError());
+    launches += 2;
+    return 0;
+}
+
+// frame_rows: the frame's row hit counts when the caller already has them: the bundle-cull mode's re-render of a frame whose
+// closest-hit pass was complete but whose shadow candidates overflowed (same hits; the exchange hook runs once per frame)
+int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32_t H, const tracer_render_opts *opts_in,
+                 uint8_t *rgb_out, const std::vector<int> *frame_rows);
+}  // namespace
+
 extern "C" {
 
 int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32_t H,
                              const tracer_render_opts *opts_in, uint8_t *rgb_out) {
+    return render_scene(s, cam, W, H, opts_in, rgb_out, nullptr);
+}
+}  // extern "C"
+
+namespace {
+int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32_t H, const tracer_render_opts *opts_in,
+                 uint8_t *rgb_out, const std::vector<int> *frame_rows) {
     if (!s || !cam || !rgb_out) return fail(TRACER_ERR_INVALID, "null argument");
     if (!s->ctx || !s->ctx->inited) return fail(TRACER_ERR_NO_DEVICE, "tracer_cuda_init not called");
     Ctx &g = *s->ctx;
@@ -889,8 +999,8 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     const int band_rows = band_count > 1 ? o.band_rows : H;
     if (band_count > 1 && (band_rows <= 0 || o.band_index < 0 || o.band_index >= band_count))
         return fail(TRACER_ERR_INVALID, "bad band selection");
-    if (o.rng_mode == TRACER_RNG_MT19937 && band_count > 1)
-        return fail(TRACER_ERR_INVALID, "TRACER_RNG_MT19937 needs the whole frame in one call (band_count <= 1)");
+    if (o.rng_mode == TRACER_RNG_MT19937 && band_count > 1 && !o.row_hits_exchange)
+        return fail(TRACER_ERR_INVALID, "TRACER_RNG_MT19937 with band_count > 1 needs opts->row_hits_exchange (the other bands' row hit counts)");
     if (o.rng_mode == TRACER_RNG_EXPLICIT && !o.faceid && s->n_lights > 0)
         return fail(TRACER_ERR_INVALID, "TRACER_RNG_EXPLICIT needs opts->faceid");
     if (o.rng_mode < 0 || o.rng_mode > 2) return fail(TRACER_ERR_INVALID, "bad rng_mode");
@@ -906,7 +1016,9 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     std::memset(&s->stats, 0, sizeof s->stats);
     s->stats.n_sms = g.n_sms;
     s->stats.n_pixels = n_px;
-    if (n_px == 0) return TRACER_OK;
+    const bool mt_exchange = o.rng_mode == TRACER_RNG_MT19937 && band_count > 1 && !frame_rows;
+    std::vector<int> mt_frame; // the frame's row hit counts (TRACER_RNG_MT19937)
+    if (n_px == 0) return mt_exchange ? mt_frame_rows(o, W, H, band_rows, band_count, {}, mt_frame) : TRACER_OK;
     if (int rc = ensure_workspace(s, n_px, o.out_occ_tri != nullptr)) return rc;
     int launches = 0;
 
@@ -954,6 +1066,21 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     const double est_default_ms = (double)n_px * (double)s->n_tris * (1.0 + 0.25 * L) / 4.0e9;
     // (the optional mode keeps every light vertex's tables resident; a light too big for that renders in the default mode)
     const bool cull = !use_bvh && s->tables_resident && (o.bundle_cull == 3 ? est_default_ms > 6.0 : o.bundle_cull != 0);
+    // the optional mode's candidate buffer (24 per ray + slack) was too small for this scene's depth complexity: render the
+    // frame again with a 4x larger one while that fits comfortably, else by the default sweeps, which need no such buffer —
+    // same bytes out either way.  rows: the frame's row hit counts when they are known to be right (see frame_rows).
+    auto rerender_after_overflow = [&](const std::vector<int> *rows) -> int {
+        tracer_render_opts o2 = o;
+        o2.struct_size = sizeof o2;
+        size_t free_b = 0, total_b = 0;
+        cudaMemGetInfo(&free_b, &total_b);
+        const size_t next_bytes = ((size_t)n_px * 24 * (size_t)s->cull_grow * 4 + ((size_t)1 << 22)) * sizeof(unsigned long long) * 3;
+        if (!std::getenv("TRACER_CAND_CAP") && s->cull_grow < 64 && next_bytes < free_b / 2 + s->cand_cap * 24)
+            s->cull_grow *= 4;
+        else
+            o2.bundle_cull = 0;
+        return render_scene(s, cam, W, H, &o2, rgb_out, rows);
+    };
     if (cull) { // candidate buffers: 24 per ray + slack (a few per ray are typical), sorted with a radix sort
         const size_t cap = (size_t)n_px * 24 * (size_t)s->cull_grow + ((size_t)1 << 22);
         if (cap > s->cand_cap) {
@@ -1124,17 +1251,25 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
         }
         CK_CUDA(cudaMemcpyAsync(s->faceid, loc.data(), loc.size() * sizeof(int), cudaMemcpyHostToDevice, st));
         CK_CUDA(cudaStreamSynchronize(st));
-    } else if (smp == 0 && L > 0 && o.rng_mode == TRACER_RNG_MT19937) {
-        trk::hitmask_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(s->hit_tri, n_px, s->mask);
-        CK_CUDA(cudaGetLastError());
+    } else if (smp == 0 && o.rng_mode == TRACER_RNG_MT19937) {
+        // a bundle-cull closest-hit pass whose candidates overflowed has lost hits: its row counts must not be used or sent,
+        // so the frame is rendered again before the exchange (read back with the row counts, at the same synchronise)
+        unsigned long long primary_overflow = 0;
+        if (cull) CK_CUDA(cudaMemcpyAsync(&primary_overflow, &s->counters->cull_overflow, sizeof primary_overflow, cudaMemcpyDeviceToHost, st));
+        std::vector<int> local;
+        if (int rc = mt_count_rows(s->mt, s->hit_tri, W, n_rows, st, local)) return rc;
         ++launches;
-        std::vector<uint8_t> hm((size_t)n_px);
-        CK_CUDA(cudaMemcpyAsync(hm.data(), s->mask, (size_t)n_px, cudaMemcpyDeviceToHost, st));
-        CK_CUDA(cudaStreamSynchronize(st));
-        std::vector<int> fid((size_t)n_px * L);
-        tracer__mt19937_scan(o.seed, L, s->h_light_F.data(), n_px, hm.data(), fid.data()); // local order == scan order
-        CK_CUDA(cudaMemcpyAsync(s->faceid, fid.data(), fid.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-        CK_CUDA(cudaStreamSynchronize(st));
+        if (primary_overflow) return rerender_after_overflow(frame_rows);
+        if (frame_rows) {
+            if (!mt::rows_valid(local.data(), n_rows, band_rows, bands.band_index, band_count, frame_rows->data(), H, W))
+                return fail(TRACER_ERR_STATE, "bundle-cull re-render: the closest-hit pass found other hits than the first pass");
+            mt_frame = *frame_rows;
+        } else if (int rc = mt_frame_rows(o, W, H, band_rows, band_count, local, mt_frame)) {
+            return rc;
+        }
+        if (int rc = mt_replay(s->mt, o.seed, s->h_light_F, mt_frame, W, band_rows, bands.band_index, band_count, n_rows, s->hit_tri,
+                               s->faceid, st, launches))
+            return rc;
     }
 
     // ---- lights: (finish k-1, set up k) -> group by light vertex -> first-occluder sweep ----
@@ -1441,21 +1576,8 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
     // of which multiply-adds that evaluate bounds (the rest is each pair's interval test and the per-triangle interval)
     s->stats.flop_primary_edges = no_flops ? 0.0 : flop_primary_edges;
     s->stats.flop_shadow_edges = no_flops ? 0.0 : 16.0 / trk::SHADOW_R;
-    if (hc.cull_overflow) {
-        // the optional mode's candidate buffer (24 per ray + slack) was too small for this scene's depth complexity: render
-        // the frame again with a 4x larger one while that fits comfortably, else by the default sweeps, which need no such
-        // buffer — same bytes out either way
-        tracer_render_opts o2 = o;
-        o2.struct_size = sizeof o2;
-        size_t free_b = 0, total_b = 0;
-        cudaMemGetInfo(&free_b, &total_b);
-        const size_t next_bytes = ((size_t)n_px * 24 * (size_t)s->cull_grow * 4 + ((size_t)1 << 22)) * sizeof(unsigned long long) * 3;
-        if (!std::getenv("TRACER_CAND_CAP") && s->cull_grow < 64 && next_bytes < free_b / 2 + s->cand_cap * 24)
-            s->cull_grow *= 4;
-        else
-            o2.bundle_cull = 0;
-        return tracer_cuda_render_scene(s, cam, W, H, &o2, rgb_out);
-    }
+    if (hc.cull_overflow) // (with TRACER_RNG_MT19937 only the shadow sweeps' candidates can have overflowed by now)
+        return rerender_after_overflow(o.rng_mode == TRACER_RNG_MT19937 ? &mt_frame : nullptr);
     if (getenv("TRACER_SHADOW_DIAG") && hc.cyc_total)
         fprintf(stderr, "shadow diag: CTA cycles %.3e total = items %.1f %% + grid barriers %.1f %% + compaction %.1f %% + other %.1f %%; %llu items in %llu runs\n",
                 (double)hc.cyc_total, 100.0 * hc.cyc_items / hc.cyc_total, 100.0 * hc.cyc_barrier / hc.cyc_total, 100.0 * hc.cyc_compact / hc.cyc_total,
@@ -1465,6 +1587,9 @@ int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int3
                 hc.cull_tiles_any, hc.cull_tiles_fallback, hc.cull_l1, (unsigned long long)(hc.tests_shadow / 4096 / cull::CTILE));
     return TRACER_OK;
 }
+}  // namespace
+
+extern "C" {
 
 int tracer_cuda_last_stats(tracer_scene_dev *s, tracer_frame_stats *out) {
     if (!s || !out) return fail(TRACER_ERR_INVALID, "null argument");
@@ -1487,6 +1612,85 @@ int tracer__bvh_prepare(tracer_scene_dev *s, double *ms_out) {
     float ms = 0.f;
     CK_CUDA(cudaEventElapsedTime(&ms, s->ev[0], s->ev[3]));
     if (ms_out) *ms_out = ms;
+    return TRACER_OK;
+}
+
+// Internal (tests, measurement): the device replay of the seeded draws, on the current device, for one whole frame's hit
+// mask in scan order (n_rows rows of W pixels).  faceid_scan [W*n_rows*L]: what tracer_mt19937_faceids gives, in scan
+// order, -1 for misses.  *ms_out (may be NULL): CUDA events around the replay, from the per-row hit count to the gather.
+int tracer__mt19937_faceids_device(uint32_t seed, int32_t L, const int32_t *faces, int32_t W, int32_t n_rows, const uint8_t *hit_scan,
+                                   int32_t *faceid_scan, double *ms_out) {
+    if (!g_cur) return fail(TRACER_ERR_NO_DEVICE, "tracer_cuda_init not called");
+    if (L < 0 || W < 1 || n_rows < 1 || (int64_t)W * n_rows * std::max(L, 1) >= ((int64_t)1 << 31) || !hit_scan || !faceid_scan || (L && !faces))
+        return fail(TRACER_ERR_INVALID, "bad argument");
+    Ctx &g = *g_cur;
+    t_pool = &g.pool;
+    CK_CUDA(cudaSetDevice(g.device));
+    cudaStream_t st = g.stream;
+    const int n_px = W * n_rows;
+    struct Bufs {
+        MtWork m;
+        int *tri = nullptr, *fid = nullptr;
+        cudaEvent_t ev[2] = {nullptr, nullptr};
+        ~Bufs() {
+            m.release(), dev_free(tri), dev_free(fid);
+            for (cudaEvent_t e : ev)
+                if (e) cudaEventDestroy(e);
+        }
+    } b;
+    std::vector<int> tri((size_t)n_px);
+    for (int k = 0; k < n_px; ++k) tri[k] = hit_scan[k] ? 0 : -1;
+    if (dev_alloc(&b.tri, (size_t)n_px) || dev_alloc(&b.fid, (size_t)n_px * std::max(L, 1))) return TRACER_ERR_NOMEM;
+    CK_CUDA(cudaEventCreate(&b.ev[0]));
+    CK_CUDA(cudaEventCreate(&b.ev[1]));
+    CK_CUDA(cudaMemcpyAsync(b.tri, tri.data(), sizeof(int) * (size_t)n_px, cudaMemcpyHostToDevice, st));
+    CK_CUDA(cudaMemsetAsync(b.fid, 0xff, sizeof(int) * (size_t)n_px * std::max(L, 1), st));
+    CK_CUDA(cudaEventRecord(b.ev[0], st));
+    std::vector<int> local, frame;
+    tracer_render_opts whole{};
+    int launches = 0;
+    if (int rc = mt_count_rows(b.m, b.tri, W, n_rows, st, local)) return rc;
+    if (int rc = mt_frame_rows(whole, W, n_rows, n_rows, 1, local, frame)) return rc;
+    if (int rc = mt_replay(b.m, seed, std::vector<int>(faces, faces + L), frame, W, n_rows, 0, 1, n_rows, b.tri, b.fid, st, launches))
+        return rc;
+    CK_CUDA(cudaEventRecord(b.ev[1], st));
+    CK_CUDA(cudaMemcpyAsync(faceid_scan, b.fid, sizeof(int) * (size_t)n_px * L, cudaMemcpyDeviceToHost, st));
+    CK_CUDA(cudaStreamSynchronize(st));
+    float ms = 0.f;
+    CK_CUDA(cudaEventElapsedTime(&ms, b.ev[0], b.ev[1]));
+    if (ms_out) *ms_out = ms;
+    return TRACER_OK;
+}
+
+// Internal (measurement): the replay's stream generator on its own, n words of std::mt19937(seed) on the current device;
+// *ms_out = CUDA events around the one launch.
+int tracer__mt19937_stream_device(uint32_t seed, int64_t n, double *ms_out) {
+    if (!g_cur) return fail(TRACER_ERR_NO_DEVICE, "tracer_cuda_init not called");
+    if (n < 1 || !ms_out) return fail(TRACER_ERR_INVALID, "bad argument");
+    Ctx &g = *g_cur;
+    t_pool = &g.pool;
+    CK_CUDA(cudaSetDevice(g.device));
+    cudaStream_t st = g.stream;
+    struct Bufs {
+        uint32_t *words = nullptr;
+        cudaEvent_t ev[2] = {nullptr, nullptr};
+        ~Bufs() {
+            dev_free(words);
+            for (cudaEvent_t e : ev)
+                if (e) cudaEventDestroy(e);
+        }
+    } b;
+    if (dev_alloc(&b.words, (size_t)n)) return TRACER_ERR_NOMEM;
+    CK_CUDA(cudaEventCreate(&b.ev[0]));
+    CK_CUDA(cudaEventCreate(&b.ev[1]));
+    CK_CUDA(cudaEventRecord(b.ev[0], st));
+    mt::stream_kernel<<<1, mt::GEN_THREADS, 0, st>>>(seed, n, b.words);
+    CK_CUDA(cudaGetLastError());
+    CK_CUDA(cudaEventRecord(b.ev[1], st));
+    CK_CUDA(cudaEventSynchronize(b.ev[1]));
+    float ms = 0.f;
+    CK_CUDA(cudaEventElapsedTime(&ms, b.ev[0], b.ev[1]));
+    *ms_out = ms;
     return TRACER_OK;
 }
 
@@ -1577,6 +1781,67 @@ int tracer_cuda_scene_create_multi(const tracer_scene_flat *sc, tracer_scene_mul
     return TRACER_OK;
 }
 
+}  // extern "C"
+
+namespace {
+// TRACER_RNG_MT19937 on several GPUs: their row hit counts summed between their threads, a barrier and a shared [H]
+// array.  A GPU whose render fails before the exchange arrives after it, with an error flag, so that no thread waits
+// forever; every GPU's exchange then fails.
+struct RowExchange {
+    std::mutex mu;
+    std::condition_variable cv;
+    int n = 0, arrived = 0;
+    bool error = false;
+    std::vector<int> sum;
+    bool arrive(int32_t *rows, int32_t H, bool failed) {
+        std::unique_lock<std::mutex> lk(mu);
+        if (failed) error = true;
+        else {
+            if ((int)sum.size() < H) sum.resize((size_t)H, 0);
+            for (int r = 0; r < H; ++r) sum[r] += rows[r];
+        }
+        if (++arrived == n) cv.notify_all();
+        else cv.wait(lk, [&] { return arrived == n; });
+        if (error) return false;
+        if (rows) std::copy(sum.begin(), sum.begin() + H, rows);
+        return true;
+    }
+};
+struct RowExchangeSeat {
+    RowExchange *x = nullptr;
+    bool arrived = false, peer_failed = false;
+};
+int32_t row_exchange_hook(void *user, int32_t H, int32_t *rows) {
+    auto *seat = (RowExchangeSeat *)user;
+    seat->arrived = true;
+    if (seat->x->arrive(rows, H, false)) return 0;
+    seat->peer_failed = true;
+    return 1;
+}
+}  // namespace
+
+extern "C" {
+
+// Internal (tests only, no GPU needed): the multi-GPU call's row-count exchange between n threads.  Thread d offers
+// rows_in[d*H ..] through the hook, or — fails[d] != 0 — arrives as a GPU whose render failed before the exchange does.
+// rows_out[d*H ..] = what thread d's hook left in its array, rc_out[d] = the hook's return (-1 for a failed thread).
+void tracer__row_exchange_host(int32_t n, int32_t H, const int32_t *rows_in, const uint8_t *fails, int32_t *rows_out, int32_t *rc_out) {
+    RowExchange xchg;
+    xchg.n = n;
+    std::vector<RowExchangeSeat> seats((size_t)n);
+    auto work = [&](int d) {
+        int32_t *rows = rows_out + (size_t)d * H;
+        std::copy(rows_in + (size_t)d * H, rows_in + (size_t)(d + 1) * H, rows);
+        seats[d].x = &xchg;
+        rc_out[d] = fails[d] ? -1 : row_exchange_hook(&seats[d], H, rows);
+        if (!seats[d].arrived) xchg.arrive(nullptr, 0, true);
+    };
+    std::vector<std::thread> th;
+    for (int d = 1; d < n; ++d) th.emplace_back(work, d);
+    work(0);
+    for (auto &t : th) t.join();
+}
+
 int tracer_cuda_render_scene_multi(tracer_scene_multi *ms, const tracer_camera *cam, int32_t W, int32_t H,
                                    const tracer_render_opts *opts_in, uint8_t *rgb_out) {
     if (!ms || !cam || !rgb_out) return fail(TRACER_ERR_INVALID, "null argument");
@@ -1615,7 +1880,11 @@ int tracer_cuda_render_scene_multi(tracer_scene_multi *ms, const tracer_camera *
     }
     std::vector<int> rc((size_t)n, 0);
     std::vector<std::string> err((size_t)n);
-    auto work = [&](int d) {
+    const bool mt = o.rng_mode == TRACER_RNG_MT19937;
+    RowExchange xchg;
+    xchg.n = n;
+    std::vector<RowExchangeSeat> seats((size_t)n);
+    auto render_on = [&](int d) {
         Ctx &g = g_ctx[d];
         uint8_t *dst = g_multi.gathered; // GPU 0
         if (d > 0) {
@@ -1633,16 +1902,22 @@ int tracer_cuda_render_scene_multi(tracer_scene_multi *ms, const tracer_camera *
         od.struct_size = sizeof od;
         od.band_rows = band_rows, od.band_index = d, od.band_count = n;
         od.rgb_out_is_device = 1, od.cuda_stream = nullptr; // the GPU's own stream: the send below is queued behind the frame
+        if (mt) seats[d].x = &xchg, od.row_hits_exchange = row_exchange_hook, od.row_hits_user = &seats[d];
         rc[d] = tracer_cuda_render_scene(ms->dev[d], cam, W, H, &od, dst);
         if (rc[d]) err[d] = g_err;
+    };
+    auto work = [&](int d) {
+        render_on(d);
+        if (mt && !seats[d].arrived) xchg.arrive(nullptr, 0, true); // failed before the exchange: release the others
     };
     std::vector<std::thread> th;
     for (int d = 1; d < n; ++d) th.emplace_back(work, d);
     work(0);
     for (auto &t : th) t.join();
-    for (int d = 0; d < n; ++d)
-        if (rc[d]) return fail(rc[d], "GPU " + std::to_string(d) + ": " + err[d]);
-    // the one exchange step: packed bands -> GPU 0
+    for (int pass = 0; pass < 2; ++pass) // the error of a GPU that failed on its own before the others' exchange failures
+        for (int d = 0; d < n; ++d)
+            if (rc[d] && (pass == 1 || !seats[d].peer_failed)) return fail(rc[d], "GPU " + std::to_string(d) + ": " + err[d]);
+    // the band gather: packed bands -> GPU 0
     ncclResult_t r = g_nccl.GroupStart();
     for (int d = 1; d < n && r == ncclSuccess; ++d) {
         const size_t bytes = (size_t)tracer_band_row_count(H, band_rows, d, n) * row_bytes;

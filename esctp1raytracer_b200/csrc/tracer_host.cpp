@@ -134,23 +134,4 @@ int tracer_mt19937_faceids(const tracer_scene_flat *scene, int32_t width, int32_
     return TRACER_OK;
 }
 
-// Internal (not in tracer_cuda.h): same draws for a hit mask already in scan order
-// (the local pixel order of an un-banded frame), F_l given per light.
-int tracer__mt19937_scan(uint32_t seed, int32_t n_lights, const int32_t *faces_per_light, int64_t n_px,
-                         const uint8_t *hit_scan, int32_t *faceid_scan) {
-    Mt19937 gen(seed);
-    for (int64_t k = 0; k < n_px; ++k) {
-        for (int l = 0; l < n_lights; ++l) {
-            int fid = -1;
-            if (hit_scan[k]) {
-                fid = gen.below((uint32_t)faces_per_light[l]);
-                (void)gen.next();
-                (void)gen.next();
-            }
-            faceid_scan[k * n_lights + l] = fid;
-        }
-    }
-    return TRACER_OK;
-}
-
 }  // extern "C"

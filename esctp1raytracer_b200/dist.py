@@ -10,6 +10,8 @@ buffers into PPM order with ``tracer_cuda_assemble_bands``.
 
 The counter-based RNG is keyed by the image index, so the assembled frame is
 byte-identical to a single-GPU frame (tests/test_gpu_parity.py, tests/test_dist_gloo.py).
+The seeded std::mt19937 mode needs one more exchange per frame: each rank's per-row hit
+counts, all-reduced (SUM) over the group, give every rank its hits' places in the stream.
 """
 from __future__ import annotations
 
@@ -55,6 +57,22 @@ def torch_stream_handle():
     return torch.cuda.current_stream().cuda_stream or 1
 
 
+def row_hits_all_reduce(group=None):
+    """The seeded mode's exchange hook for ``Renderer.trace(row_hits_exchange=...)``: every rank's per-row hit counts
+    summed over the process group, in place (each row has one owner, so the sum is the frame's counts)."""
+
+    def exchange(row_hits):
+        import torch
+        import torch.distributed as dist
+
+        dev = "cuda" if dist.get_backend(group) == "nccl" else "cpu"
+        t = torch.from_numpy(row_hits.copy()).to(dev)
+        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
+        row_hits[:] = t.cpu().numpy()
+
+    return exchange
+
+
 def render_frame(renderer, resident_scene, camera, width, height, *, rank=0, world=1, band_rows=DEFAULT_BAND_ROWS,
                  rng_mode=0, seed=1, group=None, bundle_cull=False, samples_per_pixel=0, bvh=False):
     """Render this rank's bands into HBM, gather to rank 0, assemble.  Returns
@@ -65,9 +83,10 @@ def render_frame(renderer, resident_scene, camera, width, height, *, rank=0, wor
     local = torch.zeros((rows_pad, width, 3), dtype=torch.uint8, device="cuda")
     stream = torch_stream_handle()
     bands = (band_rows, rank, world) if world > 1 else None
+    exchange = row_hits_all_reduce(group) if world > 1 and rng_mode == 1 else None  # RNG_MT19937
     fr = renderer.trace(resident_scene, camera, width, height, rng_mode=rng_mode, seed=seed, bands=bands,
                         out_device_ptr=local.data_ptr(), stream=stream, bundle_cull=bundle_cull, bvh=bvh,
-                        samples_per_pixel=samples_per_pixel)
+                        samples_per_pixel=samples_per_pixel, row_hits_exchange=exchange)
     if world == 1:
         return local, fr.stats
     gathered = gather_bands(local, rank, world, 0, group)

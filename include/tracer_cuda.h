@@ -83,8 +83,10 @@ typedef enum tracer_rng_mode {
     /* std::mt19937(seed) consumed exactly as scan_row does (main.cpp:743-754,
      * three draws per hit pixel per light, scan order h=H-1..0, w=0..W-1,
      * libstdc++ uniform_int_distribution): reproduces the seeded serial path.
-     * The draws are sequential over the whole frame's hit mask, so this mode
-     * needs the whole frame in one call (band_count <= 1). */
+     * The draws are replayed on the device.  A pixel's draws depend on the hits
+     * of every earlier row of the frame, so a call that renders bands
+     * (band_count > 1) needs opts->row_hits_exchange to learn the other rows'
+     * hit counts; 1 sample per pixel only. */
     TRACER_RNG_MT19937 = 1,
     /* faceID per (pixel, light) supplied by the caller in opts->faceid. */
     TRACER_RNG_EXPLICIT = 2
@@ -133,6 +135,17 @@ typedef struct tracer_render_opts {
                              shadow_chunks are ignored.  In this mode tests_primary / tests_shadow = strict_evals = the
                              triangle tests done at leaves, flop_* = 0, and the tree's build time is part of ms_other.
                              Appended last: callers with an older struct_size get 0. */
+
+    /* TRACER_RNG_MT19937 with band_count > 1 only (required there, ignored otherwise): the frame's per-row hit counts.
+     * The call invokes it exactly once, after its closest-hit pass, also when its band selection covers no row.  On
+     * entry row_hits[r] (r = PPM row, 0 .. height-1) holds this call's hit count for every row it renders and 0
+     * elsewhere; on return it must hold the counts of every row of the frame (each row has one owner, so an all-reduce
+     * sum over the calls that render the frame does it) and return 0.  A non-zero return fails the render with
+     * TRACER_ERR_STATE; this call's rows changed or a count outside [0, width] fails it with TRACER_ERR_INVALID.  The
+     * scene stays usable either way.  A call that fails before its closest-hit pass ends does not invoke it.
+     * Appended last: callers with an older struct_size get NULL. */
+    int32_t (*row_hits_exchange)(void *user, int32_t height, int32_t *row_hits);
+    void *row_hits_user;
 } tracer_render_opts;
 
 typedef struct tracer_frame_stats {
@@ -205,8 +218,9 @@ int tracer_cuda_last_stats(tracer_scene_dev *scene, tracer_frame_stats *out);
  * The frame's PPM rows are cut into bands of opts->band_rows (default 8) rows, band b is
  * rendered by GPU b % n_gpus, every GPU quantises its bands straight into its send
  * buffer and the packed bands are gathered on GPU 0 with grouped ncclSend/ncclRecv over
- * NVLink.  Results are byte-identical to a single-GPU frame (TRACER_RNG_HASH and
- * TRACER_RNG_EXPLICIT; TRACER_RNG_MT19937 needs the whole frame on one GPU).
+ * NVLink.  Results are byte-identical to a single-GPU frame, in every rng_mode: with
+ * TRACER_RNG_MT19937 the GPUs exchange their per-row hit counts between their threads
+ * (opts->row_hits_exchange is the call's own), and every GPU replays the draws itself.
  * After tracer_cuda_init_multi(n > 1) the drop-in tracer_cuda_render() uses all n GPUs. */
 typedef struct tracer_scene_multi tracer_scene_multi; /* opaque: one scene replica per GPU */
 int tracer_cuda_init_multi(int n_gpus);               /* devices 0 .. n_gpus-1 */
