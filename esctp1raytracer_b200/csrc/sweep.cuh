@@ -4,7 +4,8 @@
 // What the reference does per (ray, triangle) pair: full Moller-Trumbore with
 // a double-precision divide (ray_triangle.h:7-57, ~52 flop).  What this kernel
 // does per pair: half a packed add and half a three-input min (4., hot rows), plus
-// 8 ops per thread and triangle (12 with a mean q).  The saving comes from these observations.
+// 8 ops per thread and triangle (12 with a mean q); the closest-hit sweep does nothing per pair, one packed add per
+// thread and triangle on the thread's extreme rays (segment_pass).  The saving comes from these observations.
 //
 //  1. Every sweep is a bundle of rays through ONE common point.  Primary rays
 //     all start at the eye (camera.h:31-34).  A shadow ray runs from the hit
@@ -62,7 +63,8 @@
 //  * every lane of every warp reads the SAME row at the same time, so the two LDS.128 per
 //    triangle are pure broadcasts, amortised over R rays per thread held in registers
 //    (R = 64 closest hit, 32 any-hit);
-//  * each pair is ONE interval test |2*S*p + nc2| <= h2 (hot rows, below): per two pairs one packed
+//  * closest hit (MODE_SHAREDQ): one two-sided test on the thread's least and greatest 2*S*p per triangle (segment_pass);
+//  * any-hit: each pair is ONE interval test |2*S*p + nc2| <= h2 (hot rows, below): per two pairs one packed
 //    FADD2 and one FMNMX3 running minimum, no saturation, no integer op.  History on this part
 //    (cycles per pair, closest hit): round 1 sign bits through LOP3 on the half-rate ALU pipe 7.9,
 //    three saturating rows with a product accumulate 6.8, span form with two saturating adds 4.0;
@@ -393,6 +395,17 @@ __device__ __forceinline__ float fmin3_abs(float m, float a, float b) {
 // Padding rows (Cl = -SPAN_OPEN, shifted: still -1e30) give A = -1e30, B = C, h2 = -1e30 < 0: never a candidate;
 // always-candidate rows (every constant SPAN_OPEN) give A = B = C, nc2 = 0, h2 = 2C > |2*S*p|.  A NaN bound is dropped by
 // the min3 (the clamp stays), a NaN |e| by the running minimum: neither can hide a candidate.
+//
+// SEGMENT verdict (closest-hit sweep, MODE_SHAREDQ: segment_pass).  The R rays of a thread share q bit for bit, so they
+// share (nc2, h2), and the hot loop's verdict "some ray r has |fl(ps2_r + nc2)| <= h2" needs no per-ray work.  Let
+// pmin2 <= ps2_r <= pmax2 for every r (a min and a max over all R values, whatever their order).  Round-to-nearest
+// addition is monotone, a <= b => fl(a + c) <= fl(b + c), so a passing ray r gives
+//     fl(pmin2 + nc2) <= fl(ps2_r + nc2) <= h2     and     fl(pmax2 + nc2) >= fl(ps2_r + nc2) >= -h2,
+// and the two-sided test on the thread's extreme rays passes every (thread, triangle) the per-ray verdict passes: no new
+// margin, no new rounding.  It costs one FADD2 and the compares per thread and triangle in place of R/2 FADD2 + R/2
+// FMNMX3.  It is looser only where a triangle's interval falls between two neighbouring rays of the thread (narrower than
+// a pixel); the candidate path rebuilds the per-ray mask with hot_pass, so the pairs handed to the strict test are the same.
+// A NaN sum counts as a pass.  Not for the shadow sweeps: their rays are sorted by q and scattered in p.
 constexpr float HOT_CLAMP = SPAN_BOX;
 constexpr float HOT_DELTA = 8.f * 1.1920928955078125e-7f * HOT_CLAMP;
 constexpr float HOT_QD_SCALE = 1.f + 0x1p-20f;
@@ -425,6 +438,16 @@ __host__ __device__ __forceinline__ void hot_terms_qbar(const float4 lo, const f
 }
 // the hot test of one pair (ps2 = p * 2 * SPAN_S)
 __host__ __device__ __forceinline__ bool hot_pass(float nc2, float h2, float ps2) { return fabsf(ps2 + nc2) <= h2; }
+// the segment verdict of a thread's rays with a shared q (pmin2, pmax2: least and greatest ps2 over all of them; above HOT_CLAMP):
+// true whenever hot_pass holds for one of them.  Device: one packed FADD2; host: the same two RN adds.
+__host__ __device__ __forceinline__ bool segment_pass(float nc2, float h2, float pmin2, float pmax2) {
+#ifdef __CUDA_ARCH__
+    const float2 e = __fadd2_rn(make_float2(pmin2, pmax2), make_float2(nc2, nc2));
+#else
+    const float2 e = make_float2(pmin2 + nc2, pmax2 + nc2);
+#endif
+    return !(e.x > h2) && !(-e.y > h2);
+}
 // the hot test of one ray (p, its own q) on a staged hot row (candidate path of the any-hit sweeps)
 __device__ __forceinline__ bool hot_row_pass(const float4 *row, float p, float q) {
     float nc2, h2;
@@ -457,6 +480,18 @@ __device__ __forceinline__ unsigned eval_interval(const float4 *__restrict__ tp,
             m = fmin3_abs(m, e.x, e.y);
         }
         cand |= (unsigned)(m <= h2) << k;
+    }
+    return cand;
+}
+// The same verdict bits from the thread's extreme rays (segment_pass; closest-hit sweep, MODE_SHAREDQ only): per triangle
+// the set-up of hot_terms, one FADD2 and the compares, whatever R.  Bit k set = triangle k may hold a candidate.
+__device__ __forceinline__ unsigned eval_segment(const float4 *__restrict__ tp, float pmin2, float pmax2, float q) {
+    unsigned cand = 0;
+#pragma unroll
+    for (int k = 0; k < SPAN_BATCH; ++k) {
+        float nc2, h2;
+        hot_terms(tp[2 * k], tp[2 * k + 1], q, nc2, h2);
+        cand |= (unsigned)segment_pass(nc2, h2, pmin2, pmax2) << k;
     }
     return cand;
 }
@@ -521,6 +556,13 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
 #pragma unroll
     for (int r = 0; r < R; ++r) ps2[r] = rp[r] * (2.f * SPAN_S);
     const float qhot = MODE == MODE_QBAR ? qbar : rq[0], qdh = hot_qdelta(qdelta);
+    // closest hit with a shared q: the hot loop decides each triangle from the extreme rays (segment_pass)
+    constexpr bool SEGMENT = !ANYHIT && MODE == MODE_SHAREDQ;
+    float pmin2 = ps2[0], pmax2 = ps2[0];
+    if (SEGMENT) {
+#pragma unroll
+        for (int r = 1; r < R; ++r) pmin2 = fminf(pmin2, ps2[r]), pmax2 = fmaxf(pmax2, ps2[r]);
+    }
     const unsigned lane = tid & 31;
     unsigned *queue = sm.queue[tid >> 5];
 #ifndef SWEEP_NO_STRICT
@@ -571,7 +613,8 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
 #pragma unroll 1
             for (int b0 = 0; b0 < TILE; b0 += NB) {
                 unsigned cand;
-                if constexpr (SPAN) cand = eval_interval<R, MODE>(tp + ROWS * b0, ps2, qhot, qdh);
+                if constexpr (SEGMENT) cand = eval_segment(tp + ROWS * b0, pmin2, pmax2, qhot);
+                else if constexpr (SPAN) cand = eval_interval<R, MODE>(tp + ROWS * b0, ps2, qhot, qdh);
                 else cand = eval_batch<R, MODE>(tp + ROWS * b0, rp, rq, qbar, qdelta);
 #ifdef SWEEP_NO_STRICT // development microbenchmark only (tools/sweep_mb2.cu): timing without the strict path
                 if (cand) ++done;

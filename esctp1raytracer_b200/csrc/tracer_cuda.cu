@@ -109,6 +109,25 @@ extern "C" void tracer__hot_row_pass(const float *row8, int n, const float *p, c
     }
 }
 extern "C" void tracer__hot_consts(float *out3) { out3[0] = sweep::HOT_CLAMP, out3[1] = sweep::HOT_DELTA, out3[2] = sweep::HOT_QD_SCALE; }
+// n rays (p, in any order, duplicates allowed) of one closest-hit thread with the shared q against one span row (row8 as
+// span_rows makes it, stored in the hot form as the tables store it).  out2[0] = the segment verdict (sweep::segment_pass on
+// the least and greatest 2 S p, as sweep_table forms them), out2[1] = the OR of the per-ray hot tests (the verdict of the
+// per-ray loop it replaces).  terms2 (may be null) receives (nc2, h2).
+extern "C" void tracer__segment_pass(const float *row8, int n, const float *p, float q, unsigned char *out2, float *terms2) {
+    float4 lo = make_float4(row8[0], row8[1], row8[2], row8[3]), hi = make_float4(row8[4], row8[5], row8[6], row8[7]);
+    sweep::hot_row(lo, hi);
+    float nc2, h2;
+    sweep::hot_terms(lo, hi, q, nc2, h2);
+    bool any = false;
+    float pmin2 = p[0] * (2.f * sweep::SPAN_S), pmax2 = pmin2;
+    for (int i = 0; i < n; ++i) {
+        const float ps2 = p[i] * (2.f * sweep::SPAN_S);
+        pmin2 = fminf(pmin2, ps2), pmax2 = fmaxf(pmax2, ps2);
+        any |= sweep::hot_pass(nc2, h2, ps2);
+    }
+    out2[0] = sweep::segment_pass(nc2, h2, pmin2, pmax2), out2[1] = any;
+    if (terms2) terms2[0] = nc2, terms2[1] = h2;
+}
 
 // Internal (tests only): strict::powf_glibc as the device computes it, for every stride-th float bit pattern x from
 // lo_bits up to hi_bits (inclusive) -> host_out[(hi_bits - lo_bits) / stride + 1], or for n (x, y) pairs.  Runs on the
@@ -1231,7 +1250,8 @@ int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32
         // executed FP32 flops per pair: hot form half a packed FADD2 per pair (the three-input mins are no flops), and
         // per thread and triangle 4 FFMA for the bounds + the 2 FADD of nc2 and h2 (10 flops; 8 more FFMA-flops with a
         // mean q); three-row form with every ray its own q: 6 FFMA.SAT + FMUL + FFMA
-        flop_primary = qmode == sweep::MODE_OWNQ ? 15.0 : 1.0 + (qmode == sweep::MODE_QBAR ? 18.0 : 10.0) / d.R;
+        // shared q: per thread and triangle the set-up's 10 flops and one FADD2 (segment_pass), nothing per pair
+        flop_primary = qmode == sweep::MODE_OWNQ ? 15.0 : qmode == sweep::MODE_QBAR ? 1.0 + 18.0 / d.R : 12.0 / d.R;
         flop_primary_edges = qmode == sweep::MODE_OWNQ ? 12.0 : (qmode == sweep::MODE_QBAR ? 16.0 : 8.0) / d.R;
         if (int rc = launch_primary(d.R, o.exhaustive_strict != 0, qmode, p, grid, st)) return rc;
         trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(dc, bands, s->best, s->tri_verts, s->n_tris, s->spheres,

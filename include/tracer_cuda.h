@@ -164,10 +164,10 @@ typedef struct tracer_frame_stats {
     int32_t kernel_launches;
     int32_t n_sms;
     double flop_primary;    /* FP32 flops the closest-hit sweep executes per swept pair (FFMA = 2, FADD = FMUL = 1, a
-                               minimum 0).  Hot rows (no jitter: the R rays of a thread share q): per pair half a
-                               packed FADD2 (its three-input min is no flop), per thread and triangle 4 FFMA for the
-                               bounds and 2 FADD for the interval: 1 + 10/R.  Jittered samples with a shared mean q
-                               (8 FFMA): 1 + 18/R.  Three-row form (every ray its own q): 6 FFMA + FMUL + FFMA = 15.
+                               minimum 0).  Hot rows (no jitter: the R rays of a thread share q): per thread and
+                               triangle 4 FFMA for the bounds, 2 FADD for the interval and one packed FADD2 for the
+                               thread's extreme rays (segment verdict), nothing per pair: 12/R.  Jittered samples with
+                               a shared mean q (8 FFMA, and per pair half a packed FADD2): 1 + 18/R.  Three-row form (every ray its own q): 6 FFMA + FMUL + FFMA = 15.
                                0 in bundle-cull mode                                                              */
     double flop_shadow;     /* same for the any-hit sweeps (hot rows, R = 32 q-sorted rays share a mean q: 8 FFMA +
                                2 FADD per thread and triangle): 1 + 18/R                                          */

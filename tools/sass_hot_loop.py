@@ -1,5 +1,6 @@
 """SASS instruction counts of a sweep kernel's hot loops (profiles/r05_a): every straight-line block of the kernel that
-holds packed FADD2 (one per two ray-triangle pairs of the interval test), with its FP instruction counts per triangle.
+holds packed FADD2 (one per two ray-triangle pairs of the interval test, or one per triangle of the closest-hit sweep's
+segment verdict), with its instruction counts per triangle.
 
     cuobjdump -sass esctp1raytracer_b200/csrc/tracer_cuda.o | python tools/sass_hot_loop.py <mangled kernel name> [triangles per block]
 """
@@ -54,11 +55,17 @@ def main():
     for b in sorted(hot, key=lambda b: -sum(op == "FADD2" for op, _ in b)):
         c = collections.Counter(op for op, _ in b)
         fadd2 = c["FADD2"]
-        print("## hot-loop block at %s: %d instructions, %d FADD2 = %d rays per thread x %d triangles"
-              % (b[0][1].split("*/")[0] + "*/", len(b), fadd2, 2 * fadd2 // per, per))
+        if fadd2 == per and c["FMNMX3"] == 2 * per:  # segment verdict: one FADD2 per triangle, no per-pair work
+            print("## hot-loop block at %s: %d instructions, %d FADD2 = one per triangle (segment verdict) x %d triangles"
+                  % (b[0][1].split("*/")[0] + "*/", len(b), fadd2, per))
+        else:
+            print("## hot-loop block at %s: %d instructions, %d FADD2 = %d rays per thread x %d triangles"
+                  % (b[0][1].split("*/")[0] + "*/", len(b), fadd2, 2 * fadd2 // per, per))
         print("#  per triangle: " + ", ".join("%g %s" % (n / per, op) for op, n in sorted(c.items(), key=lambda x: -x[1])
-                                             if op.split(".")[0] in ("FFMA", "FADD", "FADD2", "FMNMX3", "FMNMX", "LDS", "FSETP")))
-        print("#  per FADD2 (two pairs): %g FMNMX3 besides the 2 per triangle of the set-up" % ((c["FMNMX3"] - 2 * per) / fadd2))
+                                             if op.split(".")[0] in ("FFMA", "FADD", "FADD2", "FMNMX3", "FMNMX", "LDS", "FSETP", "SEL",
+                                                                     "IADD3", "LOP3")))
+        if fadd2 != per:
+            print("#  per FADD2 (two pairs): %g FMNMX3 besides the 2 per triangle of the set-up" % ((c["FMNMX3"] - 2 * per) / fadd2))
     if hot:
         first = max(hot, key=lambda b: sum(op == "FADD2" for op, _ in b))
         print("## the widest block's first %d instructions (about one triangle)" % (len(first) // per))

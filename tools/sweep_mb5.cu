@@ -12,6 +12,9 @@
 // The FMNMX3 chain kernel times the three-input min alone, to find its issue cost and pipe.
 // F_HOT is the loop on the HOT rows the tables store now (csrc/sweep.cuh, hot_row): the +1s, the clamp and the margin
 // folded into the row, per thread and triangle 4 FFMA + 2 FMNMX3 + 2 FADD (8 FFMA with a mean q), the rays holding 2*S*p.
+// F_SEG is the segment verdict of the closest-hit sweep (csrc/sweep.cuh, segment_pass): the set-up of F_HOT, then one
+// FADD2 {pmin, pmax} + nc2 and the two-sided compare per thread and triangle, nothing per pair (round 7).  Its
+// "cyc/warp-tri" column is the loop's cost per (warp, triangle), whatever R.
 #include <cstdio>
 #include <cstdlib>
 #include <cuda_runtime.h>
@@ -19,7 +22,7 @@
 
 constexpr int TILE = 256, BATCH = 16;
 enum { MODE_SHAREDQ = 1, MODE_QBAR = 2 };
-enum { F_SPAN = 0, F_IV_FMA2 = 1, F_IV_ADD2 = 2, F_HOT = 3 };
+enum { F_SPAN = 0, F_IV_FMA2 = 1, F_IV_ADD2 = 2, F_HOT = 3, F_SEG = 4 };
 
 __device__ __forceinline__ float min3(float a, float b, float c) {
     float d;
@@ -64,7 +67,7 @@ __device__ __forceinline__ unsigned eval_span(const float4 *__restrict__ tp, con
 // the interval form: returns a bit per triangle; NCH independent min chains per triangle
 template <int R, int MODE, int FORM, int NCH>
 __device__ __forceinline__ unsigned eval_interval(const float4 *__restrict__ tp, const float (&rp)[R], const float (&ps)[R], float q, float qdelta,
-                                                  float S) {
+                                                  float S, float pmin, float pmax) {
     constexpr float P = 65536.f * 1.0625f + 1.f, DELTA = 8.f * 1.1920929e-7f * P;
     unsigned cand = 0;
 #pragma unroll
@@ -76,27 +79,34 @@ __device__ __forceinline__ unsigned eval_interval(const float4 *__restrict__ tp,
             b1 = fmaf(fabsf(hi.x), qdelta, b1), b2 = fmaf(fabsf(hi.z), qdelta, b2);
         }
         float nc, h;
-        if (FORM == F_HOT) { // (ps holds 2*S*p here)
+        if (FORM == F_HOT || FORM == F_SEG) { // (ps holds 2*S*p here)
             const float A = min3(a1, a2, P), B = min3(b1, b2, P);
             nc = A - B, h = A + B;
         } else {
             const float l = fmaxf(1.f - fminf(a1, a2), -P), u = fminf(fminf(b1, b2) - 1.f, P);
             nc = -0.5f * (l + u), h = fmaf(0.5f, u - l, DELTA);
         }
-        float m[NCH];
+        bool pass;
+        if constexpr (FORM == F_SEG) { // the thread's extreme rays only
+            const float2 e = __fadd2_rn(make_float2(pmin, pmax), make_float2(nc, nc));
+            pass = !(e.x > h) && !(-e.y > h);
+        } else {
+            float m[NCH];
 #pragma unroll
-        for (int j = 0; j < NCH; ++j) m[j] = __int_as_float(0x7f800000);
+            for (int j = 0; j < NCH; ++j) m[j] = __int_as_float(0x7f800000);
 #pragma unroll
-        for (int r = 0; r < R; r += 2) {
-            const float2 e = FORM == F_IV_FMA2 ? __ffma2_rn(make_float2(rp[r], rp[r + 1]), make_float2(S, S), make_float2(nc, nc))
-                                               : __fadd2_rn(make_float2(ps[r], ps[r + 1]), make_float2(nc, nc));
-            float &mm = m[(r / 2) % NCH];
-            mm = min3(mm, fabsf(e.x), fabsf(e.y));
+            for (int r = 0; r < R; r += 2) {
+                const float2 e = FORM == F_IV_FMA2 ? __ffma2_rn(make_float2(rp[r], rp[r + 1]), make_float2(S, S), make_float2(nc, nc))
+                                                   : __fadd2_rn(make_float2(ps[r], ps[r + 1]), make_float2(nc, nc));
+                float &mm = m[(r / 2) % NCH];
+                mm = min3(mm, fabsf(e.x), fabsf(e.y));
+            }
+            float mn = m[0];
+#pragma unroll
+            for (int j = 1; j < NCH; ++j) mn = fminf(mn, m[j]);
+            pass = mn <= h;
         }
-        float mn = m[0];
-#pragma unroll
-        for (int j = 1; j < NCH; ++j) mn = fminf(mn, m[j]);
-        cand |= (unsigned)(mn <= h) << k;
+        cand |= (unsigned)pass << k;
     }
     return cand;
 }
@@ -108,14 +118,17 @@ __global__ void __launch_bounds__(NTH, MINBLK) k_loop(const float4 *tile_g, int 
     __syncthreads();
     float rp[R], ps[R];
 #pragma unroll
-    for (int r = 0; r < R; ++r) rp[r] = seed * (threadIdx.x + 1) * (r + 1), ps[r] = rp[r] * (FORM == F_HOT ? 2.f * S : S);
+    for (int r = 0; r < R; ++r) rp[r] = seed * (threadIdx.x + 1) * (r + 1), ps[r] = rp[r] * (FORM >= F_HOT ? 2.f * S : S);
+    float pmin = ps[0], pmax = ps[0];
+#pragma unroll
+    for (int r = 1; r < R; ++r) pmin = fminf(pmin, ps[r]), pmax = fmaxf(pmax, ps[r]);
     const float q = seed * (threadIdx.x + 7) * 3, qdelta = 1e-6f * (1 + (threadIdx.x & 3));
     int hits = 0;
     for (int rep = 0; rep < reps; ++rep) {
 #pragma unroll 1
         for (int b0 = 0; b0 < TILE; b0 += BATCH) {
             const unsigned c = FORM == F_SPAN ? eval_span<R, MODE, GROUP, NACC2>(tile + 2 * b0, ps, q, qdelta)
-                                              : eval_interval<R, MODE, FORM, NACC2>(tile + 2 * b0, rp, ps, q, qdelta, S);
+                                              : eval_interval<R, MODE, FORM, NACC2>(tile + 2 * b0, rp, ps, q, qdelta, S, pmin, pmax);
             if (c) {
                 hits += 1;
                 asm volatile("" ::: "memory");
@@ -229,6 +242,14 @@ int main() {
     LOOP(64, MODE_SHAREDQ, F_IV_ADD2, 128, 2, 1, 1);
     LOOP(64, MODE_SHAREDQ, F_HOT, 128, 2, 1, 1);
     LOOP(64, MODE_SHAREDQ, F_HOT, 128, 3, 1, 1);
+    printf("-- shared q: segment verdict (closest hit, round 7) against the hot loop, R = 32 and 64, 2 and 3 CTAs/SM\n");
+    LOOP(32, MODE_SHAREDQ, F_HOT, 128, 2, 1, 1);
+    LOOP(32, MODE_SHAREDQ, F_SEG, 128, 2, 1, 1);
+    LOOP(32, MODE_SHAREDQ, F_HOT, 128, 3, 1, 1);
+    LOOP(32, MODE_SHAREDQ, F_SEG, 128, 3, 1, 1);
+    LOOP(32, MODE_SHAREDQ, F_SEG, 128, 4, 1, 1);
+    LOOP(64, MODE_SHAREDQ, F_SEG, 128, 2, 1, 1);
+    LOOP(64, MODE_SHAREDQ, F_SEG, 128, 3, 1, 1);
     printf("-- any-hit (qbar + |B| qdelta): span loop vs interval form\n");
     LOOP(16, MODE_QBAR, F_SPAN, 128, 4, 4, 4);
     LOOP(16, MODE_QBAR, F_IV_FMA2, 128, 4, 1, 1);
