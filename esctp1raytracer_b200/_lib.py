@@ -20,6 +20,7 @@ ABI_SYMBOLS = [
     "tracer_mt19937_faceids", "tracer_cuda_fp32_peak", "tracer_camera_lookat",
     "tracer_cuda_init_multi", "tracer_cuda_multi_gpu_count", "tracer_cuda_render_multi", "tracer_cuda_scene_create_multi",
     "tracer_cuda_scene_destroy_multi", "tracer_cuda_render_scene_multi", "tracer_cuda_last_stats_multi",
+    "tracer_cuda_scene_update", "tracer_cuda_scene_update_multi",
 ]
 # include/tracer_host.h
 HOST_SYMBOLS = ["tracer_scene_load_obj", "tracer_scene_host_flat", "tracer_scene_host_free", "tracer_host_last_error",
@@ -58,6 +59,15 @@ class RenderOpts(C.Structure):
         ("out_tri", C.POINTER(C.c_int32)), ("out_t", C.POINTER(C.c_float)), ("out_v", C.POINTER(C.c_float)),
         ("out_occ_tri", C.POINTER(C.c_int32)), ("out_rgb", C.POINTER(C.c_float)), ("accel", C.c_int32),
         ("row_hits_exchange", ROW_HITS_EXCHANGE), ("row_hits_user", C.c_void_p),
+    ]
+
+
+class SceneUpdate(C.Structure):
+    """tracer_scene_update; the array pointers are plain addresses (host or device, per data_is_device)"""
+    _fields_ = [
+        ("struct_size", C.c_uint32), ("data_is_device", C.c_int32), ("cuda_stream", C.c_void_p),
+        ("tri_first", C.c_int32), ("tri_count", C.c_int32), ("tri_verts", C.c_void_p), ("tri_normals", C.c_void_p),
+        ("geom_material", C.c_void_p), ("sphere_cr", C.c_void_p), ("sphere_material", C.c_void_p),
     ]
 
 
@@ -113,6 +123,8 @@ def load():
     lib.tracer_cuda_render_multi.argtypes = [C.POINTER(SceneFlat), C.POINTER(CameraC), C.c_int32, C.c_int32,
                                              C.POINTER(RenderOpts), C.c_void_p]
     lib.tracer_cuda_last_stats_multi.argtypes = [C.c_void_p, C.POINTER(FrameStats)]
+    lib.tracer_cuda_scene_update.argtypes = [C.c_void_p, C.POINTER(SceneUpdate)]
+    lib.tracer_cuda_scene_update_multi.argtypes = [C.c_void_p, C.POINTER(SceneUpdate)]
     lib.tracer_band_row_count.argtypes = [C.c_int32] * 4
     lib.tracer_band_row_count.restype = C.c_int32
     lib.tracer_cuda_assemble_bands.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,

@@ -202,6 +202,95 @@ class Frame:
     rgb: np.ndarray | None = None
 
 
+_UPDATE_ROW = dict(tri_verts=9, tri_normals=9, geom_material=13, sphere_cr=4, sphere_material=13)
+
+
+def _update_rows(name, shape, row):
+    """rows of an update array: shape [n, row] (triangles also [n, 3, 3]) or flat [n * row]"""
+    size = int(np.prod(shape)) if len(shape) else -1
+    if size < 0 or size % row or (len(shape) > 1 and int(np.prod(shape[1:])) != row):
+        raise ValueError(f"{name}: shape {tuple(shape)} is not [n, {row}]")
+    return size // row
+
+
+def _update_array(name, a):
+    """(address, rows, on the device, interface stream or None, object to keep alive) of one update argument.  A host array
+    is converted like Scene's arrays (C-contiguous float32); an object with __cuda_array_interface__ is read in place, so
+    it must already be float32 and C-contiguous."""
+    row = _UPDATE_ROW[name]
+    cai = getattr(a, "__cuda_array_interface__", None)
+    if cai is None:
+        h = np.ascontiguousarray(a, np.float32)
+        return h.ctypes.data, _update_rows(name, h.shape, row), False, None, h
+    shape = tuple(int(x) for x in cai["shape"])
+    if np.dtype(cai["typestr"]) != np.dtype(np.float32):
+        raise ValueError(f"{name}: device arrays must be float32, not {cai['typestr']}")
+    strides = cai.get("strides")
+    if strides is not None:
+        want = [4 * int(np.prod(shape[i + 1:])) for i in range(len(shape))]
+        if any(n > 1 and int(s) != w for n, s, w in zip(shape, strides, want)):
+            raise ValueError(f"{name}: device arrays must be C-contiguous (strides {tuple(strides)})")
+    return int(cai["data"][0]), _update_rows(name, shape, row), True, cai.get("stream"), a
+
+
+def _scene_update(scene: Scene, *, tri_verts=None, first_tri=0, tri_normals=None, geom_material=None, sphere_cr=None,
+                  sphere_material=None, stream=None):
+    """The tracer_scene_update of an update() call and the objects it points into.  Needs no device: every check that can
+    be made from shapes and types is made here; the library checks the range and, for device arrays, the pointers."""
+    u = _lib.SceneUpdate()
+    u.struct_size = C.sizeof(_lib.SceneUpdate)
+    given = dict(tri_verts=tri_verts, tri_normals=tri_normals, geom_material=geom_material, sphere_cr=sphere_cr,
+                 sphere_material=sphere_material)
+    keep, rows, on_device, streams = [], {}, set(), set()
+    for name, a in given.items():
+        if a is None:
+            continue
+        ptr, rows[name], dev, st, k = _update_array(name, a)
+        keep.append(k)
+        on_device.add(dev)
+        if st is not None:
+            streams.add(int(st))
+        setattr(u, name, ptr or None)
+    if len(on_device) > 1:
+        raise ValueError("an update takes host arrays or device arrays, not both")
+    n_tri = {rows[k] for k in ("tri_verts", "tri_normals") if k in rows}
+    if len(n_tri) > 1:
+        raise ValueError("tri_verts and tri_normals cover different numbers of triangles")
+    n_sph = len(scene.sphere_cr)
+    for name, want in (("geom_material", scene.n_geoms), ("sphere_cr", n_sph), ("sphere_material", n_sph)):
+        if name in rows and rows[name] != want:
+            raise ValueError(f"{name}: {rows[name]} rows, the scene has {want}")
+    if not -2 ** 31 <= int(first_tri) < 2 ** 31:
+        raise ValueError("first_tri out of range")
+    u.tri_first, u.tri_count = int(first_tri), (n_tri.pop() if n_tri else 0)
+    u.data_is_device = int(on_device == {True})
+    if stream is not None:
+        u.cuda_stream = int(stream)
+    elif u.data_is_device:
+        if len(streams) > 1:
+            raise ValueError("device arrays name different streams: pass stream=")
+        # no stream in the interface (torch's has none): the legacy default stream, behind work queued on it
+        u.cuda_stream = streams.pop() if streams else 1
+    return u, keep
+
+
+_UPDATE_DOC = """Replace vertices, normals, materials or spheres in place (tracer_cuda_scene_update{multi}); topology stays.
+
+        ``tri_verts`` / ``tri_normals``: [n, 3, 3] for triangles ``[first_tri, first_tri + n)`` (normals only for a scene
+        created with them); ``geom_material`` [n_geoms, 13]; ``sphere_cr`` [n_spheres, 4]; ``sphere_material``
+        [n_spheres, 13].  Each is a host array (converted to float32) or an object with ``__cuda_array_interface__`` such
+        as a torch CUDA tensor on {device} (float32, C-contiguous, read in place); one call takes one kind.  The copies
+        run on ``stream`` (a cudaStream_t handle), else on the interface's ``stream`` entry, else, for device arrays, on
+        the legacy default stream, so data written there first is ordered before them; a tensor written on another
+        stream needs that stream here.  The call returns when the update is complete on the device.  The next frame is
+        the frame a fresh upload of the updated arrays gives, bit for bit.
+
+        ``self.scene`` keeps describing the topology, which is all ``trace`` reads from it: its arrays are those of the
+        upload and are not kept in sync with updates.  Raises ValueError for a wrong shape or dtype, a non-contiguous
+        device array or host and device arrays mixed; TracerError when the library refuses the update (range outside
+        the scene, normals for a scene without them, a pointer not on {device}), which leaves the scene unchanged."""
+
+
 class ResidentScene:
     """A scene uploaded to HBM (tracer_cuda_scene_create)."""
 
@@ -211,6 +300,16 @@ class ResidentScene:
         self.handle = C.c_void_p()
         cs = scene.c_struct()
         _lib.check(renderer.lib.tracer_cuda_scene_create(C.byref(cs), C.byref(self.handle)))
+
+    def update(self, *, tri_verts=None, first_tri=0, tri_normals=None, geom_material=None, sphere_cr=None,
+               sphere_material=None, stream=None):
+        # keep: the arrays u points into, alive for the call
+        u, keep = _scene_update(self.scene, tri_verts=tri_verts, first_tri=first_tri, tri_normals=tri_normals,
+                                geom_material=geom_material, sphere_cr=sphere_cr, sphere_material=sphere_material,
+                                stream=stream)  # noqa: F841
+        _lib.check(self.renderer.lib.tracer_cuda_scene_update(self.handle, C.byref(u)))
+
+    update.__doc__ = _UPDATE_DOC.format(multi="", device="the scene's GPU")
 
     def close(self):
         if self.handle:
@@ -274,6 +373,17 @@ class MultiRenderer:
 class _MultiScene:
     def __init__(self, renderer, scene, handle):
         self.renderer, self.scene, self.handle = renderer, scene, handle
+
+    def update(self, *, tri_verts=None, first_tri=0, tri_normals=None, geom_material=None, sphere_cr=None,
+               sphere_material=None, stream=None):
+        # keep: the arrays u points into, alive for the call
+        u, keep = _scene_update(self.scene, tri_verts=tri_verts, first_tri=first_tri, tri_normals=tri_normals,
+                                geom_material=geom_material, sphere_cr=sphere_cr, sphere_material=sphere_material,
+                                stream=stream)  # noqa: F841
+        _lib.check(self.renderer.lib.tracer_cuda_scene_update_multi(self.handle, C.byref(u)))
+
+    update.__doc__ = _UPDATE_DOC.format(multi="_multi", device="GPU 0") + """  Every replica is updated; a refused
+        update changes none."""
 
     def close(self):
         if self.handle:

@@ -1,6 +1,7 @@
 // tracer_cuda.cu — C ABI (include/tracer_cuda.h) over the sm_100a kernels.
 // No CPU fallback: every compute entry point needs a CUDA device.
 #include <algorithm>
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -287,9 +288,10 @@ struct tracer_scene_dev {
     float4 *spheres = nullptr;
     int *light_vbase = nullptr;
     float *light_verts = nullptr;
-    std::vector<int> h_light_vbase, h_light_F;
+    std::vector<int> h_light_vbase, h_light_F, h_light_t0; // per light: first light vertex, faces, first triangle
     std::vector<float> h_light_verts;
     double bb_lo[3], bb_hi[3];
+    void *box_work = nullptr; // bbox_partial_kernel's per-block bounds, then the 6 doubles of the box
     float4 *eye_table = nullptr, *light_tables = nullptr, *allcand_table = nullptr; // 48-byte three-row tables
     float4 *eye_span = nullptr, *light_spans = nullptr, *allcand_span = nullptr;    // 32-byte span tables (same slots)
     std::vector<double> table_lmax; // per (light vertex, cube face): reach bound it was built for, < 0 = not built
@@ -528,12 +530,77 @@ Decomp pick_decomp(int64_t n_rays, int n_tiles, int n_sms, int forced_R, int ext
 }
 
 // both forms of the filter table of one origin: the 48-byte rows (jittered primary rays, bundle-cull mode) and the
-// 32-byte span rows (default sweeps)
-int build_table(const tracer_scene_dev *s, const trk::TableParam &tp, float4 *table, float4 *span, cudaStream_t st) {
+// 32-byte span rows (default sweeps).  count >= 0: only the rows of triangles [first, first + count) (a scene update; a
+// row depends on tp and its own triangle only, so they equal those of a full build); the padding rows are left alone.
+int build_table(const tracer_scene_dev *s, const trk::TableParam &tp, float4 *table, float4 *span, cudaStream_t st, int first = 0,
+                int count = -1) {
     const int th = 128;
-    trk::build_origin_table<<<(s->n_pad + th - 1) / th, th, 0, st>>>(s->tri_verts, s->n_tris, s->n_pad, tp, table, span);
+    const int n_tris = count < 0 ? s->n_tris : count, n_pad = count < 0 ? s->n_pad : count;
+    if (n_pad == 0) return 0;
+    trk::build_origin_table<<<(n_pad + th - 1) / th, th, 0, st>>>(s->tri_verts + 9 * (size_t)first, n_tris, n_pad, tp,
+                                                                  table + 3 * (size_t)first, span + 2 * (size_t)first);
     CK_CUDA(cudaGetLastError());
     return 0;
+}
+
+// ---- the scene's bounding box, on the device --------------------------------------------------------------------------------
+// What the host loop over the flat arrays gave: in order, every triangle vertex (double)x, then every sphere's x -/+ |r| in
+// double, folded with lo = std::min(lo, x), hi = std::max(hi, x) from (1e300, -1e300).  A NaN never replaces a bound (it
+// fails every comparison) and infinities count.  A parallel fold gives the same bits when each bound carries the ordinal of
+// the item that set it and, between equal values (only -0.0 and +0.0 differ in their bits), the lower ordinal wins: the
+// sequential loop keeps the first of equal values.
+struct BoxArg {
+    double v;
+    long long i; // ordinal: vertex k -> k, sphere j -> 3 n_tris + j
+};
+constexpr int BOX_THREADS = 256, BOX_MAX_BLOCKS = 1024;
+__device__ __forceinline__ void box_take(BoxArg &a, double v, long long i, bool upper) {
+    if ((upper ? v > a.v : v < a.v) || (v == a.v && i < a.i)) a.v = v, a.i = i;
+}
+// b = 0..2: lo x y z, 3..5: hi x y z; folds the block's threads into a[*] of thread 0
+__device__ void box_block_fold(BoxArg (&a)[6]) {
+    __shared__ BoxArg sh[6][BOX_THREADS];
+    for (int b = 0; b < 6; ++b) sh[b][threadIdx.x] = a[b];
+    __syncthreads();
+    for (int w = BOX_THREADS / 2; w > 0; w >>= 1) {
+        if ((int)threadIdx.x < w)
+            for (int b = 0; b < 6; ++b) {
+                const BoxArg o = sh[b][threadIdx.x + w];
+                box_take(sh[b][threadIdx.x], o.v, o.i, b >= 3);
+            }
+        __syncthreads();
+    }
+    for (int b = 0; b < 6; ++b) a[b] = sh[b][0];
+}
+__global__ void __launch_bounds__(BOX_THREADS) bbox_partial_kernel(const float *__restrict__ verts, long long n_verts,
+                                                                   const float4 *__restrict__ spheres, int n_spheres, BoxArg *partial) {
+    BoxArg a[6];
+    for (int b = 0; b < 6; ++b) a[b] = BoxArg{b < 3 ? 1e300 : -1e300, LLONG_MAX};
+    const long long n = n_verts + n_spheres, stride = (long long)gridDim.x * BOX_THREADS;
+    for (long long k = blockIdx.x * (long long)BOX_THREADS + threadIdx.x; k < n; k += stride) {
+        if (k < n_verts) {
+            for (int c = 0; c < 3; ++c) {
+                const double x = verts[3 * k + c];
+                box_take(a[c], x, k, false), box_take(a[3 + c], x, k, true);
+            }
+        } else {
+            const float4 sp = spheres[k - n_verts];
+            const double r = fabs((double)sp.w), xs[3] = {sp.x, sp.y, sp.z};
+            for (int c = 0; c < 3; ++c) box_take(a[c], xs[c] - r, k, false), box_take(a[3 + c], xs[c] + r, k, true);
+        }
+    }
+    box_block_fold(a);
+    if (threadIdx.x == 0)
+        for (int b = 0; b < 6; ++b) partial[6 * (size_t)blockIdx.x + b] = a[b];
+}
+__global__ void __launch_bounds__(BOX_THREADS) bbox_final_kernel(const BoxArg *__restrict__ partial, int n_blocks, double *out6) {
+    BoxArg a[6];
+    for (int b = 0; b < 6; ++b) a[b] = BoxArg{b < 3 ? 1e300 : -1e300, LLONG_MAX};
+    for (int k = threadIdx.x; k < n_blocks; k += BOX_THREADS)
+        for (int b = 0; b < 6; ++b) box_take(a[b], partial[6 * (size_t)k + b].v, partial[6 * (size_t)k + b].i, b >= 3);
+    box_block_fold(a);
+    if (threadIdx.x == 0)
+        for (int b = 0; b < 6; ++b) out6[b] = a[b].v;
 }
 
 // The BVH of the optional mode (bvh.cuh), on stream st: prep (boxes, sigma, bounds) -> Morton keys -> radix sort ->
@@ -611,6 +678,25 @@ trk::TableParam face_param(const float *o, int f, double lmax) {
     tp.dmax = std::sqrt(3.0);
     tp.lmax = lmax;
     return tp;
+}
+
+// s->bb_lo, s->bb_hi from the scene's device arrays (bbox_partial_kernel): two launches on st, one read-back, a synchronise
+int scene_bbox(tracer_scene_dev *s, cudaStream_t st) {
+    if (!s->box_work && !(s->box_work = t_pool->alloc(sizeof(BoxArg) * 6 * BOX_MAX_BLOCKS + sizeof(double) * 6)))
+        return fail(TRACER_ERR_NOMEM, "bounding-box scratch");
+    BoxArg *partial = (BoxArg *)s->box_work;
+    double *out6 = (double *)(partial + 6 * BOX_MAX_BLOCKS);
+    const long long n_verts = 3 * (long long)s->n_tris, n = n_verts + s->n_spheres;
+    const int blocks = (int)std::max(1LL, std::min<long long>(BOX_MAX_BLOCKS, (n + BOX_THREADS - 1) / BOX_THREADS));
+    bbox_partial_kernel<<<blocks, BOX_THREADS, 0, st>>>(s->tri_verts, n_verts, s->spheres, s->n_spheres, partial);
+    CK_CUDA(cudaGetLastError());
+    bbox_final_kernel<<<1, BOX_THREADS, 0, st>>>(partial, blocks, out6);
+    CK_CUDA(cudaGetLastError());
+    double box[6];
+    CK_CUDA(cudaMemcpyAsync(box, out6, sizeof box, cudaMemcpyDeviceToHost, st));
+    CK_CUDA(cudaStreamSynchronize(st));
+    for (int c = 0; c < 3; ++c) s->bb_lo[c] = box[c], s->bb_hi[c] = box[3 + c];
+    return 0;
 }
 
 }  // namespace
@@ -741,6 +827,7 @@ void tracer_cuda_scene_destroy(tracer_scene_dev *s) {
     t_pool->release(s->sort_tmp), t_pool->release(s->pair_tmp);
     dev_free(s->counters);
     dev_free(s->bvh_nodes), dev_free(s->bvh_keys);
+    t_pool->release(s->box_work);
     s->mt.release();
     for (auto &e : s->ev)
         if (e) cudaEventDestroy(e);
@@ -821,18 +908,8 @@ int scene_create_on(Ctx &g, const tracer_scene_flat *sc, tracer_scene_dev **out)
         TRY_CUDA(cudaMemcpy(s->sphere_material, sc->sphere_material, (size_t)sc->n_spheres * 13 * sizeof(float),
                             cudaMemcpyHostToDevice));
     }
-    // bounding box of everything a ray can start from or end at
-    for (int c = 0; c < 3; ++c) s->bb_lo[c] = 1e300, s->bb_hi[c] = -1e300;
-    for (size_t i = 0; i < (size_t)N * 3; ++i)
-        for (int c = 0; c < 3; ++c) {
-            const double x = sc->tri_verts[3 * i + c];
-            s->bb_lo[c] = std::min(s->bb_lo[c], x), s->bb_hi[c] = std::max(s->bb_hi[c], x);
-        }
-    for (int i = 0; i < sc->n_spheres; ++i)
-        for (int c = 0; c < 3; ++c) {
-            const double x = sc->sphere_cr[4 * i + c], r = std::fabs(sc->sphere_cr[4 * i + 3]);
-            s->bb_lo[c] = std::min(s->bb_lo[c], x - r), s->bb_hi[c] = std::max(s->bb_hi[c], x + r);
-        }
+    // bounding box of everything a ray can start from or end at, from the uploaded arrays (the kernel an update uses too)
+    TRY(scene_bbox(s, g.stream));
     // lights: light.vertex[faceID], faceID in [0, F) (main.cpp:743-751) = the first F de-indexed vertices
     s->h_light_vbase.assign(1, 0);
     for (int l = 0; l < sc->n_lights; ++l) {
@@ -847,6 +924,7 @@ int scene_create_on(Ctx &g, const tracer_scene_flat *sc, tracer_scene_dev **out)
             return fail(TRACER_ERR_INVALID, "light geometry has no faces");
         }
         s->h_light_F.push_back(F);
+        s->h_light_t0.push_back(t0);
         for (int f = 0; f < F; ++f)
             for (int c = 0; c < 3; ++c) s->h_light_verts.push_back(sc->tri_verts[9 * (size_t)t0 + 3 * (size_t)f + c]);
         s->h_light_vbase.push_back(s->h_light_vbase.back() + F);
@@ -1607,6 +1685,101 @@ int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32
                 hc.cull_tiles_any, hc.cull_tiles_fallback, hc.cull_l1, (unsigned long long)(hc.tests_shadow / 4096 / cull::CTILE));
     return TRACER_OK;
 }
+// ---- scene updates (tracer_cuda_scene_update) -----------------------------------------------------------------------------
+// The checks of one replica that need no device: the struct, the triangle range, data for a count, normals
+int update_check(const tracer_scene_dev *s, const tracer_scene_update *u) {
+    if (!s || !u) return fail(TRACER_ERR_INVALID, "null argument");
+    if (u->struct_size < sizeof(tracer_scene_update)) return fail(TRACER_ERR_INVALID, "tracer_scene_update.struct_size too small");
+    if (!s->ctx || !s->ctx->inited) return fail(TRACER_ERR_NO_DEVICE, "tracer_cuda_init not called");
+    if (u->tri_first < 0 || u->tri_count < 0 || (int64_t)u->tri_first + u->tri_count > s->n_tris)
+        return fail(TRACER_ERR_INVALID, "triangle range [" + std::to_string(u->tri_first) + ", +" + std::to_string(u->tri_count) +
+                                            ") outside the scene's " + std::to_string(s->n_tris) + " triangles");
+    if (u->tri_count > 0 && !u->tri_verts && !u->tri_normals) return fail(TRACER_ERR_INVALID, "tri_count > 0 needs tri_verts or tri_normals");
+    if (u->tri_normals && !s->tri_normals) return fail(TRACER_ERR_INVALID, "tri_normals given for a scene created without normals");
+    return 0;
+}
+// data_is_device: every pointer the update reads is device or managed memory of GPU `device`
+int update_check_pointers(const tracer_scene_dev *s, const tracer_scene_update *u, int device) {
+    if (!u->data_is_device) return 0;
+    const struct {
+        const void *p;
+        bool read;
+        const char *name;
+    } args[] = {{u->tri_verts, u->tri_count > 0, "tri_verts"},          {u->tri_normals, u->tri_count > 0, "tri_normals"},
+                {u->geom_material, s->n_geoms > 0, "geom_material"},    {u->sphere_cr, s->n_spheres > 0, "sphere_cr"},
+                {u->sphere_material, s->n_spheres > 0, "sphere_material"}};
+    for (const auto &a : args) {
+        if (!a.p || !a.read) continue;
+        cudaPointerAttributes at{};
+        const cudaError_t e = cudaPointerGetAttributes(&at, a.p);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            return fail(TRACER_ERR_INVALID, std::string(a.name) + ": not a CUDA pointer (" + cudaGetErrorString(e) + ")");
+        }
+        if ((at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != device)
+            return fail(TRACER_ERR_INVALID, std::string(a.name) + ": data_is_device, but not device memory of GPU " + std::to_string(device));
+    }
+    return 0;
+}
+bool update_is_noop(const tracer_scene_update *u) {
+    return u->tri_count == 0 && !u->tri_verts && !u->tri_normals && !u->geom_material && !u->sphere_cr && !u->sphere_material;
+}
+
+// The device work of a checked update on one replica, on stream st.  src_device: the GPU the data lives on, -1 = host.
+// 1. copies; 2. the box (vertices or spheres changed); 3. the light vertices, compared bit for bit with the old ones;
+// 4. resident shadow tables: a moved light vertex's six are dropped (table_lmax = -1, rebuilt lazily by the next render as
+// on a fresh scene), every other built table gets rows [tri_first, +tri_count) again, from the TableParam it was built
+// with; 5. the BVH is marked stale.  Ends with a synchronise of st.
+int update_apply(tracer_scene_dev *s, const tracer_scene_update &u, int src_device, cudaStream_t st) {
+    Ctx &g = *s->ctx;
+    t_pool = &g.pool;
+    CK_CUDA(cudaSetDevice(g.device));
+    auto copy = [&](void *dst, const void *src, size_t bytes) -> int {
+        if (!src || !bytes) return 0;
+        if (src_device >= 0 && src_device != g.device) CK_CUDA(cudaMemcpyPeerAsync(dst, g.device, src, src_device, bytes, st));
+        else CK_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDefault, st));
+        return 0;
+    };
+    const size_t tri_bytes = (size_t)u.tri_count * 9 * sizeof(float), tri0 = 9 * (size_t)u.tri_first;
+    const bool verts = u.tri_verts && u.tri_count > 0, spheres = u.sphere_cr && s->n_spheres > 0;
+    int rc = copy(s->tri_verts + tri0, u.tri_verts, tri_bytes);
+    if (!rc && u.tri_normals) rc = copy(s->tri_normals + tri0, u.tri_normals, tri_bytes);
+    if (!rc) rc = copy(s->geom_material, u.geom_material, (size_t)s->n_geoms * 13 * sizeof(float));
+    if (!rc) rc = copy(s->spheres, u.sphere_cr, (size_t)s->n_spheres * sizeof(float4));
+    if (!rc) rc = copy(s->sphere_material, u.sphere_material, (size_t)s->n_spheres * 13 * sizeof(float));
+    if (rc) return rc;
+    if (verts || spheres) {
+        if (int r = scene_bbox(s, st)) return r;
+    }
+    if (verts) {
+        if (s->V > 0) { // light l's vertices are the first 3 F floats of its geometry's triangles
+            for (int l = 0; l < s->n_lights; ++l)
+                CK_CUDA(cudaMemcpyAsync(s->light_verts + 3 * (size_t)s->h_light_vbase[l], s->tri_verts + 9 * (size_t)s->h_light_t0[l],
+                                        3 * (size_t)s->h_light_F[l] * sizeof(float), cudaMemcpyDeviceToDevice, st));
+            const std::vector<float> old = s->h_light_verts;
+            CK_CUDA(cudaMemcpyAsync(s->h_light_verts.data(), s->light_verts, old.size() * sizeof(float), cudaMemcpyDeviceToHost, st));
+            CK_CUDA(cudaStreamSynchronize(st));
+            for (int v = 0; s->tables_resident && v < s->V; ++v) {
+                const bool moved = std::memcmp(&old[3 * (size_t)v], &s->h_light_verts[3 * (size_t)v], 3 * sizeof(float)) != 0;
+                for (int face = 0; face < 6; ++face) {
+                    double &built = s->table_lmax[(size_t)v * 6 + face];
+                    if (built < 0) continue;
+                    if (moved) {
+                        built = -1.0;
+                        continue;
+                    }
+                    const trk::TableParam tp = face_param(&s->h_light_verts[3 * (size_t)v], face, built);
+                    if (int r = build_table(s, tp, s->light_tables + ((size_t)v * 6 + face) * s->table_stride,
+                                            s->light_spans + ((size_t)v * 6 + face) * s->span_stride, st, u.tri_first, u.tri_count))
+                        return r;
+                }
+            }
+        }
+        s->bvh_built = false; // rebuilt by the next BVH render (ensure_bvh)
+    }
+    CK_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
 }  // namespace
 
 extern "C" {
@@ -1614,6 +1787,21 @@ extern "C" {
 int tracer_cuda_last_stats(tracer_scene_dev *s, tracer_frame_stats *out) {
     if (!s || !out) return fail(TRACER_ERR_INVALID, "null argument");
     *out = s->stats;
+    return TRACER_OK;
+}
+
+int tracer_cuda_scene_update(tracer_scene_dev *s, const tracer_scene_update *u) {
+    if (int rc = update_check(s, u)) return rc;
+    CK_CUDA(cudaSetDevice(s->ctx->device));
+    if (int rc = update_check_pointers(s, u, s->ctx->device)) return rc;
+    if (update_is_noop(u)) return TRACER_OK;
+    return update_apply(s, *u, u->data_is_device ? s->ctx->device : -1, u->cuda_stream ? (cudaStream_t)u->cuda_stream : s->ctx->stream);
+}
+
+// Internal (tests only): the scene's bounding box as the render uses it, lo xyz then hi xyz
+int tracer__scene_bbox(tracer_scene_dev *s, double *out6) {
+    if (!s || !out6) return fail(TRACER_ERR_INVALID, "null argument");
+    for (int c = 0; c < 3; ++c) out6[c] = s->bb_lo[c], out6[3 + c] = s->bb_hi[c];
     return TRACER_OK;
 }
 
@@ -1979,6 +2167,25 @@ int tracer_cuda_render_scene_multi(tracer_scene_multi *ms, const tracer_camera *
 int tracer_cuda_last_stats_multi(tracer_scene_multi *ms, tracer_frame_stats *out) {
     if (!ms || !out) return fail(TRACER_ERR_INVALID, "null argument");
     *out = ms->stats;
+    return TRACER_OK;
+}
+
+// Every replica is checked before any changes; then they are updated one after the other.  Replica 0 goes first, on
+// cuda_stream, and its update ends with a synchronise of that stream: device data produced on it is complete before the
+// other replicas' peer copies from device 0 start on their own streams.
+int tracer_cuda_scene_update_multi(tracer_scene_multi *ms, const tracer_scene_update *u) {
+    if (!ms || !u) return fail(TRACER_ERR_INVALID, "null argument");
+    const int n = (int)ms->dev.size();
+    if (n != g_multi.n || n < 1) return fail(TRACER_ERR_STATE, "scene was created for a different GPU set");
+    for (int d = 0; d < n; ++d)
+        if (int rc = update_check(ms->dev[d], u)) return rc;
+    CK_CUDA(cudaSetDevice(0));
+    if (int rc = update_check_pointers(ms->dev[0], u, 0)) return rc;
+    if (update_is_noop(u)) return TRACER_OK;
+    for (int d = 0; d < n; ++d) {
+        const cudaStream_t st = d == 0 && u->cuda_stream ? (cudaStream_t)u->cuda_stream : g_ctx[d].stream;
+        if (int rc = update_apply(ms->dev[d], *u, u->data_is_device ? 0 : -1, st)) return fail(rc, "GPU " + std::to_string(d) + ": " + g_err);
+    }
     return TRACER_OK;
 }
 

@@ -76,7 +76,8 @@ def row_hits_all_reduce(group=None):
 def render_frame(renderer, resident_scene, camera, width, height, *, rank=0, world=1, band_rows=DEFAULT_BAND_ROWS,
                  rng_mode=0, seed=1, group=None, bundle_cull=False, samples_per_pixel=0, bvh=False):
     """Render this rank's bands into HBM, gather to rank 0, assemble.  Returns
-    (frame uint8 CUDA tensor [H, W, 3] on rank 0 else None, per-rank stats dict)."""
+    (frame uint8 CUDA tensor [H, W, 3] on rank 0 else None, per-rank stats dict).  To move geometry between frames,
+    every rank calls ``resident_scene.update(...)`` on its own scene with the same arrays before this call."""
     import torch
 
     rows_pad = padded_rows(height, band_rows, world) if world > 1 else height

@@ -129,7 +129,8 @@ typedef struct tracer_render_opts {
     float *out_rgb;       /* [n_px*3] float accumulator before quantisation */
 
     int32_t accel;        /* OPTIONAL mode: 0 = the modes above; 1 = BVH: a linear BVH over the triangles (built on the
-                             device on the first BVH render of a scene, kept until the scene is destroyed) with a
+                             device on the first BVH render of a scene, kept until the scene is destroyed or an
+                             update moves vertices, tracer_cuda_scene_update) with a
                              conservative traversal in front of the reference's own test; identical results.  Not
                              combinable with bundle_cull or exhaustive_strict (TRACER_ERR_INVALID); rays_per_thread and
                              shadow_chunks are ignored.  In this mode tests_primary / tests_shadow = strict_evals = the
@@ -211,6 +212,39 @@ int tracer_cuda_render_scene(tracer_scene_dev *scene, const tracer_camera *cam, 
                              const tracer_render_opts *opts, uint8_t *rgb_out);
 int tracer_cuda_last_stats(tracer_scene_dev *scene, tracer_frame_stats *out);
 
+/* ---- updating a resident scene between frames --------------------------------
+ * Replaces vertices, normals, materials and spheres of a resident scene in place, without re-creating it.
+ * Topology is fixed: the triangle, geometry, light and sphere counts, geom_tri_offset, light_geom and
+ * geom_has_normals stay those of the create call (changing any of them means creating a new scene), and
+ * triangle order stays the reference's iteration order.  A frame rendered after an update is the frame a
+ * freshly created scene of the updated arrays gives, in every mode, rng_mode and band selection, packed bytes
+ * and every debug output alike.
+ * The library refreshes what depends on the geometry: the scene's bounding box (on the device), the light
+ * vertices, the rows [tri_first, tri_first + tri_count) of every resident shadow filter table (tables of a
+ * light vertex that moved are dropped and rebuilt by the next render that needs them) and, when vertices
+ * changed, the BVH of the optional mode (rebuilt by the next BVH render).
+ * Every check runs before anything is copied: a NULL pointer where tri_count needs data, a range outside
+ * [0, n_tris], struct_size < sizeof(tracer_scene_update), tri_normals for a scene created without normals, and
+ * with data_is_device a pointer that is not device or managed memory of the scene's GPU (multi: device 0).
+ * A refused update returns TRACER_ERR_INVALID and leaves the scene as it was; the multi form checks every
+ * replica before it changes any.  After TRACER_ERR_CUDA the scene's contents are undefined: destroy it.
+ * The call is synchronous: it returns once the update is complete on the device, so the caller may reuse or
+ * free its buffers.  Its copies and kernels run on cuda_stream, so data produced on that stream is ordered
+ * before them (multi: cuda_stream is a stream of device 0; the other replicas wait for it, then copy from
+ * device 0 with peer copies on their own streams).  tri_count = 0 and every pointer NULL is a no-op. */
+typedef struct tracer_scene_update {
+    uint32_t struct_size;          /* = sizeof(tracer_scene_update) */
+    int32_t data_is_device;        /* 1: every pointer below is device memory on the scene's GPU (multi: device 0) */
+    void *cuda_stream;             /* stream the copies and kernels run on; NULL = the library's own */
+    int32_t tri_first, tri_count;  /* triangles [tri_first, tri_first + tri_count) */
+    const float *tri_verts;        /* [tri_count*9] new vertices, or NULL */
+    const float *tri_normals;      /* [tri_count*9] or NULL; only for scenes created with normals */
+    const float *geom_material;    /* [n_geoms*13] or NULL */
+    const float *sphere_cr;        /* [n_spheres*4] or NULL */
+    const float *sphere_material;  /* [n_spheres*13] or NULL */
+} tracer_scene_update;
+int tracer_cuda_scene_update(tracer_scene_dev *scene, const tracer_scene_update *u);
+
 /* ---- all GPUs of one box behind one call ------------------------------------
  * The reference has no multi-device path (its closest analogue is thread-per-row,
  * src/main.cpp:629-643).  One process; a context, stream and scene replica per GPU; one
@@ -232,6 +266,7 @@ void tracer_cuda_scene_destroy_multi(tracer_scene_multi *scene);
 int tracer_cuda_render_scene_multi(tracer_scene_multi *scene, const tracer_camera *cam, int32_t width, int32_t height,
                                    const tracer_render_opts *opts, uint8_t *rgb_out); /* rgb_out: host, or GPU 0 if rgb_out_is_device */
 int tracer_cuda_last_stats_multi(tracer_scene_multi *scene, tracer_frame_stats *out); /* counts summed, times of the slowest GPU */
+int tracer_cuda_scene_update_multi(tracer_scene_multi *scene, const tracer_scene_update *u); /* every replica; see tracer_cuda_scene_update */
 
 /* number of PPM rows the band selection (band_rows, band_index, band_count) covers */
 int32_t tracer_band_row_count(int32_t height, int32_t band_rows, int32_t band_index, int32_t band_count);
