@@ -20,7 +20,7 @@ ABI_SYMBOLS = [
     "tracer_mt19937_faceids", "tracer_cuda_fp32_peak", "tracer_camera_lookat",
     "tracer_cuda_init_multi", "tracer_cuda_multi_gpu_count", "tracer_cuda_render_multi", "tracer_cuda_scene_create_multi",
     "tracer_cuda_scene_destroy_multi", "tracer_cuda_render_scene_multi", "tracer_cuda_last_stats_multi",
-    "tracer_cuda_scene_update", "tracer_cuda_scene_update_multi",
+    "tracer_cuda_scene_update", "tracer_cuda_scene_update_multi", "tracer_cuda_render_views",
 ]
 # include/tracer_host.h
 HOST_SYMBOLS = ["tracer_scene_load_obj", "tracer_scene_host_flat", "tracer_scene_host_free", "tracer_host_last_error",
@@ -114,6 +114,8 @@ def load():
     lib.tracer_cuda_render.argtypes = [C.POINTER(SceneFlat), C.POINTER(CameraC), C.c_int32, C.c_int32,
                                        C.POINTER(RenderOpts), C.c_void_p]
     lib.tracer_cuda_last_stats.argtypes = [C.c_void_p, C.POINTER(FrameStats)]
+    lib.tracer_cuda_render_views.argtypes = [C.c_void_p, C.POINTER(CameraC), C.c_int32, C.c_int32, C.c_int32,
+                                             C.POINTER(RenderOpts), C.c_void_p]
     lib.tracer_cuda_init_multi.argtypes = [C.c_int]
     lib.tracer_cuda_scene_create_multi.argtypes = [C.POINTER(SceneFlat), C.POINTER(C.c_void_p)]
     lib.tracer_cuda_scene_destroy_multi.argtypes = [C.c_void_p]

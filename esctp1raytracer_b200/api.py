@@ -414,13 +414,13 @@ class Renderer:
     def upload(self, scene: Scene) -> ResidentScene:
         return ResidentScene(self, scene)
 
-    def _opts(self, scene, width, height, rng_mode, seed, faceid, bands, exhaustive, debug, n_px, keep, tuning):
+    def _opts(self, scene, width, height, rng_mode, seed, faceid, bands, exhaustive, debug, n_px, keep, tuning, n_views=1):
         o = _lib.RenderOpts()
         o.struct_size = C.sizeof(_lib.RenderOpts)
         o.rng_mode, o.seed = rng_mode, seed & 0xFFFFFFFF
         if rng_mode == RNG_EXPLICIT:
             f = np.ascontiguousarray(faceid, np.int32)
-            if f.size != width * height * scene.n_lights:
+            if f.size != n_views * width * height * scene.n_lights:
                 raise ValueError("faceid must have W*H*n_lights entries (image index order)")
             keep.append(f)
             o.faceid = _ptr(f, C.c_int32)
@@ -478,6 +478,52 @@ class Renderer:
             cs = sc.c_struct()
             _lib.check(self.lib.tracer_cuda_render(C.byref(cs), C.byref(camera.c), width, height, C.byref(o), dst))
         return Frame(rgb8=out, stats=stats, **dbg)
+
+    def trace_views(self, scene: ResidentScene, cameras, width: int, height: int, *, rng_mode=RNG_HASH, seed=1,
+                    faceid=None, exhaustive_strict=False, debug=False, out_device_ptr=None, stream=None, rays_per_thread=0,
+                    shadow_chunks=0, samples_per_pixel=0, out=None, bvh=False) -> Frame:
+        """Render one view per camera of a ResidentScene in one call (tracer_cuda_render_views).  View v is bit for bit
+        ``trace(scene, cameras[v], width, height, ...)`` with the same options; the views share the frame's
+        camera-independent work (shadow sweeps, sorts, quantise, read-backs).  ``cameras``: a non-empty sequence of
+        Camera.  ``rgb8`` is [V, H, W, 3] (PPM row order per view); with ``debug`` the arrays are [V, H*W, ...].
+        ``faceid`` (RNG_EXPLICIT): [V, W*H*L] or [V, H*W, L], image index order per view.  ``out``: optional uint8
+        [V, H, W, 3] host array; ``out_device_ptr``: leave the V packed frames in HBM at that address.  Raises
+        ValueError for a wrong shape before any library call."""
+        if not isinstance(scene, ResidentScene):
+            raise ValueError("trace_views renders a ResidentScene (Renderer.upload)")
+        cams = list(cameras) if not isinstance(cameras, Camera) else None
+        if not cams or not all(isinstance(c, Camera) for c in cams):
+            raise ValueError("cameras must be a non-empty sequence of Camera")
+        V, sc, L = len(cams), scene.scene, scene.scene.n_lights
+        if width < 2 or height < 2:
+            raise ValueError("width and height must be >= 2")
+        n_px = width * height
+        if rng_mode == RNG_EXPLICIT:
+            shape = np.shape(faceid)
+            if shape not in ((V, n_px * L), (V, n_px, L)):
+                raise ValueError(f"faceid must be [V, W*H*L] or [V, H*W, L] = [{V}, {n_px * L}] or [{V}, {n_px}, {L}], "
+                                 f"not {list(shape)}")
+        keep = []
+        o, dbg = self._opts(sc, width, height, rng_mode, seed, faceid, None, exhaustive_strict, debug, V * n_px, keep,
+                            (rays_per_thread, shadow_chunks, samples_per_pixel, 0, int(bool(bvh))), n_views=V)
+        if out_device_ptr is not None:
+            out = None
+            o.rgb_out_is_device = 1
+            dst = C.c_void_p(out_device_ptr)
+        else:
+            if out is None:
+                out = np.zeros((V, height, width, 3), np.uint8)
+            if out.dtype != np.uint8 or out.shape != (V, height, width, 3) or not out.flags.c_contiguous:
+                raise ValueError(f"out must be a C-contiguous uint8 array of shape ({V}, {height}, {width}, 3)")
+            dst = out.ctypes.data_as(C.c_void_p)
+        if stream is not None:
+            o.cuda_stream = C.c_void_p(stream)
+        carr = (_lib.CameraC * V)(*[c.c for c in cams])
+        _lib.check(self.lib.tracer_cuda_render_views(scene.handle, carr, V, width, height, C.byref(o), dst))
+        st = _lib.FrameStats()
+        _lib.check(self.lib.tracer_cuda_last_stats(scene.handle, C.byref(st)))
+        dbg = {k: a.reshape((V, n_px) + a.shape[1:]) for k, a in dbg.items()}
+        return Frame(rgb8=out, stats=st.asdict(), **dbg)
 
     def assemble_bands(self, gathered_ptr, frame_ptr, width, height, band_rows, band_count, rows_pad, stream=None):
         _lib.check(self.lib.tracer_cuda_assemble_bands(C.c_void_p(gathered_ptr), C.c_void_p(frame_ptr), width, height,

@@ -529,14 +529,15 @@ __device__ __forceinline__ void count_tests(sweep::Counters *ctr, unsigned long 
 
 // closest hit, one thread per primary ray (direction exactly as the sweeps' candidate path builds it, bands and jitter
 // included): the merged key the sweeps leave in best[], for resolve_primary_kernel
-__global__ void __launch_bounds__(128) primary_kernel(const trk::Cam cam, const trk::Bands bands, const Tree tr, float m,
+__global__ void __launch_bounds__(128) primary_kernel(const trk::Views views, const trk::Bands bands, const Tree tr, float m,
                                                       const float *__restrict__ tri_verts, unsigned long long *__restrict__ best,
                                                       sweep::Counters *ctr) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     unsigned tests = 0;
     if (k < bands.n_px) {
-        int w, h;
-        bands.map(k, w, h);
+        int w, h, local;
+        const trk::Cam &cam = views.cams[views.split(k, local)];
+        bands.map(local, w, h);
         const strict::f3 d = trk::primary_dir(cam, bands, w, h), o = strict::ld(cam.o);
         const float df[3] = {d.x, d.y, d.z};
         const RayBox r = make_ray(cam.o, df, m, 1.f);

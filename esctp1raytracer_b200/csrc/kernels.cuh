@@ -65,6 +65,18 @@ struct Bands {
     }
 };
 
+// The cameras of one call (tracer_cuda_render_views): the call's pixels run view-major, pixel k is local pixel
+// k - v * view_px of view v = k / view_px, and Bands::map maps that local index.  A one-view call has view_px = n_px.
+struct Views {
+    const Cam *cams; // [n_views], device
+    int view_px;     // pixels per view: W * n_rows
+    __device__ __forceinline__ int split(int k, int &local) const {
+        const int v = k / view_px;
+        local = k - v * view_px;
+        return v;
+    }
+};
+
 // main.cpp:709-710 + camera.h:31-34, strict
 __device__ __forceinline__ f3 primary_dir(const Cam &c, const Bands &b, int w, int h) {
     float s, tt;
@@ -320,9 +332,12 @@ __global__ void build_allcand_table(int n_tris, int n_pad, float4 *__restrict__ 
 constexpr unsigned long long KEY_NONE = 0xffffffffffffffffull;
 
 struct PrimaryParams {
-    Cam cam;
+    Views views;
+    Cam cam; // a one-view launch's camera (primary_kernel<..., false>), read as kernel parameters like the table pointer
     Bands bands;
-    const float4 *table; // eye table: span rows (MODE_SHAREDQ, MODE_QBAR) or the three-row table (MODE_OWNQ)
+    const float4 *table; // eye tables of views view0 ..: span rows (MODE_SHAREDQ, MODE_QBAR) or three-row (MODE_OWNQ)
+    long long table_stride; // float4 from one view's table to the next
+    int view0, view_blocks; // first view of this launch; ray blocks per view (n_blocks = views of the launch * view_blocks)
     int n_tiles, n_tris;
     const float *tri_verts;
     unsigned long long *best; // [n_px] merged closest-hit keys over triangles, KEY_NONE = miss
@@ -338,18 +353,22 @@ struct PrimaryParams {
 // pairs is what the serial loop ends with (t2 >= t rejects, ray_triangle.h:49, so among equal t the lowest index
 // stays), whatever the order of evaluation.  filt: the filter passed the pair (validation).  Returns true for a
 // filter miss: an accepted pair the filter did not pass.
-__device__ __noinline__ bool strict_primary(const PrimaryParams &p, int kpx, int tri, bool filt) {
+// kpx: the pixel's index within its view.  VIEWS: the launch sweeps several views (the camera comes from p.views.cams);
+// otherwise it sweeps view p.view0 with camera p.cam.
+template <bool VIEWS>
+__device__ __noinline__ bool strict_primary(const PrimaryParams &p, int view, int kpx, int tri, bool filt) {
     const float *q = p.tri_verts + 9 * (size_t)tri;
     const f3 v0 = strict::mk(__ldg(q), __ldg(q + 1), __ldg(q + 2));
     const f3 v1 = strict::mk(__ldg(q + 3), __ldg(q + 4), __ldg(q + 5));
     const f3 v2 = strict::mk(__ldg(q + 6), __ldg(q + 7), __ldg(q + 8));
-    const f3 o = strict::ld(p.cam.o);
+    const Cam &cam = VIEWS ? p.views.cams[view] : p.cam;
+    const f3 o = strict::ld(cam.o);
     int w, h;
     p.bands.map(kpx, w, h);
-    const f3 d = primary_dir(p.cam, p.bands, w, h);
+    const f3 d = primary_dir(cam, p.bands, w, h);
     float t = FLT_MAX, v = 0.f; // main.cpp:715-717
     if (!strict::intersect_triangle(o, d, v0, v1, v2, t, v)) return false;
-    atomicMin(&p.best[kpx], ((unsigned long long)__float_as_uint(t) << 32) | (unsigned)tri);
+    atomicMin(&p.best[view * p.views.view_px + kpx], ((unsigned long long)__float_as_uint(t) << 32) | (unsigned)tri);
     return !filt;
 }
 
@@ -365,7 +384,10 @@ constexpr int primary_minb(int R) { return R > 32 ? SWEEP_MINB64 : sweep::MINB; 
 // of R pixels of one image row: their q lie inside one stratum, 1/(spp_n (H-1)) wide, and the bounds are evaluated at
 // the thread's mean q plus |B| x spread (MODE_QBAR, as the shadow sweeps do); the candidate path uses each ray's own q.
 // MODE_OWNQ (three-row table, every ray its own q) remains for frames too small for the span rows' |p|,|q| range.
-template <int R, bool EXHAUSTIVE, int MODE>
+// VIEWS: the launch sweeps several views, each ray block against its own view's eye table; without it the launch sweeps
+// the one view p.view0 and takes its camera and table straight from the kernel parameters (no per-item view state: the
+// extra registers of the decode would cost the small mean-q instantiations a CTA per SM).
+template <int R, bool EXHAUSTIVE, int MODE, bool VIEWS>
 __global__ void __launch_bounds__(sweep::NT, primary_minb(R)) primary_kernel(const __grid_constant__ PrimaryParams p) {
     constexpr bool SHAREDQ = MODE == sweep::MODE_SHAREDQ;
     using Mask = sweep::RayMask<R>;
@@ -378,12 +400,19 @@ __global__ void __launch_bounds__(sweep::NT, primary_minb(R)) primary_kernel(con
     unsigned long long tests = 0;
     const int n_items = p.n_blocks * p.n_slices;
     for (;;) {
-        if (tid == 0) sm.blk = atomicAdd(p.work, 1);
+        if (tid == 0) { // sm.seg: the item's view, for the candidate path (shared memory: no register across the sweep)
+            const int it = atomicAdd(p.work, 1);
+            sm.blk = it;
+            if (VIEWS) sm.seg = p.view0 + it % p.n_blocks / p.view_blocks;
+        }
         __syncthreads();
         const int item = sm.blk;
         if (item >= n_items) break;
-        // slice-major order: all CTAs stream the same table tiles at about the same time (L2 reuse)
-        const int slice = item / p.n_blocks, blk = item - slice * p.n_blocks;
+        // slice-major order: all CTAs stream the same table tiles at about the same time (L2 reuse); within a slice,
+        // view-major: a ray block is a screen tile of one view, swept against that view's eye table
+        const int slice = item / p.n_blocks, vblk = item - slice * p.n_blocks;
+        const int vg = VIEWS ? vblk / p.view_blocks : 0, blk = vblk - vg * p.view_blocks;
+        const float4 *table = VIEWS ? p.table + vg * p.table_stride : p.table;
         const int tile_lo = (int)((long long)p.n_tiles * slice / p.n_slices);
         const int tile_hi = (int)((long long)p.n_tiles * (slice + 1) / p.n_slices);
         const int W = p.bands.W;
@@ -419,10 +448,10 @@ __global__ void __launch_bounds__(sweep::NT, primary_minb(R)) primary_kernel(con
             qdelta = fmaxf(qmax - qbar, qbar - qmin) * 1.0001f + 2.4e-7f * (fabsf(qbar) + 1.f);
         }
         sweep::sweep_table<R, MODE, false, EXHAUSTIVE>(
-            sm, p.table, tile_lo, tile_hi, p.n_tris, rp, rq, qbar, qdelta, valid, done, gtile, n_swept,
+            sm, table, tile_lo, tile_hi, p.n_tris, rp, rq, qbar, qdelta, valid, done, gtile, n_swept,
             [&](int otid, int r, int tri, bool filt, const float4 *) {
                 ++n_strict;
-                n_miss += strict_primary(p, thread_ly(otid) * W + thread_x0(otid) + r, tri, filt);
+                n_miss += strict_primary<VIEWS>(p, VIEWS ? sm.seg : p.view0, thread_ly(otid) * W + thread_x0(otid) + r, tri, filt);
                 return false;
             },
             &n_pipe_err);
@@ -461,7 +490,7 @@ struct PixelState {
 // After the sliced closest-hit sweep: unpack the merged (t, index) key, recover v by one strict
 // re-evaluation of the winning triangle (same arithmetic, same bits as in the sweep), then the
 // extension: analytic spheres, tested after all triangles in object order with the running t.
-__global__ void __launch_bounds__(256) resolve_primary_kernel(Cam cam, Bands bands, const unsigned long long *__restrict__ best,
+__global__ void __launch_bounds__(256) resolve_primary_kernel(Views views, Bands bands, const unsigned long long *__restrict__ best,
                                                               const float *__restrict__ tri_verts, int n_tris,
                                                               const float4 *__restrict__ spheres, int n_spheres,
                                                               int *__restrict__ hit_tri, float *__restrict__ hit_t,
@@ -472,8 +501,9 @@ __global__ void __launch_bounds__(256) resolve_primary_kernel(Cam cam, Bands ban
     int tri = key == KEY_NONE ? -1 : (int)(unsigned)(key & 0xffffffffu);
     float t = FLT_MAX, v = 0.f; // main.cpp:715-717
     if (tri >= 0 || n_spheres > 0) {
-        int w, h;
-        bands.map(kpx, w, h);
+        int w, h, local;
+        const Cam &cam = views.cams[views.split(kpx, local)];
+        bands.map(local, w, h);
         const f3 o = strict::ld(cam.o);
         const f3 d = primary_dir(cam, bands, w, h);
         if (tri >= 0) {
@@ -487,7 +517,7 @@ __global__ void __launch_bounds__(256) resolve_primary_kernel(Cam cam, Bands ban
 }
 
 struct LightStepParams {
-    Cam cam;
+    Views views;
     Bands bands;
     PixelState px;
     LightInfo li;
@@ -532,10 +562,12 @@ __global__ void __launch_bounds__(256) light_step_kernel(const LightStepParams p
                 if (p.dbg_occ) p.dbg_occ[(size_t)kpx * p.L + p.k] = -2;
             }
         } else {
-            int w, h;
-            p.bands.map(kpx, w, h);
-            const f3 origin = strict::ld(p.cam.o);
-            const f3 dir = primary_dir(p.cam, p.bands, w, h);
+            // the image index h*W + w (faceID hash, jitter) is the pixel's own within its view
+            int w, h, local;
+            const Cam &cam = p.views.cams[p.views.split(kpx, local)];
+            p.bands.map(local, w, h);
+            const f3 origin = strict::ld(cam.o);
+            const f3 dir = primary_dir(cam, p.bands, w, h);
             const float *mat;
             f3 N;
             float t;
@@ -569,6 +601,8 @@ __global__ void __launch_bounds__(256) light_step_kernel(const LightStepParams p
             }
             mat = (tri < p.n_tris) ? p.geom_material + 13 * (size_t)p.tri_geom[tri]
                                    : p.sphere_material + 13 * (size_t)(tri - p.n_tris);
+            // the next shadow ray's origin, before the shading: eye and direction need not live across powf_glibc
+            const f3 hit = strict::add(origin, strict::mul(dir, __fsub_rn(t, TRC_EPS)));
             const float fL = (float)p.L;
             if (p.k > 0) { // finish light k-1: main.cpp:768-788
                 const unsigned long long ok = p.px.best_occ[kpx];
@@ -603,7 +637,6 @@ __global__ void __launch_bounds__(256) light_step_kernel(const LightStepParams p
                 // P = v0 + ((v1-v0)*r1 + (v2-v0)*r2) with v1 = v2 = v0 (main.cpp:749-754)
                 const f3 zero = strict::sub(v0, v0);
                 const f3 P = strict::add(v0, strict::add(strict::mul(zero, 0.5f), strict::mul(zero, 0.5f)));
-                const f3 hit = strict::add(origin, strict::mul(dir, __fsub_rn(t, TRC_EPS)));
                 f3 Lv = strict::sub(P, hit);
                 const float len = strict::length(Lv);
                 t = __fsub_rn(len, TRC_EPS);

@@ -9,6 +9,10 @@
 // same generator and, for a given --seed, the same bytes as one GPU;
 // `--spp S` = S stratified jittered samples per pixel (extension); `--sorted` runs the reference's optional
 // flatten+sort pass (src/simplify/flatten.cpp:50-82) before rendering.
+// `--eye x,y,z` (repeatable) renders one view per eye, all looking at -l, in one tracer_cuda_render_views call on a resident
+// scene; with -o out.ppm they are written to out_0.ppm, out_1.ppm, ...  Each is the frame `-v x,y,z` gives with the same
+// --seed.  Not with -v, --gpus > 1 or --cull.
+#include <array>
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -33,7 +37,8 @@ int main(int argc, char *argv[]) {
         int device = 0, p6 = 0, bundle_cull = 0, gpus = 1, spp = 0;
         bool sorted = false;
         int accel = 0;
-        bool have_seed = false;
+        bool have_seed = false, have_v = false;
+        std::vector<std::array<float, 3>> eyes;
         unsigned seed = 0;
         int rng = TRACER_RNG_MT19937; // the serial path's generator
         for (int a = 1; a < argc; ++a) {
@@ -47,7 +52,11 @@ int main(int argc, char *argv[]) {
                 throw std::runtime_error(f + ": CPU/ISPC modes are not part of this build (GPU renderer only)");
             if (f == "-m") model = need("-m");
             else if (f == "-o") output = need("-o");
-            else if (f == "-v") parse_triple(need("-v"), eye);
+            else if (f == "-v") parse_triple(need("-v"), eye), have_v = true;
+            else if (f == "--eye") {
+                eyes.emplace_back();
+                parse_triple(need("--eye"), eyes.back().data());
+            }
             else if (f == "-l") parse_triple(need("-l"), look);
             else if (f == "-w") {
                 if (std::sscanf(need("-w"), "%d,%d", &W, &H) != 2) throw std::runtime_error("expected -w W,H");
@@ -64,6 +73,9 @@ int main(int argc, char *argv[]) {
             else if (f == "--bvh") sorted = true, accel = 1;
             else throw std::runtime_error("Unknown argument: " + f); // main.cpp:531-534
         }
+        if (!eyes.empty() && have_v) throw std::runtime_error("--eye and -v do not combine: give every view as --eye");
+        if (!eyes.empty() && gpus > 1) throw std::runtime_error("--eye renders on one GPU: --gpus must be 1");
+        if (!eyes.empty() && bundle_cull) throw std::runtime_error("--eye does not combine with --cull");
         tracer_scene_host *scene = nullptr;
         tracer_scene_flat empty{};
         const int32_t zero_off[1] = {0};
@@ -92,6 +104,38 @@ int main(int argc, char *argv[]) {
         o.samples_per_pixel = spp;
         if (spp > 1 && rng == TRACER_RNG_MT19937) o.rng_mode = rng = TRACER_RNG_HASH; // the serial replay is 1 spp only
         o.seed = have_seed ? seed : std::random_device{}(); // main.cpp:587-588
+        if (!eyes.empty()) { // one resident scene, one call for every view
+            std::vector<tracer_camera> cams(eyes.size());
+            for (size_t v = 0; v < eyes.size(); ++v) tracer_camera_lookat(eyes[v].data(), look, vup, 60.f, float(W) / H, &cams[v]);
+            tracer_scene_dev *dev = nullptr;
+            if (tracer_cuda_scene_create(flat, &dev)) throw std::runtime_error(tracer_cuda_last_error());
+            std::vector<uint8_t> rgb(eyes.size() * (size_t)W * H * 3);
+            const auto t0 = std::chrono::high_resolution_clock::now();
+            const int rc = tracer_cuda_render_views(dev, cams.data(), (int32_t)cams.size(), W, H, &o, rgb.data());
+            const auto t1 = std::chrono::high_resolution_clock::now();
+            tracer_cuda_scene_destroy(dev);
+            if (rc) throw std::runtime_error(tracer_cuda_last_error());
+            std::cerr << "\n CUDA      : true" << std::endl;
+            std::cerr << "\n Views     : " << eyes.size() << std::endl;
+            std::cerr << "\n Duration  : " << std::chrono::duration_cast<std::chrono::milliseconds>(t1 - t0).count() << std::endl;
+            if (!output.empty()) {
+                const size_t dot = output.rfind('.'), slash = output.rfind('/');
+                const bool has_ext = dot != std::string::npos && (slash == std::string::npos || dot > slash);
+                const std::string stem = has_ext ? output.substr(0, dot) : output, ext = has_ext ? output.substr(dot) : "";
+                for (size_t v = 0; v < eyes.size(); ++v) {
+                    const std::string path = stem + "_" + std::to_string(v) + ext;
+                    if (tracer_write_ppm(path.c_str(), rgb.data() + v * (size_t)W * H * 3, W, H, p6))
+                        throw std::runtime_error(tracer_host_last_error());
+                    std::cout << "Rendered image in: " << path << std::endl;
+                }
+            } else {
+                std::cout << "Nothing saved: use -o to save rendered image" << std::endl;
+            }
+            tracer_scene_host_free(sorted_scene);
+            tracer_scene_host_free(scene);
+            tracer_cuda_shutdown();
+            return 0;
+        }
         std::vector<uint8_t> rgb((size_t)W * H * 3);
         const auto t0 = std::chrono::high_resolution_clock::now(); // main.cpp:583
         if (tracer_cuda_render(flat, &cam, W, H, &o, rgb.data())) throw std::runtime_error(tracer_cuda_last_error());

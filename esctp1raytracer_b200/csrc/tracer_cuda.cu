@@ -294,6 +294,9 @@ struct tracer_scene_dev {
     void *box_work = nullptr; // bbox_partial_kernel's per-block bounds, then the 6 doubles of the box
     float4 *eye_table = nullptr, *light_tables = nullptr, *allcand_table = nullptr; // 48-byte three-row tables
     float4 *eye_span = nullptr, *light_spans = nullptr, *allcand_span = nullptr;    // 32-byte span tables (same slots)
+    int eye_cap = 1;                // views whose eye tables (both forms) eye_table / eye_span hold; grown on demand
+    trk::Cam *cams = nullptr;       // the call's cameras, one per view
+    size_t cams_cap = 0;
     std::vector<double> table_lmax; // per (light vertex, cube face): reach bound it was built for, < 0 = not built
     int table_slots = 1;            // light vertices whose 6 face tables fit at once (and per persistent-kernel launch)
     bool tables_resident = true;    // every light vertex has its own slot: tables are kept across lights and frames
@@ -365,13 +368,18 @@ int ensure_workspace(tracer_scene_dev *s, int n_px, bool want_dbg_occ) {
     return 0;
 }
 
-template <int R, bool EX, int MODE>
-int launch_primary_q(const trk::PrimaryParams &p, int grid, cudaStream_t st) {
+template <int R, bool EX, int MODE, bool VIEWS>
+int launch_primary_v(const trk::PrimaryParams &p, int grid, cudaStream_t st) {
     const size_t smem = sizeof(sweep::SmemT<sweep::Rows<MODE>::N>);
-    CK_CUDA(cudaFuncSetAttribute(trk::primary_kernel<R, EX, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    trk::primary_kernel<R, EX, MODE><<<grid, sweep::NT, smem, st>>>(p);
+    CK_CUDA(cudaFuncSetAttribute(trk::primary_kernel<R, EX, MODE, VIEWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    trk::primary_kernel<R, EX, MODE, VIEWS><<<grid, sweep::NT, smem, st>>>(p);
     CK_CUDA(cudaGetLastError());
     return 0;
+}
+// views: the launch covers several views (primary_kernel's per-item view decode); one view reads camera and table as parameters
+template <int R, bool EX, int MODE>
+int launch_primary_q(const trk::PrimaryParams &p, bool views, int grid, cudaStream_t st) {
+    return views ? launch_primary_v<R, EX, MODE, true>(p, grid, st) : launch_primary_v<R, EX, MODE, false>(p, grid, st);
 }
 int scene_create_on(Ctx &g, const tracer_scene_flat *sc, tracer_scene_dev **out);
 
@@ -463,28 +471,28 @@ int launch_shadow_light(Ctx &g, bool ex, const trk::ShadowLightParams &p, unsign
     return ex ? launch_shadow_light_t<true>(g, p, bar, st) : launch_shadow_light_t<false>(g, p, bar, st);
 }
 // qmode: sweep::MODE_SHAREDQ (no jitter), MODE_QBAR (jittered samples, span table) or MODE_OWNQ (jittered, three-row table)
-int launch_primary(int R, bool ex, int qmode, const trk::PrimaryParams &p, int grid, cudaStream_t st) {
+int launch_primary(int R, bool ex, int qmode, const trk::PrimaryParams &p, bool views, int grid, cudaStream_t st) {
     constexpr int OQ = sweep::MODE_OWNQ, SQ = sweep::MODE_SHAREDQ, QB = sweep::MODE_QBAR;
     if (qmode == OQ) { // every ray its own q, three-row table
-        if (R == 12) return ex ? launch_primary_q<12, true, OQ>(p, grid, st) : launch_primary_q<12, false, OQ>(p, grid, st);
-        if (R == 8) return ex ? launch_primary_q<8, true, OQ>(p, grid, st) : launch_primary_q<8, false, OQ>(p, grid, st);
-        if (R == 4) return ex ? launch_primary_q<4, true, OQ>(p, grid, st) : launch_primary_q<4, false, OQ>(p, grid, st);
-        return ex ? launch_primary_q<2, true, OQ>(p, grid, st) : launch_primary_q<2, false, OQ>(p, grid, st);
+        if (R == 12) return ex ? launch_primary_q<12, true, OQ>(p, views, grid, st) : launch_primary_q<12, false, OQ>(p, views, grid, st);
+        if (R == 8) return ex ? launch_primary_q<8, true, OQ>(p, views, grid, st) : launch_primary_q<8, false, OQ>(p, views, grid, st);
+        if (R == 4) return ex ? launch_primary_q<4, true, OQ>(p, views, grid, st) : launch_primary_q<4, false, OQ>(p, views, grid, st);
+        return ex ? launch_primary_q<2, true, OQ>(p, views, grid, st) : launch_primary_q<2, false, OQ>(p, views, grid, st);
     }
     if (qmode == QB) {
-        if (R == 32) return ex ? launch_primary_q<32, true, QB>(p, grid, st) : launch_primary_q<32, false, QB>(p, grid, st);
-        if (R == 16) return ex ? launch_primary_q<16, true, QB>(p, grid, st) : launch_primary_q<16, false, QB>(p, grid, st);
-        if (R == 8) return ex ? launch_primary_q<8, true, QB>(p, grid, st) : launch_primary_q<8, false, QB>(p, grid, st);
-        if (R == 4) return ex ? launch_primary_q<4, true, QB>(p, grid, st) : launch_primary_q<4, false, QB>(p, grid, st);
-        return ex ? launch_primary_q<2, true, QB>(p, grid, st) : launch_primary_q<2, false, QB>(p, grid, st);
+        if (R == 32) return ex ? launch_primary_q<32, true, QB>(p, views, grid, st) : launch_primary_q<32, false, QB>(p, views, grid, st);
+        if (R == 16) return ex ? launch_primary_q<16, true, QB>(p, views, grid, st) : launch_primary_q<16, false, QB>(p, views, grid, st);
+        if (R == 8) return ex ? launch_primary_q<8, true, QB>(p, views, grid, st) : launch_primary_q<8, false, QB>(p, views, grid, st);
+        if (R == 4) return ex ? launch_primary_q<4, true, QB>(p, views, grid, st) : launch_primary_q<4, false, QB>(p, views, grid, st);
+        return ex ? launch_primary_q<2, true, QB>(p, views, grid, st) : launch_primary_q<2, false, QB>(p, views, grid, st);
     }
-    if (R == 64) return ex ? launch_primary_q<64, true, SQ>(p, grid, st) : launch_primary_q<64, false, SQ>(p, grid, st);
-    if (R == 32) return ex ? launch_primary_q<32, true, SQ>(p, grid, st) : launch_primary_q<32, false, SQ>(p, grid, st);
-    if (R == 24) return ex ? launch_primary_q<24, true, SQ>(p, grid, st) : launch_primary_q<24, false, SQ>(p, grid, st);
-    if (R == 16) return ex ? launch_primary_q<16, true, SQ>(p, grid, st) : launch_primary_q<16, false, SQ>(p, grid, st);
-    if (R == 8) return ex ? launch_primary_q<8, true, SQ>(p, grid, st) : launch_primary_q<8, false, SQ>(p, grid, st);
-    if (R == 4) return ex ? launch_primary_q<4, true, SQ>(p, grid, st) : launch_primary_q<4, false, SQ>(p, grid, st);
-    return ex ? launch_primary_q<2, true, SQ>(p, grid, st) : launch_primary_q<2, false, SQ>(p, grid, st);
+    if (R == 64) return ex ? launch_primary_q<64, true, SQ>(p, views, grid, st) : launch_primary_q<64, false, SQ>(p, views, grid, st);
+    if (R == 32) return ex ? launch_primary_q<32, true, SQ>(p, views, grid, st) : launch_primary_q<32, false, SQ>(p, views, grid, st);
+    if (R == 24) return ex ? launch_primary_q<24, true, SQ>(p, views, grid, st) : launch_primary_q<24, false, SQ>(p, views, grid, st);
+    if (R == 16) return ex ? launch_primary_q<16, true, SQ>(p, views, grid, st) : launch_primary_q<16, false, SQ>(p, views, grid, st);
+    if (R == 8) return ex ? launch_primary_q<8, true, SQ>(p, views, grid, st) : launch_primary_q<8, false, SQ>(p, views, grid, st);
+    if (R == 4) return ex ? launch_primary_q<4, true, SQ>(p, views, grid, st) : launch_primary_q<4, false, SQ>(p, views, grid, st);
+    return ex ? launch_primary_q<2, true, SQ>(p, views, grid, st) : launch_primary_q<2, false, SQ>(p, views, grid, st);
 }
 // Work decomposition of a sweep: R rays per thread (8 preferred: best amortisation of the row loads) and
 // n_slices triangle slices, chosen so that ray blocks x slices keeps every SM busy for several items.
@@ -815,7 +823,7 @@ void tracer_cuda_scene_destroy(tracer_scene_dev *s) {
     dev_free(s->tri_verts), dev_free(s->tri_normals), dev_free(s->geom_material), dev_free(s->sphere_material);
     dev_free(s->tri_geom), dev_free(s->geom_has_normals), dev_free(s->spheres), dev_free(s->light_vbase);
     dev_free(s->light_verts), dev_free(s->eye_table), dev_free(s->light_tables), dev_free(s->allcand_table);
-    dev_free(s->eye_span), dev_free(s->light_spans), dev_free(s->allcand_span);
+    dev_free(s->eye_span), dev_free(s->light_spans), dev_free(s->allcand_span), dev_free(s->cams);
     dev_free(s->hit_tri), dev_free(s->rj), dev_free(s->best), dev_free(s->best_occ), dev_free(s->list), dev_free(s->list_b);
     dev_free(s->faceid), dev_free(s->dbg_occ), dev_free(s->cnt_b), dev_free(s->accum_total);
     dev_free(s->hit_t), dev_free(s->hit_v), dev_free(s->carry), dev_free(s->nrm), dev_free(s->accum);
@@ -1010,8 +1018,10 @@ int mt_frame_rows(const tracer_render_opts &o, int W, int H, int band_rows, int 
 }
 
 // faceid[k*L + l] of every hit local pixel k, from the frame's row counts: the stream, the automaton, the gather
+// (rank_off: where these rows' in-row ranks start in m.rank, when mt_count_rows counted more rows than these)
 int mt_replay(MtWork &m, uint32_t seed, const std::vector<int> &faces, const std::vector<int> &frame, int W, int band_rows,
-              int band_index, int band_count, int n_rows, const int *hit_tri, int *faceid, cudaStream_t st, int &launches) {
+              int band_index, int band_count, int n_rows, const int *hit_tri, int *faceid, cudaStream_t st, int &launches,
+              size_t rank_off = 0) {
     const int L = (int)faces.size(), S = 3 * L, n_px = n_rows * W;
     if (L == 0 || n_rows == 0) return 0;
     std::vector<int64_t> base((size_t)n_rows);
@@ -1049,36 +1059,67 @@ int mt_replay(MtWork &m, uint32_t seed, const std::vector<int> &faces, const std
     mt::chunk_faceids_kernel<<<(unsigned)((n_chunks + mt::AUTO_THREADS - 1) / mt::AUTO_THREADS), mt::AUTO_THREADS, 0, st>>>(
         m.words, D, C, n_chunks, T, L, m.lights, m.start, m.ord, m.fid_ord);
     CK_CUDA(cudaGetLastError());
-    mt::gather_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(hit_tri, W, n_px, L, m.base, m.rank, m.fid_ord, faceid);
+    mt::gather_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(hit_tri, W, n_px, L, m.base, m.rank + rank_off, m.fid_ord, faceid);
     CK_CUDA(cudaGetLastError());
     launches += 2;
     return 0;
 }
 
+// n_views frames of one scene, one per camera, in one call (V = 1: tracer_cuda_render_scene).  The call's pixels run view-major
+// (k = view * W * n_rows + local); every per-pixel buffer, sort and list spans all of them, and the shadow sweeps take the
+// rays of every view at once.  Only the closest-hit sweep is per view: one eye table each, in groups (DESIGN §4e).
 // frame_rows: the frame's row hit counts when the caller already has them: the bundle-cull mode's re-render of a frame whose
 // closest-hit pass was complete but whose shadow candidates overflowed (same hits; the exchange hook runs once per frame)
-int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32_t H, const tracer_render_opts *opts_in,
+int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, int32_t W, int32_t H, const tracer_render_opts *opts_in,
                  uint8_t *rgb_out, const std::vector<int> *frame_rows);
+
+// Eye tables kept per call: views in groups whose tables (both forms, n_pad x 80 B per view) fit a quarter of the free
+// device memory, one closest-hit launch per group.  (TRACER_VIEW_GROUP caps the group size: development/test knob.)
+int view_group_size(tracer_scene_dev *s, int n_views) {
+    const char *e = std::getenv("TRACER_VIEW_GROUP");
+    const int cap = e ? std::max(1, std::atoi(e)) : INT_MAX;
+    if (n_views <= s->eye_cap) return std::min(n_views, cap);
+    size_t free_b = 0, total_b = 0;
+    cudaMemGetInfo(&free_b, &total_b);
+    const size_t per_view = (s->table_stride + s->span_stride) * sizeof(float4);
+    const size_t fit = std::max<size_t>((size_t)s->eye_cap, free_b / 4 / per_view);
+    return (int)std::max<size_t>(1, std::min<size_t>({fit, (size_t)cap, (size_t)n_views}));
+}
 }  // namespace
 
 extern "C" {
 
 int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32_t H,
                              const tracer_render_opts *opts_in, uint8_t *rgb_out) {
-    return render_scene(s, cam, W, H, opts_in, rgb_out, nullptr);
+    return render_views(s, cam, 1, W, H, opts_in, rgb_out, nullptr);
+}
+
+int tracer_cuda_render_views(tracer_scene_dev *s, const tracer_camera *cams, int32_t n_views, int32_t W, int32_t H,
+                             const tracer_render_opts *opts_in, uint8_t *rgb_out) {
+    if (n_views < 1) return fail(TRACER_ERR_INVALID, "n_views must be >= 1");
+    if (!cams) return fail(TRACER_ERR_INVALID, "null cameras");
+    if (opts_in) {
+        tracer_render_opts o;
+        std::memset(&o, 0, sizeof o);
+        std::memcpy(&o, opts_in, std::min<size_t>(sizeof o, opts_in->struct_size ? opts_in->struct_size : sizeof o));
+        if (o.band_count > 1) return fail(TRACER_ERR_INVALID, "tracer_cuda_render_views renders whole views: band_count must be <= 1");
+        if (o.bundle_cull != 0) return fail(TRACER_ERR_INVALID, "tracer_cuda_render_views does not combine with bundle_cull");
+    }
+    return render_views(s, cams, n_views, W, H, opts_in, rgb_out, nullptr);
 }
 }  // extern "C"
 
 namespace {
-int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32_t H, const tracer_render_opts *opts_in,
+int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, int32_t W, int32_t H, const tracer_render_opts *opts_in,
                  uint8_t *rgb_out, const std::vector<int> *frame_rows) {
-    if (!s || !cam || !rgb_out) return fail(TRACER_ERR_INVALID, "null argument");
+    if (!s || !cams || !rgb_out) return fail(TRACER_ERR_INVALID, "null argument");
     if (!s->ctx || !s->ctx->inited) return fail(TRACER_ERR_NO_DEVICE, "tracer_cuda_init not called");
     Ctx &g = *s->ctx;
     t_pool = &g.pool;
     if (W < 2 || H < 2) return fail(TRACER_ERR_INVALID, "width and height must be >= 2 (the reference divides by W-1, H-1)");
     // per-pixel planes are indexed with int (3 planes of n_px floats): keep 3 * n_px below 2^31
-    if ((int64_t)W * H > (int64_t)700 * 1000 * 1000) return fail(TRACER_ERR_INVALID, "frame too large (limit 7e8 pixels per call; render bands)");
+    if ((int64_t)n_views * W * H > (int64_t)700 * 1000 * 1000)
+        return fail(TRACER_ERR_INVALID, "frame too large (limit 7e8 pixels per call, over all views; render bands or fewer views)");
     tracer_render_opts o;
     std::memset(&o, 0, sizeof o);
     if (opts_in) std::memcpy(&o, opts_in, std::min<size_t>(sizeof o, opts_in->struct_size ? opts_in->struct_size : sizeof o));
@@ -1106,7 +1147,7 @@ int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32
     if (use_bvh && (o.bundle_cull != 0 || o.exhaustive_strict != 0))
         return fail(TRACER_ERR_INVALID, "accel = 1 (BVH) does not combine with bundle_cull or exhaustive_strict (a debug mode of the sweeps' filter)");
     const int n_rows = tracer_band_row_count(H, band_rows, band_count > 1 ? o.band_index : 0, band_count);
-    const int n_px = n_rows * W;
+    const int view_px = n_rows * W, n_px = n_views * view_px;
     const int L = s->n_lights;
     CK_CUDA(cudaSetDevice(g.device));
     cudaStream_t st = o.cuda_stream ? (cudaStream_t)o.cuda_stream : g.stream;
@@ -1120,39 +1161,66 @@ int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32
     int launches = 0;
 
     trk::Cam dc;
-    std::memcpy(dc.o, cam->origin, 12), std::memcpy(dc.llc, cam->lower_left_corner, 12);
-    std::memcpy(dc.hor, cam->horizontal, 12), std::memcpy(dc.ver, cam->vertical, 12);
+    std::vector<trk::Cam> h_cams((size_t)n_views);
+    for (int v = 0; v < n_views; ++v) {
+        trk::Cam &c = h_cams[v];
+        std::memcpy(c.o, cams[v].origin, 12), std::memcpy(c.llc, cams[v].lower_left_corner, 12);
+        std::memcpy(c.hor, cams[v].horizontal, 12), std::memcpy(c.ver, cams[v].vertical, 12);
+    }
+    dc = h_cams[0];
+    if (dev_grow(s->cams, s->cams_cap, (size_t)n_views)) return TRACER_ERR_NOMEM;
+    CK_CUDA(cudaMemcpyAsync(s->cams, h_cams.data(), sizeof(trk::Cam) * (size_t)n_views, cudaMemcpyHostToDevice, st));
+    const trk::Views views{s->cams, view_px};
     trk::Bands bands{W, H, band_rows, band_count > 1 ? o.band_index : 0, band_count, n_px};
     bands.spp_n = spp_n, bands.sample = 0, bands.seed = o.seed;
 
-    // reach bound for shadow segments: len_k <= (k+1) * diag(bbox U eye)  (t carries over lights, main.cpp:764)
+    // reach bound for shadow segments: len_k <= (k+1) * diag(bbox U every eye)  (t carries over lights, main.cpp:764).  One
+    // bound for all views: a view's own would be smaller, and a table built for a larger bound is only looser (DESIGN §4e)
     double lo[3], hi[3], diag2 = 0;
     for (int c = 0; c < 3; ++c) {
-        lo[c] = std::min(s->bb_lo[c], (double)cam->origin[c]), hi[c] = std::max(s->bb_hi[c], (double)cam->origin[c]);
+        lo[c] = s->bb_lo[c], hi[c] = s->bb_hi[c];
+        for (int v = 0; v < n_views; ++v) lo[c] = std::min(lo[c], (double)cams[v].origin[c]), hi[c] = std::max(hi[c], (double)cams[v].origin[c]);
         if (hi[c] >= lo[c]) diag2 += (hi[c] - lo[c]) * (hi[c] - lo[c]);
     }
     // shadow segments of light k are bounded by len_k <= (k+1) * diag: t carries over lights (main.cpp:764)
     const double diag = std::sqrt(diag2) * 1.001 + 1e-30;
+    // eye tables: views [v0, v1) into slots 0 .. v1 - v0, on the image plane: d'(s,t) = (llc - origin) + s*horizontal +
+    // t*vertical (camera.h:31-34)
+    const int group = use_bvh ? n_views : view_group_size(s, n_views), n_groups = (n_views + group - 1) / group;
+    if (!use_bvh && group > s->eye_cap) {
+        dev_free(s->eye_table), dev_free(s->eye_span);
+        s->eye_cap = 0;
+        if (dev_alloc(&s->eye_table, s->table_stride * group) || dev_alloc(&s->eye_span, s->span_stride * group)) return TRACER_ERR_NOMEM;
+        s->eye_cap = group;
+    }
+    auto build_eye_tables = [&](int v0, int v1) -> int {
+        for (int v = v0; v < v1; ++v) {
+            const tracer_camera *cv = &cams[v];
+            trk::TableParam tp{};
+            for (int c = 0; c < 3; ++c) {
+                tp.o[c] = cv->origin[c], tp.U[c] = cv->horizontal[c], tp.V[c] = cv->vertical[c];
+                tp.W[c] = (double)cv->lower_left_corner[c] - (double)cv->origin[c];
+            }
+            for (int corner = 0; corner < 4; ++corner) { // |d'| is convex in (s,t): its maximum is at a corner
+                double n2 = 0;
+                for (int c = 0; c < 3; ++c) {
+                    const double x = tp.W[c] + (corner & 1) * tp.U[c] + (corner >> 1) * tp.V[c];
+                    n2 += x * x;
+                }
+                tp.dmax = std::max(tp.dmax, std::sqrt(n2));
+            }
+            tp.lmax = 0.0;
+            if (int rc = build_table(s, tp, s->eye_table + (size_t)(v - v0) * s->table_stride, s->eye_span + (size_t)(v - v0) * s->span_stride, st))
+                return rc;
+            ++launches;
+        }
+        return 0;
+    };
     CK_CUDA(cudaEventRecord(s->ev[0], st));
     if (use_bvh) {
         if (int rc = ensure_bvh(s, st)) return rc;
-    } else {   // eye table on the image plane: d'(s,t) = (llc - origin) + s*horizontal + t*vertical (camera.h:31-34)
-        trk::TableParam tp{};
-        for (int c = 0; c < 3; ++c) {
-            tp.o[c] = cam->origin[c], tp.U[c] = cam->horizontal[c], tp.V[c] = cam->vertical[c];
-            tp.W[c] = (double)cam->lower_left_corner[c] - (double)cam->origin[c];
-        }
-        for (int corner = 0; corner < 4; ++corner) { // |d'| is convex in (s,t): its maximum is at a corner
-            double n2 = 0;
-            for (int c = 0; c < 3; ++c) {
-                const double v = tp.W[c] + (corner & 1) * tp.U[c] + (corner >> 1) * tp.V[c];
-                n2 += v * v;
-            }
-            tp.dmax = std::max(tp.dmax, std::sqrt(n2));
-        }
-        tp.lmax = 0.0;
-        if (int rc = build_table(s, tp, s->eye_table, s->eye_span, st)) return rc;
-        ++launches;
+    } else if (n_groups == 1) { // one group: its tables serve every sample; otherwise each group builds its own in turn
+        if (int rc = build_eye_tables(0, n_views)) return rc;
     }
     CK_CUDA(cudaMemsetAsync(s->counters, 0, sizeof(sweep::Counters), st));
     CK_CUDA(cudaMemsetAsync(s->work, 0, sizeof(int), st));
@@ -1176,7 +1244,7 @@ int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32
             s->cull_grow *= 4;
         else
             o2.bundle_cull = 0;
-        return render_scene(s, cam, W, H, &o2, rgb_out, rows);
+        return render_views(s, cams, n_views, W, H, &o2, rgb_out, rows);
     };
     if (cull) { // candidate buffers: 24 per ray + slack (a few per ray are typical), sorted with a radix sort
         const size_t cap = (size_t)n_px * 24 * (size_t)s->cull_grow + ((size_t)1 << 22);
@@ -1258,13 +1326,14 @@ int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32
     CK_CUDA(cudaEventRecord(s->ev[1], st));
     // BVH mode: the tree's dilation m (bvh.cuh frame_margin) from the largest |coordinate| of the tree and the eye, with
     // the reach bound diag of the primary rays' hit points, (k+1) diag for light k
-    double bvh_ext = s->bvh_ext;
-    for (int c = 0; c < 3; ++c) bvh_ext = std::max(bvh_ext, (double)std::fabs(cam->origin[c]));
+    double bvh_ext = s->bvh_ext; // (every view's eye: the tree serves them all)
+    for (int v = 0; v < n_views; ++v)
+        for (int c = 0; c < 3; ++c) bvh_ext = std::max(bvh_ext, (double)std::fabs(cams[v].origin[c]));
     if (use_bvh) {
-        bvh::primary_kernel<<<(n_px + 127) / 128, 128, 0, st>>>(dc, bands, s->bvh_tree, bvh::frame_margin(bvh_ext, diag), s->tri_verts,
+        bvh::primary_kernel<<<(n_px + 127) / 128, 128, 0, st>>>(views, bands, s->bvh_tree, bvh::frame_margin(bvh_ext, diag), s->tri_verts,
                                                                  s->best, s->counters);
         CK_CUDA(cudaGetLastError());
-        trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(dc, bands, s->best, s->tri_verts, s->n_tris, s->spheres,
+        trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(views, bands, s->best, s->tri_verts, s->n_tris, s->spheres,
                                                                         s->n_spheres, s->hit_tri, s->hit_t, s->hit_v);
         CK_CUDA(cudaGetLastError());
         launches += 2;
@@ -1300,7 +1369,7 @@ int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32
         trk::strict_primary_pairs<<<8 * g.n_sms, 256, 0, st>>>(s->cand_a, s->cand_count, em_cap, dc, bands,
                                                                s->tri_verts, s->best, s->counters);
         CK_CUDA(cudaGetLastError());
-        trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(dc, bands, s->best, s->tri_verts, s->n_tris, s->spheres,
+        trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(views, bands, s->best, s->tri_verts, s->n_tris, s->spheres,
                                                                         s->n_spheres, s->hit_tri, s->hit_t, s->hit_v);
         CK_CUDA(cudaGetLastError());
         launches += 3;
@@ -1308,17 +1377,27 @@ int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32
         // no jitter: the rays of a thread share q exactly; jittered samples (extension): they share a mean q (span table)
         // unless the frame is so small that a jittered (s,t) can leave the span rows' |p|,|q| <= 1.0625 range
         const int qmode = bands.spp_n <= 1 ? sweep::MODE_SHAREDQ : (W >= 16 && H >= 16 ? sweep::MODE_QBAR : sweep::MODE_OWNQ);
-        const Decomp d = pick_decomp(n_px, n_tiles, g.n_sms, o.rays_per_thread, 0, qmode);
+        // one launch per group of views (all of them unless their eye tables did not fit at once)
+        for (int v0 = 0; v0 < n_views; v0 += group) {
+        const int nv = std::min(group, n_views - v0);
+        if (n_groups > 1) {
+            if (int rc = build_eye_tables(v0, v0 + nv)) return rc;
+            if (v0 > 0) CK_CUDA(cudaMemsetAsync(s->work, 0, sizeof(int), st));
+        }
+        const Decomp d = pick_decomp((int64_t)nv * view_px, n_tiles, g.n_sms, o.rays_per_thread, 0, qmode);
         trk::PrimaryParams p{};
-        p.cam = dc, p.bands = bands, p.table = qmode == sweep::MODE_OWNQ ? s->eye_table : s->eye_span, p.n_tiles = n_tiles, p.n_tris = s->n_tris;
+        p.views = views, p.cam = h_cams[v0], p.bands = bands, p.n_tiles = n_tiles, p.n_tris = s->n_tris;
+        p.table = qmode == sweep::MODE_OWNQ ? s->eye_table : s->eye_span;
+        p.table_stride = (long long)(qmode == sweep::MODE_OWNQ ? s->table_stride : s->span_stride), p.view0 = v0;
         p.tri_verts = s->tri_verts;
         p.best = s->best, p.counters = s->counters, p.work = s->work;
-        p.n_rows = n_rows, p.n_blocks = 0; // ray blocks = screen tiles of (TX R) x (NT / TX) pixels: least edge waste wins
+        p.n_rows = n_rows, p.view_blocks = 0; // ray blocks = screen tiles of (TX R) x (NT / TX) pixels: least edge waste wins
         for (int lg = d.R > 32 ? 2 : 3; lg <= 6; ++lg) { // (64 rays per thread: from 4 x 64 = 256 pixels wide)
             const int tw = (1 << lg) * d.R, th = sweep::NT >> lg;
             const int tx = (W + tw - 1) / tw, nb = tx * ((n_rows + th - 1) / th);
-            if (!p.n_blocks || nb < p.n_blocks) p.n_blocks = nb, p.tiles_x = tx, p.tx_log2 = lg;
+            if (!p.view_blocks || nb < p.view_blocks) p.view_blocks = nb, p.tiles_x = tx, p.tx_log2 = lg;
         }
+        p.n_blocks = nv * p.view_blocks;
         p.n_slices = d.n_slices;
         const int minb = trk::primary_minb(d.R);
         const int want_items = items_per_cta() * minb * g.n_sms;
@@ -1331,21 +1410,24 @@ int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32
         // shared q: per thread and triangle the set-up's 10 flops and one FADD2 (segment_pass), nothing per pair
         flop_primary = qmode == sweep::MODE_OWNQ ? 15.0 : qmode == sweep::MODE_QBAR ? 1.0 + 18.0 / d.R : 12.0 / d.R;
         flop_primary_edges = qmode == sweep::MODE_OWNQ ? 12.0 : (qmode == sweep::MODE_QBAR ? 16.0 : 8.0) / d.R;
-        if (int rc = launch_primary(d.R, o.exhaustive_strict != 0, qmode, p, grid, st)) return rc;
-        trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(dc, bands, s->best, s->tri_verts, s->n_tris, s->spheres,
+        if (int rc = launch_primary(d.R, o.exhaustive_strict != 0, qmode, p, nv > 1, grid, st)) return rc;
+        ++launches;
+        }
+        trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(views, bands, s->best, s->tri_verts, s->n_tris, s->spheres,
                                                                         s->n_spheres, s->hit_tri, s->hit_t, s->hit_v);
         CK_CUDA(cudaGetLastError());
-        launches += 2;
+        ++launches;
     }
     CK_CUDA(cudaEventRecord(s->ev[2], st));
 
     // ---- faceIDs ------------------------------------------------------------------------
     if (smp == 0 && L > 0 && o.rng_mode == TRACER_RNG_EXPLICIT) {
         std::vector<int> loc((size_t)n_px * L);
-        for (int k = 0; k < n_px; ++k) {
+        for (int k = 0; k < n_px; ++k) { // view v's faceids: opts->faceid[v][W*H*L], image index order
             int w, h;
-            bands.map(k, w, h);
-            std::memcpy(&loc[(size_t)k * L], o.faceid + ((size_t)h * W + w) * L, sizeof(int) * L);
+            const int v = k / view_px;
+            bands.map(k - v * view_px, w, h);
+            std::memcpy(&loc[(size_t)k * L], o.faceid + ((size_t)v * H * W + (size_t)h * W + w) * L, sizeof(int) * L);
         }
         CK_CUDA(cudaMemcpyAsync(s->faceid, loc.data(), loc.size() * sizeof(int), cudaMemcpyHostToDevice, st));
         CK_CUDA(cudaStreamSynchronize(st));
@@ -1354,20 +1436,26 @@ int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32
         // so the frame is rendered again before the exchange (read back with the row counts, at the same synchronise)
         unsigned long long primary_overflow = 0;
         if (cull) CK_CUDA(cudaMemcpyAsync(&primary_overflow, &s->counters->cull_overflow, sizeof primary_overflow, cudaMemcpyDeviceToHost, st));
-        std::vector<int> local;
-        if (int rc = mt_count_rows(s->mt, s->hit_tri, W, n_rows, st, local)) return rc;
+        // the row hits of every view in one pass (view-major rows), then each view replays its own std::mt19937(seed) draws,
+        // as a separate render of that view would
+        std::vector<int> all_rows;
+        if (int rc = mt_count_rows(s->mt, s->hit_tri, W, n_views * n_rows, st, all_rows)) return rc;
         ++launches;
         if (primary_overflow) return rerender_after_overflow(frame_rows);
-        if (frame_rows) {
-            if (!mt::rows_valid(local.data(), n_rows, band_rows, bands.band_index, band_count, frame_rows->data(), H, W))
-                return fail(TRACER_ERR_STATE, "bundle-cull re-render: the closest-hit pass found other hits than the first pass");
-            mt_frame = *frame_rows;
-        } else if (int rc = mt_frame_rows(o, W, H, band_rows, band_count, local, mt_frame)) {
-            return rc;
+        for (int v = 0; v < n_views; ++v) {
+            const std::vector<int> local(all_rows.begin() + (size_t)v * n_rows, all_rows.begin() + (size_t)(v + 1) * n_rows);
+            if (frame_rows) {
+                if (!mt::rows_valid(local.data(), n_rows, band_rows, bands.band_index, band_count, frame_rows->data(), H, W))
+                    return fail(TRACER_ERR_STATE, "bundle-cull re-render: the closest-hit pass found other hits than the first pass");
+                mt_frame = *frame_rows;
+            } else if (int rc = mt_frame_rows(o, W, H, band_rows, band_count, local, mt_frame)) {
+                return rc;
+            }
+            const size_t off = (size_t)v * view_px;
+            if (int rc = mt_replay(s->mt, o.seed, s->h_light_F, mt_frame, W, band_rows, bands.band_index, band_count, n_rows,
+                                   s->hit_tri + off, s->faceid + off * L, st, launches, off))
+                return rc;
         }
-        if (int rc = mt_replay(s->mt, o.seed, s->h_light_F, mt_frame, W, band_rows, bands.band_index, band_count, n_rows, s->hit_tri,
-                               s->faceid, st, launches))
-            return rc;
     }
 
     // ---- lights: (finish k-1, set up k) -> group by light vertex -> first-occluder sweep ----
@@ -1399,7 +1487,7 @@ int render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32
                        s->ro,   s->rd,       s->re,      s->rt,    s->rj};
     for (int k = 0; k <= L; ++k) {
         trk::LightStepParams lp{};
-        lp.cam = dc, lp.bands = bands, lp.px = px;
+        lp.views = views, lp.bands = bands, lp.px = px;
         lp.li = trk::LightInfo{s->light_vbase, s->light_verts};
         lp.k = k, lp.L = L, lp.n_tris = s->n_tris;
         lp.tri_verts = s->tri_verts, lp.tri_normals = s->tri_normals, lp.tri_geom = s->tri_geom;

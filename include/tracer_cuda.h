@@ -212,6 +212,19 @@ int tracer_cuda_render_scene(tracer_scene_dev *scene, const tracer_camera *cam, 
                              const tracer_render_opts *opts, uint8_t *rgb_out);
 int tracer_cuda_last_stats(tracer_scene_dev *scene, tracer_frame_stats *out);
 
+/* n_views frames of one resident scene, one per camera, in one call.  rgb_out: n_views * height * width * 3 bytes,
+ * view-major, each view in PPM row order (host, or device with opts->rgb_out_is_device).  Debug outputs are view-major
+ * too ([n_views * height * width] ...), and with TRACER_RNG_EXPLICIT opts->faceid is [n_views][W*H*n_lights].
+ * View v is the frame tracer_cuda_render_scene gives for cams[v] with the same opts: packed bytes, hit ids, t, v,
+ * first occluders and the float accumulator, in every rng_mode (TRACER_RNG_MT19937: each view draws from its own
+ * std::mt19937(seed), as a separate run of the serial path would), with jittered samples, in the default and the BVH
+ * mode, with exhaustive_strict.  Refused with TRACER_ERR_INVALID: n_views < 1, cams NULL, band_count > 1, bundle_cull != 0,
+ * n_views * width * height above the per-call pixel limit.  Stats (tracer_cuda_last_stats) are totals over the call.
+ * The views share the camera-independent work of a frame: the shadow rays of every view go through one sweep per light
+ * vertex batch; only the closest-hit sweep runs per view (one eye table each). */
+int tracer_cuda_render_views(tracer_scene_dev *scene, const tracer_camera *cams, int32_t n_views, int32_t width,
+                             int32_t height, const tracer_render_opts *opts, uint8_t *rgb_out);
+
 /* ---- updating a resident scene between frames --------------------------------
  * Replaces vertices, normals, materials and spheres of a resident scene in place, without re-creating it.
  * Topology is fixed: the triangle, geometry, light and sphere counts, geom_tri_offset, light_geom and
