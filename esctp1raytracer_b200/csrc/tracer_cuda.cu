@@ -8,6 +8,7 @@
 #include <condition_variable>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <unordered_map>
@@ -250,12 +251,14 @@ void dev_free(T *&p) {
     t_pool->release((void *)p);
     p = nullptr;
 }
-template <typename T>
-int dev_grow(T *&p, size_t &cap, size_t n) {
+// Buffers of one capacity cap, grown to n elements each when n > cap (the old contents are lost); cap is 0 while any may be
+// missing, so that a failed grow is tried again by the next call
+template <typename... T>
+int dev_grow(size_t &cap, size_t n, T *&...p) {
     if (n <= cap) return 0;
-    dev_free(p);
+    (dev_free(p), ...);
     cap = 0;
-    if (int rc = dev_alloc(&p, n)) return rc;
+    if ((dev_alloc(&p, n) || ...)) return TRACER_ERR_NOMEM;
     cap = n;
     return 0;
 }
@@ -271,6 +274,23 @@ struct MtWork {
         dev_free(base), dev_free(ord);
         rank_cap = rows_cap = maps_cap = start_cap = fid_cap = words_cap = lights_cap = base_cap = ord_cap = 0;
     }
+};
+
+// The per-frame buffers of a scene, per pixel of the largest call so far (npx); dbg_occ and accum_total once a call needs them
+struct Workspace {
+    int npx = 0;
+    int *hit_tri = nullptr, *rj = nullptr, *list = nullptr, *list_b = nullptr, *faceid = nullptr, *dbg_occ = nullptr;
+    unsigned long long *best = nullptr, *best_occ = nullptr;
+    float *hit_t = nullptr, *hit_v = nullptr, *carry = nullptr, *nrm = nullptr, *accum = nullptr, *ro = nullptr, *rd = nullptr,
+          *re = nullptr, *rt = nullptr, *accum_total = nullptr;
+    uint8_t *rgb8 = nullptr;
+    void release() {
+        dev_free(hit_tri), dev_free(rj), dev_free(best), dev_free(best_occ), dev_free(list), dev_free(list_b), dev_free(faceid);
+        dev_free(hit_t), dev_free(hit_v), dev_free(carry), dev_free(nrm), dev_free(accum), dev_free(ro), dev_free(rd), dev_free(re);
+        dev_free(rt), dev_free(rgb8), dev_free(dbg_occ), dev_free(accum_total);
+        npx = 0;
+    }
+    trk::PixelState px() const { return {best, best_occ, hit_tri, hit_t, hit_v, carry, nrm, accum, ro, rd, re, rt, rj}; }
 };
 
 }  // namespace
@@ -294,7 +314,7 @@ struct tracer_scene_dev {
     void *box_work = nullptr; // bbox_partial_kernel's per-block bounds, then the 6 doubles of the box
     float4 *eye_table = nullptr, *light_tables = nullptr, *allcand_table = nullptr; // 48-byte three-row tables
     float4 *eye_span = nullptr, *light_spans = nullptr, *allcand_span = nullptr;    // 32-byte span tables (same slots)
-    int eye_cap = 1;                // views whose eye tables (both forms) eye_table / eye_span hold; grown on demand
+    size_t eye_table_cap = 0, eye_span_cap = 0; // float4 of eye_table / eye_span: the eye tables of one view or more
     trk::Cam *cams = nullptr;       // the call's cameras, one per view
     size_t cams_cap = 0;
     std::vector<double> table_lmax; // per (light vertex, cube face): reach bound it was built for, < 0 = not built
@@ -302,15 +322,8 @@ struct tracer_scene_dev {
     bool tables_resident = true;    // every light vertex has its own slot: tables are kept across lights and frames
     bool allcand_built = false;
     size_t table_stride = 0, span_stride = 0; // float4 per table
-    // per-frame workspace
-    int ws_npx = 0, ws_L = 0;
-    int *hit_tri = nullptr, *rj = nullptr, *list = nullptr, *list_b = nullptr, *faceid = nullptr, *dbg_occ = nullptr;
-    unsigned long long *best = nullptr, *best_occ = nullptr;
-    float *hit_t = nullptr, *hit_v = nullptr, *carry = nullptr, *nrm = nullptr, *accum = nullptr, *ro = nullptr,
-          *rd = nullptr, *re = nullptr, *rt = nullptr;
-    uint8_t *rgb8 = nullptr;
+    Workspace ws;
     MtWork mt;
-    float *accum_total = nullptr;
     // bundle-cull mode: candidate (ray<<32|triangle) buffers, their count, radix-sort scratch
     unsigned long long *cand_a = nullptr, *cand_b = nullptr, *cand_count = nullptr, *rkey = nullptr, *rkey_sorted = nullptr;
     int *blk_cnt = nullptr;            // order-preserving compaction: survivors per (group, block of CBLK entries)
@@ -318,12 +331,12 @@ struct tracer_scene_dev {
     cull::BlockBoxes *boxes = nullptr; // two-phase bundle cull: boxes of every ray block
     size_t boxes_cap = 0;
     int *iota = nullptr;
-    size_t pair_bytes = 0;
-    void *pair_tmp = nullptr;
-    int rkey_npx = 0;
-    size_t cand_cap = 0, sort_bytes = 0;
+    size_t pair_bytes = 0, pair_cap = 0;
+    unsigned char *pair_tmp = nullptr;
+    size_t rkey_cap = 0;
+    size_t cand_cap = 0, sort_bytes = 0, sort_cap = 0, count_cap = 0;
     int cull_grow = 1; // candidate buffers hold 24 * cull_grow pairs per ray (grown after an overflow)
-    void *sort_tmp = nullptr;
+    unsigned char *sort_tmp = nullptr;
     int *seg_count = nullptr, *seg_off = nullptr, *blk_off = nullptr, *cursor = nullptr, *cnt_b = nullptr, *work = nullptr,
         *n_slices = nullptr;
     int maxF = 0;
@@ -341,29 +354,25 @@ struct tracer_scene_dev {
 
 namespace {
 
-int ensure_workspace(tracer_scene_dev *s, int n_px, bool want_dbg_occ) {
-    const int L = std::max(1, s->n_lights);
-    if (n_px > s->ws_npx) {
-        dev_free(s->hit_tri), dev_free(s->rj), dev_free(s->best), dev_free(s->best_occ), dev_free(s->list), dev_free(s->list_b);
-        dev_free(s->faceid), dev_free(s->hit_t), dev_free(s->hit_v), dev_free(s->carry), dev_free(s->nrm), dev_free(s->accum);
-        dev_free(s->ro), dev_free(s->rd), dev_free(s->re), dev_free(s->rt), dev_free(s->rgb8);
-        dev_free(s->dbg_occ), dev_free(s->accum_total);
-        s->ws_npx = 0;
+// L: faceIDs (and first occluders) per pixel
+int ensure_workspace(Workspace &w, int n_px, int L, bool want_dbg_occ) {
+    if (n_px > w.npx) {
+        w.release();
         const size_t n = (size_t)n_px;
         int rc = 0;
-        rc |= dev_alloc(&s->hit_tri, n) | dev_alloc(&s->rj, n) | dev_alloc(&s->best, n) | dev_alloc(&s->best_occ, n);
-        rc |= dev_alloc(&s->list, n);
-        rc |= dev_alloc(&s->list_b, n);
-        rc |= dev_alloc(&s->faceid, n * L);
-        rc |= dev_alloc(&s->hit_t, n) | dev_alloc(&s->hit_v, n) | dev_alloc(&s->carry, n);
-        rc |= dev_alloc(&s->nrm, 3 * n) | dev_alloc(&s->accum, 3 * n + 16) | dev_alloc(&s->ro, 3 * n);
-        rc |= dev_alloc(&s->rd, 3 * n) | dev_alloc(&s->re, 2 * n) | dev_alloc(&s->rt, n);
-        rc |= dev_alloc(&s->rgb8, 3 * n + 64);
+        rc |= dev_alloc(&w.hit_tri, n) | dev_alloc(&w.rj, n) | dev_alloc(&w.best, n) | dev_alloc(&w.best_occ, n);
+        rc |= dev_alloc(&w.list, n);
+        rc |= dev_alloc(&w.list_b, n);
+        rc |= dev_alloc(&w.faceid, n * L);
+        rc |= dev_alloc(&w.hit_t, n) | dev_alloc(&w.hit_v, n) | dev_alloc(&w.carry, n);
+        rc |= dev_alloc(&w.nrm, 3 * n) | dev_alloc(&w.accum, 3 * n + 16) | dev_alloc(&w.ro, 3 * n);
+        rc |= dev_alloc(&w.rd, 3 * n) | dev_alloc(&w.re, 2 * n) | dev_alloc(&w.rt, n);
+        rc |= dev_alloc(&w.rgb8, 3 * n + 64);
         if (rc) return TRACER_ERR_NOMEM;
-        s->ws_npx = n_px;
+        w.npx = n_px;
     }
-    if (want_dbg_occ && !s->dbg_occ) {
-        if (dev_alloc(&s->dbg_occ, (size_t)s->ws_npx * L)) return TRACER_ERR_NOMEM;
+    if (want_dbg_occ && !w.dbg_occ) {
+        if (dev_alloc(&w.dbg_occ, (size_t)w.npx * L)) return TRACER_ERR_NOMEM;
     }
     return 0;
 }
@@ -470,29 +479,33 @@ int launch_shadow_light_t(Ctx &g, const trk::ShadowLightParams &p, unsigned *bar
 int launch_shadow_light(Ctx &g, bool ex, const trk::ShadowLightParams &p, unsigned *bar, cudaStream_t st) {
     return ex ? launch_shadow_light_t<true>(g, p, bar, st) : launch_shadow_light_t<false>(g, p, bar, st);
 }
-// qmode: sweep::MODE_SHAREDQ (no jitter), MODE_QBAR (jittered samples, span table) or MODE_OWNQ (jittered, three-row table)
+// Rays per thread R of each form of the closest-hit sweep, largest first: the primary_kernel instantiations there are.
+// qmode sweep::MODE_SHAREDQ: no jitter, the rays of a thread share one exact q (span table); MODE_QBAR: jittered samples
+// sharing a mean q (span table); MODE_OWNQ: jittered, every ray its own q (three-row table)
+template <int QMODE, int... Rs>
+struct RaysPerThread {
+    static constexpr int n = sizeof...(Rs);
+    static constexpr int r[] = {Rs...};
+};
+template <typename Fn>
+auto with_rays_per_thread(int qmode, Fn &&fn) {
+    if (qmode == sweep::MODE_OWNQ) return fn(RaysPerThread<sweep::MODE_OWNQ, 12, 8, 4, 2>{});
+    if (qmode == sweep::MODE_QBAR) return fn(RaysPerThread<sweep::MODE_QBAR, 32, 16, 8, 4, 2>{});
+    return fn(RaysPerThread<sweep::MODE_SHAREDQ, 64, 32, 24, 16, 8, 4, 2>{});
+}
+// the form's instantiation for r rays per thread (its last, 2, for an r it lacks)
+template <int QMODE, int R, int... Rs>
+int launch_primary_r(int r, bool ex, const trk::PrimaryParams &p, bool views, int grid, cudaStream_t st) {
+    if constexpr (sizeof...(Rs) > 0)
+        if (r != R) return launch_primary_r<QMODE, Rs...>(r, ex, p, views, grid, st);
+    return ex ? launch_primary_q<R, true, QMODE>(p, views, grid, st) : launch_primary_q<R, false, QMODE>(p, views, grid, st);
+}
+template <int QMODE, int... Rs>
+int launch_primary_of(RaysPerThread<QMODE, Rs...>, int r, bool ex, const trk::PrimaryParams &p, bool views, int grid, cudaStream_t st) {
+    return launch_primary_r<QMODE, Rs...>(r, ex, p, views, grid, st);
+}
 int launch_primary(int R, bool ex, int qmode, const trk::PrimaryParams &p, bool views, int grid, cudaStream_t st) {
-    constexpr int OQ = sweep::MODE_OWNQ, SQ = sweep::MODE_SHAREDQ, QB = sweep::MODE_QBAR;
-    if (qmode == OQ) { // every ray its own q, three-row table
-        if (R == 12) return ex ? launch_primary_q<12, true, OQ>(p, views, grid, st) : launch_primary_q<12, false, OQ>(p, views, grid, st);
-        if (R == 8) return ex ? launch_primary_q<8, true, OQ>(p, views, grid, st) : launch_primary_q<8, false, OQ>(p, views, grid, st);
-        if (R == 4) return ex ? launch_primary_q<4, true, OQ>(p, views, grid, st) : launch_primary_q<4, false, OQ>(p, views, grid, st);
-        return ex ? launch_primary_q<2, true, OQ>(p, views, grid, st) : launch_primary_q<2, false, OQ>(p, views, grid, st);
-    }
-    if (qmode == QB) {
-        if (R == 32) return ex ? launch_primary_q<32, true, QB>(p, views, grid, st) : launch_primary_q<32, false, QB>(p, views, grid, st);
-        if (R == 16) return ex ? launch_primary_q<16, true, QB>(p, views, grid, st) : launch_primary_q<16, false, QB>(p, views, grid, st);
-        if (R == 8) return ex ? launch_primary_q<8, true, QB>(p, views, grid, st) : launch_primary_q<8, false, QB>(p, views, grid, st);
-        if (R == 4) return ex ? launch_primary_q<4, true, QB>(p, views, grid, st) : launch_primary_q<4, false, QB>(p, views, grid, st);
-        return ex ? launch_primary_q<2, true, QB>(p, views, grid, st) : launch_primary_q<2, false, QB>(p, views, grid, st);
-    }
-    if (R == 64) return ex ? launch_primary_q<64, true, SQ>(p, views, grid, st) : launch_primary_q<64, false, SQ>(p, views, grid, st);
-    if (R == 32) return ex ? launch_primary_q<32, true, SQ>(p, views, grid, st) : launch_primary_q<32, false, SQ>(p, views, grid, st);
-    if (R == 24) return ex ? launch_primary_q<24, true, SQ>(p, views, grid, st) : launch_primary_q<24, false, SQ>(p, views, grid, st);
-    if (R == 16) return ex ? launch_primary_q<16, true, SQ>(p, views, grid, st) : launch_primary_q<16, false, SQ>(p, views, grid, st);
-    if (R == 8) return ex ? launch_primary_q<8, true, SQ>(p, views, grid, st) : launch_primary_q<8, false, SQ>(p, views, grid, st);
-    if (R == 4) return ex ? launch_primary_q<4, true, SQ>(p, views, grid, st) : launch_primary_q<4, false, SQ>(p, views, grid, st);
-    return ex ? launch_primary_q<2, true, SQ>(p, views, grid, st) : launch_primary_q<2, false, SQ>(p, views, grid, st);
+    return with_rays_per_thread(qmode, [&](auto rays) { return launch_primary_of(rays, R, ex, p, views, grid, st); });
 }
 // Work decomposition of a sweep: R rays per thread (8 preferred: best amortisation of the row loads) and
 // n_slices triangle slices, chosen so that ray blocks x slices keeps every SM busy for several items.
@@ -510,24 +523,19 @@ int items_per_cta() {
     return forced > 0 ? forced : 96;
 }
 
-Decomp pick_decomp(int64_t n_rays, int n_tiles, int n_sms, int forced_R, int extra_blocks, int qmode) {
+Decomp pick_decomp(int64_t n_rays, int n_tiles, int n_sms, int forced_R, int qmode) {
     const int slices_possible = std::max(1, n_tiles / 4); // at least 4 tiles per slice
-    auto blocks_for = [&](int R) {
-        return (int)((n_rays + (int64_t)sweep::NT * R - 1) / ((int64_t)sweep::NT * R)) + extra_blocks;
-    };
+    auto blocks_for = [&](int R) { return (int)((n_rays + (int64_t)sweep::NT * R - 1) / ((int64_t)sweep::NT * R)); };
     Decomp d{2, blocks_for(2), 1};
-    // rays per thread: span form with one exact q (no jitter) 64, 32, 16, 8, 4 or 2 (24 on request); span form with a
-    // shared mean q (jittered samples) 32, 16, 8, 4 or 2; three-row form (own q) 12, 8, 4 or 2
+    // rays per thread: forced_R when the form has it, else the largest that gives enough work items (24 only on request)
     // (C4 closest-hit sweep on one B200: 997 ms at 16, 944 at 24, 905 at 32 with the saturating span loop)
-    const bool own_q = qmode == sweep::MODE_OWNQ, shared_q = qmode == sweep::MODE_SHAREDQ;
-    const int huge = shared_q ? 64 : 0, big = own_q ? 12 : 32, mid = own_q ? 8 : 16;
-    if (forced_R == 2 || forced_R == 4 || forced_R == 8 || forced_R == mid || forced_R == big ||
-        (shared_q && (forced_R == 24 || forced_R == 64))) {
+    const auto [rs, n_rs] = with_rays_per_thread(qmode, [](auto rays) { return std::make_pair(rays.r, rays.n); });
+    if (std::find(rs, rs + n_rs, forced_R) != rs + n_rs) {
         d.R = forced_R, d.n_blocks = blocks_for(forced_R);
     } else {
-        for (int R : {huge, big, mid, 8, 4, 2}) {
-            if (!R) continue;
-            d.R = R, d.n_blocks = blocks_for(R);
+        for (const int *R = rs; R != rs + n_rs; ++R) {
+            if (*R == 24) continue;
+            d.R = *R, d.n_blocks = blocks_for(*R);
             if ((int64_t)d.n_blocks * slices_possible >= 4 * (int64_t)n_sms) break;
         }
     }
@@ -688,6 +696,37 @@ trk::TableParam face_param(const float *o, int f, double lmax) {
     return tp;
 }
 
+// The shadow filter tables (both forms) of cube face `face` of light vertex vtx, in table slot `slot`: vtx itself when every
+// vertex has its own slot (tables_resident: kept across lights and frames), else its place in the batch of vertices whose
+// tables the slots hold (rebuilt every time).  A full build serves shadow segments up to `need`, with 1.5x head-room so
+// that camera moves rarely trigger a rebuild; a resident table already built for `need` or more is kept.  count >= 0 (a
+// scene update): only rows [first, first + count) of a built resident table, for the bound it was built with.
+int build_face_table(tracer_scene_dev *s, int vtx, int face, size_t slot, double need, cudaStream_t st, int &launches, int first = 0,
+                     int count = -1) {
+    double lmax = need * 1.5;
+    if (s->tables_resident) {
+        double &built = s->table_lmax[(size_t)vtx * 6 + face];
+        if (count >= 0) lmax = built;
+        else if (built >= need) return 0;
+        else built = lmax;
+    }
+    const trk::TableParam tp = face_param(&s->h_light_verts[3 * (size_t)vtx], face, lmax);
+    if (int rc = build_table(s, tp, s->light_tables + (slot * 6 + face) * s->table_stride, s->light_spans + (slot * 6 + face) * s->span_stride,
+                             st, first, count))
+        return rc;
+    ++launches;
+    return 0;
+}
+
+// The table of every light vertex's last ray group (trk::NFACE - 1), every row a candidate: built once per scene
+int ensure_allcand_table(tracer_scene_dev *s, cudaStream_t st, int &launches) {
+    if (s->allcand_built) return 0;
+    trk::build_allcand_table<<<(s->n_pad + 255) / 256, 256, 0, st>>>(s->n_tris, s->n_pad, s->allcand_table, s->allcand_span);
+    CK_CUDA(cudaGetLastError());
+    s->allcand_built = true, ++launches;
+    return 0;
+}
+
 // s->bb_lo, s->bb_hi from the scene's device arrays (bbox_partial_kernel): two launches on st, one read-back, a synchronise
 int scene_bbox(tracer_scene_dev *s, cudaStream_t st) {
     if (!s->box_work && !(s->box_work = t_pool->alloc(sizeof(BoxArg) * 6 * BOX_MAX_BLOCKS + sizeof(double) * 6)))
@@ -824,15 +863,12 @@ void tracer_cuda_scene_destroy(tracer_scene_dev *s) {
     dev_free(s->tri_geom), dev_free(s->geom_has_normals), dev_free(s->spheres), dev_free(s->light_vbase);
     dev_free(s->light_verts), dev_free(s->eye_table), dev_free(s->light_tables), dev_free(s->allcand_table);
     dev_free(s->eye_span), dev_free(s->light_spans), dev_free(s->allcand_span), dev_free(s->cams);
-    dev_free(s->hit_tri), dev_free(s->rj), dev_free(s->best), dev_free(s->best_occ), dev_free(s->list), dev_free(s->list_b);
-    dev_free(s->faceid), dev_free(s->dbg_occ), dev_free(s->cnt_b), dev_free(s->accum_total);
-    dev_free(s->hit_t), dev_free(s->hit_v), dev_free(s->carry), dev_free(s->nrm), dev_free(s->accum);
-    dev_free(s->ro), dev_free(s->rd), dev_free(s->re), dev_free(s->rt), dev_free(s->rgb8);
-    dev_free(s->seg_count), dev_free(s->seg_off), dev_free(s->blk_off), dev_free(s->cursor), dev_free(s->work);
+    s->ws.release();
+    dev_free(s->seg_count), dev_free(s->seg_off), dev_free(s->blk_off), dev_free(s->cursor), dev_free(s->cnt_b), dev_free(s->work);
     dev_free(s->n_slices);
     dev_free(s->cand_a), dev_free(s->cand_b), dev_free(s->cand_count), dev_free(s->rkey), dev_free(s->rkey_sorted), dev_free(s->iota);
     dev_free(s->boxes), dev_free(s->blk_cnt);
-    t_pool->release(s->sort_tmp), t_pool->release(s->pair_tmp);
+    dev_free(s->sort_tmp), dev_free(s->pair_tmp);
     dev_free(s->counters);
     dev_free(s->bvh_nodes), dev_free(s->bvh_keys);
     t_pool->release(s->box_work);
@@ -870,67 +906,45 @@ int scene_create_on(Ctx &g, const tracer_scene_flat *sc, tracer_scene_dev **out)
     for (int g2 = 0; g2 < G && sc->geom_has_normals; ++g2) any_normals |= sc->geom_has_normals[g2] != 0;
     if (any_normals && !sc->tri_normals) return fail(TRACER_ERR_INVALID, "geom_has_normals set but tri_normals is null");
 
+    // lives until the upload has been waited for: declared before the scene, whose destroy waits for the device
+    std::vector<int> tg((size_t)std::max(N, 1));
     CK_CUDA(cudaSetDevice(g.device));
-    auto *s = new tracer_scene_dev();
+    // destroyed on every failure return, handed out on success
+    std::unique_ptr<tracer_scene_dev, void (*)(tracer_scene_dev *)> s(new tracer_scene_dev(), tracer_cuda_scene_destroy);
     s->ctx = &g;
     s->n_geoms = G, s->n_tris = N, s->n_lights = sc->n_lights, s->n_spheres = sc->n_spheres;
     s->n_pad = std::max(1, (N + cull::CTILE - 1) / cull::CTILE) * cull::CTILE; // multiple of both tile sizes
     s->table_stride = (size_t)s->n_pad * 3, s->span_stride = (size_t)s->n_pad * 2;
-#define TRY(x)                         \
-    do {                               \
-        int rc_ = (x);                 \
-        if (rc_) {                     \
-            tracer_cuda_scene_destroy(s); \
-            return rc_;                \
-        }                              \
-    } while (0)
-#define TRY_CUDA(call)                                                                                      \
-    do {                                                                                                    \
-        cudaError_t e_ = (call);                                                                            \
-        if (e_ != cudaSuccess) {                                                                            \
-            tracer_cuda_scene_destroy(s);                                                                   \
-            return fail(TRACER_ERR_CUDA, std::string(#call) + " failed (tracer_cuda.cu:" + std::to_string(__LINE__) + "): " + cudaGetErrorString(e_)); \
-        }                                                                                                   \
-    } while (0)
-    TRY(dev_alloc(&s->tri_verts, (size_t)N * 9));
-    TRY_CUDA(cudaMemcpyAsync(s->tri_verts, sc->tri_verts, (size_t)N * 9 * sizeof(float), cudaMemcpyHostToDevice, g.stream));
+    if (int rc = dev_alloc(&s->tri_verts, (size_t)N * 9)) return rc;
+    CK_CUDA(cudaMemcpyAsync(s->tri_verts, sc->tri_verts, (size_t)N * 9 * sizeof(float), cudaMemcpyHostToDevice, g.stream));
     if (any_normals) {
-        TRY(dev_alloc(&s->tri_normals, (size_t)N * 9));
-        TRY_CUDA(cudaMemcpyAsync(s->tri_normals, sc->tri_normals, (size_t)N * 9 * sizeof(float), cudaMemcpyHostToDevice, g.stream));
-        TRY(dev_alloc(&s->geom_has_normals, (size_t)G));
-        TRY_CUDA(cudaMemcpyAsync(s->geom_has_normals, sc->geom_has_normals, (size_t)G * sizeof(int), cudaMemcpyHostToDevice, g.stream));
+        if (int rc = dev_alloc(&s->tri_normals, (size_t)N * 9)) return rc;
+        CK_CUDA(cudaMemcpyAsync(s->tri_normals, sc->tri_normals, (size_t)N * 9 * sizeof(float), cudaMemcpyHostToDevice, g.stream));
+        if (int rc = dev_alloc(&s->geom_has_normals, (size_t)G)) return rc;
+        CK_CUDA(cudaMemcpyAsync(s->geom_has_normals, sc->geom_has_normals, (size_t)G * sizeof(int), cudaMemcpyHostToDevice, g.stream));
     }
-    TRY(dev_alloc(&s->geom_material, (size_t)G * 13));
-    TRY_CUDA(cudaMemcpyAsync(s->geom_material, sc->geom_material, (size_t)G * 13 * sizeof(float), cudaMemcpyHostToDevice, g.stream));
-    std::vector<int> tg((size_t)std::max(N, 1)); // lives until the upload has been waited for
-    {
-        for (int g2 = 0; g2 < G; ++g2)
-            for (int t = sc->geom_tri_offset[g2]; t < sc->geom_tri_offset[g2 + 1]; ++t) tg[t] = g2;
-        TRY(dev_alloc(&s->tri_geom, (size_t)N));
-        TRY_CUDA(cudaMemcpyAsync(s->tri_geom, tg.data(), (size_t)N * sizeof(int), cudaMemcpyHostToDevice, g.stream));
-    }
+    if (int rc = dev_alloc(&s->geom_material, (size_t)G * 13)) return rc;
+    CK_CUDA(cudaMemcpyAsync(s->geom_material, sc->geom_material, (size_t)G * 13 * sizeof(float), cudaMemcpyHostToDevice, g.stream));
+    for (int g2 = 0; g2 < G; ++g2)
+        for (int t = sc->geom_tri_offset[g2]; t < sc->geom_tri_offset[g2 + 1]; ++t) tg[t] = g2;
+    if (int rc = dev_alloc(&s->tri_geom, (size_t)N)) return rc;
+    CK_CUDA(cudaMemcpyAsync(s->tri_geom, tg.data(), (size_t)N * sizeof(int), cudaMemcpyHostToDevice, g.stream));
     if (sc->n_spheres > 0) {
-        TRY(dev_alloc(&s->spheres, (size_t)sc->n_spheres));
-        TRY_CUDA(cudaMemcpyAsync(s->spheres, sc->sphere_cr, (size_t)sc->n_spheres * 4 * sizeof(float), cudaMemcpyHostToDevice, g.stream));
-        TRY(dev_alloc(&s->sphere_material, (size_t)sc->n_spheres * 13));
-        TRY_CUDA(cudaMemcpy(s->sphere_material, sc->sphere_material, (size_t)sc->n_spheres * 13 * sizeof(float),
+        if (int rc = dev_alloc(&s->spheres, (size_t)sc->n_spheres)) return rc;
+        CK_CUDA(cudaMemcpyAsync(s->spheres, sc->sphere_cr, (size_t)sc->n_spheres * 4 * sizeof(float), cudaMemcpyHostToDevice, g.stream));
+        if (int rc = dev_alloc(&s->sphere_material, (size_t)sc->n_spheres * 13)) return rc;
+        CK_CUDA(cudaMemcpy(s->sphere_material, sc->sphere_material, (size_t)sc->n_spheres * 13 * sizeof(float),
                             cudaMemcpyHostToDevice));
     }
     // bounding box of everything a ray can start from or end at, from the uploaded arrays (the kernel an update uses too)
-    TRY(scene_bbox(s, g.stream));
+    if (int rc = scene_bbox(s.get(), g.stream)) return rc;
     // lights: light.vertex[faceID], faceID in [0, F) (main.cpp:743-751) = the first F de-indexed vertices
     s->h_light_vbase.assign(1, 0);
     for (int l = 0; l < sc->n_lights; ++l) {
         const int lg = sc->light_geom[l];
-        if (lg < 0 || lg >= G) {
-            tracer_cuda_scene_destroy(s);
-            return fail(TRACER_ERR_INVALID, "light_geom index out of range");
-        }
+        if (lg < 0 || lg >= G) return fail(TRACER_ERR_INVALID, "light_geom index out of range");
         const int t0 = sc->geom_tri_offset[lg], F = sc->geom_tri_offset[lg + 1] - t0;
-        if (F <= 0) {
-            tracer_cuda_scene_destroy(s);
-            return fail(TRACER_ERR_INVALID, "light geometry has no faces");
-        }
+        if (F <= 0) return fail(TRACER_ERR_INVALID, "light geometry has no faces");
         s->h_light_F.push_back(F);
         s->h_light_t0.push_back(t0);
         for (int f = 0; f < F; ++f)
@@ -939,10 +953,10 @@ int scene_create_on(Ctx &g, const tracer_scene_flat *sc, tracer_scene_dev **out)
         s->maxF = std::max(s->maxF, F);
     }
     s->V = s->h_light_vbase.back();
-    TRY(dev_alloc(&s->light_vbase, s->h_light_vbase.size()));
-    TRY_CUDA(cudaMemcpyAsync(s->light_vbase, s->h_light_vbase.data(), s->h_light_vbase.size() * sizeof(int), cudaMemcpyHostToDevice, g.stream));
-    TRY(dev_alloc(&s->light_verts, s->h_light_verts.size()));
-    TRY_CUDA(cudaMemcpyAsync(s->light_verts, s->h_light_verts.data(), s->h_light_verts.size() * sizeof(float), cudaMemcpyHostToDevice, g.stream));
+    if (int rc = dev_alloc(&s->light_vbase, s->h_light_vbase.size())) return rc;
+    CK_CUDA(cudaMemcpyAsync(s->light_vbase, s->h_light_vbase.data(), s->h_light_vbase.size() * sizeof(int), cudaMemcpyHostToDevice, g.stream));
+    if (int rc = dev_alloc(&s->light_verts, s->h_light_verts.size())) return rc;
+    CK_CUDA(cudaMemcpyAsync(s->light_verts, s->h_light_verts.data(), s->h_light_verts.size() * sizeof(float), cudaMemcpyHostToDevice, g.stream));
     {   // Filter tables of the shadow sweeps: 6 cube-face tables of 48 B per triangle for every light vertex.  Two quad
         // lights need 0.6 GB at 1M triangles; an emissive MESH with hundreds of faces would need more than the GPU has.
         // Budget = half of the free HBM: when all vertices fit, every vertex owns a slot and its tables are built once
@@ -958,33 +972,29 @@ int scene_create_on(Ctx &g, const tracer_scene_flat *sc, tracer_scene_dev **out)
         s->tables_resident = (size_t)s->V <= fit;
         s->table_slots = (int)std::min<size_t>(fit, (size_t)trk::SL_MAXF / trk::NFACE);
     }
-    TRY(dev_alloc(&s->eye_table, s->table_stride));
-    TRY(dev_alloc(&s->light_tables, s->table_stride * 6 * (size_t)std::max(1, s->tables_resident ? s->V : s->table_slots)));
-    TRY(dev_alloc(&s->allcand_table, s->table_stride));
-    TRY(dev_alloc(&s->eye_span, s->span_stride));
-    TRY(dev_alloc(&s->light_spans, s->span_stride * 6 * (size_t)std::max(1, s->tables_resident ? s->V : s->table_slots)));
-    TRY(dev_alloc(&s->allcand_span, s->span_stride));
+    if (int rc = dev_grow(s->eye_table_cap, s->table_stride, s->eye_table)) return rc;
+    if (int rc = dev_alloc(&s->light_tables, s->table_stride * 6 * (size_t)std::max(1, s->tables_resident ? s->V : s->table_slots))) return rc;
+    if (int rc = dev_alloc(&s->allcand_table, s->table_stride)) return rc;
+    if (int rc = dev_grow(s->eye_span_cap, s->span_stride, s->eye_span)) return rc;
+    if (int rc = dev_alloc(&s->light_spans, s->span_stride * 6 * (size_t)std::max(1, s->tables_resident ? s->V : s->table_slots))) return rc;
+    if (int rc = dev_alloc(&s->allcand_span, s->span_stride)) return rc;
     s->table_lmax.assign((size_t)6 * s->V, -1.0);
     const size_t n_groups = (size_t)s->maxF * trk::NFACE;
-    TRY(dev_alloc(&s->seg_count, n_groups + 1));
-    TRY(dev_alloc(&s->seg_off, n_groups + 2));
-    TRY(dev_alloc(&s->blk_off, n_groups + 2));
-    TRY(dev_alloc(&s->cursor, n_groups + 1));
-    TRY(dev_alloc(&s->cnt_b, n_groups + 1));
-    TRY(dev_alloc(&s->work, (size_t)WORK_INTS));
-    TRY(dev_alloc(&s->n_slices, 1));
-    TRY(dev_alloc(&s->counters, 1));
-    for (auto &e : s->ev) TRY_CUDA(cudaEventCreate(&e));
+    if (int rc = dev_alloc(&s->seg_count, n_groups + 1)) return rc;
+    if (int rc = dev_alloc(&s->seg_off, n_groups + 2)) return rc;
+    if (int rc = dev_alloc(&s->blk_off, n_groups + 2)) return rc;
+    if (int rc = dev_alloc(&s->cursor, n_groups + 1)) return rc;
+    if (int rc = dev_alloc(&s->cnt_b, n_groups + 1)) return rc;
+    if (int rc = dev_alloc(&s->work, (size_t)WORK_INTS)) return rc;
+    if (int rc = dev_alloc(&s->n_slices, 1)) return rc;
+    if (int rc = dev_alloc(&s->counters, 1)) return rc;
+    for (auto &e : s->ev) CK_CUDA(cudaEventCreate(&e));
     s->ev_shadow.resize(2 * (size_t)std::max(1, s->n_lights));
-    for (auto &e : s->ev_shadow) TRY_CUDA(cudaEventCreate(&e));
+    for (auto &e : s->ev_shadow) CK_CUDA(cudaEventCreate(&e));
     // uploads were queued on the context's stream (truly asynchronous from pinned host memory): one wait for all
-    if (cudaError_t e_ = cudaStreamSynchronize(g.stream); e_ != cudaSuccess) {
-        tracer_cuda_scene_destroy(s);
+    if (cudaError_t e_ = cudaStreamSynchronize(g.stream); e_ != cudaSuccess)
         return fail(TRACER_ERR_CUDA, std::string("scene upload failed: ") + cudaGetErrorString(e_));
-    }
-#undef TRY
-#undef TRY_CUDA
-    *out = s;
+    *out = s.release();
     return TRACER_OK;
 }
 }  // namespace
@@ -995,7 +1005,7 @@ namespace {
 int mt_count_rows(MtWork &m, const int *hit_tri, int W, int n_rows, cudaStream_t st, std::vector<int> &local) {
     local.assign((size_t)n_rows, 0);
     if (n_rows == 0) return 0;
-    if (dev_grow(m.rank, m.rank_cap, (size_t)n_rows * W) || dev_grow(m.row_hits, m.rows_cap, (size_t)n_rows)) return TRACER_ERR_NOMEM;
+    if (dev_grow(m.rank_cap, (size_t)n_rows * W, m.rank) || dev_grow(m.rows_cap, (size_t)n_rows, m.row_hits)) return TRACER_ERR_NOMEM;
     mt::row_rank_kernel<<<n_rows, mt::SCAN_THREADS, 0, st>>>(hit_tri, W, m.rank, m.row_hits);
     CK_CUDA(cudaGetLastError());
     CK_CUDA(cudaMemcpyAsync(local.data(), m.row_hits, sizeof(int) * (size_t)n_rows, cudaMemcpyDeviceToHost, st));
@@ -1029,8 +1039,8 @@ int mt_replay(MtWork &m, uint32_t seed, const std::vector<int> &faces, const std
     if (T == 0) return 0;
     std::vector<uint32_t> lights((size_t)2 * L);
     for (int l = 0; l < L; ++l) lights[l] = (uint32_t)faces[l], lights[L + l] = mt::threshold((uint32_t)faces[l]);
-    if (dev_grow(m.lights, m.lights_cap, lights.size()) || dev_grow(m.base, m.base_cap, base.size()) ||
-        dev_grow(m.fid_ord, m.fid_cap, (size_t)T * L))
+    if (dev_grow(m.lights_cap, lights.size(), m.lights) || dev_grow(m.base_cap, base.size(), m.base) ||
+        dev_grow(m.fid_cap, (size_t)T * L, m.fid_ord))
         return TRACER_ERR_NOMEM;
     CK_CUDA(cudaMemcpyAsync(m.lights, lights.data(), sizeof(uint32_t) * lights.size(), cudaMemcpyHostToDevice, st));
     CK_CUDA(cudaMemcpyAsync(m.base, base.data(), sizeof(int64_t) * base.size(), cudaMemcpyHostToDevice, st));
@@ -1038,8 +1048,8 @@ int mt_replay(MtWork &m, uint32_t seed, const std::vector<int> &faces, const std
     int64_t D = 3 * (int64_t)L * T, C = 0, n_chunks = 0;
     for (;;) {
         C = std::max<int64_t>(256, (D + 2047) / 2048), n_chunks = (D + C - 1) / C;
-        if (dev_grow(m.words, m.words_cap, (size_t)D) || dev_grow(m.maps, m.maps_cap, (size_t)(2 * n_chunks * S)) ||
-            dev_grow(m.start, m.start_cap, (size_t)n_chunks) || dev_grow(m.ord, m.ord_cap, (size_t)n_chunks + 1))
+        if (dev_grow(m.words_cap, (size_t)D, m.words) || dev_grow(m.maps_cap, (size_t)(2 * n_chunks * S), m.maps) ||
+            dev_grow(m.start_cap, (size_t)n_chunks, m.start) || dev_grow(m.ord_cap, (size_t)n_chunks + 1, m.ord))
             return TRACER_ERR_NOMEM;
         mt::stream_kernel<<<1, mt::GEN_THREADS, 0, st>>>(seed, D, m.words);
         CK_CUDA(cudaGetLastError());
@@ -1065,114 +1075,119 @@ int mt_replay(MtWork &m, uint32_t seed, const std::vector<int> &faces, const std
     return 0;
 }
 
-// n_views frames of one scene, one per camera, in one call (V = 1: tracer_cuda_render_scene).  The call's pixels run view-major
-// (k = view * W * n_rows + local); every per-pixel buffer, sort and list spans all of them, and the shadow sweeps take the
-// rays of every view at once.  Only the closest-hit sweep is per view: one eye table each, in groups (DESIGN §4e).
-// frame_rows: the frame's row hit counts when the caller already has them: the bundle-cull mode's re-render of a frame whose
-// closest-hit pass was complete but whose shadow candidates overflowed (same hits; the exchange hook runs once per frame)
-int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, int32_t W, int32_t H, const tracer_render_opts *opts_in,
-                 uint8_t *rgb_out, const std::vector<int> *frame_rows);
-
 // Eye tables kept per call: views in groups whose tables (both forms, n_pad x 80 B per view) fit a quarter of the free
 // device memory, one closest-hit launch per group.  (TRACER_VIEW_GROUP caps the group size: development/test knob.)
 int view_group_size(tracer_scene_dev *s, int n_views) {
     const char *e = std::getenv("TRACER_VIEW_GROUP");
     const int cap = e ? std::max(1, std::atoi(e)) : INT_MAX;
-    if (n_views <= s->eye_cap) return std::min(n_views, cap);
+    const size_t held = s->eye_table_cap / s->table_stride; // views whose tables the scene already holds
+    if ((size_t)n_views <= held) return std::min(n_views, cap);
     size_t free_b = 0, total_b = 0;
     cudaMemGetInfo(&free_b, &total_b);
     const size_t per_view = (s->table_stride + s->span_stride) * sizeof(float4);
-    const size_t fit = std::max<size_t>((size_t)s->eye_cap, free_b / 4 / per_view);
+    const size_t fit = std::max<size_t>(held, free_b / 4 / per_view);
     return (int)std::max<size_t>(1, std::min<size_t>({fit, (size_t)cap, (size_t)n_views}));
 }
-}  // namespace
 
-extern "C" {
-
-int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32_t H,
-                             const tracer_render_opts *opts_in, uint8_t *rgb_out) {
-    return render_views(s, cam, 1, W, H, opts_in, rgb_out, nullptr);
-}
-
-int tracer_cuda_render_views(tracer_scene_dev *s, const tracer_camera *cams, int32_t n_views, int32_t W, int32_t H,
-                             const tracer_render_opts *opts_in, uint8_t *rgb_out) {
-    if (n_views < 1) return fail(TRACER_ERR_INVALID, "n_views must be >= 1");
-    if (!cams) return fail(TRACER_ERR_INVALID, "null cameras");
-    if (opts_in) {
-        tracer_render_opts o;
-        std::memset(&o, 0, sizeof o);
-        std::memcpy(&o, opts_in, std::min<size_t>(sizeof o, opts_in->struct_size ? opts_in->struct_size : sizeof o));
-        if (o.band_count > 1) return fail(TRACER_ERR_INVALID, "tracer_cuda_render_views renders whole views: band_count must be <= 1");
-        if (o.bundle_cull != 0) return fail(TRACER_ERR_INVALID, "tracer_cuda_render_views does not combine with bundle_cull");
-    }
-    return render_views(s, cams, n_views, W, H, opts_in, rgb_out, nullptr);
-}
-}  // extern "C"
-
-namespace {
-int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, int32_t W, int32_t H, const tracer_render_opts *opts_in,
-                 uint8_t *rgb_out, const std::vector<int> *frame_rows) {
-    if (!s || !cams || !rgb_out) return fail(TRACER_ERR_INVALID, "null argument");
-    if (!s->ctx || !s->ctx->inited) return fail(TRACER_ERR_NO_DEVICE, "tracer_cuda_init not called");
-    Ctx &g = *s->ctx;
-    t_pool = &g.pool;
-    if (W < 2 || H < 2) return fail(TRACER_ERR_INVALID, "width and height must be >= 2 (the reference divides by W-1, H-1)");
-    // per-pixel planes are indexed with int (3 planes of n_px floats): keep 3 * n_px below 2^31
-    if ((int64_t)n_views * W * H > (int64_t)700 * 1000 * 1000)
-        return fail(TRACER_ERR_INVALID, "frame too large (limit 7e8 pixels per call, over all views; render bands or fewer views)");
+// The caller's options; fields past a caller's struct_size are 0
+tracer_render_opts read_opts(const tracer_render_opts *in) {
     tracer_render_opts o;
     std::memset(&o, 0, sizeof o);
-    if (opts_in) std::memcpy(&o, opts_in, std::min<size_t>(sizeof o, opts_in->struct_size ? opts_in->struct_size : sizeof o));
-    // extension (parity unpinned): samples_per_pixel = n*n stratified jittered samples per pixel
-    int spp_n = 1;
-    if (o.samples_per_pixel > 1) {
-        spp_n = (int)std::lround(std::sqrt((double)o.samples_per_pixel));
-        if (spp_n * spp_n != o.samples_per_pixel || spp_n > 16)
-            return fail(TRACER_ERR_INVALID, "samples_per_pixel must be a square number <= 256");
-        if (o.rng_mode == TRACER_RNG_MT19937)
-            return fail(TRACER_ERR_INVALID, "TRACER_RNG_MT19937 reproduces the 1-sample serial path only");
-    }
-    const int S = spp_n * spp_n;
-    const int band_count = o.band_count <= 1 ? 1 : o.band_count;
-    const int band_rows = band_count > 1 ? o.band_rows : H;
-    if (band_count > 1 && (band_rows <= 0 || o.band_index < 0 || o.band_index >= band_count))
-        return fail(TRACER_ERR_INVALID, "bad band selection");
-    if (o.rng_mode == TRACER_RNG_MT19937 && band_count > 1 && !o.row_hits_exchange)
-        return fail(TRACER_ERR_INVALID, "TRACER_RNG_MT19937 with band_count > 1 needs opts->row_hits_exchange (the other bands' row hit counts)");
-    if (o.rng_mode == TRACER_RNG_EXPLICIT && !o.faceid && s->n_lights > 0)
-        return fail(TRACER_ERR_INVALID, "TRACER_RNG_EXPLICIT needs opts->faceid");
-    if (o.rng_mode < 0 || o.rng_mode > 2) return fail(TRACER_ERR_INVALID, "bad rng_mode");
-    if (o.accel < 0 || o.accel > 1) return fail(TRACER_ERR_INVALID, "bad accel (0 = sweeps, 1 = BVH)");
-    const bool use_bvh = o.accel == 1;
-    if (use_bvh && (o.bundle_cull != 0 || o.exhaustive_strict != 0))
-        return fail(TRACER_ERR_INVALID, "accel = 1 (BVH) does not combine with bundle_cull or exhaustive_strict (a debug mode of the sweeps' filter)");
-    const int n_rows = tracer_band_row_count(H, band_rows, band_count > 1 ? o.band_index : 0, band_count);
-    const int view_px = n_rows * W, n_px = n_views * view_px;
-    const int L = s->n_lights;
+    if (in) std::memcpy(&o, in, std::min<size_t>(sizeof o, in->struct_size ? in->struct_size : sizeof o));
+    return o;
+}
+
+// ---- one render call: n_views frames of one scene, one per camera (V = 1: tracer_cuda_render_scene) -------------------------
+// The call's pixels run view-major (k = view * W * n_rows + local); every per-pixel buffer, sort and list spans all of them,
+// and the shadow sweeps take the rays of every view at once.  Only the closest-hit sweep is per view: one eye table each, in
+// groups (DESIGN §4e).  Per sample: closest hit, faceIDs (first sample), then per light a light step and a shadow sweep.
+
+// The render modes.  The values are light_step_kernel's cull_cells: which shadow-ray sort key it writes.
+enum Mode { BVH = 0, CULL = 1, SWEEPS = 2 };
+// Frame::render's outcome when the bundle-cull candidate buffer overflowed (not a status code: render_views renders again)
+constexpr int CAND_OVERFLOW = 1;
+
+// One attempt at the frames of one call: the scene, the checked options, what follows from them, and the counts it adds up
+struct Frame {
+    tracer_scene_dev *s;
+    Ctx &g;
+    const tracer_render_opts &o;
+    const tracer_camera *cams;
+    cudaStream_t st;
+    int W, H, n_rows, view_px, n_px, n_views, L, S; // S: samples per pixel
+    trk::Bands bands;
+    trk::Views views{};
+    std::vector<trk::Cam> h_cams;
+    double diag = 0;    // reach bound of a primary ray's hit point; light k's shadow segments are bounded by (k+1) * diag
+    double bvh_ext = 0; // BVH mode: largest |coordinate| of the tree and every eye
+    Mode mode = SWEEPS;
+    bool two_phase = false;        // bundle-cull mode: block lists first (cull.cuh), not only the streaming kernels
+    int group = 1, n_groups = 1;   // eye tables: n_groups groups of up to `group` views
+    unsigned long long em_cap = 0; // candidate pairs the bundle-cull kernels may emit
+    int tri_bits = 1;              // bits of a triangle index in a block-list key
+    trk::PixelState px{};
+    int launches = 0;
+    int64_t host_tests_primary = 0, host_tests_shadow = 0; // pairs considered by two-phase sweeps (every block x every triangle)
+    double flop_primary = 0.0;       // executed FP32 flops per swept pair of the closest-hit sweep (default mode)
+    double flop_primary_edges = 0.0; // of which bound-evaluating multiply-adds
+    double ms_primary = 0, ms_shadow = 0; // event times, summed over the samples
+
+    int render(uint8_t *rgb_out, std::vector<int> &frame_rows, bool &rows_known);
+    int setup();
+    int build_eye_tables(int v0, int v1);
+    int closest_hit();
+    int primary_sweeps();
+    int primary_cull();
+    int primary_bvh();
+    int block_lists(cull::L0Params lp, int max_blocks, long long &n_keys);
+    int faceids(std::vector<int> &frame_rows, bool &rows_known);
+    int light(int k, uint32_t seed);
+    int order_shadow_rays(int F);
+    int shadow_sweeps(int k);
+    int shadow_cull(int k);
+    int shadow_bvh(int k);
+    int accumulate(int smp);
+    void add_sample_times();
+    int finish_frame(uint8_t *rgb_out);
+};
+
+// frame_rows, rows_known: the frame's row hit counts (TRACER_RNG_MT19937), known once the exchange hook has run; a render
+// again after an overflow checks its own against them (the hook runs once per frame)
+int Frame::render(uint8_t *rgb_out, std::vector<int> &frame_rows, bool &rows_known) {
     CK_CUDA(cudaSetDevice(g.device));
-    cudaStream_t st = o.cuda_stream ? (cudaStream_t)o.cuda_stream : g.stream;
     std::memset(&s->stats, 0, sizeof s->stats);
     s->stats.n_sms = g.n_sms;
     s->stats.n_pixels = n_px;
-    const bool mt_exchange = o.rng_mode == TRACER_RNG_MT19937 && band_count > 1 && !frame_rows;
-    std::vector<int> mt_frame; // the frame's row hit counts (TRACER_RNG_MT19937)
-    if (n_px == 0) return mt_exchange ? mt_frame_rows(o, W, H, band_rows, band_count, {}, mt_frame) : TRACER_OK;
-    if (int rc = ensure_workspace(s, n_px, o.out_occ_tri != nullptr)) return rc;
-    int launches = 0;
+    if (n_px == 0)
+        return o.rng_mode == TRACER_RNG_MT19937 && bands.band_count > 1 ? mt_frame_rows(o, W, H, bands.band_rows, bands.band_count, {}, frame_rows)
+                                                                         : TRACER_OK;
+    if (int rc = setup()) return rc;
+    for (int smp = 0; smp < S; ++smp) {
+        bands.sample = smp;
+        if (int rc = closest_hit()) return rc;
+        if (smp == 0)
+            if (int rc = faceids(frame_rows, rows_known)) return rc;
+        const uint32_t seed = o.seed + (uint32_t)smp * 0x9e3779b1u; // faceID stream of this sample
+        for (int k = 0; k <= L; ++k)
+            if (int rc = light(k, seed)) return rc;
+        if (S > 1)
+            if (int rc = accumulate(smp)) return rc;
+    }
+    return finish_frame(rgb_out);
+}
 
-    trk::Cam dc;
-    std::vector<trk::Cam> h_cams((size_t)n_views);
+// Workspace, cameras, reach bound, mode, and the buffers and tables the mode needs before the first sample
+int Frame::setup() {
+    if (int rc = ensure_workspace(s->ws, n_px, std::max(1, L), o.out_occ_tri != nullptr)) return rc;
+    h_cams.resize((size_t)n_views);
     for (int v = 0; v < n_views; ++v) {
         trk::Cam &c = h_cams[v];
         std::memcpy(c.o, cams[v].origin, 12), std::memcpy(c.llc, cams[v].lower_left_corner, 12);
         std::memcpy(c.hor, cams[v].horizontal, 12), std::memcpy(c.ver, cams[v].vertical, 12);
     }
-    dc = h_cams[0];
-    if (dev_grow(s->cams, s->cams_cap, (size_t)n_views)) return TRACER_ERR_NOMEM;
+    if (dev_grow(s->cams_cap, (size_t)n_views, s->cams)) return TRACER_ERR_NOMEM;
     CK_CUDA(cudaMemcpyAsync(s->cams, h_cams.data(), sizeof(trk::Cam) * (size_t)n_views, cudaMemcpyHostToDevice, st));
-    const trk::Views views{s->cams, view_px};
-    trk::Bands bands{W, H, band_rows, band_count > 1 ? o.band_index : 0, band_count, n_px};
-    bands.spp_n = spp_n, bands.sample = 0, bands.seed = o.seed;
+    views = trk::Views{s->cams, view_px};
 
     // reach bound for shadow segments: len_k <= (k+1) * diag(bbox U every eye)  (t carries over lights, main.cpp:764).  One
     // bound for all views: a view's own would be smaller, and a table built for a larger bound is only looser (DESIGN §4e)
@@ -1182,42 +1197,22 @@ int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, in
         for (int v = 0; v < n_views; ++v) lo[c] = std::min(lo[c], (double)cams[v].origin[c]), hi[c] = std::max(hi[c], (double)cams[v].origin[c]);
         if (hi[c] >= lo[c]) diag2 += (hi[c] - lo[c]) * (hi[c] - lo[c]);
     }
-    // shadow segments of light k are bounded by len_k <= (k+1) * diag: t carries over lights (main.cpp:764)
-    const double diag = std::sqrt(diag2) * 1.001 + 1e-30;
-    // eye tables: views [v0, v1) into slots 0 .. v1 - v0, on the image plane: d'(s,t) = (llc - origin) + s*horizontal +
-    // t*vertical (camera.h:31-34)
-    const int group = use_bvh ? n_views : view_group_size(s, n_views), n_groups = (n_views + group - 1) / group;
-    if (!use_bvh && group > s->eye_cap) {
-        dev_free(s->eye_table), dev_free(s->eye_span);
-        s->eye_cap = 0;
-        if (dev_alloc(&s->eye_table, s->table_stride * group) || dev_alloc(&s->eye_span, s->span_stride * group)) return TRACER_ERR_NOMEM;
-        s->eye_cap = group;
-    }
-    auto build_eye_tables = [&](int v0, int v1) -> int {
-        for (int v = v0; v < v1; ++v) {
-            const tracer_camera *cv = &cams[v];
-            trk::TableParam tp{};
-            for (int c = 0; c < 3; ++c) {
-                tp.o[c] = cv->origin[c], tp.U[c] = cv->horizontal[c], tp.V[c] = cv->vertical[c];
-                tp.W[c] = (double)cv->lower_left_corner[c] - (double)cv->origin[c];
-            }
-            for (int corner = 0; corner < 4; ++corner) { // |d'| is convex in (s,t): its maximum is at a corner
-                double n2 = 0;
-                for (int c = 0; c < 3; ++c) {
-                    const double x = tp.W[c] + (corner & 1) * tp.U[c] + (corner >> 1) * tp.V[c];
-                    n2 += x * x;
-                }
-                tp.dmax = std::max(tp.dmax, std::sqrt(n2));
-            }
-            tp.lmax = 0.0;
-            if (int rc = build_table(s, tp, s->eye_table + (size_t)(v - v0) * s->table_stride, s->eye_span + (size_t)(v - v0) * s->span_stride, st))
-                return rc;
-            ++launches;
-        }
-        return 0;
-    };
+    diag = std::sqrt(diag2) * 1.001 + 1e-30;
+
+    // bundle_cull: 1 two-phase, 2 streaming, 3 auto = two-phase unless the default sweeps are estimated to be the
+    // faster of the two (tiny scenes: the mode has a fixed cost of a few ms in sorts and count read-backs)
+    const double est_default_ms = (double)n_px * (double)s->n_tris * (1.0 + 0.25 * L) / 4.0e9;
+    // (the optional mode keeps every light vertex's tables resident; a light too big for that renders in the default mode)
+    if (o.accel == 1) mode = BVH;
+    else if (s->tables_resident && (o.bundle_cull == 3 ? est_default_ms > 6.0 : o.bundle_cull != 0)) mode = CULL;
+    two_phase = mode == CULL && o.bundle_cull != 2;
+
+    group = mode == BVH ? n_views : view_group_size(s, n_views), n_groups = (n_views + group - 1) / group;
+    if (mode != BVH && (dev_grow(s->eye_table_cap, s->table_stride * group, s->eye_table) ||
+                        dev_grow(s->eye_span_cap, s->span_stride * group, s->eye_span)))
+        return TRACER_ERR_NOMEM;
     CK_CUDA(cudaEventRecord(s->ev[0], st));
-    if (use_bvh) {
+    if (mode == BVH) {
         if (int rc = ensure_bvh(s, st)) return rc;
     } else if (n_groups == 1) { // one group: its tables serve every sample; otherwise each group builds its own in turn
         if (int rc = build_eye_tables(0, n_views)) return rc;
@@ -1225,172 +1220,142 @@ int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, in
     CK_CUDA(cudaMemsetAsync(s->counters, 0, sizeof(sweep::Counters), st));
     CK_CUDA(cudaMemsetAsync(s->work, 0, sizeof(int), st));
 
-    const int n_tiles = s->n_pad / sweep::TILE;
-    // bundle_cull: 1 two-phase, 2 streaming, 3 auto = two-phase unless the default sweeps are estimated to be the
-    // faster of the two (tiny scenes: the mode has a fixed cost of a few ms in sorts and count read-backs)
-    const double est_default_ms = (double)n_px * (double)s->n_tris * (1.0 + 0.25 * L) / 4.0e9;
-    // (the optional mode keeps every light vertex's tables resident; a light too big for that renders in the default mode)
-    const bool cull = !use_bvh && s->tables_resident && (o.bundle_cull == 3 ? est_default_ms > 6.0 : o.bundle_cull != 0);
-    // the optional mode's candidate buffer (24 per ray + slack) was too small for this scene's depth complexity: render the
-    // frame again with a 4x larger one while that fits comfortably, else by the default sweeps, which need no such buffer —
-    // same bytes out either way.  rows: the frame's row hit counts when they are known to be right (see frame_rows).
-    auto rerender_after_overflow = [&](const std::vector<int> *rows) -> int {
-        tracer_render_opts o2 = o;
-        o2.struct_size = sizeof o2;
-        size_t free_b = 0, total_b = 0;
-        cudaMemGetInfo(&free_b, &total_b);
-        const size_t next_bytes = ((size_t)n_px * 24 * (size_t)s->cull_grow * 4 + ((size_t)1 << 22)) * sizeof(unsigned long long) * 3;
-        if (!std::getenv("TRACER_CAND_CAP") && s->cull_grow < 64 && next_bytes < free_b / 2 + s->cand_cap * 24)
-            s->cull_grow *= 4;
-        else
-            o2.bundle_cull = 0;
-        return render_views(s, cams, n_views, W, H, &o2, rgb_out, rows);
-    };
-    if (cull) { // candidate buffers: 24 per ray + slack (a few per ray are typical), sorted with a radix sort
+    if (mode == CULL) { // candidate buffers: 24 per ray + slack (a few per ray are typical), sorted with a radix sort
         const size_t cap = (size_t)n_px * 24 * (size_t)s->cull_grow + ((size_t)1 << 22);
         if (cap > s->cand_cap) {
-            dev_free(s->cand_a), dev_free(s->cand_b), dev_free(s->cand_count);
-            t_pool->release(s->sort_tmp);
-            s->sort_tmp = nullptr, s->cand_cap = 0;
-            if (dev_alloc(&s->cand_a, cap) || dev_alloc(&s->cand_b, cap) || dev_alloc(&s->cand_count, 1)) return TRACER_ERR_NOMEM;
+            if (dev_grow(s->cand_cap, cap, s->cand_a, s->cand_b)) return TRACER_ERR_NOMEM;
             CK_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, s->sort_bytes, s->cand_a, s->cand_b, cap, 0, 64, st));
-            if (!(s->sort_tmp = t_pool->alloc(s->sort_bytes))) return fail(TRACER_ERR_NOMEM, "sort scratch");
-            s->cand_cap = cap;
         }
+        if (dev_grow(s->count_cap, 1, s->cand_count) || dev_grow(s->sort_cap, s->sort_bytes, s->sort_tmp)) return TRACER_ERR_NOMEM;
     }
-    // default mode: shadow rays ordered by (group, q) so that the rays of a thread can share a q-term (sweep::MODE_QBAR);
-    // bundle-cull mode: ordered by (group, Morton code of (p,q)).  Either way a radix sort of (key, pixel) pairs.
-    if (!use_bvh && s->rkey_npx < n_px) {
-        dev_free(s->rkey), dev_free(s->rkey_sorted), dev_free(s->iota);
-        t_pool->release(s->pair_tmp);
-        s->pair_tmp = nullptr;
-        if (dev_alloc(&s->rkey, (size_t)n_px) || dev_alloc(&s->rkey_sorted, (size_t)n_px) || dev_alloc(&s->iota, (size_t)n_px)) return TRACER_ERR_NOMEM;
-        CK_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, s->pair_bytes, s->rkey, s->rkey_sorted, s->iota, s->list, n_px, 0, 64, st));
-        if (!(s->pair_tmp = t_pool->alloc(s->pair_bytes))) return fail(TRACER_ERR_NOMEM, "sort scratch");
-        trk::iota_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(s->iota, n_px);
-        CK_CUDA(cudaGetLastError());
-        s->rkey_npx = n_px;
+    // shadow rays ordered by a radix sort of (key, pixel) pairs (order_shadow_rays)
+    if (mode != BVH) {
+        if ((size_t)n_px > s->rkey_cap) {
+            if (dev_grow(s->rkey_cap, (size_t)n_px, s->rkey, s->rkey_sorted, s->iota)) return TRACER_ERR_NOMEM;
+            CK_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, s->pair_bytes, s->rkey, s->rkey_sorted, s->iota, s->ws.list, n_px, 0, 64, st));
+            trk::iota_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(s->iota, n_px);
+            CK_CUDA(cudaGetLastError());
+        }
+        if (dev_grow(s->pair_cap, s->pair_bytes, s->pair_tmp)) return TRACER_ERR_NOMEM;
     }
-    // two-phase bundle cull (cull.cuh "block lists"): phase A emits block<<32|triangle into cand_a; the sorted
-    // keys land in cand_b, which phase B reads while it emits its ray<<32|triangle candidates into cand_a again.
-    // Returns the number of keys, or -1 when the survivor lists would not fit (then the streaming kernels run).
     // test knob: pretend the bundle-cull candidate buffer holds only this many pairs (exercises the overflow fallback)
     const char *cand_env = std::getenv("TRACER_CAND_CAP");
-    const unsigned long long em_cap = cand_env ? std::min<unsigned long long>((unsigned long long)std::atoll(cand_env), s->cand_cap) : (unsigned long long)s->cand_cap;
-    double flop_primary = 0.0; // executed FP32 flops per swept pair of the closest-hit sweep (default mode)
-    double flop_primary_edges = 0.0; // of which bound-evaluating multiply-adds
-    const bool two_phase = cull && o.bundle_cull != 2;
-    int64_t host_tests_primary = 0, host_tests_shadow = 0; // pairs considered by two-phase sweeps (every block x every triangle)
-    auto ensure_boxes = [&](size_t n_blocks) -> int {
-        if (n_blocks <= s->boxes_cap) return 0;
-        dev_free(s->boxes);
-        s->boxes_cap = 0;
-        if (dev_alloc(&s->boxes, n_blocks)) return TRACER_ERR_NOMEM;
-        s->boxes_cap = n_blocks;
-        return 0;
-    };
-    int tri_bits = 1;
+    em_cap = cand_env ? std::min<unsigned long long>((unsigned long long)std::atoll(cand_env), s->cand_cap) : (unsigned long long)s->cand_cap;
     while (((int64_t)1 << tri_bits) < s->n_pad) ++tri_bits;
-    auto block_lists = [&](cull::L0Params lp, int max_blocks, long long &n_keys) -> int {
-        lp.boxes = s->boxes, lp.keys = s->cand_a, lp.count = s->cand_count, lp.cap = (unsigned long long)s->cand_cap; /* phase-A keys: their own limit (TRACER_L0_CAP) */
-        lp.n_tris = s->n_tris, lp.tri_bits = tri_bits, lp.diag = s->counters;
-        CK_CUDA(cudaMemsetAsync(s->cand_count, 0, sizeof(unsigned long long), st));
-        const dim3 grid((unsigned)((s->n_tris + cull::L0_THREADS - 1) / cull::L0_THREADS), (unsigned)lp.n_groups);
-        cull::cull_l0_kernel<<<grid, cull::L0_THREADS, 0, st>>>(lp);
-        CK_CUDA(cudaGetLastError());
-        unsigned long long n = 0;
-        CK_CUDA(cudaMemcpyAsync(&n, s->cand_count, sizeof n, cudaMemcpyDeviceToHost, st));
-        CK_CUDA(cudaStreamSynchronize(st));
-        CK_CUDA(cudaMemsetAsync(s->cand_count, 0, sizeof(unsigned long long), st));
-        launches += 2;
-        if (getenv("TRACER_CULL_DIAG")) fprintf(stderr, "cull diag: phase A kept %llu (block, triangle) pairs over %d groups, <= %d blocks\n", n, lp.n_groups, max_blocks);
-        const char *cap_env = getenv("TRACER_L0_CAP"); // development/test knob: pretend the key buffer is this small
-        if (n > s->cand_cap || (cap_env && n > (unsigned long long)std::atoll(cap_env))) {
-            n_keys = -1;
-            return 0;
-        }
-        int blk_bits = 1;
-        while ((1 << blk_bits) < max_blocks * (sweep::THREADS / 32)) ++blk_bits; // keys name a (block, warp)
-        if (n) CK_CUDA(cub::DeviceRadixSort::SortKeys(s->sort_tmp, s->sort_bytes, s->cand_a, s->cand_b, n, 0, tri_bits + blk_bits, st));
-        n_keys = (long long)n;
-        return 0;
-    };
-    double ms_primary_acc = 0, ms_shadow_acc = 0;
-    if (S > 1 && !s->accum_total && dev_alloc(&s->accum_total, 3 * (size_t)s->ws_npx)) return TRACER_ERR_NOMEM;
-    for (int smp = 0; smp < S; ++smp) {
-    bands.sample = smp;
-    const uint32_t seed_s = o.seed + (uint32_t)smp * 0x9e3779b1u; // faceID stream of this sample
-    // ---- primary: raygen + closest hit ----------------------------------------------
-    CK_CUDA(cudaMemsetAsync(s->work, 0, sizeof(int), st));
-    CK_CUDA(cudaMemsetAsync(s->best, 0xff, sizeof(unsigned long long) * (size_t)n_px, st));
-    CK_CUDA(cudaEventRecord(s->ev[1], st));
+    if (S > 1 && !s->ws.accum_total && dev_alloc(&s->ws.accum_total, 3 * (size_t)s->ws.npx)) return TRACER_ERR_NOMEM;
+    px = s->ws.px();
     // BVH mode: the tree's dilation m (bvh.cuh frame_margin) from the largest |coordinate| of the tree and the eye, with
     // the reach bound diag of the primary rays' hit points, (k+1) diag for light k
-    double bvh_ext = s->bvh_ext; // (every view's eye: the tree serves them all)
+    bvh_ext = s->bvh_ext; // (every view's eye: the tree serves them all)
     for (int v = 0; v < n_views; ++v)
         for (int c = 0; c < 3; ++c) bvh_ext = std::max(bvh_ext, (double)std::fabs(cams[v].origin[c]));
-    if (use_bvh) {
-        bvh::primary_kernel<<<(n_px + 127) / 128, 128, 0, st>>>(views, bands, s->bvh_tree, bvh::frame_margin(bvh_ext, diag), s->tri_verts,
-                                                                 s->best, s->counters);
-        CK_CUDA(cudaGetLastError());
-        trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(views, bands, s->best, s->tri_verts, s->n_tris, s->spheres,
-                                                                        s->n_spheres, s->hit_tri, s->hit_t, s->hit_v);
-        CK_CUDA(cudaGetLastError());
-        launches += 2;
-    } else if (cull) { // OPTIONAL bundle-cull mode: screen tiles of 128 x 32 pixels -> candidates -> sort -> strict
-        trk::PrimaryCullParams p{};
-        const int c_tiles = s->n_pad / cull::CTILE;
-        p.cam = dc, p.bands = bands, p.table = s->eye_table, p.n_tiles = c_tiles, p.n_tris = s->n_tris, p.n_rows = n_rows;
-        p.tiles_x = (W + 127) / 128, p.tiles_y = (n_rows + 31) / 32;
-        const int blocks = p.tiles_x * p.tiles_y;
-        p.n_slices = blocks >= 12 * g.n_sms ? 1 : std::max(1, std::min((12 * g.n_sms + blocks - 1) / blocks, std::max(1, c_tiles / 8)));
-        p.em = cull::Emitter{s->cand_a, s->cand_count, em_cap};
-        p.counters = s->counters, p.work = s->work;
-        long long n_keys = -1;
-        if (two_phase) {
-            if (int rc = ensure_boxes((size_t)blocks)) return rc;
-            trk::primary_boxes_kernel<<<blocks, sweep::THREADS, 0, st>>>(p, s->boxes, s->blk_off);
-            CK_CUDA(cudaGetLastError());
-            cull::L0Params lp{};
-            lp.tables = s->eye_table, lp.n_groups = 1, lp.nface = 0, lp.blk_off = s->blk_off;
-            if (int rc = block_lists(lp, blocks, n_keys)) return rc;
+    return 0;
+}
+
+// eye tables: views [v0, v1) into slots 0 .. v1 - v0, on the image plane: d'(s,t) = (llc - origin) + s*horizontal +
+// t*vertical (camera.h:31-34)
+int Frame::build_eye_tables(int v0, int v1) {
+    for (int v = v0; v < v1; ++v) {
+        const tracer_camera *cv = &cams[v];
+        trk::TableParam tp{};
+        for (int c = 0; c < 3; ++c) {
+            tp.o[c] = cv->origin[c], tp.U[c] = cv->horizontal[c], tp.V[c] = cv->vertical[c];
+            tp.W[c] = (double)cv->lower_left_corner[c] - (double)cv->origin[c];
         }
-        if (n_keys >= 0) {
-            trk::primary_cull2_kernel<<<2 * g.n_sms, sweep::THREADS, 0, st>>>(p, trk::BlockLists{s->boxes, s->cand_b, (unsigned long long)n_keys, tri_bits});
-            CK_CUDA(cudaGetLastError());
-            host_tests_primary += (int64_t)n_px * s->n_tris;
-        } else {
-            CK_CUDA(cudaMemsetAsync(s->cand_count, 0, sizeof(unsigned long long), st));
-            const size_t smem = sizeof(cull::EmitSmem);
-            CK_CUDA(cudaFuncSetAttribute(trk::primary_cull_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            trk::primary_cull_kernel<<<std::min(blocks * p.n_slices, 2 * g.n_sms), sweep::THREADS, smem, st>>>(p);
-            CK_CUDA(cudaGetLastError());
+        for (int corner = 0; corner < 4; ++corner) { // |d'| is convex in (s,t): its maximum is at a corner
+            double n2 = 0;
+            for (int c = 0; c < 3; ++c) {
+                const double x = tp.W[c] + (corner & 1) * tp.U[c] + (corner >> 1) * tp.V[c];
+                n2 += x * x;
+            }
+            tp.dmax = std::max(tp.dmax, std::sqrt(n2));
         }
-        trk::strict_primary_pairs<<<8 * g.n_sms, 256, 0, st>>>(s->cand_a, s->cand_count, em_cap, dc, bands,
-                                                               s->tri_verts, s->best, s->counters);
+        tp.lmax = 0.0;
+        if (int rc = build_table(s, tp, s->eye_table + (size_t)(v - v0) * s->table_stride, s->eye_span + (size_t)(v - v0) * s->span_stride, st))
+            return rc;
+        ++launches;
+    }
+    return 0;
+}
+
+// ---- primary: raygen + closest hit -> hit_tri, hit_t, hit_v -------------------------------------------------------------
+int Frame::closest_hit() {
+    CK_CUDA(cudaMemsetAsync(s->work, 0, sizeof(int), st));
+    CK_CUDA(cudaMemsetAsync(s->ws.best, 0xff, sizeof(unsigned long long) * (size_t)n_px, st));
+    CK_CUDA(cudaEventRecord(s->ev[1], st));
+    if (int rc = mode == BVH ? primary_bvh() : mode == CULL ? primary_cull() : primary_sweeps()) return rc;
+    trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(views, bands, s->ws.best, s->tri_verts, s->n_tris, s->spheres,
+                                                                    s->n_spheres, s->ws.hit_tri, s->ws.hit_t, s->ws.hit_v);
+    CK_CUDA(cudaGetLastError());
+    ++launches;
+    CK_CUDA(cudaEventRecord(s->ev[2], st));
+    return 0;
+}
+
+int Frame::primary_bvh() {
+    bvh::primary_kernel<<<(n_px + 127) / 128, 128, 0, st>>>(views, bands, s->bvh_tree, bvh::frame_margin(bvh_ext, diag), s->tri_verts,
+                                                             s->ws.best, s->counters);
+    CK_CUDA(cudaGetLastError());
+    ++launches;
+    return 0;
+}
+
+// OPTIONAL bundle-cull mode: screen tiles of 128 x 32 pixels -> candidates -> sort -> strict
+int Frame::primary_cull() {
+    trk::PrimaryCullParams p{};
+    const int c_tiles = s->n_pad / cull::CTILE;
+    p.cam = h_cams[0], p.bands = bands, p.table = s->eye_table, p.n_tiles = c_tiles, p.n_tris = s->n_tris, p.n_rows = n_rows;
+    p.tiles_x = (W + 127) / 128, p.tiles_y = (n_rows + 31) / 32;
+    const int blocks = p.tiles_x * p.tiles_y;
+    p.n_slices = blocks >= 12 * g.n_sms ? 1 : std::max(1, std::min((12 * g.n_sms + blocks - 1) / blocks, std::max(1, c_tiles / 8)));
+    p.em = cull::Emitter{s->cand_a, s->cand_count, em_cap};
+    p.counters = s->counters, p.work = s->work;
+    long long n_keys = -1;
+    if (two_phase) {
+        if (dev_grow(s->boxes_cap, (size_t)blocks, s->boxes)) return TRACER_ERR_NOMEM;
+        trk::primary_boxes_kernel<<<blocks, sweep::THREADS, 0, st>>>(p, s->boxes, s->blk_off);
         CK_CUDA(cudaGetLastError());
-        trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(views, bands, s->best, s->tri_verts, s->n_tris, s->spheres,
-                                                                        s->n_spheres, s->hit_tri, s->hit_t, s->hit_v);
+        cull::L0Params lp{};
+        lp.tables = s->eye_table, lp.n_groups = 1, lp.nface = 0, lp.blk_off = s->blk_off;
+        if (int rc = block_lists(lp, blocks, n_keys)) return rc;
+    }
+    if (n_keys >= 0) {
+        trk::primary_cull2_kernel<<<2 * g.n_sms, sweep::THREADS, 0, st>>>(p, trk::BlockLists{s->boxes, s->cand_b, (unsigned long long)n_keys, tri_bits});
         CK_CUDA(cudaGetLastError());
-        launches += 3;
+        host_tests_primary += (int64_t)n_px * s->n_tris;
     } else {
-        // no jitter: the rays of a thread share q exactly; jittered samples (extension): they share a mean q (span table)
-        // unless the frame is so small that a jittered (s,t) can leave the span rows' |p|,|q| <= 1.0625 range
-        const int qmode = bands.spp_n <= 1 ? sweep::MODE_SHAREDQ : (W >= 16 && H >= 16 ? sweep::MODE_QBAR : sweep::MODE_OWNQ);
-        // one launch per group of views (all of them unless their eye tables did not fit at once)
-        for (int v0 = 0; v0 < n_views; v0 += group) {
+        CK_CUDA(cudaMemsetAsync(s->cand_count, 0, sizeof(unsigned long long), st));
+        const size_t smem = sizeof(cull::EmitSmem);
+        CK_CUDA(cudaFuncSetAttribute(trk::primary_cull_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        trk::primary_cull_kernel<<<std::min(blocks * p.n_slices, 2 * g.n_sms), sweep::THREADS, smem, st>>>(p);
+        CK_CUDA(cudaGetLastError());
+    }
+    trk::strict_primary_pairs<<<8 * g.n_sms, 256, 0, st>>>(s->cand_a, s->cand_count, em_cap, h_cams[0], bands, s->tri_verts, s->ws.best,
+                                                           s->counters);
+    CK_CUDA(cudaGetLastError());
+    launches += 2;
+    return 0;
+}
+
+// Default mode: one primary_kernel launch per group of views (all of them unless their eye tables did not fit at once)
+int Frame::primary_sweeps() {
+    const int n_tiles = s->n_pad / sweep::TILE;
+    // no jitter: the rays of a thread share q exactly; jittered samples (extension): they share a mean q (span table)
+    // unless the frame is so small that a jittered (s,t) can leave the span rows' |p|,|q| <= 1.0625 range
+    const int qmode = bands.spp_n <= 1 ? sweep::MODE_SHAREDQ : (W >= 16 && H >= 16 ? sweep::MODE_QBAR : sweep::MODE_OWNQ);
+    for (int v0 = 0; v0 < n_views; v0 += group) {
         const int nv = std::min(group, n_views - v0);
         if (n_groups > 1) {
             if (int rc = build_eye_tables(v0, v0 + nv)) return rc;
             if (v0 > 0) CK_CUDA(cudaMemsetAsync(s->work, 0, sizeof(int), st));
         }
-        const Decomp d = pick_decomp((int64_t)nv * view_px, n_tiles, g.n_sms, o.rays_per_thread, 0, qmode);
+        const Decomp d = pick_decomp((int64_t)nv * view_px, n_tiles, g.n_sms, o.rays_per_thread, qmode);
         trk::PrimaryParams p{};
         p.views = views, p.cam = h_cams[v0], p.bands = bands, p.n_tiles = n_tiles, p.n_tris = s->n_tris;
         p.table = qmode == sweep::MODE_OWNQ ? s->eye_table : s->eye_span;
         p.table_stride = (long long)(qmode == sweep::MODE_OWNQ ? s->table_stride : s->span_stride), p.view0 = v0;
         p.tri_verts = s->tri_verts;
-        p.best = s->best, p.counters = s->counters, p.work = s->work;
+        p.best = s->ws.best, p.counters = s->counters, p.work = s->work;
         p.n_rows = n_rows, p.view_blocks = 0; // ray blocks = screen tiles of (TX R) x (NT / TX) pixels: least edge waste wins
         for (int lg = d.R > 32 ? 2 : 3; lg <= 6; ++lg) { // (64 rays per thread: from 4 x 64 = 256 pixels wide)
             const int tw = (1 << lg) * d.R, th = sweep::NT >> lg;
@@ -1412,16 +1377,41 @@ int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, in
         flop_primary_edges = qmode == sweep::MODE_OWNQ ? 12.0 : (qmode == sweep::MODE_QBAR ? 16.0 : 8.0) / d.R;
         if (int rc = launch_primary(d.R, o.exhaustive_strict != 0, qmode, p, nv > 1, grid, st)) return rc;
         ++launches;
-        }
-        trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(views, bands, s->best, s->tri_verts, s->n_tris, s->spheres,
-                                                                        s->n_spheres, s->hit_tri, s->hit_t, s->hit_v);
-        CK_CUDA(cudaGetLastError());
-        ++launches;
     }
-    CK_CUDA(cudaEventRecord(s->ev[2], st));
+    return 0;
+}
 
-    // ---- faceIDs ------------------------------------------------------------------------
-    if (smp == 0 && L > 0 && o.rng_mode == TRACER_RNG_EXPLICIT) {
+// two-phase bundle cull (cull.cuh "block lists"): phase A emits block<<32|triangle into cand_a; the sorted
+// keys land in cand_b, which phase B reads while it emits its ray<<32|triangle candidates into cand_a again.
+// n_keys = the number of keys, or -1 when the survivor lists would not fit (then the streaming kernels run).
+int Frame::block_lists(cull::L0Params lp, int max_blocks, long long &n_keys) {
+    lp.boxes = s->boxes, lp.keys = s->cand_a, lp.count = s->cand_count, lp.cap = (unsigned long long)s->cand_cap; /* phase-A keys: their own limit (TRACER_L0_CAP) */
+    lp.n_tris = s->n_tris, lp.tri_bits = tri_bits, lp.diag = s->counters;
+    CK_CUDA(cudaMemsetAsync(s->cand_count, 0, sizeof(unsigned long long), st));
+    const dim3 grid((unsigned)((s->n_tris + cull::L0_THREADS - 1) / cull::L0_THREADS), (unsigned)lp.n_groups);
+    cull::cull_l0_kernel<<<grid, cull::L0_THREADS, 0, st>>>(lp);
+    CK_CUDA(cudaGetLastError());
+    unsigned long long n = 0;
+    CK_CUDA(cudaMemcpyAsync(&n, s->cand_count, sizeof n, cudaMemcpyDeviceToHost, st));
+    CK_CUDA(cudaStreamSynchronize(st));
+    CK_CUDA(cudaMemsetAsync(s->cand_count, 0, sizeof(unsigned long long), st));
+    launches += 2;
+    if (getenv("TRACER_CULL_DIAG")) fprintf(stderr, "cull diag: phase A kept %llu (block, triangle) pairs over %d groups, <= %d blocks\n", n, lp.n_groups, max_blocks);
+    const char *cap_env = getenv("TRACER_L0_CAP"); // development/test knob: pretend the key buffer is this small
+    if (n > s->cand_cap || (cap_env && n > (unsigned long long)std::atoll(cap_env))) {
+        n_keys = -1;
+        return 0;
+    }
+    int blk_bits = 1;
+    while ((1 << blk_bits) < max_blocks * (sweep::THREADS / 32)) ++blk_bits; // keys name a (block, warp)
+    if (n) CK_CUDA(cub::DeviceRadixSort::SortKeys(s->sort_tmp, s->sort_bytes, s->cand_a, s->cand_b, n, 0, tri_bits + blk_bits, st));
+    n_keys = (long long)n;
+    return 0;
+}
+
+// ---- faceIDs (first sample): the caller's (TRACER_RNG_EXPLICIT) or the seeded draws' (TRACER_RNG_MT19937) --------------
+int Frame::faceids(std::vector<int> &frame_rows, bool &rows_known) {
+    if (L > 0 && o.rng_mode == TRACER_RNG_EXPLICIT) {
         std::vector<int> loc((size_t)n_px * L);
         for (int k = 0; k < n_px; ++k) { // view v's faceids: opts->faceid[v][W*H*L], image index order
             int w, h;
@@ -1429,297 +1419,269 @@ int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, in
             bands.map(k - v * view_px, w, h);
             std::memcpy(&loc[(size_t)k * L], o.faceid + ((size_t)v * H * W + (size_t)h * W + w) * L, sizeof(int) * L);
         }
-        CK_CUDA(cudaMemcpyAsync(s->faceid, loc.data(), loc.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+        CK_CUDA(cudaMemcpyAsync(s->ws.faceid, loc.data(), loc.size() * sizeof(int), cudaMemcpyHostToDevice, st));
         CK_CUDA(cudaStreamSynchronize(st));
-    } else if (smp == 0 && o.rng_mode == TRACER_RNG_MT19937) {
+    } else if (o.rng_mode == TRACER_RNG_MT19937) {
         // a bundle-cull closest-hit pass whose candidates overflowed has lost hits: its row counts must not be used or sent,
         // so the frame is rendered again before the exchange (read back with the row counts, at the same synchronise)
         unsigned long long primary_overflow = 0;
-        if (cull) CK_CUDA(cudaMemcpyAsync(&primary_overflow, &s->counters->cull_overflow, sizeof primary_overflow, cudaMemcpyDeviceToHost, st));
+        if (mode == CULL) CK_CUDA(cudaMemcpyAsync(&primary_overflow, &s->counters->cull_overflow, sizeof primary_overflow, cudaMemcpyDeviceToHost, st));
         // the row hits of every view in one pass (view-major rows), then each view replays its own std::mt19937(seed) draws,
         // as a separate render of that view would
         std::vector<int> all_rows;
-        if (int rc = mt_count_rows(s->mt, s->hit_tri, W, n_views * n_rows, st, all_rows)) return rc;
+        if (int rc = mt_count_rows(s->mt, s->ws.hit_tri, W, n_views * n_rows, st, all_rows)) return rc;
         ++launches;
-        if (primary_overflow) return rerender_after_overflow(frame_rows);
+        if (primary_overflow) return CAND_OVERFLOW;
         for (int v = 0; v < n_views; ++v) {
             const std::vector<int> local(all_rows.begin() + (size_t)v * n_rows, all_rows.begin() + (size_t)(v + 1) * n_rows);
-            if (frame_rows) {
-                if (!mt::rows_valid(local.data(), n_rows, band_rows, bands.band_index, band_count, frame_rows->data(), H, W))
+            if (rows_known) {
+                if (!mt::rows_valid(local.data(), n_rows, bands.band_rows, bands.band_index, bands.band_count, frame_rows.data(), H, W))
                     return fail(TRACER_ERR_STATE, "bundle-cull re-render: the closest-hit pass found other hits than the first pass");
-                mt_frame = *frame_rows;
-            } else if (int rc = mt_frame_rows(o, W, H, band_rows, band_count, local, mt_frame)) {
+            } else if (int rc = mt_frame_rows(o, W, H, bands.band_rows, bands.band_count, local, frame_rows)) {
                 return rc;
             }
             const size_t off = (size_t)v * view_px;
-            if (int rc = mt_replay(s->mt, o.seed, s->h_light_F, mt_frame, W, band_rows, bands.band_index, band_count, n_rows,
-                                   s->hit_tri + off, s->faceid + off * L, st, launches, off))
+            if (int rc = mt_replay(s->mt, o.seed, s->h_light_F, frame_rows, W, bands.band_rows, bands.band_index, bands.band_count, n_rows,
+                                   s->ws.hit_tri + off, s->ws.faceid + off * L, st, launches, off))
                 return rc;
         }
+        rows_known = true;
     }
+    return 0;
+}
 
-    // ---- lights: (finish k-1, set up k) -> group by light vertex -> first-occluder sweep ----
-    auto build_face_tables = [&](int k, const std::vector<int> &group_cnt) -> int { // lazily, for groups that have rays
-        for (int gi = 0; gi < (int)group_cnt.size(); ++gi) {
-            if (!group_cnt[gi]) continue;
-            const int face = gi % trk::NFACE, vtx = s->h_light_vbase[k] + gi / trk::NFACE;
-            if (face == trk::NFACE - 1) {
-                if (!s->allcand_built) {
-                    trk::build_allcand_table<<<(s->n_pad + 255) / 256, 256, 0, st>>>(s->n_tris, s->n_pad, s->allcand_table, s->allcand_span);
-                    CK_CUDA(cudaGetLastError());
-                    s->allcand_built = true, ++launches;
-                }
-                continue;
-            }
-            double &built = s->table_lmax[(size_t)vtx * 6 + face];
-            const double need = (k + 1) * diag;
-            if (built >= need) continue;
-            built = need * 1.5; // head-room so that camera moves rarely trigger a rebuild
-            const trk::TableParam tp = face_param(&s->h_light_verts[3 * (size_t)vtx], face, built);
-            if (int rc = build_table(s, tp, s->light_tables + ((size_t)vtx * 6 + face) * s->table_stride,
-                                     s->light_spans + ((size_t)vtx * 6 + face) * s->span_stride, st))
-                return rc;
-            ++launches;
-        }
-        return 0;
-    };
-    trk::PixelState px{s->best, s->best_occ, s->hit_tri, s->hit_t, s->hit_v, s->carry, s->nrm, s->accum,
-                       s->ro,   s->rd,       s->re,      s->rt,    s->rj};
-    for (int k = 0; k <= L; ++k) {
-        trk::LightStepParams lp{};
-        lp.views = views, lp.bands = bands, lp.px = px;
-        lp.li = trk::LightInfo{s->light_vbase, s->light_verts};
-        lp.k = k, lp.L = L, lp.n_tris = s->n_tris;
-        lp.tri_verts = s->tri_verts, lp.tri_normals = s->tri_normals, lp.tri_geom = s->tri_geom;
-        lp.geom_has_normals = s->geom_has_normals, lp.geom_material = s->geom_material;
-        lp.sphere_material = s->sphere_material, lp.spheres = s->spheres;
-        lp.rng_mode = o.rng_mode, lp.seed = seed_s, lp.faceid = s->faceid, lp.lmax = (k + 1) * diag;
-        lp.seg_count = s->seg_count, lp.counters = s->counters;
-        lp.dbg_occ = o.out_occ_tri ? s->dbg_occ : nullptr;
-        lp.cull_cells = use_bvh ? 0 : (cull ? 1 : 2), lp.rkey = s->rkey;
-        if (k < L) CK_CUDA(cudaMemsetAsync(s->seg_count, 0, sizeof(int) * ((size_t)s->maxF * trk::NFACE + 1), st));
-        trk::light_step_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(lp);
+// ---- light k: (finish k-1, set up k) -> group by light vertex -> first-occluder sweep; k = L only finishes L-1 --------------
+int Frame::light(int k, uint32_t seed) {
+    trk::LightStepParams lp{};
+    lp.views = views, lp.bands = bands, lp.px = px;
+    lp.li = trk::LightInfo{s->light_vbase, s->light_verts};
+    lp.k = k, lp.L = L, lp.n_tris = s->n_tris;
+    lp.tri_verts = s->tri_verts, lp.tri_normals = s->tri_normals, lp.tri_geom = s->tri_geom;
+    lp.geom_has_normals = s->geom_has_normals, lp.geom_material = s->geom_material;
+    lp.sphere_material = s->sphere_material, lp.spheres = s->spheres;
+    lp.rng_mode = o.rng_mode, lp.seed = seed, lp.faceid = s->ws.faceid, lp.lmax = (k + 1) * diag;
+    lp.seg_count = s->seg_count, lp.counters = s->counters;
+    lp.dbg_occ = o.out_occ_tri ? s->ws.dbg_occ : nullptr;
+    lp.cull_cells = mode, lp.rkey = s->rkey;
+    if (k < L) CK_CUDA(cudaMemsetAsync(s->seg_count, 0, sizeof(int) * ((size_t)s->maxF * trk::NFACE + 1), st));
+    trk::light_step_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(lp);
+    CK_CUDA(cudaGetLastError());
+    ++launches;
+    if (k == L) return 0;
+    if (int rc = mode == BVH ? shadow_bvh(k) : mode == CULL ? shadow_cull(k) : shadow_sweeps(k)) return rc;
+    CK_CUDA(cudaEventRecord(s->ev_shadow[2 * k + 1], st));
+    return 0;
+}
+
+// The shadow rays of one light in list order, grouped by ray group (light vertex, cube face): seg_off = where each group
+// starts, cursor = its count, best_occ = no occluder yet.  Keys (light_step_kernel): default mode (group, q), so that the rays
+// of a thread can share a q-term (sweep::MODE_QBAR); bundle-cull mode (group, Morton code of (p,q)).  Pixels without a
+// shadow ray carry the all-ones key and sort last.
+int Frame::order_shadow_rays(int F) {
+    trk::list_prefix_kernel<<<1, 32, 0, st>>>(s->seg_count, F, s->seg_off, s->cursor);
+    CK_CUDA(cudaGetLastError());
+    int group_bits = 1;
+    while ((1 << group_bits) < F) ++group_bits;
+    CK_CUDA(cub::DeviceRadixSort::SortPairs(s->pair_tmp, s->pair_bytes, s->rkey, s->rkey_sorted, s->iota, s->ws.list, n_px, 0,
+                                            32 + group_bits + 1, st));
+    CK_CUDA(cudaMemcpyAsync(s->cursor, s->seg_count, sizeof(int) * F, cudaMemcpyDeviceToDevice, st));
+    CK_CUDA(cudaMemsetAsync(s->ws.best_occ, 0xff, sizeof(unsigned long long) * (size_t)n_px, st));
+    return 0;
+}
+
+// one thread per pixel: first occluder through the tree, then the spheres
+int Frame::shadow_bvh(int k) {
+    CK_CUDA(cudaEventRecord(s->ev_shadow[2 * k], st));
+    bvh::shadow_kernel<<<(n_px + 127) / 128, 128, 0, st>>>(s->bvh_tree, px, n_px, bvh::frame_margin(bvh_ext, (k + 1) * diag), s->tri_verts,
+                                                            s->spheres, s->n_spheres, s->n_tris, s->counters);
+    CK_CUDA(cudaGetLastError());
+    ++launches;
+    return 0;
+}
+
+// OPTIONAL bundle-cull mode: rays sorted by (group, Morton code of (p,q)), one culled sweep over all triangles per light
+int Frame::shadow_cull(int k) {
+    const int F = s->h_light_F[k] * trk::NFACE; // ray groups: (light vertex, cube face)
+    const int rpb = sweep::THREADS * 8;
+    if (int rc = order_shadow_rays(F)) return rc;
+    trk::chunk_prefix_kernel<<<1, 32, 0, st>>>(s->seg_count, F, rpb, s->n_pad / cull::CTILE, 2 * g.n_sms, s->blk_off, s->cnt_b, s->work,
+                                               s->n_slices, 24, 16);
+    CK_CUDA(cudaGetLastError());
+    std::vector<int> gcnt((size_t)F);
+    CK_CUDA(cudaMemcpyAsync(gcnt.data(), s->cursor, sizeof(int) * F, cudaMemcpyDeviceToHost, st));
+    CK_CUDA(cudaStreamSynchronize(st));
+    CK_CUDA(cudaEventRecord(s->ev_shadow[2 * k], st));
+    for (int gi = 0; gi < F; ++gi) { // the tables of the groups that have rays
+        if (!gcnt[gi]) continue;
+        const int face = gi % trk::NFACE, vtx = s->h_light_vbase[k] + gi / trk::NFACE;
+        if (int rc = face == trk::NFACE - 1 ? ensure_allcand_table(s, st, launches) : build_face_table(s, vtx, face, vtx, (k + 1) * diag, st, launches))
+            return rc;
+    }
+    trk::ShadowCullParams sp{};
+    sp.tables = s->light_tables + (size_t)s->h_light_vbase[k] * 6 * s->table_stride, sp.table_stride = s->table_stride;
+    sp.allcand = s->allcand_table, sp.n_tiles = s->n_pad / cull::CTILE, sp.n_tris = s->n_tris, sp.n_groups = F, sp.n_px = n_px;
+    sp.cells_per_group = 0, sp.n_slices = s->n_slices;
+    sp.list = s->ws.list, sp.seg_off = s->seg_off, sp.seg_cnt = s->cursor, sp.blk_off = s->blk_off, sp.px = px;
+    sp.counters = s->counters, sp.work = s->work;
+    sp.em = cull::Emitter{s->cand_a, s->cand_count, em_cap};
+    long long n_keys = -1;
+    if (two_phase) {
+        const int max_blocks = n_px / rpb + F + 1;
+        if (dev_grow(s->boxes_cap, (size_t)max_blocks, s->boxes)) return TRACER_ERR_NOMEM;
+        trk::shadow_boxes_kernel<<<max_blocks, sweep::THREADS, 0, st>>>(sp, s->boxes);
+        CK_CUDA(cudaGetLastError());
+        cull::L0Params lp{};
+        lp.tables = sp.tables, lp.allcand = sp.allcand, lp.table_stride = sp.table_stride;
+        lp.n_groups = F, lp.nface = trk::NFACE, lp.blk_off = s->blk_off;
+        if (int rc = block_lists(lp, max_blocks, n_keys)) return rc;
+    }
+    if (n_keys >= 0) {
+        trk::shadow_cull2_kernel<<<2 * g.n_sms, sweep::THREADS, 0, st>>>(sp, trk::BlockLists{s->boxes, s->cand_b, (unsigned long long)n_keys, tri_bits});
+        CK_CUDA(cudaGetLastError());
+        for (int c : gcnt) host_tests_shadow += (int64_t)c * s->n_pad;
+    } else {
+        CK_CUDA(cudaMemsetAsync(s->cand_count, 0, sizeof(unsigned long long), st));
+        const size_t smem = sizeof(cull::EmitSmem);
+        CK_CUDA(cudaFuncSetAttribute(trk::shadow_cull_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        trk::shadow_cull_kernel<<<2 * g.n_sms, sweep::THREADS, smem, st>>>(sp);
+        CK_CUDA(cudaGetLastError());
+    }
+    trk::strict_shadow_pairs<<<8 * g.n_sms, 256, 0, st>>>(s->cand_a, s->cand_count, em_cap, px, n_px, s->tri_verts, s->counters);
+    CK_CUDA(cudaGetLastError());
+    launches += 4;
+    if (s->n_spheres > 0) {
+        const dim3 sgrid((unsigned)std::min(1024, (n_px + 255) / 256), (unsigned)F);
+        trk::shadow_spheres_kernel<<<sgrid, 256, 0, st>>>(s->ws.list, s->seg_off, s->cursor, F, px, n_px, s->spheres, s->n_spheres, s->n_tris);
         CK_CUDA(cudaGetLastError());
         ++launches;
-        if (k == L) break;
-        if (use_bvh) { // one thread per pixel: first occluder through the tree, then the spheres
-            CK_CUDA(cudaEventRecord(s->ev_shadow[2 * k], st));
-            bvh::shadow_kernel<<<(n_px + 127) / 128, 128, 0, st>>>(s->bvh_tree, px, n_px, bvh::frame_margin(bvh_ext, (k + 1) * diag),
-                                                                    s->tri_verts, s->spheres, s->n_spheres, s->n_tris, s->counters);
-            CK_CUDA(cudaGetLastError());
-            ++launches;
-            CK_CUDA(cudaEventRecord(s->ev_shadow[2 * k + 1], st));
-            continue;
+    }
+    return 0;
+}
+
+// Triangle chunks of the default shadow sweep: after each one the still-unoccluded rays are compacted (early exit,
+// main.cpp:324).  Equal chunks keep the pairs swept past a ray's occluder lowest (x1.056 at 64 chunks; x1.11 at 32) and win
+// when a light has many shadow rays.  32 of them: at 32 rays per thread an item is twice as long and so is each chunk's tail
+// (C4: 189 ms of shadow sweep at 32 chunks, 192 at 48, 199 at 64; profiles/r05_d).  With few rays (small frames, one band
+// share of a multi-GPU frame) a chunk's fixed cost (three grid barriers, the compaction passes, the sweep's tail: ~0.1 ms)
+// weighs more, and 20 chunks that start fine (1/64 of the triangles: most occluded rays find their occluder early) and
+// coarsen win (x1.10).  The kernel picks the scheme from the live-ray count it finds.  opts.shadow_chunks asks for that many
+// equal chunks.
+void chunk_schemes(trk::ShadowLightParams &sp, int n_tiles, int shadow_chunks) {
+    const int nc = std::min({n_tiles, trk::SL_MAXCHUNK, shadow_chunks > 0 ? shadow_chunks : std::max(1, std::min(32, n_tiles / 8))});
+    sp.n_chunks[1] = nc;
+    for (int c = 0; c <= nc; ++c) sp.bounds[1][c] = (int)((int64_t)n_tiles * c / nc);
+    if (shadow_chunks > 0 || n_tiles < 64) {
+        sp.n_chunks[0] = nc;
+        std::memcpy(sp.bounds[0], sp.bounds[1], sizeof sp.bounds[0]);
+    } else {
+        std::vector<int> fr{0, 1, 2, 3, 4, 5, 6, 7, 8, 10, 12, 14, 16, 20, 24, 28, 32, 40, 48, 56, 64};
+        int den = 64;
+        if (const char *e = std::getenv("TRACER_GEO")) { // development knob: "den,f1,f2,...,den"
+            fr.assign(1, 0);
+            den = std::atoi(e);
+            for (const char *q = std::strchr(e, ','); q; q = std::strchr(q + 1, ',')) fr.push_back(std::atoi(q + 1));
         }
-        const int F = s->h_light_F[k] * trk::NFACE; // ray groups: (light vertex, cube face)
-        if (cull) {
-            // OPTIONAL bundle-cull mode: rays sorted by (group, Morton code of (p,q)), one culled sweep over all triangles per light
-            const int rpb = sweep::THREADS * 8;
-            int group_bits = 1;
-            while ((1 << group_bits) < F) ++group_bits;
-            trk::list_prefix_kernel<<<1, 32, 0, st>>>(s->seg_count, F, s->seg_off, s->cursor);
-            CK_CUDA(cudaGetLastError());
-            trk::chunk_prefix_kernel<<<1, 32, 0, st>>>(s->seg_count, F, rpb, s->n_pad / cull::CTILE, 2 * g.n_sms, s->blk_off, s->cnt_b, s->work,
-                                                       s->n_slices, 24, 16);
-            CK_CUDA(cudaGetLastError());
-            CK_CUDA(cub::DeviceRadixSort::SortPairs(s->pair_tmp, s->pair_bytes, s->rkey, s->rkey_sorted, s->iota, s->list, n_px, 0,
-                                                    32 + group_bits + 1, st));
-            CK_CUDA(cudaMemcpyAsync(s->cursor, s->seg_count, sizeof(int) * F, cudaMemcpyDeviceToDevice, st));
-            CK_CUDA(cudaMemsetAsync(s->best_occ, 0xff, sizeof(unsigned long long) * (size_t)n_px, st));
-            std::vector<int> gcnt((size_t)F);
-            CK_CUDA(cudaMemcpyAsync(gcnt.data(), s->cursor, sizeof(int) * F, cudaMemcpyDeviceToHost, st));
+        sp.n_chunks[0] = (int)fr.size() - 1;
+        for (size_t c = 0; c < fr.size(); ++c) sp.bounds[0][c] = (int)((int64_t)n_tiles * fr[c] / den);
+    }
+}
+
+// ---- default mode: q-sorted lists, then ONE persistent cooperative kernel per batch of light vertices ----
+int Frame::shadow_sweeps(int k) {
+    const int F = s->h_light_F[k] * trk::NFACE, n_tiles = s->n_pad / sweep::TILE; // ray groups: (light vertex, cube face)
+    if (int rc = order_shadow_rays(F)) return rc;
+    launches += 2;
+    if (dev_grow(s->blk_cnt_cap, (size_t)n_px / trk::CBLK + (size_t)F + 2, s->blk_cnt)) return TRACER_ERR_NOMEM;
+    CK_CUDA(cudaEventRecord(s->ev_shadow[2 * k], st));
+    if (int rc = ensure_allcand_table(s, st, launches)) return rc;
+    trk::ShadowLightParams sp{};
+    chunk_schemes(sp, n_tiles, o.shadow_chunks);
+    sp.many_rays = (long long)1 << 20;
+    sp.items_per_cta = items_per_cta();
+    sp.run_pairs = std::getenv("TRACER_RUN_PAIRS") ? std::max(1ll, std::atoll(std::getenv("TRACER_RUN_PAIRS"))) : 6000000ll;
+    sp.min_tiles = std::getenv("TRACER_MIN_TILES") ? std::max(1, std::atoi(std::getenv("TRACER_MIN_TILES"))) : 1;
+    sp.allcand = s->allcand_span, sp.table_stride = s->span_stride; // the default sweeps read the span tables
+    sp.n_tris = s->n_tris, sp.n_tiles = n_tiles, sp.n_px = n_px, sp.tri_verts = s->tri_verts;
+    sp.list[0] = s->ws.list, sp.list[1] = s->ws.list_b;
+    sp.blk_cnt = s->blk_cnt, sp.px = px, sp.spheres = s->spheres, sp.n_spheres = s->n_spheres;
+    sp.counters = s->counters;
+    // light vertices in batches: as many as have table slots (all of them unless the light is a big mesh)
+    const int Fk = s->h_light_F[k], vb = s->h_light_vbase[k];
+    for (int b0 = 0; b0 < Fk; b0 += s->table_slots) {
+        const int b1 = std::min(Fk, b0 + s->table_slots);
+        for (int v = b0; v < b1; ++v)
+            for (int face = 0; face < 6; ++face)
+                if (int rc = build_face_table(s, vb + v, face, s->tables_resident ? vb + v : v - b0, (k + 1) * diag, st, launches)) return rc;
+        sp.tables = s->light_spans + (s->tables_resident ? (size_t)(vb + b0) : 0) * 6 * s->span_stride;
+        sp.F = (b1 - b0) * trk::NFACE;
+        sp.seg_off = s->seg_off + b0 * trk::NFACE;
+        sp.cnt[0] = s->cursor + b0 * trk::NFACE, sp.cnt[1] = s->cnt_b + b0 * trk::NFACE;
+        sp.work = s->work;
+        CK_CUDA(cudaMemsetAsync(s->work, 0, sizeof(int) * WORK_INTS, st));
+        // development: TRACER_SHADOW_DIAG=2 dumps, for every light, when each CTA ran out of sweep items in each chunk
+        static const bool want_timeline = std::getenv("TRACER_SHADOW_DIAG") && std::atoi(std::getenv("TRACER_SHADOW_DIAG")) >= 2;
+        const size_t tl_n = (size_t)trk::SL_MAXCHUNK * 8 * (size_t)g.n_sms * 2;
+        unsigned long long *tl = nullptr;
+        if (want_timeline) {
+            tl = (unsigned long long *)t_pool->alloc(tl_n * sizeof(unsigned long long));
+            if (tl) CK_CUDA(cudaMemsetAsync(tl, 0, tl_n * sizeof(unsigned long long), st));
+        }
+        sp.timeline = tl;
+        if (int rc = launch_shadow_light(g, o.exhaustive_strict != 0, sp, (unsigned *)(s->work + trk::SL_MAXCHUNK), st)) return rc;
+        ++launches;
+        if (tl) {
+            std::vector<unsigned long long> h(tl_n);
+            CK_CUDA(cudaMemcpyAsync(h.data(), tl, tl_n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
             CK_CUDA(cudaStreamSynchronize(st));
-            CK_CUDA(cudaEventRecord(s->ev_shadow[2 * k], st));
-            if (int rc = build_face_tables(k, gcnt)) return rc;
-            trk::ShadowCullParams sp{};
-            sp.tables = s->light_tables + (size_t)s->h_light_vbase[k] * 6 * s->table_stride, sp.table_stride = s->table_stride;
-            sp.allcand = s->allcand_table, sp.n_tiles = s->n_pad / cull::CTILE, sp.n_tris = s->n_tris, sp.n_groups = F, sp.n_px = n_px;
-            sp.cells_per_group = 0, sp.n_slices = s->n_slices;
-            sp.list = s->list, sp.seg_off = s->seg_off, sp.seg_cnt = s->cursor, sp.blk_off = s->blk_off, sp.px = px;
-            sp.counters = s->counters, sp.work = s->work;
-            sp.em = cull::Emitter{s->cand_a, s->cand_count, em_cap};
-            long long n_keys = -1;
-            if (two_phase) {
-                const int max_blocks = n_px / rpb + F + 1;
-                if (int rc = ensure_boxes((size_t)max_blocks)) return rc;
-                trk::shadow_boxes_kernel<<<max_blocks, sweep::THREADS, 0, st>>>(sp, s->boxes);
-                CK_CUDA(cudaGetLastError());
-                cull::L0Params lp{};
-                lp.tables = sp.tables, lp.allcand = sp.allcand, lp.table_stride = sp.table_stride;
-                lp.n_groups = F, lp.nface = trk::NFACE, lp.blk_off = s->blk_off;
-                if (int rc = block_lists(lp, max_blocks, n_keys)) return rc;
+            t_pool->release(tl);
+            char name[128];
+            std::snprintf(name, sizeof name, "gpurun_out/shadow_timeline_light%d.bin", k);
+            if (FILE *f = std::fopen(name, "wb")) {
+                const int hdr[2] = {trk::SL_MAXCHUNK, 8 * g.n_sms};
+                std::fwrite(hdr, sizeof hdr, 1, f), std::fwrite(h.data(), sizeof(unsigned long long), h.size(), f), std::fclose(f);
             }
-            if (n_keys >= 0) {
-                trk::shadow_cull2_kernel<<<2 * g.n_sms, sweep::THREADS, 0, st>>>(sp, trk::BlockLists{s->boxes, s->cand_b, (unsigned long long)n_keys, tri_bits});
-                CK_CUDA(cudaGetLastError());
-                for (int c : gcnt) host_tests_shadow += (int64_t)c * s->n_pad;
-            } else {
-                CK_CUDA(cudaMemsetAsync(s->cand_count, 0, sizeof(unsigned long long), st));
-                const size_t smem = sizeof(cull::EmitSmem);
-                CK_CUDA(cudaFuncSetAttribute(trk::shadow_cull_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                trk::shadow_cull_kernel<<<2 * g.n_sms, sweep::THREADS, smem, st>>>(sp);
-                CK_CUDA(cudaGetLastError());
-            }
-            trk::strict_shadow_pairs<<<8 * g.n_sms, 256, 0, st>>>(s->cand_a, s->cand_count, em_cap, px, n_px,
-                                                                  s->tri_verts, s->counters);
-            CK_CUDA(cudaGetLastError());
-            launches += 4;
-            if (s->n_spheres > 0) {
-                const dim3 sgrid((unsigned)std::min(1024, (n_px + 255) / 256), (unsigned)F);
-                trk::shadow_spheres_kernel<<<sgrid, 256, 0, st>>>(s->list, s->seg_off, s->cursor, F, px, n_px, s->spheres, s->n_spheres,
-                                                                   s->n_tris);
-                CK_CUDA(cudaGetLastError());
-                ++launches;
-            }
-            CK_CUDA(cudaEventRecord(s->ev_shadow[2 * k + 1], st));
-            continue;
-        }
-        // ---- default mode: q-sorted lists, then ONE persistent cooperative kernel per batch of light vertices ----
-        trk::list_prefix_kernel<<<1, 32, 0, st>>>(s->seg_count, F, s->seg_off, s->cursor);
-        CK_CUDA(cudaGetLastError());
-        { // group-major, q-minor order (pixels without a shadow ray carry the all-ones key and sort last)
-            int group_bits = 1;
-            while ((1 << group_bits) < F) ++group_bits;
-            CK_CUDA(cub::DeviceRadixSort::SortPairs(s->pair_tmp, s->pair_bytes, s->rkey, s->rkey_sorted, s->iota, s->list, n_px, 0,
-                                                    32 + group_bits + 1, st));
-            CK_CUDA(cudaMemcpyAsync(s->cursor, s->seg_count, sizeof(int) * F, cudaMemcpyDeviceToDevice, st));
-            const size_t need = (size_t)n_px / trk::CBLK + (size_t)F + 2;
-            if (need > s->blk_cnt_cap) {
-                dev_free(s->blk_cnt);
-                s->blk_cnt_cap = 0;
-                if (dev_alloc(&s->blk_cnt, need)) return TRACER_ERR_NOMEM;
-                s->blk_cnt_cap = need;
-            }
-        }
-        launches += 2;
-        CK_CUDA(cudaMemsetAsync(s->best_occ, 0xff, sizeof(unsigned long long) * (size_t)n_px, st));
-        CK_CUDA(cudaEventRecord(s->ev_shadow[2 * k], st));
-        if (!s->allcand_built) {
-            trk::build_allcand_table<<<(s->n_pad + 255) / 256, 256, 0, st>>>(s->n_tris, s->n_pad, s->allcand_table, s->allcand_span);
-            CK_CUDA(cudaGetLastError());
-            s->allcand_built = true, ++launches;
-        }
-        // Triangle chunks: after each one the still-unoccluded rays are compacted (early exit, main.cpp:324).  Equal chunks
-        // keep the pairs swept past a ray's occluder lowest (x1.056 at 64 chunks; x1.11 at 32) and win when a light has many
-        // shadow rays.  32 of them: at 32 rays per thread an item is twice as long and so is each chunk's tail (C4: 189 ms
-        // of shadow sweep at 32 chunks, 192 at 48, 199 at 64; profiles/r05_d).  With few rays (small frames, one band share of
-        // a multi-GPU frame) a chunk's fixed cost (three grid barriers, the compaction passes, the sweep's tail: ~0.1 ms)
-        // weighs more, and 20 chunks that start fine (1/64 of the triangles: most occluded rays find their occluder early) and coarsen win (x1.10).  The kernel picks the scheme from
-        // the live-ray count it finds.  opts.shadow_chunks asks for that many equal chunks.
-        trk::ShadowLightParams sp{};
-        {
-            const int nc = std::min({n_tiles, trk::SL_MAXCHUNK, o.shadow_chunks > 0 ? o.shadow_chunks : std::max(1, std::min(32, n_tiles / 8))});
-            sp.n_chunks[1] = nc;
-            for (int c = 0; c <= nc; ++c) sp.bounds[1][c] = (int)((int64_t)n_tiles * c / nc);
-            if (o.shadow_chunks > 0 || n_tiles < 64) {
-                sp.n_chunks[0] = nc;
-                std::memcpy(sp.bounds[0], sp.bounds[1], sizeof sp.bounds[0]);
-            } else {
-                std::vector<int> fr{0, 1, 2, 3, 4, 5, 6, 7, 8, 10, 12, 14, 16, 20, 24, 28, 32, 40, 48, 56, 64};
-                int den = 64;
-                if (const char *e = std::getenv("TRACER_GEO")) { // development knob: "den,f1,f2,...,den"
-                    fr.assign(1, 0);
-                    den = std::atoi(e);
-                    for (const char *q = std::strchr(e, ','); q; q = std::strchr(q + 1, ',')) fr.push_back(std::atoi(q + 1));
-                }
-                sp.n_chunks[0] = (int)fr.size() - 1;
-                for (size_t c = 0; c < fr.size(); ++c) sp.bounds[0][c] = (int)((int64_t)n_tiles * fr[c] / den);
-            }
-        }
-        sp.many_rays = (long long)1 << 20;
-        sp.items_per_cta = items_per_cta();
-        sp.run_pairs = std::getenv("TRACER_RUN_PAIRS") ? std::max(1ll, std::atoll(std::getenv("TRACER_RUN_PAIRS"))) : 6000000ll;
-        sp.min_tiles = std::getenv("TRACER_MIN_TILES") ? std::max(1, std::atoi(std::getenv("TRACER_MIN_TILES"))) : 1;
-        sp.allcand = s->allcand_span, sp.table_stride = s->span_stride; // the default sweeps read the span tables
-        sp.n_tris = s->n_tris, sp.n_tiles = n_tiles, sp.n_px = n_px, sp.tri_verts = s->tri_verts;
-        sp.list[0] = s->list, sp.list[1] = s->list_b;
-        sp.blk_cnt = s->blk_cnt, sp.px = px, sp.spheres = s->spheres, sp.n_spheres = s->n_spheres;
-        sp.counters = s->counters;
-        // light vertices in batches: as many as have table slots (all of them unless the light is a big mesh)
-        const int Fk = s->h_light_F[k], vb = s->h_light_vbase[k];
-        for (int b0 = 0; b0 < Fk; b0 += s->table_slots) {
-            const int b1 = std::min(Fk, b0 + s->table_slots);
-            for (int v = b0; v < b1; ++v)
-                for (int face = 0; face < 6; ++face) {
-                    // every vertex has its own slot when they all fit (tables are then kept across frames and lights);
-                    // otherwise the slots are reused batch by batch and rebuilt every time
-                    const size_t slot = s->tables_resident ? (size_t)(vb + v) : (size_t)(v - b0);
-                    const double need = (k + 1) * diag;
-                    if (s->tables_resident) {
-                        double &built = s->table_lmax[slot * 6 + face];
-                        if (built >= need) continue;
-                        built = need * 1.5; // head-room so that camera moves rarely trigger a rebuild
-                    }
-                    const trk::TableParam tp = face_param(&s->h_light_verts[3 * (size_t)(vb + v)], face, need * 1.5);
-                    if (int rc = build_table(s, tp, s->light_tables + (slot * 6 + face) * s->table_stride,
-                                             s->light_spans + (slot * 6 + face) * s->span_stride, st))
-                        return rc;
-                    ++launches;
-                }
-            sp.tables = s->light_spans + (s->tables_resident ? (size_t)(vb + b0) : 0) * 6 * s->span_stride;
-            sp.F = (b1 - b0) * trk::NFACE;
-            sp.seg_off = s->seg_off + b0 * trk::NFACE;
-            sp.cnt[0] = s->cursor + b0 * trk::NFACE, sp.cnt[1] = s->cnt_b + b0 * trk::NFACE;
-            sp.work = s->work;
-            CK_CUDA(cudaMemsetAsync(s->work, 0, sizeof(int) * WORK_INTS, st));
-            // development: TRACER_SHADOW_DIAG=2 dumps, for every light, when each CTA ran out of sweep items in each chunk
-            static const bool want_timeline = std::getenv("TRACER_SHADOW_DIAG") && std::atoi(std::getenv("TRACER_SHADOW_DIAG")) >= 2;
-            const size_t tl_n = (size_t)trk::SL_MAXCHUNK * 8 * (size_t)g.n_sms * 2;
-            unsigned long long *tl = nullptr;
-            if (want_timeline) {
-                tl = (unsigned long long *)t_pool->alloc(tl_n * sizeof(unsigned long long));
-                if (tl) CK_CUDA(cudaMemsetAsync(tl, 0, tl_n * sizeof(unsigned long long), st));
-            }
-            sp.timeline = tl;
-            if (int rc = launch_shadow_light(g, o.exhaustive_strict != 0, sp, (unsigned *)(s->work + trk::SL_MAXCHUNK), st)) return rc;
-            ++launches;
-            if (tl) {
-                std::vector<unsigned long long> h(tl_n);
-                CK_CUDA(cudaMemcpyAsync(h.data(), tl, tl_n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-                CK_CUDA(cudaStreamSynchronize(st));
-                t_pool->release(tl);
-                char name[128];
-                std::snprintf(name, sizeof name, "gpurun_out/shadow_timeline_light%d.bin", k);
-                if (FILE *f = std::fopen(name, "wb")) {
-                    const int hdr[2] = {trk::SL_MAXCHUNK, 8 * g.n_sms};
-                    std::fwrite(hdr, sizeof hdr, 1, f), std::fwrite(h.data(), sizeof(unsigned long long), h.size(), f), std::fclose(f);
-                }
-            }
-        }
-        CK_CUDA(cudaEventRecord(s->ev_shadow[2 * k + 1], st));
-    }
-    if (S > 1) { // sum the samples in a fixed order; the last pass divides by S
-        const size_t n3 = 3 * (size_t)n_px;
-        trk::accumulate_kernel<<<(unsigned)((n3 + 255) / 256), 256, 0, st>>>(s->accum, s->accum_total, n3, smp == 0, smp == S - 1,
-                                                                              (float)S);
-        CK_CUDA(cudaGetLastError());
-        ++launches;
-        CK_CUDA(cudaStreamSynchronize(st));
-        float msx = 0;
-        cudaEventElapsedTime(&msx, s->ev[1], s->ev[2]);
-        ms_primary_acc += msx;
-        for (int k = 0; k < L; ++k) {
-            cudaEventElapsedTime(&msx, s->ev_shadow[2 * k], s->ev_shadow[2 * k + 1]);
-            ms_shadow_acc += msx;
         }
     }
-    } // samples
+    return 0;
+}
 
-    // ---- quantise + pack ------------------------------------------------------------------
-    uint8_t *dst8 = o.rgb_out_is_device ? rgb_out : s->rgb8;
-    const float *final_accum = S > 1 ? s->accum_total : s->accum;
+// S > 1: sum the samples in a fixed order; the last pass divides by S
+int Frame::accumulate(int smp) {
+    const size_t n3 = 3 * (size_t)n_px;
+    trk::accumulate_kernel<<<(unsigned)((n3 + 255) / 256), 256, 0, st>>>(s->ws.accum, s->ws.accum_total, n3, smp == 0, smp == S - 1, (float)S);
+    CK_CUDA(cudaGetLastError());
+    ++launches;
+    CK_CUDA(cudaStreamSynchronize(st));
+    add_sample_times();
+    return 0;
+}
+
+// The event times of the sample just rendered (after a synchronise): its closest-hit pass and its shadow sweeps
+void Frame::add_sample_times() {
+    float ms = 0;
+    cudaEventElapsedTime(&ms, s->ev[1], s->ev[2]);
+    ms_primary += ms;
+    for (int k = 0; k < L; ++k) {
+        cudaEventElapsedTime(&ms, s->ev_shadow[2 * k], s->ev_shadow[2 * k + 1]);
+        ms_shadow += ms;
+    }
+}
+
+// ---- quantise + pack, read-backs, stats --------------------------------------------------------------------------------
+int Frame::finish_frame(uint8_t *rgb_out) {
+    uint8_t *dst8 = o.rgb_out_is_device ? rgb_out : s->ws.rgb8;
+    const float *final_accum = S > 1 ? s->ws.accum_total : s->ws.accum;
     trk::quantise_kernel<<<((n_px + 15) / 16 + 127) / 128, 128, 0, st>>>(final_accum, n_px, dst8);
     CK_CUDA(cudaGetLastError());
     ++launches;
     CK_CUDA(cudaEventRecord(s->ev[3], st));
-    if (!o.rgb_out_is_device) CK_CUDA(cudaMemcpyAsync(rgb_out, s->rgb8, (size_t)n_px * 3, cudaMemcpyDeviceToHost, st));
-
-    // ---- optional debug read-backs -----------------------------------------------------------
-    if (o.out_tri) CK_CUDA(cudaMemcpyAsync(o.out_tri, s->hit_tri, (size_t)n_px * 4, cudaMemcpyDeviceToHost, st));
-    if (o.out_t) CK_CUDA(cudaMemcpyAsync(o.out_t, s->hit_t, (size_t)n_px * 4, cudaMemcpyDeviceToHost, st));
-    if (o.out_v) CK_CUDA(cudaMemcpyAsync(o.out_v, s->hit_v, (size_t)n_px * 4, cudaMemcpyDeviceToHost, st));
+    if (!o.rgb_out_is_device) CK_CUDA(cudaMemcpyAsync(rgb_out, s->ws.rgb8, (size_t)n_px * 3, cudaMemcpyDeviceToHost, st));
+    // optional debug read-backs
+    if (o.out_tri) CK_CUDA(cudaMemcpyAsync(o.out_tri, s->ws.hit_tri, (size_t)n_px * 4, cudaMemcpyDeviceToHost, st));
+    if (o.out_t) CK_CUDA(cudaMemcpyAsync(o.out_t, s->ws.hit_t, (size_t)n_px * 4, cudaMemcpyDeviceToHost, st));
+    if (o.out_v) CK_CUDA(cudaMemcpyAsync(o.out_v, s->ws.hit_v, (size_t)n_px * 4, cudaMemcpyDeviceToHost, st));
     if (o.out_occ_tri && L > 0)
-        CK_CUDA(cudaMemcpyAsync(o.out_occ_tri, s->dbg_occ, (size_t)n_px * L * 4, cudaMemcpyDeviceToHost, st));
+        CK_CUDA(cudaMemcpyAsync(o.out_occ_tri, s->ws.dbg_occ, (size_t)n_px * L * 4, cudaMemcpyDeviceToHost, st));
     std::vector<float> acc;
     if (o.out_rgb) {
         acc.resize((size_t)n_px * 3);
@@ -1735,16 +1697,10 @@ int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, in
     float ms = 0;
     cudaEventElapsedTime(&ms, s->ev[0], s->ev[3]);
     s->stats.ms_total = ms;
-    cudaEventElapsedTime(&ms, s->ev[1], s->ev[2]);
-    s->stats.ms_primary = S > 1 ? ms_primary_acc : ms;
-    double sh = 0;
-    for (int k = 0; k < L; ++k) {
-        cudaEventElapsedTime(&ms, s->ev_shadow[2 * k], s->ev_shadow[2 * k + 1]);
-        sh += ms;
-    }
-    if (S > 1) sh = ms_shadow_acc;
-    s->stats.ms_shadow = sh;
-    s->stats.ms_other = s->stats.ms_total - s->stats.ms_primary - sh;
+    if (S == 1) add_sample_times();
+    s->stats.ms_primary = ms_primary;
+    s->stats.ms_shadow = ms_shadow;
+    s->stats.ms_other = s->stats.ms_total - s->stats.ms_primary - ms_shadow;
     s->stats.n_primary_rays = (int64_t)n_px * S;
     s->stats.n_shadow_rays = (int64_t)hc.n_hits * L;
     s->stats.tests_primary = (int64_t)hc.tests_primary + host_tests_primary;
@@ -1757,13 +1713,12 @@ int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, in
     // FP32 flops the sweeps' formulation needs per swept pair (FFMA = 2, FADD = FMUL = 1, a minimum 0).  Interval form: half
     // a packed FADD2 per pair, plus per thread and triangle the bound FFMAs, 4 (one exact q) or 8 (mean q + |B| * spread:
     // shadow sweeps, jittered primary samples), and the interval's centre and half width (7 flops), over the R rays.
-    const bool no_flops = cull || use_bvh; // the optional modes: no fixed per-pair cost
+    const bool no_flops = mode != SWEEPS; // the optional modes: no fixed per-pair cost
     s->stats.flop_primary = no_flops ? 0.0 : flop_primary, s->stats.flop_shadow = no_flops ? 0.0 : 1.0 + 18.0 / trk::SHADOW_R;
     // of which multiply-adds that evaluate bounds (the rest is each pair's interval test and the per-triangle interval)
     s->stats.flop_primary_edges = no_flops ? 0.0 : flop_primary_edges;
     s->stats.flop_shadow_edges = no_flops ? 0.0 : 16.0 / trk::SHADOW_R;
-    if (hc.cull_overflow) // (with TRACER_RNG_MT19937 only the shadow sweeps' candidates can have overflowed by now)
-        return rerender_after_overflow(o.rng_mode == TRACER_RNG_MT19937 ? &mt_frame : nullptr);
+    if (hc.cull_overflow) return CAND_OVERFLOW; // (with TRACER_RNG_MT19937 only the shadow sweeps' candidates can have overflowed by now)
     if (getenv("TRACER_SHADOW_DIAG") && hc.cyc_total)
         fprintf(stderr, "shadow diag: CTA cycles %.3e total = items %.1f %% + grid barriers %.1f %% + compaction %.1f %% + other %.1f %%; %llu items in %llu runs\n",
                 (double)hc.cyc_total, 100.0 * hc.cyc_items / hc.cyc_total, 100.0 * hc.cyc_barrier / hc.cyc_total, 100.0 * hc.cyc_compact / hc.cyc_total,
@@ -1773,6 +1728,84 @@ int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, in
                 hc.cull_tiles_any, hc.cull_tiles_fallback, hc.cull_l1, (unsigned long long)(hc.tests_shadow / 4096 / cull::CTILE));
     return TRACER_OK;
 }
+
+// Checks the call, then renders it: again after a bundle-cull candidate overflow, with a 4x larger candidate buffer while
+// that fits comfortably, else by the default sweeps, which need no such buffer (same bytes out either way).  The stats are
+// those of the last attempt.
+int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, int32_t W, int32_t H, const tracer_render_opts *opts_in,
+                 uint8_t *rgb_out) {
+    if (!s || !cams || !rgb_out) return fail(TRACER_ERR_INVALID, "null argument");
+    if (!s->ctx || !s->ctx->inited) return fail(TRACER_ERR_NO_DEVICE, "tracer_cuda_init not called");
+    Ctx &g = *s->ctx;
+    t_pool = &g.pool;
+    if (W < 2 || H < 2) return fail(TRACER_ERR_INVALID, "width and height must be >= 2 (the reference divides by W-1, H-1)");
+    // per-pixel planes are indexed with int (3 planes of n_px floats): keep 3 * n_px below 2^31
+    if ((int64_t)n_views * W * H > (int64_t)700 * 1000 * 1000)
+        return fail(TRACER_ERR_INVALID, "frame too large (limit 7e8 pixels per call, over all views; render bands or fewer views)");
+    tracer_render_opts o = read_opts(opts_in);
+    // extension (parity unpinned): samples_per_pixel = n*n stratified jittered samples per pixel
+    int spp_n = 1;
+    if (o.samples_per_pixel > 1) {
+        spp_n = (int)std::lround(std::sqrt((double)o.samples_per_pixel));
+        if (spp_n * spp_n != o.samples_per_pixel || spp_n > 16)
+            return fail(TRACER_ERR_INVALID, "samples_per_pixel must be a square number <= 256");
+        if (o.rng_mode == TRACER_RNG_MT19937)
+            return fail(TRACER_ERR_INVALID, "TRACER_RNG_MT19937 reproduces the 1-sample serial path only");
+    }
+    const int band_count = o.band_count <= 1 ? 1 : o.band_count;
+    const int band_rows = band_count > 1 ? o.band_rows : H;
+    if (band_count > 1 && (band_rows <= 0 || o.band_index < 0 || o.band_index >= band_count))
+        return fail(TRACER_ERR_INVALID, "bad band selection");
+    if (o.rng_mode == TRACER_RNG_MT19937 && band_count > 1 && !o.row_hits_exchange)
+        return fail(TRACER_ERR_INVALID, "TRACER_RNG_MT19937 with band_count > 1 needs opts->row_hits_exchange (the other bands' row hit counts)");
+    if (o.rng_mode == TRACER_RNG_EXPLICIT && !o.faceid && s->n_lights > 0)
+        return fail(TRACER_ERR_INVALID, "TRACER_RNG_EXPLICIT needs opts->faceid");
+    if (o.rng_mode < 0 || o.rng_mode > 2) return fail(TRACER_ERR_INVALID, "bad rng_mode");
+    if (o.accel < 0 || o.accel > 1) return fail(TRACER_ERR_INVALID, "bad accel (0 = sweeps, 1 = BVH)");
+    if (o.accel == 1 && (o.bundle_cull != 0 || o.exhaustive_strict != 0))
+        return fail(TRACER_ERR_INVALID, "accel = 1 (BVH) does not combine with bundle_cull or exhaustive_strict (a debug mode of the sweeps' filter)");
+    const int band_index = band_count > 1 ? o.band_index : 0;
+    const int n_rows = tracer_band_row_count(H, band_rows, band_index, band_count);
+    const int view_px = n_rows * W, n_px = n_views * view_px;
+    trk::Bands bands{W, H, band_rows, band_index, band_count, n_px};
+    bands.spp_n = spp_n, bands.sample = 0, bands.seed = o.seed;
+    const cudaStream_t st = o.cuda_stream ? (cudaStream_t)o.cuda_stream : g.stream;
+    std::vector<int> frame_rows;
+    bool rows_known = false;
+    for (;;) {
+        Frame f{s, g, o, cams, st, W, H, n_rows, view_px, n_px, n_views, s->n_lights, spp_n * spp_n, bands};
+        const int rc = f.render(rgb_out, frame_rows, rows_known);
+        if (rc != CAND_OVERFLOW) return rc;
+        size_t free_b = 0, total_b = 0;
+        cudaMemGetInfo(&free_b, &total_b);
+        const size_t next_bytes = ((size_t)n_px * 24 * (size_t)s->cull_grow * 4 + ((size_t)1 << 22)) * sizeof(unsigned long long) * 3;
+        if (!std::getenv("TRACER_CAND_CAP") && s->cull_grow < 64 && next_bytes < free_b / 2 + s->cand_cap * 24)
+            s->cull_grow *= 4;
+        else
+            o.bundle_cull = 0;
+    }
+}
+}  // namespace
+
+extern "C" {
+
+int tracer_cuda_render_scene(tracer_scene_dev *s, const tracer_camera *cam, int32_t W, int32_t H,
+                             const tracer_render_opts *opts_in, uint8_t *rgb_out) {
+    return render_views(s, cam, 1, W, H, opts_in, rgb_out);
+}
+
+int tracer_cuda_render_views(tracer_scene_dev *s, const tracer_camera *cams, int32_t n_views, int32_t W, int32_t H,
+                             const tracer_render_opts *opts_in, uint8_t *rgb_out) {
+    if (n_views < 1) return fail(TRACER_ERR_INVALID, "n_views must be >= 1");
+    if (!cams) return fail(TRACER_ERR_INVALID, "null cameras");
+    const tracer_render_opts o = read_opts(opts_in);
+    if (o.band_count > 1) return fail(TRACER_ERR_INVALID, "tracer_cuda_render_views renders whole views: band_count must be <= 1");
+    if (o.bundle_cull != 0) return fail(TRACER_ERR_INVALID, "tracer_cuda_render_views does not combine with bundle_cull");
+    return render_views(s, cams, n_views, W, H, opts_in, rgb_out);
+}
+}  // extern "C"
+
+namespace {
 // ---- scene updates (tracer_cuda_scene_update) -----------------------------------------------------------------------------
 // The checks of one replica that need no device: the struct, the triangle range, data for a count, normals
 int update_check(const tracer_scene_dev *s, const tracer_scene_update *u) {
@@ -1847,6 +1880,7 @@ int update_apply(tracer_scene_dev *s, const tracer_scene_update &u, int src_devi
             const std::vector<float> old = s->h_light_verts;
             CK_CUDA(cudaMemcpyAsync(s->h_light_verts.data(), s->light_verts, old.size() * sizeof(float), cudaMemcpyDeviceToHost, st));
             CK_CUDA(cudaStreamSynchronize(st));
+            int launches = 0; // (an update keeps no launch count)
             for (int v = 0; s->tables_resident && v < s->V; ++v) {
                 const bool moved = std::memcmp(&old[3 * (size_t)v], &s->h_light_verts[3 * (size_t)v], 3 * sizeof(float)) != 0;
                 for (int face = 0; face < 6; ++face) {
@@ -1856,10 +1890,7 @@ int update_apply(tracer_scene_dev *s, const tracer_scene_update &u, int src_devi
                         built = -1.0;
                         continue;
                     }
-                    const trk::TableParam tp = face_param(&s->h_light_verts[3 * (size_t)v], face, built);
-                    if (int r = build_table(s, tp, s->light_tables + ((size_t)v * 6 + face) * s->table_stride,
-                                            s->light_spans + ((size_t)v * 6 + face) * s->span_stride, st, u.tri_first, u.tri_count))
-                        return r;
+                    if (int r = build_face_table(s, v, face, v, built, st, launches, u.tri_first, u.tri_count)) return r;
                 }
             }
         }
@@ -2148,9 +2179,7 @@ int tracer_cuda_render_scene_multi(tracer_scene_multi *ms, const tracer_camera *
         ms->stats = ms->dev[0]->stats;
         return rc;
     }
-    tracer_render_opts o;
-    std::memset(&o, 0, sizeof o);
-    if (opts_in) std::memcpy(&o, opts_in, std::min<size_t>(sizeof o, opts_in->struct_size ? opts_in->struct_size : sizeof o));
+    const tracer_render_opts o = read_opts(opts_in);
     if (o.band_count > 1) return fail(TRACER_ERR_INVALID, "the multi-GPU call partitions the frame itself: leave band_count at 0");
     if (o.out_tri || o.out_t || o.out_v || o.out_occ_tri || o.out_rgb) return fail(TRACER_ERR_INVALID, "debug outputs are per-GPU: use tracer_cuda_render_scene with bands");
     if (W < 2 || H < 2 || (int64_t)W * H > (int64_t)2000 * 1000 * 1000) return fail(TRACER_ERR_INVALID, "bad frame size");
@@ -2162,18 +2191,8 @@ int tracer_cuda_render_scene_multi(tracer_scene_multi *ms, const tracer_camera *
     Ctx &g0 = g_ctx[0];
     CK_CUDA(cudaSetDevice(0));
     t_pool = &g0.pool;
-    if (g_multi.gathered_cap < pad_bytes * n + 64) {
-        dev_free(g_multi.gathered);
-        g_multi.gathered_cap = 0;
-        if (dev_alloc(&g_multi.gathered, pad_bytes * n + 64)) return TRACER_ERR_NOMEM;
-        g_multi.gathered_cap = pad_bytes * n + 64;
-    }
-    if (g_multi.frame_cap < frame_bytes + 64) {
-        dev_free(g_multi.frame);
-        g_multi.frame_cap = 0;
-        if (dev_alloc(&g_multi.frame, frame_bytes + 64)) return TRACER_ERR_NOMEM;
-        g_multi.frame_cap = frame_bytes + 64;
-    }
+    if (dev_grow(g_multi.gathered_cap, pad_bytes * n + 64, g_multi.gathered) || dev_grow(g_multi.frame_cap, frame_bytes + 64, g_multi.frame))
+        return TRACER_ERR_NOMEM;
     std::vector<int> rc((size_t)n, 0);
     std::vector<std::string> err((size_t)n);
     const bool mt = o.rng_mode == TRACER_RNG_MT19937;
@@ -2186,12 +2205,7 @@ int tracer_cuda_render_scene_multi(tracer_scene_multi *ms, const tracer_camera *
         if (d > 0) {
             if (cudaSetDevice(d) != cudaSuccess) { rc[d] = TRACER_ERR_CUDA, err[d] = "cudaSetDevice"; return; }
             t_pool = &g.pool;
-            if (g_multi.band_cap[d] < pad_bytes + 64) {
-                dev_free(g_multi.band_buf[d]);
-                g_multi.band_cap[d] = 0;
-                if (dev_alloc(&g_multi.band_buf[d], pad_bytes + 64)) { rc[d] = TRACER_ERR_NOMEM, err[d] = g_err; return; }
-                g_multi.band_cap[d] = pad_bytes + 64;
-            }
+            if (dev_grow(g_multi.band_cap[d], pad_bytes + 64, g_multi.band_buf[d])) { rc[d] = TRACER_ERR_NOMEM, err[d] = g_err; return; }
             dst = g_multi.band_buf[d];
         }
         tracer_render_opts od = o;
