@@ -59,6 +59,7 @@ class RenderOpts(C.Structure):
         ("out_tri", C.POINTER(C.c_int32)), ("out_t", C.POINTER(C.c_float)), ("out_v", C.POINTER(C.c_float)),
         ("out_occ_tri", C.POINTER(C.c_int32)), ("out_rgb", C.POINTER(C.c_float)), ("accel", C.c_int32),
         ("row_hits_exchange", ROW_HITS_EXCHANGE), ("row_hits_user", C.c_void_p),
+        ("crop_x", C.c_int32), ("crop_y", C.c_int32), ("crop_w", C.c_int32), ("crop_h", C.c_int32),
     ]
 
 

@@ -17,6 +17,7 @@ there is no CPU path here.
 from __future__ import annotations
 
 import ctypes as C
+import operator
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -189,6 +190,19 @@ def hash_faceids(seed: int, width: int, height: int, faces_per_light) -> np.ndar
 
 def band_row_count(height, band_rows, band_index, band_count) -> int:
     return int(_lib.load().tracer_band_row_count(height, band_rows, band_index, band_count))
+
+
+def _crop_window(crop, width, height, bands):
+    """(x, y, w, h) of a crop window inside the width x height frame, or ValueError"""
+    try:
+        x, y, w, h = (operator.index(c) for c in crop)
+    except (TypeError, ValueError):
+        raise ValueError(f"crop must be four integers (x, y, w, h), not {crop!r}") from None
+    if w < 1 or h < 1 or x < 0 or y < 0 or x + w > width or y + h > height:
+        raise ValueError(f"crop window {(x, y, w, h)} is not inside the {width} x {height} frame")
+    if bands is not None:
+        raise ValueError("a crop window does not combine with bands")
+    return x, y, w, h
 
 
 @dataclass
@@ -440,7 +454,7 @@ class Renderer:
     def trace(self, scene, camera: Camera, width: int, height: int, *, rng_mode=RNG_HASH, seed=1, faceid=None,
               bands=None, exhaustive_strict=False, debug=False, out_device_ptr=None, stream=None,
               rays_per_thread=0, shadow_chunks=0, samples_per_pixel=0, bundle_cull=False, out=None, bvh=False,
-              row_hits_exchange=None) -> Frame:
+              row_hits_exchange=None, crop=None) -> Frame:
         """Render; ``scene`` is a Scene (one-shot: upload + render, the drop-in call) or a
         ResidentScene.  ``bvh``: the optional BVH mode (opts.accel = 1): the resident scene builds its tree on the
         first such render and keeps it; same bytes as the default mode.  ``bands`` = (band_rows, band_index, band_count).  With
@@ -448,21 +462,35 @@ class Renderer:
         caller-owned uint8 [rows, W, 3] host array (e.g. pinned) to receive them.  ``row_hits_exchange``: with
         ``RNG_MT19937`` and bands, a callable ``(row_hits: np.ndarray[int32, H]) -> None`` that completes this call's
         per-row hit counts into the frame's, in place (opts.row_hits_exchange; an all-reduce sum over the calls that render
-        the frame does it).  An exception inside it fails the render with TracerError."""
+        the frame does it).  An exception inside it fails the render with TracerError.
+
+        ``crop`` = (x, y, w, h): render only columns [x, x+w) of PPM rows [y, y+h) (row 0 at the top) of the width x
+        height frame.  ``rgb8`` is then [h, w, 3] and the debug arrays [h*w, ...], bit for bit the same pixels of the whole
+        frame, in every mode; ``faceid`` (RNG_EXPLICIT) stays the whole frame's.  Raises ValueError for a window that is not
+        inside the frame, a crop with ``bands`` or an ``out`` that is not uint8 [h, w, 3], before any library call."""
+        window = None if crop is None else _crop_window(crop, width, height, bands)
+        if window is not None and out is not None and out_device_ptr is None and (
+                out.dtype != np.uint8 or out.shape != (window[3], window[2], 3) or not out.flags.c_contiguous):
+            raise ValueError(f"out must be a C-contiguous uint8 array of shape ({window[3]}, {window[2]}, 3)")
         sc = scene.scene if isinstance(scene, ResidentScene) else scene
         rows = height if bands is None else band_row_count(height, *bands)
-        n_px = rows * width
+        cols = width
+        if window is not None:
+            cols, rows = window[2], window[3]
+        n_px = rows * cols
         keep = []
         o, dbg = self._opts(sc, width, height, rng_mode, seed, faceid, bands, exhaustive_strict, debug, n_px, keep,
                             (rays_per_thread, shadow_chunks, samples_per_pixel, int(bundle_cull), int(bool(bvh))))
+        if window is not None:
+            o.crop_x, o.crop_y, o.crop_w, o.crop_h = window
         if out_device_ptr is not None:
             out = None
             o.rgb_out_is_device = 1
             dst = C.c_void_p(out_device_ptr)
         else:
             if out is None:
-                out = np.zeros((rows, width, 3), np.uint8)
-            assert out.dtype == np.uint8 and out.size == rows * width * 3 and out.flags.c_contiguous
+                out = np.zeros((rows, cols, 3), np.uint8)
+            assert out.dtype == np.uint8 and out.size == rows * cols * 3 and out.flags.c_contiguous
             dst = out.ctypes.data_as(C.c_void_p)
         if stream is not None:
             o.cuda_stream = C.c_void_p(stream)

@@ -30,11 +30,14 @@ __host__ __device__ __forceinline__ uint32_t mix32(uint32_t x) {
     return x;
 }
 
+// W, H: the whole frame's size (image-plane (s, t) and image index h*W + w).  The call renders local rows of crop_w pixels,
+// columns crop_x .. crop_x + crop_w - 1, from PPM row crop_y on: (0, W, 0) without a crop window (a crop has one band).
 struct Bands {
     int W, H, band_rows, band_index, band_count, n_px;
     // extension (parity unpinned): spp_n x spp_n stratified jitter; sample = 0 .. spp_n^2-1
     int spp_n, sample;
     uint32_t seed;
+    int crop_x, crop_w, crop_y;
     // image-plane parameters of pixel (w,h): the reference's s = w/(W-1), t = h/(H-1) (main.cpp:709-710);
     // with jitter, w and h are displaced inside the pixel's stratum first.  Strict arithmetic: the
     // restatement (oracle/restated.c:pixel_st) computes the same bits.
@@ -53,15 +56,16 @@ struct Bands {
         s = __fdiv_rn(fw, (float)(W - 1));
         t = __fdiv_rn(fh, (float)(H - 1));
     }
+    // local pixel k -> the whole frame's (w, h)
     __host__ __device__ __forceinline__ void map(int k, int &w, int &h) const {
-        const int lr = k / W;
-        w = k - lr * W;
+        const int lr = k / crop_w;
+        w = crop_x + (k - lr * crop_w);
         int pr = lr;
         if (band_count > 1) {
             const int lb = lr / band_rows;
             pr = (band_index + lb * band_count) * band_rows + (lr - lb * band_rows);
         }
-        h = H - 1 - pr; // PPM row 0 is h = H-1 (main.cpp:662)
+        h = H - 1 - crop_y - pr; // PPM row 0 is h = H-1 (main.cpp:662)
     }
 };
 
@@ -415,7 +419,7 @@ __global__ void __launch_bounds__(sweep::NT, primary_minb(R)) primary_kernel(con
         const float4 *table = VIEWS ? p.table + vg * p.table_stride : p.table;
         const int tile_lo = (int)((long long)p.n_tiles * slice / p.n_slices);
         const int tile_hi = (int)((long long)p.n_tiles * (slice + 1) / p.n_slices);
-        const int W = p.bands.W;
+        const int W = p.bands.crop_w; // local rows: the crop window's width (the frame's without one)
         const int tile_y = blk / p.tiles_x, tile_x = blk - tile_y * p.tiles_x;
         const int txn = 1 << p.tx_log2;
         // first pixel (x, local row) of thread t's R rays
@@ -514,6 +518,23 @@ __global__ void __launch_bounds__(256) resolve_primary_kernel(Views views, Bands
             if (strict::intersect_sphere(o, d, __ldg(&spheres[s]), t)) tri = n_tris + s;
     }
     hit_tri[kpx] = tri, hit_t[kpx] = t, hit_v[kpx] = v;
+}
+
+// A crop window with seeded faceIDs: its pixels' hits and faceIDs (faceid[k*L + l], hit pixels only) from those of its
+// covering rows, the whole frame's PPM rows from 0 on at full width (pixel (w, h) at (H-1-h) * W + w)
+__global__ void __launch_bounds__(256) crop_gather_kernel(Bands crop, const int *__restrict__ c_tri, const float *__restrict__ c_t,
+                                                          const float *__restrict__ c_v, const int *__restrict__ c_fid, int L,
+                                                          int *__restrict__ hit_tri, float *__restrict__ hit_t,
+                                                          float *__restrict__ hit_v, int *__restrict__ faceid) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= crop.n_px) return;
+    int w, h;
+    crop.map(k, w, h);
+    const int c = (crop.H - 1 - h) * crop.W + w;
+    const int tri = c_tri[c];
+    hit_tri[k] = tri, hit_t[k] = c_t[c], hit_v[k] = c_v[c];
+    if (tri >= 0)
+        for (int l = 0; l < L; ++l) faceid[(size_t)k * L + l] = c_fid[(size_t)c * L + l];
 }
 
 struct LightStepParams {
@@ -1158,7 +1179,7 @@ struct PrimaryCullParams {
 template <int R>
 __device__ __forceinline__ void load_primary_bundle(const PrimaryCullParams &p, int blk, int warp, float (&rp)[R], float (&rq)[R],
                                                     float (&rl)[R], int (&kp)[R], unsigned &valid) {
-    const int lane = threadIdx.x & 31, W = p.bands.W;
+    const int lane = threadIdx.x & 31, W = p.bands.crop_w; // local row length
     const int ty = blk / p.tiles_x, tx = blk - ty * p.tiles_x;
     const int x = tx * 128 + (warp & 3) * 32 + lane, y0 = ty * 32 + (warp >> 2) * 8;
     valid = 0;

@@ -12,6 +12,9 @@
 // `--eye x,y,z` (repeatable) renders one view per eye, all looking at -l, in one tracer_cuda_render_views call on a resident
 // scene; with -o out.ppm they are written to out_0.ppm, out_1.ppm, ...  Each is the frame `-v x,y,z` gives with the same
 // --seed.  Not with -v, --gpus > 1 or --cull.
+// `--crop x,y,w,h` renders only that window of the -w frame (columns x .. x+w-1 of PPM rows y .. y+h-1, row 0 at the top) and
+// writes a w x h PPM: the same pixels as the whole frame's, in every --rng mode, with --cull and --bvh.  Not with --eye or
+// --gpus > 1.
 #include <array>
 #include <chrono>
 #include <cstdio>
@@ -37,7 +40,8 @@ int main(int argc, char *argv[]) {
         int device = 0, p6 = 0, bundle_cull = 0, gpus = 1, spp = 0;
         bool sorted = false;
         int accel = 0;
-        bool have_seed = false, have_v = false;
+        int crop[4] = {0, 0, 0, 0}; // x, y, w, h; all 0 = the whole frame
+        bool have_seed = false, have_v = false, have_crop = false;
         std::vector<std::array<float, 3>> eyes;
         unsigned seed = 0;
         int rng = TRACER_RNG_MT19937; // the serial path's generator
@@ -71,11 +75,18 @@ int main(int argc, char *argv[]) {
             else if (f == "--spp") spp = std::atoi(need("--spp"));
             else if (f == "--sorted") sorted = true;
             else if (f == "--bvh") sorted = true, accel = 1;
-            else throw std::runtime_error("Unknown argument: " + f); // main.cpp:531-534
+            else if (f == "--crop") {
+                if (std::sscanf(need("--crop"), "%d,%d,%d,%d", &crop[0], &crop[1], &crop[2], &crop[3]) != 4)
+                    throw std::runtime_error("expected --crop x,y,w,h");
+                if (crop[2] < 1 || crop[3] < 1) throw std::runtime_error("--crop needs a width and height >= 1");
+                have_crop = true;
+            } else throw std::runtime_error("Unknown argument: " + f); // main.cpp:531-534
         }
         if (!eyes.empty() && have_v) throw std::runtime_error("--eye and -v do not combine: give every view as --eye");
         if (!eyes.empty() && gpus > 1) throw std::runtime_error("--eye renders on one GPU: --gpus must be 1");
         if (!eyes.empty() && bundle_cull) throw std::runtime_error("--eye does not combine with --cull");
+        if (have_crop && !eyes.empty()) throw std::runtime_error("--crop does not combine with --eye");
+        if (have_crop && gpus > 1) throw std::runtime_error("--crop renders on one GPU: --gpus must be 1");
         tracer_scene_host *scene = nullptr;
         tracer_scene_flat empty{};
         const int32_t zero_off[1] = {0};
@@ -136,7 +147,9 @@ int main(int argc, char *argv[]) {
             tracer_cuda_shutdown();
             return 0;
         }
-        std::vector<uint8_t> rgb((size_t)W * H * 3);
+        o.crop_x = crop[0], o.crop_y = crop[1], o.crop_w = crop[2], o.crop_h = crop[3];
+        const int out_w = have_crop ? crop[2] : W, out_h = have_crop ? crop[3] : H;
+        std::vector<uint8_t> rgb((size_t)out_w * out_h * 3);
         const auto t0 = std::chrono::high_resolution_clock::now(); // main.cpp:583
         if (tracer_cuda_render(flat, &cam, W, H, &o, rgb.data())) throw std::runtime_error(tracer_cuda_last_error());
         const auto t1 = std::chrono::high_resolution_clock::now();
@@ -144,7 +157,7 @@ int main(int argc, char *argv[]) {
         std::cerr << "\n GPUs      : " << gpus << std::endl;
         std::cerr << "\n Duration  : " << std::chrono::duration_cast<std::chrono::milliseconds>(t1 - t0).count() << std::endl;
         if (!output.empty()) {
-            if (tracer_write_ppm(output.c_str(), rgb.data(), W, H, p6)) throw std::runtime_error(tracer_host_last_error());
+            if (tracer_write_ppm(output.c_str(), rgb.data(), out_w, out_h, p6)) throw std::runtime_error(tracer_host_last_error());
             std::cout << "Rendered image in: " << output << std::endl; // main.cpp:688
         } else {
             std::cout << "Nothing saved: use -o to save rendered image" << std::endl;

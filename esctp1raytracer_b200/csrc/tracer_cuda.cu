@@ -269,10 +269,16 @@ struct MtWork {
     uint32_t *words = nullptr, *lights = nullptr;
     int64_t *base = nullptr, *ord = nullptr;
     size_t rank_cap = 0, rows_cap = 0, maps_cap = 0, start_cap = 0, fid_cap = 0, words_cap = 0, lights_cap = 0, base_cap = 0, ord_cap = 0;
+    // a crop window's covering rows: the closest-hit pass's merged keys and hits, and the faceIDs replayed for them
+    unsigned long long *cov_best = nullptr;
+    int *cov_tri = nullptr, *cov_fid = nullptr;
+    float *cov_t = nullptr, *cov_v = nullptr;
+    size_t cov_cap = 0, cov_fid_cap = 0;
     void release() {
         dev_free(rank), dev_free(row_hits), dev_free(maps), dev_free(start), dev_free(fid_ord), dev_free(words), dev_free(lights);
         dev_free(base), dev_free(ord);
-        rank_cap = rows_cap = maps_cap = start_cap = fid_cap = words_cap = lights_cap = base_cap = ord_cap = 0;
+        dev_free(cov_best), dev_free(cov_tri), dev_free(cov_fid), dev_free(cov_t), dev_free(cov_v);
+        rank_cap = rows_cap = maps_cap = start_cap = fid_cap = words_cap = lights_cap = base_cap = ord_cap = cov_cap = cov_fid_cap = 0;
     }
 };
 
@@ -1096,6 +1102,8 @@ tracer_render_opts read_opts(const tracer_render_opts *in) {
     if (in) std::memcpy(&o, in, std::min<size_t>(sizeof o, in->struct_size ? in->struct_size : sizeof o));
     return o;
 }
+// any crop field set: the call renders a window of the frame (render_views checks it)
+bool has_crop(const tracer_render_opts &o) { return o.crop_x || o.crop_y || o.crop_w || o.crop_h; }
 
 // ---- one render call: n_views frames of one scene, one per camera (V = 1: tracer_cuda_render_scene) -------------------------
 // The call's pixels run view-major (k = view * W * n_rows + local); every per-pixel buffer, sort and list spans all of them,
@@ -1107,6 +1115,17 @@ enum Mode { BVH = 0, CULL = 1, SWEEPS = 2 };
 // Frame::render's outcome when the bundle-cull candidate buffer overflowed (not a status code: render_views renders again)
 constexpr int CAND_OVERFLOW = 1;
 
+// A closest-hit pass: its pixels (bands.n_px, in local rows of bands.crop_w), the local rows they span, and the planes it
+// leaves its merged keys and hits in
+struct HitPass {
+    trk::Bands bands;
+    trk::Views views;
+    int n_rows;
+    unsigned long long *best;
+    int *hit_tri;
+    float *hit_t, *hit_v;
+};
+
 // One attempt at the frames of one call: the scene, the checked options, what follows from them, and the counts it adds up
 struct Frame {
     tracer_scene_dev *s;
@@ -1114,8 +1133,11 @@ struct Frame {
     const tracer_render_opts &o;
     const tracer_camera *cams;
     cudaStream_t st;
-    int W, H, n_rows, view_px, n_px, n_views, L, S; // S: samples per pixel
+    int W, H, n_rows, view_px, n_px, n_views, L, S; // S: samples per pixel; n_rows, view_px: local rows of bands.crop_w pixels
     trk::Bands bands;
+    // a crop window with TRACER_RNG_MT19937: the closest-hit pass covers PPM rows [0, cover_rows) at full width, whose hits
+    // fix the crop's faceIDs (DESIGN §4f); 0 = the pass covers the call's own pixels
+    int cover_rows;
     trk::Views views{};
     std::vector<trk::Cam> h_cams;
     double diag = 0;    // reach bound of a primary ray's hit point; light k's shadow segments are bounded by (k+1) * diag
@@ -1135,10 +1157,12 @@ struct Frame {
     int render(uint8_t *rgb_out, std::vector<int> &frame_rows, bool &rows_known);
     int setup();
     int build_eye_tables(int v0, int v1);
+    size_t hit_px() const { return cover_rows ? (size_t)W * cover_rows : (size_t)n_px; }
+    HitPass hit_pass() const;
     int closest_hit();
-    int primary_sweeps();
-    int primary_cull();
-    int primary_bvh();
+    int primary_sweeps(const HitPass &hp);
+    int primary_cull(const HitPass &hp);
+    int primary_bvh(const HitPass &hp);
     int block_lists(cull::L0Params lp, int max_blocks, long long &n_keys);
     int faceids(std::vector<int> &frame_rows, bool &rows_known);
     int light(int k, uint32_t seed);
@@ -1220,8 +1244,14 @@ int Frame::setup() {
     CK_CUDA(cudaMemsetAsync(s->counters, 0, sizeof(sweep::Counters), st));
     CK_CUDA(cudaMemsetAsync(s->work, 0, sizeof(int), st));
 
+    if (cover_rows) { // the covering pass's planes
+        const size_t n = hit_px();
+        if (dev_grow(s->mt.cov_cap, n, s->mt.cov_best, s->mt.cov_tri, s->mt.cov_t, s->mt.cov_v) ||
+            dev_grow(s->mt.cov_fid_cap, n * std::max(1, L), s->mt.cov_fid))
+            return TRACER_ERR_NOMEM;
+    }
     if (mode == CULL) { // candidate buffers: 24 per ray + slack (a few per ray are typical), sorted with a radix sort
-        const size_t cap = (size_t)n_px * 24 * (size_t)s->cull_grow + ((size_t)1 << 22);
+        const size_t cap = hit_px() * 24 * (size_t)s->cull_grow + ((size_t)1 << 22);
         if (cap > s->cand_cap) {
             if (dev_grow(s->cand_cap, cap, s->cand_a, s->cand_b)) return TRACER_ERR_NOMEM;
             CK_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, s->sort_bytes, s->cand_a, s->cand_b, cap, 0, 64, st));
@@ -1279,33 +1309,44 @@ int Frame::build_eye_tables(int v0, int v1) {
 }
 
 // ---- primary: raygen + closest hit -> hit_tri, hit_t, hit_v -------------------------------------------------------------
+// The call's own pixels into the workspace, or a seeded crop's covering rows (the whole frame's first cover_rows PPM rows,
+// full width) into their own planes
+HitPass Frame::hit_pass() const {
+    if (!cover_rows) return {bands, views, n_rows, s->ws.best, s->ws.hit_tri, s->ws.hit_t, s->ws.hit_v};
+    trk::Bands b = bands;
+    b.crop_x = 0, b.crop_w = W, b.crop_y = 0, b.n_px = (int)hit_px();
+    return {b, trk::Views{s->cams, b.n_px}, cover_rows, s->mt.cov_best, s->mt.cov_tri, s->mt.cov_t, s->mt.cov_v};
+}
+
 int Frame::closest_hit() {
+    const HitPass hp = hit_pass();
+    const int n = hp.bands.n_px;
     CK_CUDA(cudaMemsetAsync(s->work, 0, sizeof(int), st));
-    CK_CUDA(cudaMemsetAsync(s->ws.best, 0xff, sizeof(unsigned long long) * (size_t)n_px, st));
+    CK_CUDA(cudaMemsetAsync(hp.best, 0xff, sizeof(unsigned long long) * (size_t)n, st));
     CK_CUDA(cudaEventRecord(s->ev[1], st));
-    if (int rc = mode == BVH ? primary_bvh() : mode == CULL ? primary_cull() : primary_sweeps()) return rc;
-    trk::resolve_primary_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(views, bands, s->ws.best, s->tri_verts, s->n_tris, s->spheres,
-                                                                    s->n_spheres, s->ws.hit_tri, s->ws.hit_t, s->ws.hit_v);
+    if (int rc = mode == BVH ? primary_bvh(hp) : mode == CULL ? primary_cull(hp) : primary_sweeps(hp)) return rc;
+    trk::resolve_primary_kernel<<<(n + 255) / 256, 256, 0, st>>>(hp.views, hp.bands, hp.best, s->tri_verts, s->n_tris, s->spheres,
+                                                                 s->n_spheres, hp.hit_tri, hp.hit_t, hp.hit_v);
     CK_CUDA(cudaGetLastError());
     ++launches;
     CK_CUDA(cudaEventRecord(s->ev[2], st));
     return 0;
 }
 
-int Frame::primary_bvh() {
-    bvh::primary_kernel<<<(n_px + 127) / 128, 128, 0, st>>>(views, bands, s->bvh_tree, bvh::frame_margin(bvh_ext, diag), s->tri_verts,
-                                                             s->ws.best, s->counters);
+int Frame::primary_bvh(const HitPass &hp) {
+    bvh::primary_kernel<<<(hp.bands.n_px + 127) / 128, 128, 0, st>>>(hp.views, hp.bands, s->bvh_tree, bvh::frame_margin(bvh_ext, diag),
+                                                                      s->tri_verts, hp.best, s->counters);
     CK_CUDA(cudaGetLastError());
     ++launches;
     return 0;
 }
 
 // OPTIONAL bundle-cull mode: screen tiles of 128 x 32 pixels -> candidates -> sort -> strict
-int Frame::primary_cull() {
+int Frame::primary_cull(const HitPass &hp) {
     trk::PrimaryCullParams p{};
     const int c_tiles = s->n_pad / cull::CTILE;
-    p.cam = h_cams[0], p.bands = bands, p.table = s->eye_table, p.n_tiles = c_tiles, p.n_tris = s->n_tris, p.n_rows = n_rows;
-    p.tiles_x = (W + 127) / 128, p.tiles_y = (n_rows + 31) / 32;
+    p.cam = h_cams[0], p.bands = hp.bands, p.table = s->eye_table, p.n_tiles = c_tiles, p.n_tris = s->n_tris, p.n_rows = hp.n_rows;
+    p.tiles_x = (hp.bands.crop_w + 127) / 128, p.tiles_y = (hp.n_rows + 31) / 32;
     const int blocks = p.tiles_x * p.tiles_y;
     p.n_slices = blocks >= 12 * g.n_sms ? 1 : std::max(1, std::min((12 * g.n_sms + blocks - 1) / blocks, std::max(1, c_tiles / 8)));
     p.em = cull::Emitter{s->cand_a, s->cand_count, em_cap};
@@ -1322,7 +1363,7 @@ int Frame::primary_cull() {
     if (n_keys >= 0) {
         trk::primary_cull2_kernel<<<2 * g.n_sms, sweep::THREADS, 0, st>>>(p, trk::BlockLists{s->boxes, s->cand_b, (unsigned long long)n_keys, tri_bits});
         CK_CUDA(cudaGetLastError());
-        host_tests_primary += (int64_t)n_px * s->n_tris;
+        host_tests_primary += (int64_t)hp.bands.n_px * s->n_tris;
     } else {
         CK_CUDA(cudaMemsetAsync(s->cand_count, 0, sizeof(unsigned long long), st));
         const size_t smem = sizeof(cull::EmitSmem);
@@ -1330,7 +1371,7 @@ int Frame::primary_cull() {
         trk::primary_cull_kernel<<<std::min(blocks * p.n_slices, 2 * g.n_sms), sweep::THREADS, smem, st>>>(p);
         CK_CUDA(cudaGetLastError());
     }
-    trk::strict_primary_pairs<<<8 * g.n_sms, 256, 0, st>>>(s->cand_a, s->cand_count, em_cap, h_cams[0], bands, s->tri_verts, s->ws.best,
+    trk::strict_primary_pairs<<<8 * g.n_sms, 256, 0, st>>>(s->cand_a, s->cand_count, em_cap, h_cams[0], hp.bands, s->tri_verts, hp.best,
                                                            s->counters);
     CK_CUDA(cudaGetLastError());
     launches += 2;
@@ -1338,8 +1379,8 @@ int Frame::primary_cull() {
 }
 
 // Default mode: one primary_kernel launch per group of views (all of them unless their eye tables did not fit at once)
-int Frame::primary_sweeps() {
-    const int n_tiles = s->n_pad / sweep::TILE;
+int Frame::primary_sweeps(const HitPass &hp) {
+    const int n_tiles = s->n_pad / sweep::TILE, row_w = hp.bands.crop_w;
     // no jitter: the rays of a thread share q exactly; jittered samples (extension): they share a mean q (span table)
     // unless the frame is so small that a jittered (s,t) can leave the span rows' |p|,|q| <= 1.0625 range
     const int qmode = bands.spp_n <= 1 ? sweep::MODE_SHAREDQ : (W >= 16 && H >= 16 ? sweep::MODE_QBAR : sweep::MODE_OWNQ);
@@ -1349,17 +1390,17 @@ int Frame::primary_sweeps() {
             if (int rc = build_eye_tables(v0, v0 + nv)) return rc;
             if (v0 > 0) CK_CUDA(cudaMemsetAsync(s->work, 0, sizeof(int), st));
         }
-        const Decomp d = pick_decomp((int64_t)nv * view_px, n_tiles, g.n_sms, o.rays_per_thread, qmode);
+        const Decomp d = pick_decomp((int64_t)nv * hp.views.view_px, n_tiles, g.n_sms, o.rays_per_thread, qmode);
         trk::PrimaryParams p{};
-        p.views = views, p.cam = h_cams[v0], p.bands = bands, p.n_tiles = n_tiles, p.n_tris = s->n_tris;
+        p.views = hp.views, p.cam = h_cams[v0], p.bands = hp.bands, p.n_tiles = n_tiles, p.n_tris = s->n_tris;
         p.table = qmode == sweep::MODE_OWNQ ? s->eye_table : s->eye_span;
         p.table_stride = (long long)(qmode == sweep::MODE_OWNQ ? s->table_stride : s->span_stride), p.view0 = v0;
         p.tri_verts = s->tri_verts;
-        p.best = s->ws.best, p.counters = s->counters, p.work = s->work;
-        p.n_rows = n_rows, p.view_blocks = 0; // ray blocks = screen tiles of (TX R) x (NT / TX) pixels: least edge waste wins
+        p.best = hp.best, p.counters = s->counters, p.work = s->work;
+        p.n_rows = hp.n_rows, p.view_blocks = 0; // ray blocks = screen tiles of (TX R) x (NT / TX) pixels: least edge waste wins
         for (int lg = d.R > 32 ? 2 : 3; lg <= 6; ++lg) { // (64 rays per thread: from 4 x 64 = 256 pixels wide)
             const int tw = (1 << lg) * d.R, th = sweep::NT >> lg;
-            const int tx = (W + tw - 1) / tw, nb = tx * ((n_rows + th - 1) / th);
+            const int tx = (row_w + tw - 1) / tw, nb = tx * ((hp.n_rows + th - 1) / th);
             if (!p.view_blocks || nb < p.view_blocks) p.view_blocks = nb, p.tiles_x = tx, p.tx_log2 = lg;
         }
         p.n_blocks = nv * p.view_blocks;
@@ -1427,25 +1468,35 @@ int Frame::faceids(std::vector<int> &frame_rows, bool &rows_known) {
         unsigned long long primary_overflow = 0;
         if (mode == CULL) CK_CUDA(cudaMemcpyAsync(&primary_overflow, &s->counters->cull_overflow, sizeof primary_overflow, cudaMemcpyDeviceToHost, st));
         // the row hits of every view in one pass (view-major rows), then each view replays its own std::mt19937(seed) draws,
-        // as a separate render of that view would
+        // as a separate render of that view would.  A crop window: those of its covering rows (full-width rows from PPM row 0,
+        // the prefix of a whole frame), then its own pixels' hits and faceIDs are gathered from them.
+        const HitPass hp = hit_pass();
+        const int rows = hp.n_rows, vpx = hp.views.view_px;
+        int *const fid = cover_rows ? s->mt.cov_fid : s->ws.faceid;
         std::vector<int> all_rows;
-        if (int rc = mt_count_rows(s->mt, s->ws.hit_tri, W, n_views * n_rows, st, all_rows)) return rc;
+        if (int rc = mt_count_rows(s->mt, hp.hit_tri, W, n_views * rows, st, all_rows)) return rc;
         ++launches;
         if (primary_overflow) return CAND_OVERFLOW;
         for (int v = 0; v < n_views; ++v) {
-            const std::vector<int> local(all_rows.begin() + (size_t)v * n_rows, all_rows.begin() + (size_t)(v + 1) * n_rows);
+            const std::vector<int> local(all_rows.begin() + (size_t)v * rows, all_rows.begin() + (size_t)(v + 1) * rows);
             if (rows_known) {
-                if (!mt::rows_valid(local.data(), n_rows, bands.band_rows, bands.band_index, bands.band_count, frame_rows.data(), H, W))
+                if (!mt::rows_valid(local.data(), rows, bands.band_rows, bands.band_index, bands.band_count, frame_rows.data(), H, W))
                     return fail(TRACER_ERR_STATE, "bundle-cull re-render: the closest-hit pass found other hits than the first pass");
             } else if (int rc = mt_frame_rows(o, W, H, bands.band_rows, bands.band_count, local, frame_rows)) {
                 return rc;
             }
-            const size_t off = (size_t)v * view_px;
-            if (int rc = mt_replay(s->mt, o.seed, s->h_light_F, frame_rows, W, bands.band_rows, bands.band_index, bands.band_count, n_rows,
-                                   s->ws.hit_tri + off, s->ws.faceid + off * L, st, launches, off))
+            const size_t off = (size_t)v * vpx;
+            if (int rc = mt_replay(s->mt, o.seed, s->h_light_F, frame_rows, W, bands.band_rows, bands.band_index, bands.band_count, rows,
+                                   hp.hit_tri + off, fid + off * L, st, launches, off))
                 return rc;
         }
         rows_known = true;
+        if (cover_rows) {
+            trk::crop_gather_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(bands, hp.hit_tri, hp.hit_t, hp.hit_v, fid, L, s->ws.hit_tri,
+                                                                        s->ws.hit_t, s->ws.hit_v, s->ws.faceid);
+            CK_CUDA(cudaGetLastError());
+            ++launches;
+        }
     }
     return 0;
 }
@@ -1701,7 +1752,7 @@ int Frame::finish_frame(uint8_t *rgb_out) {
     s->stats.ms_primary = ms_primary;
     s->stats.ms_shadow = ms_shadow;
     s->stats.ms_other = s->stats.ms_total - s->stats.ms_primary - ms_shadow;
-    s->stats.n_primary_rays = (int64_t)n_px * S;
+    s->stats.n_primary_rays = (int64_t)hit_px() * S;
     s->stats.n_shadow_rays = (int64_t)hc.n_hits * L;
     s->stats.tests_primary = (int64_t)hc.tests_primary + host_tests_primary;
     s->stats.tests_shadow = (int64_t)hc.tests_shadow + host_tests_shadow;
@@ -1739,10 +1790,22 @@ int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, in
     Ctx &g = *s->ctx;
     t_pool = &g.pool;
     if (W < 2 || H < 2) return fail(TRACER_ERR_INVALID, "width and height must be >= 2 (the reference divides by W-1, H-1)");
-    // per-pixel planes are indexed with int (3 planes of n_px floats): keep 3 * n_px below 2^31
-    if ((int64_t)n_views * W * H > (int64_t)700 * 1000 * 1000)
-        return fail(TRACER_ERR_INVALID, "frame too large (limit 7e8 pixels per call, over all views; render bands or fewer views)");
     tracer_render_opts o = read_opts(opts_in);
+    const bool crop = has_crop(o);
+    if (crop && (o.crop_w < 1 || o.crop_h < 1 || o.crop_x < 0 || o.crop_y < 0 || (int64_t)o.crop_x + o.crop_w > W ||
+                 (int64_t)o.crop_y + o.crop_h > H))
+        return fail(TRACER_ERR_INVALID, "crop window (" + std::to_string(o.crop_x) + ", " + std::to_string(o.crop_y) + ") " +
+                                            std::to_string(o.crop_w) + " x " + std::to_string(o.crop_h) + " is not inside the " +
+                                            std::to_string(W) + " x " + std::to_string(H) + " frame");
+    // per-pixel planes are indexed with int (3 planes of n_px floats): keep 3 * n_px below 2^31
+    constexpr int64_t PX_LIMIT = (int64_t)700 * 1000 * 1000;
+    if ((crop ? (int64_t)o.crop_w * o.crop_h : (int64_t)n_views * W * H) > PX_LIMIT)
+        return fail(TRACER_ERR_INVALID, "frame too large (limit 7e8 pixels per call, over all views; render bands or fewer views)");
+    if (crop && (int64_t)W * H >= ((int64_t)1 << 31)) // a crop pixel's image index h*W + w is an int
+        return fail(TRACER_ERR_INVALID, "a crop window needs a frame of fewer than 2^31 pixels");
+    if (crop && o.rng_mode == TRACER_RNG_MT19937 && (int64_t)W * (o.crop_y + o.crop_h) > PX_LIMIT)
+        return fail(TRACER_ERR_INVALID, "seeded crop window too low in the frame: its covering rows (every PPM row down to its last, "
+                                        "full width) exceed the limit of 7e8 pixels per call");
     // extension (parity unpinned): samples_per_pixel = n*n stratified jittered samples per pixel
     int spp_n = 1;
     if (o.samples_per_pixel > 1) {
@@ -1756,6 +1819,7 @@ int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, in
     const int band_rows = band_count > 1 ? o.band_rows : H;
     if (band_count > 1 && (band_rows <= 0 || o.band_index < 0 || o.band_index >= band_count))
         return fail(TRACER_ERR_INVALID, "bad band selection");
+    if (crop && band_count > 1) return fail(TRACER_ERR_INVALID, "a crop window does not combine with bands (band_count > 1)");
     if (o.rng_mode == TRACER_RNG_MT19937 && band_count > 1 && !o.row_hits_exchange)
         return fail(TRACER_ERR_INVALID, "TRACER_RNG_MT19937 with band_count > 1 needs opts->row_hits_exchange (the other bands' row hit counts)");
     if (o.rng_mode == TRACER_RNG_EXPLICIT && !o.faceid && s->n_lights > 0)
@@ -1765,20 +1829,23 @@ int render_views(tracer_scene_dev *s, const tracer_camera *cams, int n_views, in
     if (o.accel == 1 && (o.bundle_cull != 0 || o.exhaustive_strict != 0))
         return fail(TRACER_ERR_INVALID, "accel = 1 (BVH) does not combine with bundle_cull or exhaustive_strict (a debug mode of the sweeps' filter)");
     const int band_index = band_count > 1 ? o.band_index : 0;
-    const int n_rows = tracer_band_row_count(H, band_rows, band_index, band_count);
-    const int view_px = n_rows * W, n_px = n_views * view_px;
+    const int n_rows = crop ? o.crop_h : tracer_band_row_count(H, band_rows, band_index, band_count);
+    const int row_w = crop ? o.crop_w : W;
+    const int view_px = n_rows * row_w, n_px = n_views * view_px;
     trk::Bands bands{W, H, band_rows, band_index, band_count, n_px};
     bands.spp_n = spp_n, bands.sample = 0, bands.seed = o.seed;
+    bands.crop_x = crop ? o.crop_x : 0, bands.crop_w = row_w, bands.crop_y = crop ? o.crop_y : 0;
+    const int cover_rows = crop && o.rng_mode == TRACER_RNG_MT19937 ? o.crop_y + o.crop_h : 0;
     const cudaStream_t st = o.cuda_stream ? (cudaStream_t)o.cuda_stream : g.stream;
     std::vector<int> frame_rows;
     bool rows_known = false;
     for (;;) {
-        Frame f{s, g, o, cams, st, W, H, n_rows, view_px, n_px, n_views, s->n_lights, spp_n * spp_n, bands};
+        Frame f{s, g, o, cams, st, W, H, n_rows, view_px, n_px, n_views, s->n_lights, spp_n * spp_n, bands, cover_rows};
         const int rc = f.render(rgb_out, frame_rows, rows_known);
         if (rc != CAND_OVERFLOW) return rc;
         size_t free_b = 0, total_b = 0;
         cudaMemGetInfo(&free_b, &total_b);
-        const size_t next_bytes = ((size_t)n_px * 24 * (size_t)s->cull_grow * 4 + ((size_t)1 << 22)) * sizeof(unsigned long long) * 3;
+        const size_t next_bytes = (f.hit_px() * 24 * (size_t)s->cull_grow * 4 + ((size_t)1 << 22)) * sizeof(unsigned long long) * 3;
         if (!std::getenv("TRACER_CAND_CAP") && s->cull_grow < 64 && next_bytes < free_b / 2 + s->cand_cap * 24)
             s->cull_grow *= 4;
         else
@@ -1801,6 +1868,7 @@ int tracer_cuda_render_views(tracer_scene_dev *s, const tracer_camera *cams, int
     const tracer_render_opts o = read_opts(opts_in);
     if (o.band_count > 1) return fail(TRACER_ERR_INVALID, "tracer_cuda_render_views renders whole views: band_count must be <= 1");
     if (o.bundle_cull != 0) return fail(TRACER_ERR_INVALID, "tracer_cuda_render_views does not combine with bundle_cull");
+    if (has_crop(o)) return fail(TRACER_ERR_INVALID, "tracer_cuda_render_views renders whole views: no crop window");
     return render_views(s, cams, n_views, W, H, opts_in, rgb_out);
 }
 }  // extern "C"
@@ -2174,12 +2242,13 @@ int tracer_cuda_render_scene_multi(tracer_scene_multi *ms, const tracer_camera *
     if (!ms || !cam || !rgb_out) return fail(TRACER_ERR_INVALID, "null argument");
     const int n = (int)ms->dev.size();
     if (n != g_multi.n || n < 1) return fail(TRACER_ERR_STATE, "scene was created for a different GPU set");
+    const tracer_render_opts o = read_opts(opts_in);
+    if (has_crop(o)) return fail(TRACER_ERR_INVALID, "the multi-GPU call renders whole frames: use tracer_cuda_render_scene for a crop window");
     if (n == 1) {
         const int rc = tracer_cuda_render_scene(ms->dev[0], cam, W, H, opts_in, rgb_out);
         ms->stats = ms->dev[0]->stats;
         return rc;
     }
-    const tracer_render_opts o = read_opts(opts_in);
     if (o.band_count > 1) return fail(TRACER_ERR_INVALID, "the multi-GPU call partitions the frame itself: leave band_count at 0");
     if (o.out_tri || o.out_t || o.out_v || o.out_occ_tri || o.out_rgb) return fail(TRACER_ERR_INVALID, "debug outputs are per-GPU: use tracer_cuda_render_scene with bands");
     if (W < 2 || H < 2 || (int64_t)W * H > (int64_t)2000 * 1000 * 1000) return fail(TRACER_ERR_INVALID, "bad frame size");
@@ -2293,6 +2362,8 @@ int tracer_cuda_scene_update_multi(tracer_scene_multi *ms, const tracer_scene_up
 
 int tracer_cuda_render_multi(const tracer_scene_flat *scene, const tracer_camera *cam, int32_t width, int32_t height,
                              const tracer_render_opts *opts, uint8_t *rgb_out) {
+    if (has_crop(read_opts(opts)))
+        return fail(TRACER_ERR_INVALID, "the multi-GPU call renders whole frames: use tracer_cuda_render_scene for a crop window");
     tracer_scene_multi *ms = nullptr;
     if (int rc = tracer_cuda_scene_create_multi(scene, &ms)) return rc;
     const int rc = tracer_cuda_render_scene_multi(ms, cam, width, height, opts, rgb_out);

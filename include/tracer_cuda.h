@@ -101,7 +101,8 @@ typedef struct tracer_render_opts {
     /* Row-band partition for multi-GPU (1 process per GPU).  The frame's PPM
      * rows (row 0 = h=H-1, main.cpp:662) are cut into bands of band_rows
      * rows; this call renders the bands b with b % band_count == band_index,
-     * packed back to back in the output.  band_count<=1 renders everything. */
+     * packed back to back in the output.  band_count<=1 renders everything (or, with crop_x .. crop_h at the end
+     * of this struct, one rectangular window of the frame). */
     int32_t band_rows;
     int32_t band_index;
     int32_t band_count;
@@ -147,6 +148,19 @@ typedef struct tracer_render_opts {
      * Appended last: callers with an older struct_size get NULL. */
     int32_t (*row_hits_exchange)(void *user, int32_t height, int32_t *row_hits);
     void *row_hits_user;
+
+    /* Crop window: render only columns [crop_x, crop_x + crop_w) of PPM rows [crop_y, crop_y + crop_h) (PPM row 0 =
+     * h = H-1, as for bands).  The frame is still width x height: the camera, the image-plane (s, t), the faceID hash,
+     * the jitter and the explicit faceid array (still [W*H*n_lights]) are those of the whole frame.  rgb_out holds
+     * crop_h rows of crop_w pixels in PPM order, and the debug outputs are indexed k = local_row * crop_w + column.
+     * Contract: every byte and debug value equals the same pixel of the whole frame rendered with the same options, in
+     * every mode, rng_mode and sample count and with exhaustive_strict.  With TRACER_RNG_MT19937 a pixel's draws depend
+     * on the hits of every pixel before it in scan order, so the call first runs the closest-hit pass over the covering
+     * rows [0, crop_y + crop_h) at full width; tests_primary, strict_evals and n_primary_rays count that pass, n_pixels
+     * counts the crop.  All four 0 = the whole frame.  Refused with TRACER_ERR_INVALID: a window not inside the frame,
+     * crop_w < 1 or crop_h < 1 while any field is set, band_count > 1, tracer_cuda_render_views and the multi-GPU calls.
+     * Appended last: callers with an older struct_size get 0. */
+    int32_t crop_x, crop_y, crop_w, crop_h;
 } tracer_render_opts;
 
 typedef struct tracer_frame_stats {
@@ -154,8 +168,8 @@ typedef struct tracer_frame_stats {
     double ms_primary;      /* closest-hit sweep                                       */
     double ms_shadow;       /* any-hit sweeps, all lights                              */
     double ms_other;        /* table build, ray set-up, shading, quantise              */
-    int64_t n_pixels;       /* pixels rendered by this call                            */
-    int64_t n_primary_rays;
+    int64_t n_pixels;       /* pixels rendered by this call (a crop's)                 */
+    int64_t n_primary_rays; /* (a seeded crop: those of its covering rows)             */
     int64_t n_shadow_rays;
     int64_t tests_primary;  /* ray-triangle pairs swept (filter evaluations), primary  */
     int64_t tests_shadow;   /* same, shadow sweeps                                     */
@@ -199,7 +213,7 @@ const char *tracer_cuda_last_error(void);
 int tracer_cuda_device_info(tracer_device_info *out);
 
 /* ---- the drop-in call: host buffers in, packed 8-bit RGB out --------------
- * rgb_out: caller-owned, n_rows_of_this_call * W * 3 bytes, PPM row order,
+ * rgb_out: caller-owned, n_rows_of_this_call * W * 3 bytes (a crop: crop_h * crop_w * 3), PPM row order,
  * fully overwritten (unlike ispc::trace, which += into an un-zeroed malloc,
  * trace.ispc:262-265 / main.cpp:593).  Uploads the scene, renders, downloads. */
 int tracer_cuda_render(const tracer_scene_flat *scene, const tracer_camera *cam, int32_t width, int32_t height,
@@ -219,7 +233,7 @@ int tracer_cuda_last_stats(tracer_scene_dev *scene, tracer_frame_stats *out);
  * first occluders and the float accumulator, in every rng_mode (TRACER_RNG_MT19937: each view draws from its own
  * std::mt19937(seed), as a separate run of the serial path would), with jittered samples, in the default and the BVH
  * mode, with exhaustive_strict.  Refused with TRACER_ERR_INVALID: n_views < 1, cams NULL, band_count > 1, bundle_cull != 0,
- * n_views * width * height above the per-call pixel limit.  Stats (tracer_cuda_last_stats) are totals over the call.
+ * a crop window, n_views * width * height above the per-call pixel limit.  Stats (tracer_cuda_last_stats) are totals over the call.
  * The views share the camera-independent work of a frame: the shadow rays of every view go through one sweep per light
  * vertex batch; only the closest-hit sweep runs per view (one eye table each). */
 int tracer_cuda_render_views(tracer_scene_dev *scene, const tracer_camera *cams, int32_t n_views, int32_t width,
