@@ -725,6 +725,31 @@ __global__ void list_prefix_kernel(const int *seg_count, int F, int *seg_off, in
     }
 }
 
+// Default mode: entries per stripe of the shadow-ray order (order_shadow_rays).  Measured at C4 (profiles/r11_b): 128 gives
+// the fastest shadow sweeps.  Longer stripes make a thread's cell narrower in p but taller in q, and past ~200 entries the
+// |B| * qdelta widening of the mean-q bounds costs more queued pairs than the narrower cell saves.
+constexpr int SHADOW_STRIPE = 128;
+
+// Default mode, after the (group, q) sort: the key that reorders every stripe of L consecutive entries of a group by p,
+// ascending in even stripes and descending in odd ones (serpentine), so that consecutive entries stay close in (p, q)
+// across stripe boundaries too.  key = stripe's first list position << 32 | p's order bits (inverted in odd stripes);
+// pixels without a shadow ray (all-ones key, last) keep it.  The list stays a permutation of each group's rays.
+__global__ void stripe_key_kernel(const unsigned long long *__restrict__ key_sorted, const int *__restrict__ list, const float *__restrict__ re,
+                                  const int *__restrict__ seg_off, int n_px, int L, unsigned long long *__restrict__ key_out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_px) return;
+    const unsigned j = (unsigned)(key_sorted[i] >> 32);
+    if (j == 0xffffffffu) {
+        key_out[i] = ~0ull;
+        return;
+    }
+    const int s = (i - seg_off[j]) / L;
+    const unsigned pb = __float_as_uint(re[list[i]]);
+    unsigned pk = (pb & 0x80000000u) ? ~pb : (pb | 0x80000000u);
+    if (s & 1) pk = ~pk;
+    key_out[i] = (unsigned long long)(unsigned)(seg_off[j] + s * L) << 32 | pk;
+}
+
 // before each triangle chunk: live-ray counts per ray group -> ray-block offsets; reset the
 // survivors' counters and the work counter
 // The triangle-slice count of the chunk is chosen here, on the device, from the live block count (so the
@@ -764,7 +789,7 @@ __global__ void iota_kernel(int *a, int n) {
 // the loop at all: block offsets, slice counts, the chunk scheme and the early stop ("every ray has its occluder")
 // are decided on the device.  Round 1 ran A/B/C as 4 launches per chunk with host read-backs in between.
 constexpr int SHADOW_R = 32;    // rays per thread of a full shadow-ray block (blocks of NT * SHADOW_R consecutive list entries).
-                                // Each thread pays 12 set-up instructions per triangle (mean q), amortised over R rays; with
+                                // Each thread pays 12 set-up instructions and one FADD2 per triangle (mean q, segment verdict); with
                                 // the candidate pairs drained warp-wide (sweep.cuh) a thread's strict evaluations no longer
                                 // serialise over its rays, which is what made 32 slower than 16 in the per-thread form.
                                 // 64 measured slower (C4: 238 against 199 ms of shadow sweep, 2 CTAs per SM).
@@ -820,14 +845,16 @@ __device__ __noinline__ bool strict_shadow(const PixelState &px, const float *__
     return true;
 }
 
-// one (ray block, triangle slice) work item with RR rays per thread.  The list is ordered by q inside each group
-// (and compaction keeps it so); a thread takes RR CONSECUTIVE rays, whose q differ by ~1e-6, and evaluates them
-// with one q-term per edge row (sweep::MODE_QBAR).  Only 2*S*p stays in registers: the candidate path reads a
-// queued ray's own (p, q) back through the list.
+// one (ray block, triangle slice) work item with RR rays per thread.  The list is ordered by q inside each group, then by
+// p in serpentine stripes of SHADOW_STRIPE entries (and compaction keeps that order); a thread takes RR CONSECUTIVE rays,
+// evaluates them with one q-term per edge row (sweep::MODE_QBAR) and decides each triangle from its least and greatest p
+// (the mean-q segment verdict, sweep.cuh).  Only 2*S*p stays in registers: the candidate path reads a queued ray's own
+// (p, q) back through the list.
 template <int RR, bool EXHAUSTIVE>
 __device__ __forceinline__ void shadow_item(sweep::SmemT<2> &sm, const ShadowLightParams &p, const int *__restrict__ list_in, int base,
                                             int seg_end, int lo, int hi, const float4 *__restrict__ tab, unsigned &gtile,
-                                            unsigned &n_strict, unsigned &n_miss, unsigned long long &tests, unsigned &n_pipe_err) {
+                                            unsigned &n_strict, unsigned &n_miss, unsigned long long &tests, unsigned &n_pipe_err,
+                                            unsigned long long &n_flag, unsigned long long &n_queue) {
     using Mask = sweep::RayMask<RR>;
     const int tid = threadIdx.x, n = p.n_px;
     float rp[RR], rq[RR];
@@ -849,7 +876,7 @@ __device__ __forceinline__ void shadow_item(sweep::SmemT<2> &sm, const ShadowLig
     const float qbar = 0.5f * (qmin + qmax);
     // >= max |q_r - qbar| with room for the roundings of this line and of the one extra FFMA per row
     const float qdelta = fmaxf(qmax - qbar, qbar - qmin) * 1.0001f + 2.4e-7f * (fabsf(qbar) + 1.f);
-    unsigned swept = 0;
+    unsigned swept = 0, flagged = 0, queued = 0;
     sweep::sweep_table<RR, sweep::MODE_QBAR, true, EXHAUSTIVE>(
         sm, tab, lo, hi, p.n_tris, rp, rq, qbar, qdelta, valid, done, gtile, swept,
         [&](int otid, int r, int tri, bool filt, const float4 *row) {
@@ -863,8 +890,9 @@ __device__ __forceinline__ void shadow_item(sweep::SmemT<2> &sm, const ShadowLig
             n_miss += acc && !filt;
             return acc;
         },
-        &n_pipe_err);
+        &n_pipe_err, &flagged, &queued);
     tests += (unsigned long long)swept * sweep::TILE * __popcll((unsigned long long)valid);
+    n_flag += flagged, n_queue += queued;
 }
 
 // exclusive prefix over the F groups of ceil(cnt[j] / unit), by the whole CTA into shared memory; returns the total
@@ -939,7 +967,7 @@ __global__ void __launch_bounds__(sweep::NT, SHADOW_MINB) shadow_light_kernel(co
     const int tid = threadIdx.x, F = p.F;
     sweep::smem_init(sm);
     unsigned gtile = 0, n_strict = 0, n_miss = 0, epoch = 0, n_pipe_err = 0;
-    unsigned long long tests = 0;
+    unsigned long long tests = 0, n_flag = 0, n_queue = 0;
     long long c_items = 0, c_bar = 0, c_comp = 0, n_it = 0, n_run = 0; // time split (thread 0)
     const long long c_begin = clock64();
     // chunk scheme: equal chunks keep the pairs swept past a ray's occluder lowest and win when the light has many
@@ -1000,15 +1028,15 @@ __global__ void __launch_bounds__(sweep::NT, SHADOW_MINB) shadow_light_kernel(co
                 const int cnt = seg_end - base;
                 static_assert(SHADOW_R == 32, "the part-filled block sizes below follow SHADOW_R");
                 if (cnt > 16 * sweep::NT)
-                    shadow_item<SHADOW_R, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err);
+                    shadow_item<SHADOW_R, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue);
                 else if (cnt > 8 * sweep::NT)
-                    shadow_item<16, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err);
+                    shadow_item<16, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue);
                 else if (cnt > 4 * sweep::NT)
-                    shadow_item<8, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err);
+                    shadow_item<8, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue);
                 else if (cnt > 2 * sweep::NT)
-                    shadow_item<4, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err);
+                    shadow_item<4, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue);
                 else
-                    shadow_item<2, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err);
+                    shadow_item<2, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue);
                 __syncthreads(); // every warp is out of the tile pipeline before the next run re-arms it
             }
             c_items += clock64() - c_run;
@@ -1129,6 +1157,7 @@ __global__ void __launch_bounds__(sweep::NT, SHADOW_MINB) shadow_light_kernel(co
     }
     atomicAdd(&p.counters->tests_shadow, tests);
     atomicAdd(&p.counters->strict_evals, (unsigned long long)n_strict);
+    atomicAdd(&p.counters->n_flagged, n_flag), atomicAdd(&p.counters->n_queued, n_queue);
     if (EXHAUSTIVE) atomicAdd(&p.counters->filter_misses, (unsigned long long)n_miss);
     if (EXHAUSTIVE && n_pipe_err) atomicAdd(&p.counters->pipeline_errors, (unsigned long long)n_pipe_err);
     if (tid == 0) {

@@ -4,8 +4,8 @@
 // What the reference does per (ray, triangle) pair: full Moller-Trumbore with
 // a double-precision divide (ray_triangle.h:7-57, ~52 flop).  What this kernel
 // does per pair: half a packed add and half a three-input min (4., hot rows), plus
-// 8 ops per thread and triangle (12 with a mean q); the closest-hit sweep does nothing per pair, one packed add per
-// thread and triangle on the thread's extreme rays (segment_pass).  The saving comes from these observations.
+// 8 ops per thread and triangle (12 with a mean q); the closest-hit and shadow sweeps do nothing per pair, one packed add
+// per thread and triangle on the thread's extreme rays (segment_pass).  The saving comes from these observations.
 //
 //  1. Every sweep is a bundle of rays through ONE common point.  Primary rays
 //     all start at the eye (camera.h:31-34).  A shadow ray runs from the hit
@@ -42,8 +42,8 @@
 //
 //  3. The R rays of a thread share q.  Closest-hit ray blocks are screen tiles in which a
 //     thread holds R consecutive pixels of one image row: same q exactly (MODE_SHAREDQ).
-//     Shadow-ray lists are sorted by q, a thread takes R consecutive rays and evaluates the
-//     q-dependent terms at qbar with |B|*qdelta added, qdelta >= max|q_r - qbar|, which is
+//     Shadow-ray lists are sorted by q, then by p in short serpentine stripes; a thread takes R consecutive
+//     rays and evaluates the q-dependent terms at qbar with |B|*qdelta added, qdelta >= max|q_r - qbar|, which is
 //     >= every ray's own term, so the test stays a necessary condition (MODE_QBAR; also used
 //     for jittered primary samples, whose q lie inside one stratum).
 //
@@ -63,8 +63,9 @@
 //  * every lane of every warp reads the SAME row at the same time, so the two LDS.128 per
 //    triangle are pure broadcasts, amortised over R rays per thread held in registers
 //    (R = 64 closest hit, 32 any-hit);
-//  * closest hit (MODE_SHAREDQ): one two-sided test on the thread's least and greatest 2*S*p per triangle (segment_pass);
-//  * any-hit: each pair is ONE interval test |2*S*p + nc2| <= h2 (hot rows, below): per two pairs one packed
+//  * closest hit (MODE_SHAREDQ) and any-hit (MODE_QBAR): one two-sided test on the thread's least and greatest 2*S*p per
+//    triangle (segment_pass);
+//  * jittered primary samples: each pair is ONE interval test |2*S*p + nc2| <= h2 (hot rows, below): per two pairs one packed
 //    FADD2 and one FMNMX3 running minimum, no saturation, no integer op.  History on this part
 //    (cycles per pair, closest hit): round 1 sign bits through LOP3 on the half-rate ALU pipe 7.9,
 //    three saturating rows with a product accumulate 6.8, span form with two saturating adds 4.0;
@@ -175,6 +176,8 @@ struct Counters {
     // shadow_light_kernel time split, SM cycles summed over CTAs (thread 0's clock; TRACER_SHADOW_DIAG prints them):
     // inside work items, waiting at grid barriers, compaction passes, everything else (work-queue pops, prefix sums)
     unsigned long long cyc_items, cyc_barrier, cyc_compact, cyc_total, n_items, n_runs;
+    // shadow_light_kernel: (thread, triangle) verdicts the hot loop flagged, and (ray, triangle) pairs queued for the drain
+    unsigned long long n_flagged, n_queued;
 };
 
 template <int ROWS>
@@ -405,7 +408,20 @@ __device__ __forceinline__ float fmin3_abs(float m, float a, float b) {
 // margin, no new rounding.  It costs one FADD2 and the compares per thread and triangle in place of R/2 FADD2 + R/2
 // FMNMX3.  It is looser only where a triangle's interval falls between two neighbouring rays of the thread (narrower than
 // a pixel); the candidate path rebuilds the per-ray mask with hot_pass, so the pairs handed to the strict test are the same.
-// A NaN sum counts as a pass.  Not for the shadow sweeps: their rays are sorted by q and scattered in p.
+// A NaN sum counts as a pass.
+//
+// MEAN-q SEGMENT verdict (shadow sweeps, MODE_QBAR with ANYHIT: the same segment_pass after hot_terms_qbar).  The R rays of
+// a shadow thread do not share q, but the per-ray loop already gives them one (nc2, h2): hot_terms_qbar at the thread's qbar
+// with the bounds widened by |B| * qdh, qdh = hot_qdelta(qdelta), qdelta >= max |q_r - qbar| over all R values (shadow_item's
+// formula: the spread times 1.0001 plus 2.4e-7 (|qbar| + 1) covers the roundings of qbar and of the spread for any spread).
+// The hot-row proof above already takes any qdelta: its qdelta step bounds G' - G with |z| <= (1 + 2u)(|G| + |Bl| qd) and the
+// HOT_QD_SCALE term, neither of which assumes qd small, and a large qd only moves A_i, B_i towards the clamp C.  So every pair
+// the exact row passes, at the ray's own q, passes |fl(ps2_r + nc2)| <= h2 with these shared (nc2, h2), and the monotonicity
+// argument above then carries over word for word: pmin2 <= ps2_r <= pmax2 over the thread's R values gives
+// fl(pmin2 + nc2) <= h2 and fl(pmax2 + nc2) >= -h2 for any passing ray.  No new margin, no new rounding.  The R values include
+// the duplicated tail entries of a short list and rays already done: both only widen [pmin2, pmax2], so only loosen it.
+// It pays once a thread's rays form a compact cell in (p, q): the default mode's shadow lists are sorted by q, then by p in
+// serpentine stripes (order_shadow_rays), so qdelta is ~1e-3 instead of ~1e-6 and [pmin2, pmax2] a few triangle widths.
 constexpr float HOT_CLAMP = SPAN_BOX;
 constexpr float HOT_DELTA = 8.f * 1.1920928955078125e-7f * HOT_CLAMP;
 constexpr float HOT_QD_SCALE = 1.f + 0x1p-20f;
@@ -483,14 +499,17 @@ __device__ __forceinline__ unsigned eval_interval(const float4 *__restrict__ tp,
     }
     return cand;
 }
-// The same verdict bits from the thread's extreme rays (segment_pass; closest-hit sweep, MODE_SHAREDQ only): per triangle
-// the set-up of hot_terms, one FADD2 and the compares, whatever R.  Bit k set = triangle k may hold a candidate.
-__device__ __forceinline__ unsigned eval_segment(const float4 *__restrict__ tp, float pmin2, float pmax2, float q) {
+// The same verdict bits from the thread's extreme rays (segment_pass; closest-hit sweep with MODE_SHAREDQ, shadow sweeps with
+// MODE_QBAR): per triangle the set-up of hot_terms (hot_terms_qbar), one FADD2 and the compares, whatever R.  Bit k set =
+// triangle k may hold a candidate.
+template <int MODE>
+__device__ __forceinline__ unsigned eval_segment(const float4 *__restrict__ tp, float pmin2, float pmax2, float q, float qdh) {
     unsigned cand = 0;
 #pragma unroll
     for (int k = 0; k < SPAN_BATCH; ++k) {
         float nc2, h2;
-        hot_terms(tp[2 * k], tp[2 * k + 1], q, nc2, h2);
+        if (MODE == MODE_QBAR) hot_terms_qbar(tp[2 * k], tp[2 * k + 1], q, qdh, nc2, h2);
+        else hot_terms(tp[2 * k], tp[2 * k + 1], q, nc2, h2);
         cand |= (unsigned)segment_pass(nc2, h2, pmin2, pmax2) << k;
     }
     return cand;
@@ -531,11 +550,13 @@ __device__ __forceinline__ unsigned eval_batch_lop3(const float4 *__restrict__ t
 // strict(otid, r, tri, filt, row) -> accepted: the reference's own test of ray r of thread otid (a thread of the calling
 //        lane's warp) against triangle tri (kernels.cuh), run by whichever lane drains the pair; filt = the filter passed
 //        the pair (false only in EXHAUSTIVE validation mode), row = the triangle's staged row (still resident)
+// n_flag, n_queue (may be null; not counted in EXHAUSTIVE mode): add this thread's flagged (thread, triangle) verdicts and the
+//        pairs it queued
 template <int R, int MODE, bool ANYHIT, bool EXHAUSTIVE, class Strict>
 __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const float4 *__restrict__ table, int tile_lo, int tile_hi, int n_tris,
                                             const float (&rp)[R], const float (&rq)[R], float qbar, float qdelta, RayMask<R> valid,
                                             RayMask<R> &done, unsigned &gtile, unsigned &n_tiles_swept, Strict &&strict,
-                                            unsigned *n_pipe_err = nullptr) {
+                                            unsigned *n_pipe_err = nullptr, unsigned *n_flag = nullptr, unsigned *n_queue = nullptr) {
     using Mask = RayMask<R>;
     static_assert(R <= 32 || MODE != MODE_OWNQ, "the three-row form's rays fit one 32-bit mask");
     constexpr int ROWS = Rows<MODE>::N;
@@ -556,8 +577,9 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
 #pragma unroll
     for (int r = 0; r < R; ++r) ps2[r] = rp[r] * (2.f * SPAN_S);
     const float qhot = MODE == MODE_QBAR ? qbar : rq[0], qdh = hot_qdelta(qdelta);
-    // closest hit with a shared q: the hot loop decides each triangle from the extreme rays (segment_pass)
-    constexpr bool SEGMENT = !ANYHIT && MODE == MODE_SHAREDQ;
+    // closest hit with a shared q, and the shadow sweeps (mean q): the hot loop decides each triangle from the extreme rays
+    // (segment_pass); jittered primary samples (MODE_QBAR, closest hit) keep the per-ray loop
+    constexpr bool SEGMENT = (!ANYHIT && MODE == MODE_SHAREDQ) || (ANYHIT && MODE == MODE_QBAR);
     float pmin2 = ps2[0], pmax2 = ps2[0];
     if (SEGMENT) {
 #pragma unroll
@@ -613,7 +635,7 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
 #pragma unroll 1
             for (int b0 = 0; b0 < TILE; b0 += NB) {
                 unsigned cand;
-                if constexpr (SEGMENT) cand = eval_segment(tp + ROWS * b0, pmin2, pmax2, qhot);
+                if constexpr (SEGMENT) cand = eval_segment<MODE>(tp + ROWS * b0, pmin2, pmax2, qhot, qdh);
                 else if constexpr (SPAN) cand = eval_interval<R, MODE>(tp + ROWS * b0, ps2, qhot, qdh);
                 else cand = eval_batch<R, MODE>(tp + ROWS * b0, rp, rq, qbar, qdelta);
 #ifdef SWEEP_NO_STRICT // development microbenchmark only (tools/sweep_mb2.cu): timing without the strict path
@@ -622,6 +644,7 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
                 // validation mode: every triangle goes to the strict path; the hot loop's own verdict is kept so that an
                 // accepted pair whose triangle (group) it would have skipped counts as a filter miss too
                 const unsigned cand_hot = cand;
+                if (!EXHAUSTIVE && n_flag) *n_flag += __popc(cand);
                 if (EXHAUSTIVE) cand = NB / UNIT == 32 ? 0xffffffffu : (1u << (NB / UNIT)) - 1u;
                 // rare: some lane flagged a triangle (group of UNIT triangles).  The warp rebuilds, lane by lane, the per-ray
                 // candidate mask of each flagged triangle, queues the (owner lane, ray, triangle) pairs and drains the queue one
@@ -659,6 +682,7 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
                             }
                             const Mask live = valid & ~done;
                             Mask pend = mine ? (EXHAUSTIVE ? live : filt & live) : (Mask)0;
+                            if (!EXHAUSTIVE && n_queue) *n_queue += __popcll((unsigned long long)pend);
                             while (__any_sync(0xffffffffu, pend != 0)) {
                                 // this lane's pairs go to queue slots [fill + before, ...): as many as fit, the rest after a drain
                                 const int n = __popcll((unsigned long long)pend);

@@ -130,6 +130,29 @@ extern "C" void tracer__segment_pass(const float *row8, int n, const float *p, f
     out2[0] = sweep::segment_pass(nc2, h2, pmin2, pmax2), out2[1] = any;
     if (terms2) terms2[0] = nc2, terms2[1] = h2;
 }
+// The same for n rays (p, q) of one shadow-sweep thread (mean-q form): (nc2, h2) from hot_terms_qbar at qbar with the bounds
+// widened by hot_qdelta(qdelta), as shadow_item and sweep_table form them.  out3[0] = the segment verdict, out3[1] = the OR of
+// the per-ray hot tests at qbar (the per-ray loop it replaces), out3[2] = the OR of the hot tests with each ray's own q (the
+// drain's test).  terms2 (may be null) receives (nc2, h2).
+extern "C" void tracer__segment_pass_qbar(const float *row8, int n, const float *p, const float *q, float qbar, float qdelta,
+                                          unsigned char *out3, float *terms2) {
+    float4 lo = make_float4(row8[0], row8[1], row8[2], row8[3]), hi = make_float4(row8[4], row8[5], row8[6], row8[7]);
+    sweep::hot_row(lo, hi);
+    float nc2, h2;
+    sweep::hot_terms_qbar(lo, hi, qbar, sweep::hot_qdelta(qdelta), nc2, h2);
+    bool any = false, own = false;
+    float pmin2 = p[0] * (2.f * sweep::SPAN_S), pmax2 = pmin2;
+    for (int i = 0; i < n; ++i) {
+        const float ps2 = p[i] * (2.f * sweep::SPAN_S);
+        pmin2 = fminf(pmin2, ps2), pmax2 = fmaxf(pmax2, ps2);
+        any |= sweep::hot_pass(nc2, h2, ps2);
+        float rnc2, rh2;
+        sweep::hot_terms(lo, hi, q[i], rnc2, rh2);
+        own |= sweep::hot_pass(rnc2, rh2, ps2);
+    }
+    out3[0] = sweep::segment_pass(nc2, h2, pmin2, pmax2), out3[1] = any, out3[2] = own;
+    if (terms2) terms2[0] = nc2, terms2[1] = h2;
+}
 
 // Internal (tests only): strict::powf_glibc as the device computes it, for every stride-th float bit pattern x from
 // lo_bits up to hi_bits (inclusive) -> host_out[(hi_bits - lo_bits) / stride + 1], or for n (x, y) pairs.  Runs on the
@@ -1527,14 +1550,29 @@ int Frame::light(int k, uint32_t seed) {
 // The shadow rays of one light in list order, grouped by ray group (light vertex, cube face): seg_off = where each group
 // starts, cursor = its count, best_occ = no occluder yet.  Keys (light_step_kernel): default mode (group, q), so that the rays
 // of a thread can share a q-term (sweep::MODE_QBAR); bundle-cull mode (group, Morton code of (p,q)).  Pixels without a
-// shadow ray carry the all-ones key and sort last.
+// shadow ray carry the all-ones key and sort last.  Default mode then cuts each group's q-sorted run into stripes of
+// SHADOW_STRIPE entries and sorts every stripe by p, serpentine (stripe_key_kernel): a thread's SHADOW_R consecutive entries
+// span a quarter of the stripe's p range instead of all of it, at a q spread that the mean-q bounds still absorb.
+// TRACER_SHADOW_STRIPE (development) sets another stripe length; 1 gives the plain (group, q) order.
 int Frame::order_shadow_rays(int F) {
     trk::list_prefix_kernel<<<1, 32, 0, st>>>(s->seg_count, F, s->seg_off, s->cursor);
     CK_CUDA(cudaGetLastError());
     int group_bits = 1;
     while ((1 << group_bits) < F) ++group_bits;
-    CK_CUDA(cub::DeviceRadixSort::SortPairs(s->pair_tmp, s->pair_bytes, s->rkey, s->rkey_sorted, s->iota, s->ws.list, n_px, 0,
+    int *first = mode == SWEEPS ? s->ws.list_b : s->ws.list;
+    CK_CUDA(cub::DeviceRadixSort::SortPairs(s->pair_tmp, s->pair_bytes, s->rkey, s->rkey_sorted, s->iota, first, n_px, 0,
                                             32 + group_bits + 1, st));
+    if (mode == SWEEPS) {
+        const char *e = std::getenv("TRACER_SHADOW_STRIPE");
+        const int len = e ? std::max(1, std::atoi(e)) : trk::SHADOW_STRIPE;
+        trk::stripe_key_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(s->rkey_sorted, first, s->ws.re, s->seg_off, n_px, len, s->rkey);
+        CK_CUDA(cudaGetLastError());
+        int pos_bits = 1;
+        while (((int64_t)1 << pos_bits) < n_px) ++pos_bits;
+        CK_CUDA(cub::DeviceRadixSort::SortPairs(s->pair_tmp, s->pair_bytes, s->rkey, s->rkey_sorted, first, s->ws.list, n_px, 0,
+                                                32 + pos_bits, st));
+        launches += 2;
+    }
     CK_CUDA(cudaMemcpyAsync(s->cursor, s->seg_count, sizeof(int) * F, cudaMemcpyDeviceToDevice, st));
     CK_CUDA(cudaMemsetAsync(s->ws.best_occ, 0xff, sizeof(unsigned long long) * (size_t)n_px, st));
     return 0;
@@ -1761,19 +1799,21 @@ int Frame::finish_frame(uint8_t *rgb_out) {
     s->stats.filter_misses = (int64_t)hc.filter_misses;
     s->stats.pipeline_errors = (int64_t)hc.pipeline_errors;
     s->stats.kernel_launches = launches;
-    // FP32 flops the sweeps' formulation needs per swept pair (FFMA = 2, FADD = FMUL = 1, a minimum 0).  Interval form: half
-    // a packed FADD2 per pair, plus per thread and triangle the bound FFMAs, 4 (one exact q) or 8 (mean q + |B| * spread:
-    // shadow sweeps, jittered primary samples), and the interval's centre and half width (7 flops), over the R rays.
+    // FP32 flops the sweeps' formulation needs per swept pair (FFMA = 2, FADD = FMUL = 1, a minimum 0).  Shadow sweeps: the
+    // segment verdict, per thread and triangle 8 bound FFMAs (mean q + |B| * spread), 2 FADD for the interval and one packed
+    // FADD2 on the thread's extreme rays, over the R rays; nothing per pair.
     const bool no_flops = mode != SWEEPS; // the optional modes: no fixed per-pair cost
-    s->stats.flop_primary = no_flops ? 0.0 : flop_primary, s->stats.flop_shadow = no_flops ? 0.0 : 1.0 + 18.0 / trk::SHADOW_R;
+    s->stats.flop_primary = no_flops ? 0.0 : flop_primary, s->stats.flop_shadow = no_flops ? 0.0 : 20.0 / trk::SHADOW_R;
     // of which multiply-adds that evaluate bounds (the rest is each pair's interval test and the per-triangle interval)
     s->stats.flop_primary_edges = no_flops ? 0.0 : flop_primary_edges;
     s->stats.flop_shadow_edges = no_flops ? 0.0 : 16.0 / trk::SHADOW_R;
     if (hc.cull_overflow) return CAND_OVERFLOW; // (with TRACER_RNG_MT19937 only the shadow sweeps' candidates can have overflowed by now)
     if (getenv("TRACER_SHADOW_DIAG") && hc.cyc_total)
-        fprintf(stderr, "shadow diag: CTA cycles %.3e total = items %.1f %% + grid barriers %.1f %% + compaction %.1f %% + other %.1f %%; %llu items in %llu runs\n",
+        fprintf(stderr, "shadow diag: CTA cycles %.3e total = items %.1f %% + grid barriers %.1f %% + compaction %.1f %% + other %.1f %%; %llu items in %llu runs; "
+                        "flagged (thread, triangle) %llu, queued pairs %llu, strict evals %llu\n",
                 (double)hc.cyc_total, 100.0 * hc.cyc_items / hc.cyc_total, 100.0 * hc.cyc_barrier / hc.cyc_total, 100.0 * hc.cyc_compact / hc.cyc_total,
-                100.0 * ((double)hc.cyc_total - hc.cyc_items - hc.cyc_barrier - hc.cyc_compact) / hc.cyc_total, hc.n_items, hc.n_runs);
+                100.0 * ((double)hc.cyc_total - hc.cyc_items - hc.cyc_barrier - hc.cyc_compact) / hc.cyc_total, hc.n_items, hc.n_runs,
+                hc.n_flagged, hc.n_queued, hc.strict_evals);
     if (getenv("TRACER_CULL_DIAG"))
         fprintf(stderr, "cull diag (shadow): l0 survivors %llu, tiles with any %llu, fallback tiles %llu, l1 warp-passes %llu, item-tiles %llu\n", hc.cull_l0,
                 hc.cull_tiles_any, hc.cull_tiles_fallback, hc.cull_l1, (unsigned long long)(hc.tests_shadow / 4096 / cull::CTILE));

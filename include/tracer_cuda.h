@@ -184,8 +184,9 @@ typedef struct tracer_frame_stats {
                                thread's extreme rays (segment verdict), nothing per pair: 12/R.  Jittered samples with
                                a shared mean q (8 FFMA, and per pair half a packed FADD2): 1 + 18/R.  Three-row form (every ray its own q): 6 FFMA + FMUL + FFMA = 15.
                                0 in bundle-cull mode                                                              */
-    double flop_shadow;     /* same for the any-hit sweeps (hot rows, R = 32 q-sorted rays share a mean q: 8 FFMA +
-                               2 FADD per thread and triangle): 1 + 18/R                                          */
+    double flop_shadow;     /* same for the any-hit sweeps (hot rows, R = 32 rays of one (p, q) cell share a mean q:
+                               8 FFMA + 2 FADD per thread and triangle and one packed FADD2 for the thread's extreme
+                               rays (segment verdict), nothing per pair): 20/R                                    */
     /* of which the multiply-adds that evaluate the bounds / edge rows (the rest is each pair's conjunction) */
     double flop_primary_edges;
     double flop_shadow_edges;
