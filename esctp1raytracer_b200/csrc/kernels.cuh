@@ -725,15 +725,21 @@ __global__ void list_prefix_kernel(const int *seg_count, int F, int *seg_off, in
     }
 }
 
-// Default mode: entries per stripe of the shadow-ray order (order_shadow_rays).  Measured at C4 (profiles/r11_b): 128 gives
-// the fastest shadow sweeps.  Longer stripes make a thread's cell narrower in p but taller in q, and past ~200 entries the
-// |B| * qdelta widening of the mean-q bounds costs more queued pairs than the narrower cell saves.
-constexpr int SHADOW_STRIPE = 128;
+// Default mode: the stripe length of a group of n shadow rays (order_shadow_rays) is max(32, ceil(sqrt(SHADOW_CELL_C * n))),
+// so a group's stripes keep their shape in the (p, q) plane whatever its ray count, and a thread's SHADOW_R consecutive rays
+// form a compact cell.  Taller cells widen the mean-q bounds (more flagged verdicts per cell), narrower ones flag more
+// cells; the candidate path rebuilds with each ray's own q, so the pairs queued do not depend on the order.  Measured at C4
+// (profiles/r12_b, r12_c, at 32 chunks): c = 128 gives the fastest shadow sweeps of c = 8, 32, 128, 512 and of fixed
+// stripes of 128 to 8192.
+#ifndef SHADOW_CELL_C
+#define SHADOW_CELL_C 128
+#endif
 
 // Default mode, after the (group, q) sort: the key that reorders every stripe of L consecutive entries of a group by p,
 // ascending in even stripes and descending in odd ones (serpentine), so that consecutive entries stay close in (p, q)
-// across stripe boundaries too.  key = stripe's first list position << 32 | p's order bits (inverted in odd stripes);
-// pixels without a shadow ray (all-ones key, last) keep it.  The list stays a permutation of each group's rays.
+// across stripe boundaries too.  L > 0: every group's stripe length; L = 0: each group's own (SHADOW_CELL_C above).
+// key = stripe's first list position << 32 | p's order bits (inverted in odd stripes); pixels without a shadow ray
+// (all-ones key, last) keep it.  The list stays a permutation of each group's rays.
 __global__ void stripe_key_kernel(const unsigned long long *__restrict__ key_sorted, const int *__restrict__ list, const float *__restrict__ re,
                                   const int *__restrict__ seg_off, int n_px, int L, unsigned long long *__restrict__ key_out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -743,6 +749,7 @@ __global__ void stripe_key_kernel(const unsigned long long *__restrict__ key_sor
         key_out[i] = ~0ull;
         return;
     }
+    if (L == 0) L = max(32, (int)ceil(sqrt((double)SHADOW_CELL_C * (seg_off[j + 1] - seg_off[j]))));
     const int s = (i - seg_off[j]) / L;
     const unsigned pb = __float_as_uint(re[list[i]]);
     unsigned pk = (pb & 0x80000000u) ? ~pb : (pb | 0x80000000u);
@@ -798,6 +805,8 @@ constexpr int SHADOW_R = 32;    // rays per thread of a full shadow-ray block (b
 #ifndef SHADOW_MINB
 #define SHADOW_MINB 3
 #endif
+// dynamic shared memory of shadow_light_kernel: the tile pipeline, then the current item's rays (shadow_item)
+constexpr size_t SHADOW_SMEM = sizeof(sweep::SmemT<2>) + sizeof(float2) * sweep::NT * SHADOW_R;
 constexpr int SL_MAXF = 1022;   // ray groups per launch (the host batches bigger lights: 146 vertices x NFACE)
 constexpr int SL_MAXCHUNK = 64;
 constexpr int CBLK = 1024;      // list entries per compaction block
@@ -846,15 +855,15 @@ __device__ __noinline__ bool strict_shadow(const PixelState &px, const float *__
 }
 
 // one (ray block, triangle slice) work item with RR rays per thread.  The list is ordered by q inside each group, then by
-// p in serpentine stripes of SHADOW_STRIPE entries (and compaction keeps that order); a thread takes RR CONSECUTIVE rays,
-// evaluates them with one q-term per edge row (sweep::MODE_QBAR) and decides each triangle from its least and greatest p
-// (the mean-q segment verdict, sweep.cuh).  Only 2*S*p stays in registers: the candidate path reads a queued ray's own
-// (p, q) back through the list.
+// p in serpentine stripes (stripe_key_kernel; compaction keeps that order); a thread takes RR CONSECUTIVE rays, evaluates
+// them with one q-term per edge row (sweep::MODE_QBAR) and decides each triangle from its least and greatest p (the mean-q
+// segment verdict, sweep.cuh).  The rays' (2*S*p, q) go to shared memory (rays: NT * RR float2), from which the candidate
+// path rebuilds a flagged triangle's pairs with each ray's own q, one ray per lane.
 template <int RR, bool EXHAUSTIVE>
-__device__ __forceinline__ void shadow_item(sweep::SmemT<2> &sm, const ShadowLightParams &p, const int *__restrict__ list_in, int base,
+__device__ __forceinline__ void shadow_item(sweep::SmemT<2> &sm, float2 *rays, const ShadowLightParams &p, const int *__restrict__ list_in, int base,
                                             int seg_end, int lo, int hi, const float4 *__restrict__ tab, unsigned &gtile,
                                             unsigned &n_strict, unsigned &n_miss, unsigned long long &tests, unsigned &n_pipe_err,
-                                            unsigned long long &n_flag, unsigned long long &n_queue) {
+                                            unsigned long long &n_flag, unsigned long long &n_queue, unsigned long long &n_cyc) {
     using Mask = sweep::RayMask<RR>;
     const int tid = threadIdx.x, n = p.n_px;
     float rp[RR], rq[RR];
@@ -865,6 +874,7 @@ __device__ __forceinline__ void shadow_item(sweep::SmemT<2> &sm, const ShadowLig
         if (e0 + r < seg_end) valid |= (Mask)1 << r;
         const int k = list_in[min(e0 + r, seg_end - 1)];
         rp[r] = p.px.re[k], rq[r] = p.px.re[n + k];
+        rays[tid * RR + ((r + tid) & (RR - 1))] = make_float2(rp[r] * (2.f * sweep::SPAN_S), rq[r]);
         // an earlier slice may already have published an occluder below this slice: nothing to do
         const unsigned long long seen = p.px.best_occ[k];
         if (seen != KEY_NONE && (int)(unsigned)(seen >> 32) < lo * sweep::TILE) done |= (Mask)1 << r;
@@ -876,21 +886,18 @@ __device__ __forceinline__ void shadow_item(sweep::SmemT<2> &sm, const ShadowLig
     const float qbar = 0.5f * (qmin + qmax);
     // >= max |q_r - qbar| with room for the roundings of this line and of the one extra FFMA per row
     const float qdelta = fmaxf(qmax - qbar, qbar - qmin) * 1.0001f + 2.4e-7f * (fabsf(qbar) + 1.f);
+    __syncwarp(); // the staged rays are read by the other lanes of the warp
     unsigned swept = 0, flagged = 0, queued = 0;
     sweep::sweep_table<RR, sweep::MODE_QBAR, true, EXHAUSTIVE>(
         sm, tab, lo, hi, p.n_tris, rp, rq, qbar, qdelta, valid, done, gtile, swept,
-        [&](int otid, int r, int tri, bool filt, const float4 *row) {
+        [&](int otid, int r, int tri, bool filt, const float4 *) {
             const int k = list_in[min(base + otid * RR + r, seg_end - 1)];
-            // each ray's own q: the widening of the shared-q bounds, ~10 % of a pixel over 16 consecutive rays of a
-            // q-sorted list, would cost ~5 % more strict evaluations
-            filt = filt && sweep::hot_row_pass(row, p.px.re[k], p.px.re[n + k]);
-            if (!EXHAUSTIVE && !filt) return false;
             ++n_strict;
             const bool acc = strict_shadow(p.px, p.tri_verts, n, k, tri);
             n_miss += acc && !filt;
             return acc;
         },
-        &n_pipe_err, &flagged, &queued);
+        &n_pipe_err, &flagged, &queued, &n_cyc, rays);
     tests += (unsigned long long)swept * sweep::TILE * __popcll((unsigned long long)valid);
     n_flag += flagged, n_queue += queued;
 }
@@ -963,11 +970,13 @@ __global__ void __launch_bounds__(sweep::NT, SHADOW_MINB) shadow_light_kernel(co
     constexpr int R = SHADOW_R, CPT = CBLK / sweep::NT; // rays per thread of a full ray block; list entries per thread of a compaction block
     extern __shared__ __align__(128) unsigned char smem_raw[];
     sweep::SmemT<2> &sm = *reinterpret_cast<sweep::SmemT<2> *>(smem_raw); // the any-hit sweeps read span tables only
+    // the rays of the current item (shadow_item), after SmemT: the closest-hit kernels share SmemT<2> and do not need them
+    float2 *rays = reinterpret_cast<float2 *>(smem_raw + sizeof(sweep::SmemT<2>));
     __shared__ int s_blk_off[SL_MAXF + 1], s_cblk_off[SL_MAXF + 1], s_scratch[sweep::NT / 32], s_off;
     const int tid = threadIdx.x, F = p.F;
     sweep::smem_init(sm);
     unsigned gtile = 0, n_strict = 0, n_miss = 0, epoch = 0, n_pipe_err = 0;
-    unsigned long long tests = 0, n_flag = 0, n_queue = 0;
+    unsigned long long tests = 0, n_flag = 0, n_queue = 0, c_cand = 0; // c_cand: lane 0's candidate-path cycles
     long long c_items = 0, c_bar = 0, c_comp = 0, n_it = 0, n_run = 0; // time split (thread 0)
     const long long c_begin = clock64();
     // chunk scheme: equal chunks keep the pairs swept past a ray's occluder lowest and win when the light has many
@@ -1028,15 +1037,15 @@ __global__ void __launch_bounds__(sweep::NT, SHADOW_MINB) shadow_light_kernel(co
                 const int cnt = seg_end - base;
                 static_assert(SHADOW_R == 32, "the part-filled block sizes below follow SHADOW_R");
                 if (cnt > 16 * sweep::NT)
-                    shadow_item<SHADOW_R, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue);
+                    shadow_item<SHADOW_R, EXHAUSTIVE>(sm, rays, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue, c_cand);
                 else if (cnt > 8 * sweep::NT)
-                    shadow_item<16, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue);
+                    shadow_item<16, EXHAUSTIVE>(sm, rays, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue, c_cand);
                 else if (cnt > 4 * sweep::NT)
-                    shadow_item<8, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue);
+                    shadow_item<8, EXHAUSTIVE>(sm, rays, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue, c_cand);
                 else if (cnt > 2 * sweep::NT)
-                    shadow_item<4, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue);
+                    shadow_item<4, EXHAUSTIVE>(sm, rays, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue, c_cand);
                 else
-                    shadow_item<2, EXHAUSTIVE>(sm, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue);
+                    shadow_item<2, EXHAUSTIVE>(sm, rays, p, list_in, base, seg_end, lo, hi, tab, gtile, n_strict, n_miss, tests, n_pipe_err, n_flag, n_queue, c_cand);
                 __syncthreads(); // every warp is out of the tile pipeline before the next run re-arms it
             }
             c_items += clock64() - c_run;
@@ -1158,6 +1167,7 @@ __global__ void __launch_bounds__(sweep::NT, SHADOW_MINB) shadow_light_kernel(co
     atomicAdd(&p.counters->tests_shadow, tests);
     atomicAdd(&p.counters->strict_evals, (unsigned long long)n_strict);
     atomicAdd(&p.counters->n_flagged, n_flag), atomicAdd(&p.counters->n_queued, n_queue);
+    if ((tid & 31) == 0) atomicAdd(&p.counters->cyc_cand, c_cand);
     if (EXHAUSTIVE) atomicAdd(&p.counters->filter_misses, (unsigned long long)n_miss);
     if (EXHAUSTIVE && n_pipe_err) atomicAdd(&p.counters->pipeline_errors, (unsigned long long)n_pipe_err);
     if (tid == 0) {

@@ -178,6 +178,8 @@ struct Counters {
     unsigned long long cyc_items, cyc_barrier, cyc_compact, cyc_total, n_items, n_runs;
     // shadow_light_kernel: (thread, triangle) verdicts the hot loop flagged, and (ray, triangle) pairs queued for the drain
     unsigned long long n_flagged, n_queued;
+    // shadow_light_kernel: SM cycles of the candidate path (from a batch's first flag to its last drain), lane 0 of every warp
+    unsigned long long cyc_cand;
 };
 
 template <int ROWS>
@@ -421,7 +423,8 @@ __device__ __forceinline__ float fmin3_abs(float m, float a, float b) {
 // fl(pmin2 + nc2) <= h2 and fl(pmax2 + nc2) >= -h2 for any passing ray.  No new margin, no new rounding.  The R values include
 // the duplicated tail entries of a short list and rays already done: both only widen [pmin2, pmax2], so only loosen it.
 // It pays once a thread's rays form a compact cell in (p, q): the default mode's shadow lists are sorted by q, then by p in
-// serpentine stripes (order_shadow_rays), so qdelta is ~1e-3 instead of ~1e-6 and [pmin2, pmax2] a few triangle widths.
+// serpentine stripes of about sqrt(128 n) entries (order_shadow_rays), so [pmin2, pmax2] spans a few triangle widths.  The
+// widened bounds pass most of a flagged thread's rays, so the candidate path rebuilds with each ray's own q (sweep_table).
 constexpr float HOT_CLAMP = SPAN_BOX;
 constexpr float HOT_DELTA = 8.f * 1.1920928955078125e-7f * HOT_CLAMP;
 constexpr float HOT_QD_SCALE = 1.f + 0x1p-20f;
@@ -463,12 +466,6 @@ __host__ __device__ __forceinline__ bool segment_pass(float nc2, float h2, float
     const float2 e = make_float2(pmin2 + nc2, pmax2 + nc2);
 #endif
     return !(e.x > h2) && !(-e.y > h2);
-}
-// the hot test of one ray (p, its own q) on a staged hot row (candidate path of the any-hit sweeps)
-__device__ __forceinline__ bool hot_row_pass(const float4 *row, float p, float q) {
-    float nc2, h2;
-    hot_terms(lds128_opaque(row), lds128_opaque(row + 1), q, nc2, h2);
-    return hot_pass(nc2, h2, p * (2.f * SPAN_S));
 }
 
 // ray masks of the sweeps: a bit per ray of a thread
@@ -552,11 +549,15 @@ __device__ __forceinline__ unsigned eval_batch_lop3(const float4 *__restrict__ t
 //        the pair (false only in EXHAUSTIVE validation mode), row = the triangle's staged row (still resident)
 // n_flag, n_queue (may be null; not counted in EXHAUSTIVE mode): add this thread's flagged (thread, triangle) verdicts and the
 //        pairs it queued
+// n_cyc (may be null): lane 0 adds the SM cycles its warp spends in the candidate path
+// own (any-hit MODE_QBAR only, required there): the rays of every thread of the CTA in shared memory, (2*S*p, q) of ray r of
+//        thread t at own[t * R + ((r + t) & (R - 1))] (rotated by the lane, so that neither the stores nor the loads conflict)
 template <int R, int MODE, bool ANYHIT, bool EXHAUSTIVE, class Strict>
 __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const float4 *__restrict__ table, int tile_lo, int tile_hi, int n_tris,
                                             const float (&rp)[R], const float (&rq)[R], float qbar, float qdelta, RayMask<R> valid,
                                             RayMask<R> &done, unsigned &gtile, unsigned &n_tiles_swept, Strict &&strict,
-                                            unsigned *n_pipe_err = nullptr, unsigned *n_flag = nullptr, unsigned *n_queue = nullptr) {
+                                            unsigned *n_pipe_err = nullptr, unsigned *n_flag = nullptr, unsigned *n_queue = nullptr,
+                                            unsigned long long *n_cyc = nullptr, const float2 *own = nullptr) {
     using Mask = RayMask<R>;
     static_assert(R <= 32 || MODE != MODE_OWNQ, "the three-row form's rays fit one 32-bit mask");
     constexpr int ROWS = Rows<MODE>::N;
@@ -580,6 +581,9 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
     // closest hit with a shared q, and the shadow sweeps (mean q): the hot loop decides each triangle from the extreme rays
     // (segment_pass); jittered primary samples (MODE_QBAR, closest hit) keep the per-ray loop
     constexpr bool SEGMENT = (!ANYHIT && MODE == MODE_SHAREDQ) || (ANYHIT && MODE == MODE_QBAR);
+    // the shadow sweeps rebuild a flagged triangle's candidates with each ray's own q, one ray per lane (below)
+    constexpr bool OWNQ_REBUILD = ANYHIT && MODE == MODE_QBAR;
+    static_assert(!OWNQ_REBUILD || 32 % R == 0, "a warp rebuilds whole threads' rays");
     float pmin2 = ps2[0], pmax2 = ps2[0];
     if (SEGMENT) {
 #pragma unroll
@@ -632,6 +636,11 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
             // triangles per hot-loop call, and per bit of its verdict: the interval form (span rows) flags single
             // triangles, the three-row form groups of GROUP
             constexpr int NB = SPAN ? SPAN_BATCH : BATCH, UNIT = SPAN ? 1 : Batch<SPAN ? 2 : R>::GROUP;
+            // pairs in this warp's queue.  The shadow sweeps keep them across the tile's batches and drain when the queue is
+            // full and at the end of the tile: a drain is a chain of dependent loads and FP64 work, and fewer, fuller drains
+            // hide more of it.  A ray that finds its occluder meanwhile only adds strict tests of later triangles, which the
+            // minimum merge ignores.  The other sweeps drain after each batch.
+            int fill = 0;
 #pragma unroll 1
             for (int b0 = 0; b0 < TILE; b0 += NB) {
                 unsigned cand;
@@ -651,61 +660,116 @@ __device__ __forceinline__ void sweep_table(SmemT<Rows<MODE>::N> &sm, const floa
                 // pair per lane, so a thread's candidates no longer serialise while the rest of the warp idles.
                 unsigned wcand = __reduce_or_sync(0xffffffffu, cand);
                 if (wcand) {
-                    int fill = 0;
-                    while (wcand) {
-                        const int gq = __ffs(wcand) - 1; // ascending triangle order
-                        wcand &= wcand - 1;
-                        const bool mine = (cand >> gq) & 1u;
-#pragma unroll 1
-                        for (int kk = 0; kk < UNIT; ++kk) {
-                            const int k = b0 + gq * UNIT + kk;
-                            if ((tile_lo + it) * TILE + k >= n_tris) break; // padding (warp-uniform)
-                            Mask filt = 0;
-                            if (mine) {
-                                // The rows are re-read through opaque loads so that the compiler cannot merge this with the
-                                // hot evaluation.
-                                if (SPAN) {
-                                    // the hot loop's own test, ray by ray: it passes every pair span_pass passes (hot_row); exact
-                                    // with a common q.  Shadow rays are tested again with their own q when the queue drains.
-                                    const float4 lo = lds128_opaque(&tp[2 * k]), hi = lds128_opaque(&tp[2 * k + 1]);
-                                    float nc2, h2;
-                                    if (MODE == MODE_QBAR) hot_terms_qbar(lo, hi, qhot, qdh, nc2, h2);
-                                    else hot_terms(lo, hi, qhot, nc2, h2);
-#pragma unroll
-                                    for (int r = 0; r < R; ++r) filt |= (Mask)hot_pass(nc2, h2, ps2[r]) << r;
-                                } else {
-                                    const float4 rb = lds128_opaque(&tp[3 * k]), rc = lds128_opaque(&tp[3 * k + 1]), rd = lds128_opaque(&tp[3 * k + 2]);
-#pragma unroll
-                                    for (int r = 0; r < R; ++r) filt |= (Mask)edge_pass(rb, rc, rd, rp[r], rq[r]) << r;
-                                }
-                                if (EXHAUSTIVE && !((cand_hot >> gq) & 1u)) filt = 0;
-                            }
+                    const long long c_cand = n_cyc ? clock64() : 0;
+                    if constexpr (OWNQ_REBUILD) {
+                        // Shadow sweeps: the thread's verdict used the mean-q bounds widened over all its rays, so most
+                        // flagged rays fail their own test.  Each flagged (owner lane, triangle) is rebuilt one ray per lane:
+                        // lane = slot * R + r tests ray r of the slot's owner, read from shared memory, with the exact test at
+                        // its own q (hot_terms, hot_pass), and the pairs that pass and are live go straight to the queue.
+                        // Every pair the reference accepts passes this test (hot_row), so the drain needs no second filter.
+                        constexpr int OPW = 32 / R; // owner lanes per round
+                        const int slot = lane / R, r = lane & (R - 1);
+                        while (wcand) {
+                            const int gq = __ffs(wcand) - 1, k = b0 + gq; // ascending triangle order
+                            wcand &= wcand - 1;
+                            if ((tile_lo + it) * TILE + k >= n_tris) break; // padding (warp-uniform), and so is the rest
+                            const float4 lo = lds128_opaque(&tp[2 * k]), hi = lds128_opaque(&tp[2 * k + 1]);
                             const Mask live = valid & ~done;
-                            Mask pend = mine ? (EXHAUSTIVE ? live : filt & live) : (Mask)0;
-                            if (!EXHAUSTIVE && n_queue) *n_queue += __popcll((unsigned long long)pend);
-                            while (__any_sync(0xffffffffu, pend != 0)) {
-                                // this lane's pairs go to queue slots [fill + before, ...): as many as fit, the rest after a drain
-                                const int n = __popcll((unsigned long long)pend);
-                                int incl = n;
+                            unsigned owners = __ballot_sync(0xffffffffu, (cand >> gq) & 1u);
+                            while (owners) {
+                                unsigned m = owners;
+                                for (int i = 0; i < slot; ++i) m &= m - 1;
+                                const int o = m ? __ffs(m) - 1 : 0;
+                                const Mask olive = __shfl_sync(0xffffffffu, live, o);
+                                const unsigned ohot = __shfl_sync(0xffffffffu, cand_hot, o);
+                                bool filt = false, in = false;
+                                if (m) {
+                                    const float2 pq = own[((tid & ~31) | o) * R + ((r + o) & (R - 1))];
+                                    float nc2, h2;
+                                    hot_terms(lo, hi, pq.y, nc2, h2);
+                                    filt = hot_pass(nc2, h2, pq.x) && (!EXHAUSTIVE || ((ohot >> gq) & 1u));
+                                    in = ((olive >> r) & 1u) && (EXHAUSTIVE || filt);
+                                }
+                                const unsigned ins = __ballot_sync(0xffffffffu, in);
+                                const int n = __popc(ins), pos = fill + __popc(ins & ((1u << lane) - 1u));
+                                const unsigned e = (unsigned)r | (unsigned)o << 6 | (unsigned)k << 11 | (unsigned)filt << 19;
+                                if (in && pos < QCAP) queue[pos] = e;
+                                if (fill + n >= QCAP) {
+                                    drain(tp, it, QCAP);
+                                    if (in && pos >= QCAP) queue[pos - QCAP] = e;
+                                    fill += n - QCAP;
+                                } else {
+                                    fill += n;
+                                }
+                                if (!EXHAUSTIVE && n_queue) *n_queue += in;
 #pragma unroll
-                                for (int o = 1; o < 32; o <<= 1) {
-                                    const int y = __shfl_up_sync(0xffffffffu, incl, o);
-                                    if (lane >= o) incl += y;
+                                for (int i = 0; i < OPW; ++i) owners &= owners - 1;
+                            }
+                        }
+                    } else {
+                        while (wcand) {
+                            const int gq = __ffs(wcand) - 1; // ascending triangle order
+                            wcand &= wcand - 1;
+                            const bool mine = (cand >> gq) & 1u;
+#pragma unroll 1
+                            for (int kk = 0; kk < UNIT; ++kk) {
+                                const int k = b0 + gq * UNIT + kk;
+                                if ((tile_lo + it) * TILE + k >= n_tris) break; // padding (warp-uniform)
+                                Mask filt = 0;
+                                if (mine) {
+                                    // The rows are re-read through opaque loads so that the compiler cannot merge this with the
+                                    // hot evaluation.
+                                    if (SPAN) {
+                                        // the hot loop's own test, ray by ray: it passes every pair span_pass passes (hot_row); exact
+                                        // with a common q
+                                        const float4 lo = lds128_opaque(&tp[2 * k]), hi = lds128_opaque(&tp[2 * k + 1]);
+                                        float nc2, h2;
+                                        if (MODE == MODE_QBAR) hot_terms_qbar(lo, hi, qhot, qdh, nc2, h2);
+                                        else hot_terms(lo, hi, qhot, nc2, h2);
+#pragma unroll
+                                        for (int r = 0; r < R; ++r) filt |= (Mask)hot_pass(nc2, h2, ps2[r]) << r;
+                                    } else {
+                                        const float4 rb = lds128_opaque(&tp[3 * k]), rc = lds128_opaque(&tp[3 * k + 1]), rd = lds128_opaque(&tp[3 * k + 2]);
+#pragma unroll
+                                        for (int r = 0; r < R; ++r) filt |= (Mask)edge_pass(rb, rc, rd, rp[r], rq[r]) << r;
+                                    }
+                                    if (EXHAUSTIVE && !((cand_hot >> gq) & 1u)) filt = 0;
                                 }
-                                for (int slot = fill + incl - n; pend && slot < QCAP; ++slot) {
-                                    const int r = lowest_ray(pend);
-                                    pend &= pend - 1;
-                                    queue[slot] = (unsigned)r | lane << 6 | (unsigned)k << 11 | (unsigned)((filt >> r) & 1u) << 19;
+                                const Mask live = valid & ~done;
+                                Mask pend = mine ? (EXHAUSTIVE ? live : filt & live) : (Mask)0;
+                                if (!EXHAUSTIVE && n_queue) *n_queue += __popcll((unsigned long long)pend);
+                                while (__any_sync(0xffffffffu, pend != 0)) {
+                                    // this lane's pairs go to queue slots [fill + before, ...): as many as fit, the rest after a drain
+                                    const int n = __popcll((unsigned long long)pend);
+                                    int incl = n;
+#pragma unroll
+                                    for (int o = 1; o < 32; o <<= 1) {
+                                        const int y = __shfl_up_sync(0xffffffffu, incl, o);
+                                        if (lane >= o) incl += y;
+                                    }
+                                    for (int slot = fill + incl - n; pend && slot < QCAP; ++slot) {
+                                        const int r = lowest_ray(pend);
+                                        pend &= pend - 1;
+                                        queue[slot] = (unsigned)r | lane << 6 | (unsigned)k << 11 | (unsigned)((filt >> r) & 1u) << 19;
+                                    }
+                                    fill = min(QCAP, fill + __shfl_sync(0xffffffffu, incl, 31));
+                                    if (fill == QCAP) drain(tp, it, fill), fill = 0;
                                 }
-                                fill = min(QCAP, fill + __shfl_sync(0xffffffffu, incl, 31));
-                                if (fill == QCAP) drain(tp, it, fill), fill = 0;
                             }
                         }
                     }
-                    if (fill) drain(tp, it, fill);
+                    if (!OWNQ_REBUILD && fill) drain(tp, it, fill), fill = 0;
+                    if (n_cyc && lane == 0) *n_cyc += clock64() - c_cand;
                 }
 #endif
             }
+#ifndef SWEEP_NO_STRICT
+            if (OWNQ_REBUILD && __any_sync(0xffffffffu, fill != 0)) {
+                const long long c_cand = n_cyc ? clock64() : 0;
+                drain(tp, it, fill);
+                if (n_cyc && lane == 0) *n_cyc += clock64() - c_cand;
+            }
+#endif
         }
         if (EXHAUSTIVE && n_pipe_err && tile_differs() && (tid & 31) == 0) ++*n_pipe_err;
         // No block-wide barrier per tile: every warp counts itself out of stage s, and the LAST one refills it.

@@ -493,7 +493,7 @@ constexpr int WORK_INTS = trk::SL_MAXCHUNK + 8; // per-chunk work counters + the
 
 template <bool EX>
 int launch_shadow_light_t(Ctx &g, const trk::ShadowLightParams &p, unsigned *bar, cudaStream_t st) {
-    const size_t smem = sizeof(sweep::SmemT<2>);
+    const size_t smem = trk::SHADOW_SMEM;
     int &ctas_per_sm = g.sl_ctas[EX ? 1 : 0]; // co-resident CTAs: a cooperative launch may not exceed them
     if (!ctas_per_sm) {
         CK_CUDA(cudaFuncSetAttribute(trk::shadow_light_kernel<EX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1550,10 +1550,10 @@ int Frame::light(int k, uint32_t seed) {
 // The shadow rays of one light in list order, grouped by ray group (light vertex, cube face): seg_off = where each group
 // starts, cursor = its count, best_occ = no occluder yet.  Keys (light_step_kernel): default mode (group, q), so that the rays
 // of a thread can share a q-term (sweep::MODE_QBAR); bundle-cull mode (group, Morton code of (p,q)).  Pixels without a
-// shadow ray carry the all-ones key and sort last.  Default mode then cuts each group's q-sorted run into stripes of
-// SHADOW_STRIPE entries and sorts every stripe by p, serpentine (stripe_key_kernel): a thread's SHADOW_R consecutive entries
-// span a quarter of the stripe's p range instead of all of it, at a q spread that the mean-q bounds still absorb.
-// TRACER_SHADOW_STRIPE (development) sets another stripe length; 1 gives the plain (group, q) order.
+// shadow ray carry the all-ones key and sort last.  Default mode then cuts each group's q-sorted run into stripes of about
+// sqrt(128 n) entries (n: the group's rays; SHADOW_CELL_C) and sorts every stripe by p, serpentine (stripe_key_kernel): a
+// thread's SHADOW_R consecutive entries form a compact cell in (p, q).
+// TRACER_SHADOW_STRIPE (development) sets one stripe length for every group; 1 gives the plain (group, q) order.
 int Frame::order_shadow_rays(int F) {
     trk::list_prefix_kernel<<<1, 32, 0, st>>>(s->seg_count, F, s->seg_off, s->cursor);
     CK_CUDA(cudaGetLastError());
@@ -1564,7 +1564,7 @@ int Frame::order_shadow_rays(int F) {
                                             32 + group_bits + 1, st));
     if (mode == SWEEPS) {
         const char *e = std::getenv("TRACER_SHADOW_STRIPE");
-        const int len = e ? std::max(1, std::atoi(e)) : trk::SHADOW_STRIPE;
+        const int len = e ? std::max(1, std::atoi(e)) : 0; // 0: each group's own stripe length
         trk::stripe_key_kernel<<<(n_px + 255) / 256, 256, 0, st>>>(s->rkey_sorted, first, s->ws.re, s->seg_off, n_px, len, s->rkey);
         CK_CUDA(cudaGetLastError());
         int pos_bits = 1;
@@ -1649,14 +1649,15 @@ int Frame::shadow_cull(int k) {
 
 // Triangle chunks of the default shadow sweep: after each one the still-unoccluded rays are compacted (early exit,
 // main.cpp:324).  Equal chunks keep the pairs swept past a ray's occluder lowest (x1.056 at 64 chunks; x1.11 at 32) and win
-// when a light has many shadow rays.  32 of them: at 32 rays per thread an item is twice as long and so is each chunk's tail
-// (C4: 189 ms of shadow sweep at 32 chunks, 192 at 48, 199 at 64; profiles/r05_d).  With few rays (small frames, one band
+// when a light has many shadow rays.  8 of them: since flagged triangles are rebuilt with each ray's own q, a chunk's grid
+// barriers and tail cost more than the pairs swept past occluders that more chunks would save (C4: 142 ms of shadow sweep
+// at 8 chunks, 146 at 10 and 12, 153 at 6, 170 with 32 chunks and the earlier run cap; profiles/r12_e).  With few rays (small frames, one band
 // share of a multi-GPU frame) a chunk's fixed cost (three grid barriers, the compaction passes, the sweep's tail: ~0.1 ms)
 // weighs more, and 20 chunks that start fine (1/64 of the triangles: most occluded rays find their occluder early) and
 // coarsen win (x1.10).  The kernel picks the scheme from the live-ray count it finds.  opts.shadow_chunks asks for that many
 // equal chunks.
 void chunk_schemes(trk::ShadowLightParams &sp, int n_tiles, int shadow_chunks) {
-    const int nc = std::min({n_tiles, trk::SL_MAXCHUNK, shadow_chunks > 0 ? shadow_chunks : std::max(1, std::min(32, n_tiles / 8))});
+    const int nc = std::min({n_tiles, trk::SL_MAXCHUNK, shadow_chunks > 0 ? shadow_chunks : std::max(1, std::min(8, n_tiles / 8))});
     sp.n_chunks[1] = nc;
     for (int c = 0; c <= nc; ++c) sp.bounds[1][c] = (int)((int64_t)n_tiles * c / nc);
     if (shadow_chunks > 0 || n_tiles < 64) {
@@ -1687,8 +1688,10 @@ int Frame::shadow_sweeps(int k) {
     chunk_schemes(sp, n_tiles, o.shadow_chunks);
     sp.many_rays = (long long)1 << 20;
     sp.items_per_cta = items_per_cta();
-    sp.run_pairs = std::getenv("TRACER_RUN_PAIRS") ? std::max(1ll, std::atoll(std::getenv("TRACER_RUN_PAIRS"))) : 6000000ll;
-    sp.min_tiles = std::getenv("TRACER_MIN_TILES") ? std::max(1, std::atoi(std::getenv("TRACER_MIN_TILES"))) : 1;
+    // run cap and smallest slice measured together with the chunk count at C4 (profiles/r12_e): 24 M pairs and 4 tiles at
+    // 8 chunks; 6 M and 1 tile (the values for 32 chunks) cost 16 ms more
+    sp.run_pairs = std::getenv("TRACER_RUN_PAIRS") ? std::max(1ll, std::atoll(std::getenv("TRACER_RUN_PAIRS"))) : 24000000ll;
+    sp.min_tiles = std::getenv("TRACER_MIN_TILES") ? std::max(1, std::atoi(std::getenv("TRACER_MIN_TILES"))) : 4;
     sp.allcand = s->allcand_span, sp.table_stride = s->span_stride; // the default sweeps read the span tables
     sp.n_tris = s->n_tris, sp.n_tiles = n_tiles, sp.n_px = n_px, sp.tri_verts = s->tri_verts;
     sp.list[0] = s->ws.list, sp.list[1] = s->ws.list_b;
@@ -1810,10 +1813,10 @@ int Frame::finish_frame(uint8_t *rgb_out) {
     if (hc.cull_overflow) return CAND_OVERFLOW; // (with TRACER_RNG_MT19937 only the shadow sweeps' candidates can have overflowed by now)
     if (getenv("TRACER_SHADOW_DIAG") && hc.cyc_total)
         fprintf(stderr, "shadow diag: CTA cycles %.3e total = items %.1f %% + grid barriers %.1f %% + compaction %.1f %% + other %.1f %%; %llu items in %llu runs; "
-                        "flagged (thread, triangle) %llu, queued pairs %llu, strict evals %llu\n",
+                        "flagged (thread, triangle) %llu, queued pairs %llu, strict evals %llu; candidate path %.1f %% of item cycles; %d CTAs per SM\n",
                 (double)hc.cyc_total, 100.0 * hc.cyc_items / hc.cyc_total, 100.0 * hc.cyc_barrier / hc.cyc_total, 100.0 * hc.cyc_compact / hc.cyc_total,
                 100.0 * ((double)hc.cyc_total - hc.cyc_items - hc.cyc_barrier - hc.cyc_compact) / hc.cyc_total, hc.n_items, hc.n_runs,
-                hc.n_flagged, hc.n_queued, hc.strict_evals);
+                hc.n_flagged, hc.n_queued, hc.strict_evals, 100.0 * hc.cyc_cand / (sweep::NT / 32) / std::max(1.0, (double)hc.cyc_items), g.sl_ctas[0]);
     if (getenv("TRACER_CULL_DIAG"))
         fprintf(stderr, "cull diag (shadow): l0 survivors %llu, tiles with any %llu, fallback tiles %llu, l1 warp-passes %llu, item-tiles %llu\n", hc.cull_l0,
                 hc.cull_tiles_any, hc.cull_tiles_fallback, hc.cull_l1, (unsigned long long)(hc.tests_shadow / 4096 / cull::CTILE));

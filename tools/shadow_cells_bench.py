@@ -5,7 +5,7 @@ the median closest-hit time, the frame hashes and, with TRACER_SHADOW_DIAG=1 in 
 line of the last frame (flagged (thread, triangle) verdicts, queued pairs, strict evaluations, the item/barrier/compaction
 split).  --profile adds one frame under torch.profiler and prints the kernel time of the shadow-ray ordering
 (order_shadow_rays: the radix sorts, stripe_key_kernel, list_prefix_kernel).  The stripe length is the library's
-TRACER_SHADOW_STRIPE (unset: SHADOW_STRIPE in kernels.cuh), so a stripe sweep is one process per value.
+TRACER_SHADOW_STRIPE (unset: each group's own, from SHADOW_CELL_C in kernels.cuh), so a stripe sweep is one process per value.
 
     python tools/shadow_cells_bench.py <repository root> <tag> [--chunks 32,48] [--frames 3] [--profile]
 """
